@@ -4,14 +4,20 @@ per second (BASELINE.json's metric) on synthetic graphs of the named shapes.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
                     [--workload c3_human] [--vertices V] [--line-order shuffled|id]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (records -> CSR -> repeat marks ->
 polymorphic/inconsistent marks) over one synthetic graph.  `value` times it
 with inputs already resident in HBM; `e2e` times the same call through the
 C ABI with HOST buffers (H2D of records/vertices and D2H of vertex/edge states
 inside the timed region).  `--impl reference` times the reference's own
-single-threaded C (oracle/_ref, compiled from /root/reference) on a bounded
-sample of the same workload on the host cores.
+single-threaded C (oracle/_ref, compiled from the reference's sources) on a
+bounded sample of the same workload on the host cores.
+
+`--dump-outputs DIR` writes what the last timed step computed -- the edges and
+vertex states a caller of gtsb_pipeline fetches -- as DIR/<name>.npy (see
+dump_outputs).  The synthetic inputs are seeded, so two builds run with the same
+arguments can be compared array for array.
 """
 from __future__ import annotations
 
@@ -152,6 +158,65 @@ def device_lines(torch, root):
     return root[start[:-1].long()].contiguous(), start.contiguous()
 
 
+DUMP_EDGES, DUMP_VERTICES, DUMP_SEED = 1 << 19, 1 << 20, 0x5CAFF01D      # at most 36 MB of .npy files
+
+
+def dump_ids(n, limit, seed):
+    """The ids a dump keeps out of n: all of them, or a fixed, seeded sample of `limit`, ascending."""
+    import numpy as np
+    if n <= limit:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, limit, replace=False))
+
+
+def dump_outputs(directory, edges, E, vstate):
+    """Write a result as .npy files for comparing two builds: counts = (vertices, edges); edge_* = the
+    edges of dump_ids(E, DUMP_EDGES, DUMP_SEED) by eid (graph->edges[] order, whatever the device's
+    slot order); vertex_* = the vertex states of dump_ids(V, DUMP_VERTICES, DUMP_SEED + 1).  `edges`
+    holds eid and the attributes of at least those edges, in any order.  flags keeps the edge's own
+    sense and same bits, the part the reference stores (the device keeps its twin's in bits 2-3).
+    Values as float64 (ids, distances) or float32 (std_dev, flags, states): exact."""
+    import numpy as np
+    V = len(vstate)
+    eids = dump_ids(E, DUMP_EDGES, DUMP_SEED)
+    vids = dump_ids(V, DUMP_VERTICES, DUMP_SEED + 1)
+    slot = np.full(E, -1, np.int64)
+    slot[np.asarray(edges["eid"], np.int64)] = np.arange(len(edges["eid"]))
+    at = slot[eids]
+    if (at < 0).any():
+        raise RuntimeError("--dump-outputs: edges of the sample are missing from the result")
+    out = {"counts": np.array([V, E], np.float64), "edge_eid": eids.astype(np.float64),
+           "vertex_id": vids.astype(np.float64), "vertex_state": np.asarray(vstate)[vids].astype(np.float32)}
+    for k in ("src", "dst", "dist"):
+        out["edge_" + k] = np.asarray(edges[k])[at].astype(np.float64)
+    out["edge_std_dev"] = np.asarray(edges["std_dev"])[at].astype(np.float32)
+    out["edge_flags"] = (np.asarray(edges["flags"])[at] & 3).astype(np.float32)
+    out["edge_estate"] = np.asarray(edges["estate"])[at].astype(np.float32)
+    os.makedirs(directory, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
+def dump_device_result(args, g, torch, dist, rank, world, dev):
+    """dump_outputs of the graph `g` holds.  Partitioned over `world` ranks: every rank sends its
+    edges of the sample to rank 0, which writes them with the vertex states (each rank has all)."""
+    import numpy as np
+    e, vstate = g.edges(), g.vstate()
+    if world == 1:
+        dump_outputs(args.dump_outputs, e, len(e["eid"]), vstate)
+        return
+    n = torch.tensor([len(e["eid"])], dtype=torch.int64, device=dev)
+    dist.all_reduce(n, op=dist.ReduceOp.SUM)
+    E = int(n.item())
+    want = np.zeros(E, bool)
+    want[dump_ids(E, DUMP_EDGES, DUMP_SEED)] = True
+    keep = want[np.asarray(e["eid"], np.int64)]
+    parts = [None] * world
+    dist.all_gather_object(parts, {k: v[keep] for k, v in e.items()})
+    if rank == 0:
+        dump_outputs(args.dump_outputs, {k: np.concatenate([p[k] for p in parts]) for k in e}, E, vstate)
+
+
 def parity_check(pkg, torch, dist, rank, world, local, uid, args, ref_result):
     """The product path (partitioned over `world` ranks when world > 1) on the CPU leg's sample
     graph against the reference's result on the same arrays: vertex states on every rank, and --
@@ -267,11 +332,16 @@ def c4_leg():
 
 
 def run_reference_arm(args, pkg):
+    import numpy as np
     rank, world, _ = dist_env()
     if rank != 0:
         return
     cb, sec, E = cpu_reference_leg(pkg, args.workload, args.cpu_sample_vertices, args.line_order,
-                                   steps=max(1, args.steps), warmup=min(args.warmup, 1))
+                                   steps=max(1, args.steps), warmup=min(args.warmup, 1),
+                                   want_result=bool(args.dump_outputs))
+    if args.dump_outputs:
+        r = cpu_reference_leg.result
+        dump_outputs(args.dump_outputs, dict(r, eid=np.arange(len(r["src"]))), len(r["src"]), r["vstate"])
     line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT,
             "n_gpus": args.gpus, "steps": max(1, args.steps), "warmup": min(args.warmup, 1),
             "ms_per_step": sec * 1e3, "higher_is_better": True, "scaling": "weak",
@@ -378,6 +448,8 @@ def run_b200_arm(args, pkg):
     st = g.stats()
     launches = (st["kernel_launches"] - launches0) // max(1, args.steps)
     E = st["nof_edges"]
+    if args.dump_outputs:
+        dump_device_result(args, g, torch, dist, rank, world, dev)
 
     # ---- per-kernel device time (CUDA events on the launching stream), 2 extra steps
     g.set_profile(True)
@@ -551,7 +623,11 @@ def main():
                     help="N = 1, default workload: skip the config-4 (hubs) leg that runs after the headline measurement")
     ap.add_argument("--records", default="lines", choices=["lines", "flat"],
                     help="device-resident record input of the timed step at N = 1")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     pkg = importlib.import_module("gt-scaffold_b200")

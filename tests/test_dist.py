@@ -76,7 +76,7 @@ def test_partitioned_pipeline_matches_the_oracle():
     import torch
     n = torch.cuda.device_count()
     if n < 2:
-        pytest.skip("needs >= 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs >= 2 GPUs")
     world = 2
     r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={world}",
                         "--master-addr", "127.0.0.1", "--master-port", "29517",
@@ -92,7 +92,7 @@ def test_a_failing_rank_stops_all_ranks():
     """ADVICE r1: an allocation failure on one rank must not leave its peers in a collective."""
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs >= 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs >= 2 GPUs")
     r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2",
                         "--master-addr", "127.0.0.1", "--master-port", "29519",
                         os.path.join(HERE, "dist_fail_check.py")], cwd=ROOT, stdout=subprocess.PIPE,

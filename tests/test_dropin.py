@@ -20,7 +20,7 @@ STAGES = ["mark_repeats", "filter", "removecycles", "makescaffold"]
 OUTPUTS = [f"gt_scaffolder_algorithms_test_{s}.dot" for s in STAGES] + ["gt_scaffolder_new_write.scaf"]
 
 needs_bin = pytest.mark.skipif(not os.path.exists(B200_TESTX),
-                               reason="integration/_build/test_b200.x not built (needs /root/reference)")
+                               reason="integration/_build/test_b200.x not built (needs the reference's sources)")
 
 
 def _run(exe, args, cwd, tokeniser=None):

@@ -126,7 +126,7 @@ def _built():
     O.build_oracles()
 
 
-@pytest.mark.skipif(not O.have_ref() and not __import__("os").path.isdir("/root/reference"),
+@pytest.mark.skipif(not O.have_ref(),
                     reason="compiled reference (oracle/_ref) not available")
 @pytest.mark.parametrize("kind", ["one_line", "any"])
 def test_restatement_equals_reference_on_every_small_case(kind, synth):

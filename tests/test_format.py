@@ -16,7 +16,7 @@ import parse_emul as PE
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 C1 = os.path.join(HERE, "golden", "c1")
-needs_ref = pytest.mark.skipif(not (O.have_ref() or os.path.isdir("/root/reference")),
+needs_ref = pytest.mark.skipif(not O.have_ref(),
                                reason="compiled reference (oracle/_ref) not available")
 
 

@@ -85,7 +85,6 @@ def test_host_build_equals_the_reference(kind, rf, seed):
             assert got[3] * 20 < got[2], "the ranking keeps too many thetas: %d of %d" % (got[3], got[2])
 
 
-@needs_ref
 def test_negative_probability_is_refused():
     pmf = np.array([0.2, 0.5, -0.1, 0.4])
     frag = np.array([[0, 2]], np.int64)

@@ -21,7 +21,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 C1 = os.path.join(HERE, "golden", "c1")
 STAGES = ["mark_repeats", "filter", "removecycles", "makescaffold"]
 
-needs_ref = pytest.mark.skipif(not (O.have_ref() or os.path.isdir("/root/reference")),
+needs_ref = pytest.mark.skipif(not O.have_ref(),
                                reason="compiled reference (oracle/_ref) not available")
 
 

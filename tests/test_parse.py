@@ -19,7 +19,7 @@ import pytest
 import oracle_lib as O
 import parse_emul as PE
 
-needs_ref = pytest.mark.skipif(not (O.have_ref() or os.path.isdir("/root/reference")),
+needs_ref = pytest.mark.skipif(not O.have_ref(),
                                reason="compiled reference (oracle/_ref) not available")
 libc = C.CDLL("libc.so.6")
 libc.strtof.restype = C.c_float
