@@ -150,32 +150,6 @@ int await_records(gtsb_context *c) {
   return 0;
 }
 
-void l2_pin(gtsb_context *c, const void *p, size_t bytes) {
-  if (!c->l2_mode || c->l2_persist_max == 0 || p == nullptr || bytes == 0) return;
-  cudaStreamAttrValue v{};
-  const size_t win = bytes < c->l2_window_max ? bytes : c->l2_window_max;
-  v.accessPolicyWindow.base_ptr = const_cast<void *>(p);
-  v.accessPolicyWindow.num_bytes = win;
-  // a window larger than the set-aside keeps a random subset of its lines instead of thrashing
-  const double r = (double) c->l2_persist_max / (double) win;
-  v.accessPolicyWindow.hitRatio = r >= 1.0 ? 1.0f : (float) r;
-  v.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-  v.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-  if (cudaStreamSetAttribute(c->stream, cudaStreamAttributeAccessPolicyWindow, &v) != cudaSuccess) {
-    cudaGetLastError();
-    return;
-  }
-  c->l2_pinned = true;
-}
-
-void l2_unpin(gtsb_context *c) {
-  if (!c->l2_pinned) return;
-  cudaStreamAttrValue v{};
-  v.accessPolicyWindow.num_bytes = 0;
-  cudaStreamSetAttribute(c->stream, cudaStreamAttributeAccessPolicyWindow, &v);
-  c->l2_pinned = false;
-}
-
 // the copy stream may only start once the main stream is done with the buffers it overwrites
 int copy_stream_follows_main(gtsb_context *c) {
   CK(cudaEventRecord(c->ev_order, c->stream));
@@ -325,8 +299,8 @@ int do_build_lines(gtsb_context *c) {
   ENSURE(c->rf, R);
   ENSURE(c->cnt_in, (V + 2) * 4);
   ENSURE(c->bptr2, (V + 2) * 4);
-  const uint64_t ngrp = (V >> GROUP_SHIFT) + 2;
-  ENSURE(c->cursor2, ngrp * 4);
+  const uint64_t nsg = (V >> RSEG_SHIFT) + 2;
+  ENSURE(c->cursor2, nsg * 4);
   ENSURE(c->tmp_ent, R * sizeof(uint4));
   ENSURE(c->tmp_dest, R * 4);
   ENSURE(c->tmp_cursor, (NB_COARSE2 + 2) * 4);
@@ -345,7 +319,7 @@ int do_build_lines(gtsb_context *c) {
   CK(cudaMemsetAsync(c->pos.p, 0xFF, (V + 1) * 4, s));
   CK(cudaMemsetAsync(c->cnt_in.p, 0, (V + 2) * 4, s));
   CK(cudaMemsetAsync(c->nown.p, 0, (V + 2) * 4, s));
-  CK(cudaMemsetAsync(c->cursor2.p, 0, ngrp * 4, s));
+  CK(cudaMemsetAsync(c->cursor2.p, 0, nsg * 4, s));
   CK(cudaMemsetAsync(c->estate.p, 0, 2 * R ? 2 * R : 1, s));   // GIS_UNVISITED, graph.c:162
   CK(cudaMemsetAsync(c->vstate.p, 0, V ? V : 1, s));
 
@@ -354,16 +328,7 @@ int do_build_lines(gtsb_context *c) {
   a.V = (uint32_t) V;
   a.Vg = (uint32_t) V;
   a.sm_count = c->sm_count;
-  {
-    // dev switch.  0: the per-entry scatter passes; 3: per-entry pass A into NB_COARSE2 bins, tile-sorted pass B
-    const char *e = getenv("GTSB_MAIL");
-    a.mail_sorted = e != nullptr ? atoi(e) : 1;
-  }
-  a.nb_coarse = a.mail_sorted ? NB_COARSE2 : NB_COARSE;
-  if (a.mail_sorted && getenv("GTSB_NB") != nullptr) {   // dev switch: fewer coarse bins (64 .. NB_COARSE2)
-    const int nb = atoi(getenv("GTSB_NB"));
-    if (nb >= 64 && nb <= NB_COARSE2) a.nb_coarse = (uint32_t) nb;
-  }
+  a.nb_coarse = NB_COARSE2;
   uint32_t shift = 0;
   while (((V ? V - 1 : 0) >> shift) >= (uint64_t) a.nb_coarse) shift++;
   a.coarse_shift = shift;
@@ -680,9 +645,7 @@ int do_filter(gtsb_context *c, float pcutoff, float cncutoff, int64_t ocutoff, b
   CK(cudaMemsetAsync(c->fstat.p, 0x0C, V + 1, s));      // rows without slots: decided, nothing fires
   // phase 1: who proposes whom (+ the static overlap answer of every small row)
   launch_vertex_facts(a, fused ? 1 : 0, cn_cutoff, astat_cutoff, use_cn, s);
-  l2_pin(c, a.vinfo, (size_t) V * sizeof(uint2));
   launch_pairs(a, s);
-  l2_unpin(c);
   c->stats.kernel_launches += (V ? 1 : 0) + (E ? 1 : 0) + (E && c->n_big_rows ? 1 : 0);
   if (read_counters(c) != 0) return -1;
   if (c->h_counters[CNT_ERROR] & 4u) return fail(c, "gtsb_filter: a contig is longer than 2^31-1");
@@ -766,9 +729,7 @@ int do_filter(gtsb_context *c, float pcutoff, float cncutoff, int64_t ocutoff, b
     n_in = n_next;
   }
   launch_vres(a, s);
-  l2_pin(c, a.vres, (size_t) V * 4);
   launch_finalize(a, s);
-  l2_unpin(c);
   c->stats.kernel_launches += (V ? 1 : 0) + (E ? 1 : 0) + (E && c->n_big_rows ? 1 : 0);
   CK(cudaGetLastError());
   return 0;
@@ -842,33 +803,6 @@ int gtsb_create(gtsb_context **out, int device) {
   cudaDeviceProp prop;
   if (cudaGetDeviceProperties(&prop, device) == cudaSuccess) {
     c->sm_count = prop.multiProcessorCount;
-    const char *e = getenv("GTSB_L2_PIN");
-    c->l2_mode = e != nullptr ? atoi(e) : 0;   // measured slower on C3 (profiles/r02_l2_persistence_experiment.json)
-    if (c->l2_mode && prop.persistingL2CacheMaxSize > 0) {
-      // set-aside for persisting lines: a share of L2 the gathered per-vertex tables may keep
-      size_t want = (size_t) prop.persistingL2CacheMaxSize;
-      const char *f = getenv("GTSB_L2_PIN_MB");
-      if (f != nullptr && (size_t) atol(f) * 1048576 < want) want = (size_t) atol(f) * 1048576;
-      if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want) == cudaSuccess) {
-        c->l2_persist_max = want;
-        c->l2_window_max = (size_t) prop.accessPolicyMaxWindowSize;
-      } else {
-        cudaGetLastError();
-      }
-    }
-    // dev switch: how much the L2 fetches from HBM on a miss (32 / 64 / 128 bytes; a hint, device-wide).
-    // The per-vertex gathers use 4-8 bytes of every sector they fetch.
-    const char *fg = getenv("GTSB_L2_FETCH");
-    if (fg != nullptr && atoi(fg) > 0 &&
-        cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t) atoi(fg)) != cudaSuccess)
-      cudaGetLastError();
-    if (getenv("GTSB_TRACE") != nullptr) {
-      size_t gran = 0;
-      if (cudaDeviceGetLimit(&gran, cudaLimitMaxL2FetchGranularity) != cudaSuccess) cudaGetLastError();
-      fprintf(stderr, "[gtsb] L2 %d MB, persisting max %d MB, window max %d MB, pin %zu MB, fetch granularity %zu B\n",
-              prop.l2CacheSize >> 20, prop.persistingL2CacheMaxSize >> 20, prop.accessPolicyMaxWindowSize >> 20,
-              c->l2_persist_max >> 20, gran);
-    }
   }
   if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess) { delete c; return -1; }
   if (cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking) != cudaSuccess ||

@@ -33,7 +33,7 @@
 // of a box (gtsb_dist.cu): positions are then global (pos_base = the rank's
 // first position), creator ranks start at k_base, k2_classify counts mail per
 // destination RANK, k2_partition stores it into the owning rank's receive
-// buffers, and k2_deliver reads what the ranks sent here.
+// buffers, and k2_deliver2 sorts and delivers what the ranks sent here.
 #include "gtsb_common.cuh"
 #include "gtsb_scan.cuh"
 #include "gtsb_kernels.h"
@@ -463,49 +463,16 @@ __global__ void __launch_bounds__(256) k2_init_group_cursors(Build2Args a, int g
   if (p < a.V) a.cursor[grp] = a.bptr[p];
 }
 
-// pass D-B: stream the coarsely sorted entries into the mailbox region of
-// their destination GROUP of 2^GROUP_SHIFT positions (k2_resolve sorts a
-// segment's mail by line in shared memory).  One cursor per group: few enough
-// to stay cache-resident, enough of them that the atomics of the threads in
-// flight do not queue up on the same address (measured: ~70 ns per queued
-// same-address atomic).
-__global__ void __launch_bounds__(256) k2_deliver(Build2Args a) {
-  if (a.counters[CNT_FALLBACK] | a.counters[CNT_ERROR]) return;
-  constexpr int ILP = 4;
-  const uint32_t n = a.bptr[a.V];
-  const uint32_t stride = gridDim.x * blockDim.x;
-  for (uint32_t e0 = blockIdx.x * blockDim.x + threadIdx.x; e0 < n; e0 += stride * ILP) {
-    uint32_t pc[ILP], at[ILP];
-    uint4 ent[ILP];
-#pragma unroll
-    for (int k = 0; k < ILP; k++) {
-      const uint32_t e = e0 + k * stride;
-      pc[k] = e < n ? a.mail_dest[e] - a.pos_base : UNSET;
-      if (e < n) ent[k] = a.mail_ent[e];
-    }
-#pragma unroll
-    for (int k = 0; k < ILP; k++)
-      if (pc[k] != UNSET) {
-        at[k] = atomicAdd(&a.cursor[pc[k] >> GROUP_SHIFT], 1u);     // cursors start at the group's offset
-      }
-#pragma unroll
-    for (int k = 0; k < ILP; k++)
-      if (pc[k] != UNSET) {
-        a.bucket[at[k]] = ent[k];
-        a.bucket_line[at[k]] = (uint8_t) (pc[k] & (SEG_LINES - 1));
-      }
-  }
-}
-
-// ------------------------------------------------------------------ mail, tile-sorted (single device)
+// ------------------------------------------------------------------ mail, tile-sorted
 //
-// The two passes above move every entry with one 16-byte store of its own (and k2_deliver one
-// returning atomic per entry): 1.2e8 scattered L2 transactions for 4e7 entries, which is what
-// bounds them (profiles/r01_microbench_scatter.txt: 16-byte scatters run at 30-50 G/s whatever the
-// window).  The tile-sorted variants counting-sort a tile of entries by bin in shared memory, take
-// ONE cursor atomic per (tile, non-empty bin) and store the sorted tile with consecutive threads,
-// so that entries of a bin leave as runs: pass A bins by NB_COARSE2 position ranges, pass B by
-// resolve segment (RSEG_LINES positions) inside the few coarse bins a tile touches.
+// Moving the mail entry by entry -- a 16-byte store and a returning cursor atomic per entry --
+// costs 1.2e8 scattered L2 transactions for 4e7 entries, which is what bounds such a pass
+// (profiles/r01_microbench_scatter.txt: 16-byte scatters run at 30-50 G/s whatever the window).
+// The passes below counting-sort a tile of entries by bin in shared memory, take ONE cursor atomic
+// per (tile, non-empty bin) and store the sorted tile with consecutive threads, so that entries of
+// a bin leave as runs: pass A (k2_partition2, single device) bins by NB_COARSE2 position ranges,
+// pass B (k2_deliver2) by resolve segment (RSEG_LINES positions) inside the few coarse bins a tile
+// touches.
 
 constexpr int P2_THREADS = 512;
 constexpr uint32_t P2_ENT_CAP = 2432;        // entries staged per flush of pass A (>= SEG_REC_CAP)
@@ -514,8 +481,6 @@ constexpr int P2_SEGS = 12;                  // 128-line segments per block of p
 constexpr int D2_THREADS = 512;
 constexpr uint32_t D2_TILE = 3072;           // entries per block of pass B
 constexpr uint32_t D2_BINS = 2048;           // resolve segments a tile of pass B may span
-constexpr int RSEG_SHIFT = 6;
-static_assert((1 << RSEG_SHIFT) == RSEG_LINES, "RSEG_SHIFT");
 
 // Counting sort of n staged items by key (< nbins) and reservation of their output ranges:
 // s_perm[t] = item at sorted place t, s_off[b] = first sorted place of bin b (s_off[nbins] = n),
@@ -1095,7 +1060,7 @@ int launch_b2_partition(const Build2Args &a, cudaStream_t s) {
   if (nseg == 0) return 0;
   KernelTimer t_("k2_partition", s);
   k2_init_cursors<<<(a.nb_coarse + 128) / 128, 128, 0, s>>>(a);
-  if (a.mail_sorted == 1 && a.nranks == 0)
+  if (a.nranks == 0)
     k2_partition2<<<(nseg + P2_SEGS - 1) / P2_SEGS, P2_THREADS, build2_smem_partition2(), s>>>(a);
   else
     k2_partition<<<nseg, SEG_THREADS, build2_smem_partition(), s>>>(a);
@@ -1127,18 +1092,12 @@ int launch_b2_deliver_resolve(const Build2Args &a, cudaStream_t s) {
   if (nseg == 0) return 0;
   {
     KernelTimer t_("k2_deliver", s);
-    if (a.mail_sorted) {
-      const uint32_t nsg = (a.V >> RSEG_SHIFT) + 1;
-      k2_init_group_cursors<<<(nsg + 255) / 256, 256, 0, s>>>(a, RSEG_SHIFT);
-      // the grid covers every record (an upper bound of the mail the device knows only after the scan),
-      // or the mail count the ranks exchanged
-      const uint64_t tiles = ((a.nranks ? (uint64_t) a.n_mail : a.R) + D2_TILE - 1) / D2_TILE;
-      k2_deliver2<false><<<(uint32_t) (tiles ? tiles : 1), D2_THREADS, build2_smem_deliver2(), s>>>(a, 0u);
-    } else {
-      const uint32_t ngrp = (a.V >> GROUP_SHIFT) + 1;
-      k2_init_group_cursors<<<(ngrp + 255) / 256, 256, 0, s>>>(a, GROUP_SHIFT);
-      k2_deliver<<<a.sm_count * 8, 256, 0, s>>>(a);
-    }
+    const uint32_t nsg = (a.V >> RSEG_SHIFT) + 1;
+    k2_init_group_cursors<<<(nsg + 255) / 256, 256, 0, s>>>(a, RSEG_SHIFT);
+    // the grid covers every record (an upper bound of the mail the device knows only after the scan),
+    // or the mail count the ranks exchanged
+    const uint64_t tiles = ((a.nranks ? (uint64_t) a.n_mail : a.R) + D2_TILE - 1) / D2_TILE;
+    k2_deliver2<false><<<(uint32_t) (tiles ? tiles : 1), D2_THREADS, build2_smem_deliver2(), s>>>(a, 0u);
   }
   KernelTimer t_("k2_resolve", s);
   k2_resolve<<<(a.V + RSEG_LINES - 1) / RSEG_LINES, SEG_THREADS, build2_smem_resolve(), s>>>(a);

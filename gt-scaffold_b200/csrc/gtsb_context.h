@@ -106,11 +106,6 @@ struct gtsb_context {
   uint32_t row_base = 0;            // global position of local row 0
   uint64_t Vloc = 0;                // rows held by this rank (== V when world == 1)
 
-  // L2 residency of the table a flat pass gathers from (access-policy window on the stream)
-  int l2_mode = 0;                  // GTSB_L2_PIN: 0 off, 1 on
-  size_t l2_persist_max = 0, l2_window_max = 0;
-  bool l2_pinned = false;
-
   // cached ambiguous-order thresholds
   bool ambig_valid = false;
   float ambig_cutoff = 0.f;
@@ -132,10 +127,6 @@ int ensure_filter_buffers(gtsb_context *c, uint64_t Vg, uint64_t E, gtsb::Filter
 int await_vertices(gtsb_context *c);      // the main stream waits for late copies (no host sync)
 int await_records(gtsb_context *c);
 int ensure_root_column(gtsb_context *c);
-// keep [p, p + bytes) L2-resident for the kernels launched next on the stream (the slot columns a
-// flat pass streams are evict-first; the table it gathers from per slot should survive them)
-void l2_pin(gtsb_context *c, const void *p, size_t bytes);
-void l2_unpin(gtsb_context *c);
 
 struct ProfScope {                      // routes KernelTimer to the context's profiler while alive
   gtsb_context *c;

@@ -581,7 +581,7 @@ int dist_build(gtsb_context *c, DistState *D, Plan &P, int inputs_rc) {
     ENSURE(c->bptr2, cap_rows * 4);
     ENSURE(c->row_ptr, cap_rows * 4);
     ENSURE(c->big_rows, cap_rows * 4);
-    ENSURE(c->cursor2, ((cap_rows >> GROUP_SHIFT) + 2) * 4);
+    ENSURE(c->cursor2, ((cap_rows >> RSEG_SHIFT) + 2) * 4);
     ENSURE(c->lineless_flag, Vg + 1);
     ENSURE(c->lineless_rank, (Vg + 2) * 4);
     const uint64_t scan_n = Vg > R ? Vg : R;
@@ -601,7 +601,7 @@ int dist_build(gtsb_context *c, DistState *D, Plan &P, int inputs_rc) {
     CK(cudaMemsetAsync(c->vstate.p, 0, Vg ? Vg : 1, s));
     CK(cudaMemsetAsync(c->nown.p, 0, cap_rows * 4, s));
     CK(cudaMemsetAsync(c->cnt_in.p, 0, cap_rows * 4, s));
-    CK(cudaMemsetAsync(c->cursor2.p, 0, ((cap_rows >> GROUP_SHIFT) + 2) * 4, s));
+    CK(cudaMemsetAsync(c->cursor2.p, 0, ((cap_rows >> RSEG_SHIFT) + 2) * 4, s));
     CK(cudaMemsetAsync(D->rank_cnt.p, 0, (MAX_RANKS + 2) * 4, s));
     return 0;
   }();
@@ -695,9 +695,6 @@ int dist_build(gtsb_context *c, DistState *D, Plan &P, int inputs_rc) {
   }
   tr.mark(me, "classify+exchange");
 
-  // received mail is sorted by coarse bin first (tile sort), so that counting and delivering it
-  // work inside L2-sized windows; GTSB_MAIL=0: counted and delivered entry by entry (dev switch)
-  const bool mail_sorted = !(getenv("GTSB_MAIL") != nullptr && atoi(getenv("GTSB_MAIL")) == 0);
   // ---- receive buffers, then the messages: k2_partition stores every rank's mail straight into
   // that rank's buffers (peer memory over NVLink) while it computes the next ones
   bool grew = false, rx_grew = false;
@@ -709,10 +706,8 @@ int dist_build(gtsb_context *c, DistState *D, Plan &P, int inputs_rc) {
     grew |= rx_grew;
     ENSURE_U(c->bucket, (M_max + 1) * sizeof(uint4));
     ENSURE_U(c->bucket_line, M_max + 16);
-    if (mail_sorted) {                                   // the coarsely sorted copy of the received mail
-      ENSURE_U(c->tmp_ent, (M_max + 1) * sizeof(uint4));
-      ENSURE_U(c->tmp_dest, (M_max + 1) * 4);
-    }
+    ENSURE_U(c->tmp_ent, (M_max + 1) * sizeof(uint4));      // the coarsely sorted copy of the received mail
+    ENSURE_U(c->tmp_dest, (M_max + 1) * 4);
     const uint64_t max_rows = (M_max + creators_max + 1) / 2 + 1;      // slots = mail + own creators
     if (c->srcp.cap < 2 * max_rows * 4 + 256 || c->estate.cap < 2 * max_rows) {
       grew = true;
@@ -751,10 +746,9 @@ int dist_build(gtsb_context *c, DistState *D, Plan &P, int inputs_rc) {
 
   tr.mark(me, "partition+alltoall");
   // ---- receiver side: mailboxes of my rows, rows
-  a.mail_ent = D->rx_ent.as<uint4>();
-  a.mail_dest = D->rx_dest.as<uint32_t>();
-  if (mail_sorted) {
-    a.mail_sorted = 1;
+  // received mail is sorted by coarse bin first (tile sort), so that counting and delivering it
+  // work inside L2-sized windows
+  {
     a.nb_coarse = NB_COARSE2;
     uint32_t shift = 0;
     while (((P.Vloc ? P.Vloc - 1 : 0u) >> shift) >= (uint32_t) NB_COARSE2) shift++;
@@ -1004,9 +998,7 @@ int dist_filter(gtsb_context *c, DistState *D, const Plan &P, float cn_cutoff, f
   // the final pass reads a neighbour's fire bits and repeat predicate from the byte summary (and its
   // polyTime from poly_cur, which every rank holds complete): one byte per vertex crosses NVLink
   launch_vres(a, s);
-  static const bool summary = !(getenv("GTSB_FINAL") != nullptr && atoi(getenv("GTSB_FINAL")) == 1);
   if (allgatherv(c, "nccl_allgather_vsum", c->vsum.p, 1, P.lo) != 0) return -1;
-  if (!summary && allgatherv(c, "nccl_allgather_vres", c->vres.p, 4, P.lo) != 0) return -1;     // dev switch
   launch_finalize(a, s);
   c->stats.kernel_launches += 2 + (c->n_big_rows ? 1 : 0);
   return 0;

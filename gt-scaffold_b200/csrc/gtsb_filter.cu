@@ -455,81 +455,17 @@ struct PairsState {
   uint8_t es;
 };
 
-__global__ void __launch_bounds__(32 * WARPS, 8) k4_pairs(FilterArgs a) {
-  const GraphArgs &g = a.g;
-  const uint32_t lane = lane_id();
-  for_each_window<1>(g,
-    [&](uint32_t start, uint32_t n) {
-      PairsState t;
-      t.start = start;
-      t.n = n;
-      const bool valid = lane < n;
-      const uint32_t s = start + lane;
-      // slot columns are read once: evict-first, so that the gathered tables stay in L2
-      t.sp = valid ? __ldcs(g.srcp + s) : NONE;
-      t.dst = valid ? __ldcs(g.dst + s) : 0u;
-      t.fl = valid ? __ldcs(g.flags + s) : 0u;
-      t.me.dist = valid ? __ldcs(g.dist + s) : 0;
-      t.me.std_dev = valid ? __ldcs(g.std_dev + s) : 0.f;
-      t.es = (valid && !a.fused_repeats) ? __ldcs(g.estate + s) : (uint8_t) 0;
-      return t;
-    },
-    [&](PairsState &t) {
-      const bool valid = lane < t.n;
-      t.own_y = valid ? a.vinfo[t.sp & S_POS].y : VI_MARKED;
-      t.vi = valid ? a.vinfo[t.dst] : make_uint2(0u, 0u);
-    },
-    [&](PairsState &t) {
-      const Window W = open_window(t.start, t.n, t.sp);
-      // rows that cannot propose or fire: marked on entry (algorithms.c:279), < 2 edges
-      const bool act = W.valid && !(t.own_y & VI_MARKED) && (W.ve - W.vb) >= 2u;
-      if (!__any_sync(FULL, act)) return;
-      SlotFacts me = t.me;
-      me.cn = __uint_as_float(t.vi.x);
-      me.len = t.vi.y & ~VI_MARKED;
-      const bool wm = (t.vi.y & VI_MARKED) != 0;
-      const bool ok = act && (a.fused_repeats ? !wm : !edge_state_marked(t.es));
-      const bool sense = (t.fl & F_SENSE) != 0;
-      const uint32_t A = __ballot_sync(FULL, act), S = __ballot_sync(FULL, act && sense);
-      const uint32_t OK = __ballot_sync(FULL, ok);
-      const uint32_t higher = lane == 31u ? 0u : FULL << (lane + 1u);
-      const uint32_t P = act ? (W.rowmask & higher & (sense ? S : (A & ~S))) : 0u;
-      uint32_t prop_mask = 0, fire_mask = 0;
-      for_each_pair(P, [&](bool live, uint32_t i, uint32_t j) {
-        const SlotFacts e1 = shfl_facts(me, i), e2 = shfl_facts(me, j);   // e1 = earlier adjacency slot
-        uint32_t hit = 0, fire = 0;
-        if (live) {
-          // check_mark_polymorphic, algorithms.c:232-238
-          if (__fadd_rn(e1.cn, e2.cn) < a.cncutoff &&
-              ambiguous_order(e1.dist, e1.std_dev, e2.dist, e2.std_dev, a.ambig))
-            hit = 1u << (e1.cn < e2.cn ? i : j);
-          if (((OK >> i) & (OK >> j) & 1u) && a.ocutoff >= 0 &&
-              interval_overlap(e1.dist, e1.len, e2.dist, e2.len) > a.ocutoff)
-            fire = 1u << i;
-        }
-        prop_mask |= __reduce_or_sync(FULL, hit);
-        fire_mask |= __reduce_or_sync(FULL, fire);
-      });
-      // proposals (target must be unmarked, algorithms.c:242)
-      warp_append2(act && ((prop_mask >> lane) & 1u) && !wm, make_uint2(W.row, t.dst), a.proposals,
-                   a.proposals_cap, &g.counters[CNT_PROPOSALS], &g.counters[CNT_OVERFLOW]);
-      const uint32_t g1 = fire_mask & W.rowmask & S, g0 = fire_mask & W.rowmask & ~S;
-      if (W.head && act && (g0 | g1)) a.gbits[W.row] = (uint8_t) ((g0 ? 1u : 0u) | (g1 ? 2u : 0u));
-    });
-}
-
-// The same pass with far fewer pair evaluations.  All that phase 2 needs from a (row, direction)
-// is whether SOME pair of unmarked edges overlaps by more than ocutoff, and most groups have such a
-// pair among neighbouring slots.  Step A: every unmarked slot is tested against the NEXT unmarked
-// slot of its group -- one pair per lane, partner by shuffle, no dealing.  Step B deals out only
+// Most pairs need no evaluation.  All that phase 2 needs from a (row, direction) is whether SOME
+// pair of unmarked edges overlaps by more than ocutoff, and most groups have such a pair among
+// neighbouring slots.  Step A: every unmarked slot is tested against the NEXT unmarked slot of
+// its group -- one pair per lane, partner by shuffle, no dealing.  Step B deals out only
 // what is left: the other pairs of the groups that have not fired yet, and (for the polymorphic
 // test, algorithms.c:232-238) the pairs with a member of low copy number -- a pair can propose only
 // if cn1 + cn2 < cncutoff, so one of the two lies below cncutoff / 2 (taken with a margin that
 // covers the rounding of the float sum; the exact test decides).
-// (Walking ALL pairs per slot, lane i stepping through its partners, measured slower than dealing
-// them: 1.86 vs 1.59 ms at C3.)
-template <int MINB>
-__global__ void __launch_bounds__(32 * WARPS, MINB) k4_pairs3(FilterArgs a) {
+// (Dealing out every pair took the same 1.59 ms at C3 with 11 % more instructions; walking ALL
+// pairs per slot, lane i stepping through its partners, measured slower: 1.86 ms.)
+__global__ void __launch_bounds__(32 * WARPS, 8) k4_pairs3(FilterArgs a) {
   const GraphArgs &g = a.g;
   const uint32_t lane = lane_id();
   const float half = __fmul_rn(a.cncutoff, 0.5f);
@@ -851,20 +787,7 @@ void launch_pairs(const FilterArgs &a, cudaStream_t s) {
   if (a.g.E == 0) return;
   {
     KernelTimer t_("k4_pairs", s);
-    static const int pruned = [] {
-      const char *e = getenv("GTSB_PAIRS");              // 1: every pair dealt to the lanes (dev switch)
-      return (e != nullptr && atoi(e) == 1) ? 0 : 1;
-    }();
-    static const int occ6 = [] {
-      const char *e = getenv("GTSB_PAIRS_OCC");          // 6: 40 registers, 6 blocks per SM (dev switch)
-      return (e != nullptr && atoi(e) == 6) ? 1 : 0;
-    }();
-    if (pruned && occ6)
-      k4_pairs3<6><<<host_flat_grid(a.g.n_windows), 32 * WARPS, 0, s>>>(a);
-    else if (pruned)
-      k4_pairs3<8><<<host_flat_grid(a.g.n_windows), 32 * WARPS, 0, s>>>(a);
-    else
-      k4_pairs<<<host_flat_grid(a.g.n_windows), 32 * WARPS, 0, s>>>(a);
+    k4_pairs3<<<host_flat_grid(a.g.n_windows), 32 * WARPS, 0, s>>>(a);
   }
   if (a.g.n_big_rows) {
     KernelTimer t_("k4_pairs_big", s);
@@ -1487,48 +1410,7 @@ __device__ __forceinline__ void final_state(const FilterArgs &a, uint32_t s, uin
   }
 }
 
-struct FinalState {
-  uint32_t start, n, sp, dst, fl, own, ru;
-};
-
-__global__ void __launch_bounds__(32 * WARPS, 8) k4_finalize(FilterArgs a) {
-  const GraphArgs &g = a.g;
-  const uint32_t lane = lane_id();
-  for_each_window<1>(g,
-    [&](uint32_t start, uint32_t n) {
-      FinalState t;
-      t.start = start;
-      t.n = n;
-      const bool valid = lane < n;
-      const uint32_t s = start + lane;
-      t.sp = valid ? __ldcs(g.srcp + s) : NONE;
-      t.dst = valid ? __ldcs(g.dst + s) : 0u;
-      t.fl = valid ? __ldcs(g.flags + s) : 0u;
-      return t;
-    },
-    [&](FinalState &t) {
-      const bool valid = lane < t.n;
-      t.own = valid ? a.vres[t.sp & S_POS] : 0u;
-      t.ru = valid ? a.vres[t.dst] : 0u;
-    },
-    [&](FinalState &t) {
-      const Window W = open_window(t.start, t.n, t.sp);
-      const uint32_t f = t.fl, ru = t.ru;
-      // pass 1: latest neighbour that fired into (row, direction)
-      int inc0 = -1, inc1 = -1;
-      const bool fin = W.valid && (ru & ((f & F_RSENSE) ? VR_F1 : VR_F0));
-      const int id = fin ? (int) id_at(g, t.dst) : -1;
-      const uint32_t dir = twin_dir((f & F_RSENSE) != 0, (f & F_RSAME) != 0) ? 1u : 0u;
-      if (__any_sync(FULL, fin)) {
-        inc0 = row_max(fin && !dir ? id : -1, W.vb, W.ve);
-        inc1 = row_max(fin && dir ? id : -1, W.vb, W.ve);
-      }
-      // pass 2
-      if (W.valid) final_state(a, W.s, f, ru, t.own, W.row, inc0, inc1);
-    });
-}
-
-// The final pass with the neighbour facts read from the one-byte summary.  A window without a
+// The final pass reads the neighbour facts from the one-byte summary.  A window without a
 // polymorphic vertex in or next to its rows (most of them) needs no vertex ids and no row maxima:
 // an edge is INCONSISTENT iff anything fired into its (row, direction) or its own row fired.  The
 // other windows take the exact route: polyTime of the neighbours that have one (poly_cur, by
@@ -1643,14 +1525,7 @@ void launch_finalize(const FilterArgs &a, cudaStream_t s) {
   if (a.g.V == 0 || a.g.E == 0) return;
   {
     KernelTimer t_("k4_finalize", s);
-    static const int summary = [] {
-      const char *e = getenv("GTSB_FINAL");              // 1: neighbour facts from the 4-byte table (dev switch)
-      return (e != nullptr && atoi(e) == 1) ? 0 : 1;
-    }();
-    if (summary)
-      k4_finalize2<<<host_flat_grid(a.g.n_windows), 32 * WARPS, 0, s>>>(a);
-    else
-      k4_finalize<<<host_flat_grid(a.g.n_windows), 32 * WARPS, 0, s>>>(a);
+    k4_finalize2<<<host_flat_grid(a.g.n_windows), 32 * WARPS, 0, s>>>(a);
   }
   if (a.g.n_big_rows) {
     KernelTimer t_("k4_finalize_big", s);

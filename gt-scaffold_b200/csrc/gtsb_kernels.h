@@ -55,11 +55,12 @@ constexpr int SEG_LINES = 128;            // lines (positions) per block
 constexpr int SEG_THREADS = 256;
 constexpr uint32_t SEG_REC_CAP = 2048;    // staged records per segment
 constexpr int RSEG_LINES = 64;            // k2_resolve works on half segments (more blocks per SM)
+constexpr int RSEG_SHIFT = 6;
+static_assert((1 << RSEG_SHIFT) == RSEG_LINES, "RSEG_SHIFT");
 constexpr uint32_t RSEG_REC_CAP = 1024, RSEG_ENT_CAP = 768;
 constexpr uint32_t MAX_LINE_RECS = 64;         // longest line the per-thread scans accept
-constexpr int NB_COARSE = 64;             // coarse bins of the mailbox partition
-constexpr int NB_COARSE2 = 512;           // ... of its tile-sorted variant (single device)
-constexpr int GROUP_SHIFT = 3;            // mail is delivered to groups of 8 positions
+constexpr int NB_COARSE = 64;             // bins of k2_partition (partitioned build: one per destination rank)
+constexpr int NB_COARSE2 = 512;           // coarse bins of the tile-sorted mail passes
 
 constexpr int MAX_RANKS = 64;
 struct Build2Args {
@@ -71,9 +72,9 @@ struct Build2Args {
   int nranks;                               // 0: single device
   const uint32_t *rank_bounds;              // [nranks + 1] first global position of every rank
   uint32_t *rank_cnt;                       // [nranks] mail this rank sends to every rank
-  const uint4 *mail_ent;                    // the stream k2_deliver reads (tmp_ent, or what the ranks sent us)
+  const uint4 *mail_ent;                    // the coarsely sorted stream k2_deliver2 reads (tmp_ent)
   const uint32_t *mail_dest;
-  const uint4 *rx_ent;                      // partitioned build with mail_sorted: what the ranks sent us, in no order
+  const uint4 *rx_ent;                      // partitioned build: what the ranks sent us, in no order
   const uint32_t *rx_dest;                  // (k2_deliver2<COARSE> sorts it into tmp_ent / tmp_dest)
   uint32_t n_mail;                          // its length
   // partitioned build: k2_partition stores each rank's mail straight into that rank's receive
@@ -83,8 +84,9 @@ struct Build2Args {
   const long long *peer_shift;
   int sm_count;
   uint32_t coarse_shift, corrections_cap;
-  uint32_t nb_coarse;                       // coarse bins in use: NB_COARSE, or NB_COARSE2 with mail_sorted
-  int mail_sorted;                          // single device: tile-sorted mail passes (k2_partition2 / k2_deliver2)
+  uint32_t nb_coarse;                       // coarse bins of the tile-sorted mail passes: NB_COARSE2
+  int mail_sorted;                          // no reader; removing it re-packs the struct and changes the code of
+                                            // the hot build kernels -- do it with a change that re-measures them
   const uint32_t *root, *ctg;
   const int32_t *dist;
   const float *std_dev;
@@ -93,7 +95,7 @@ struct Build2Args {
   uint32_t *tile_cnt, *tile_off;            // head tiles
   uint8_t *rf;                              // [R] RF_UP | RF_FIRST
   uint32_t *cnt_in, *bptr;                  // [V+1] mailbox sizes / offsets
-  uint32_t *cursor;                         // [V >> GROUP_SHIFT] fill of every group's mailbox region
+  uint32_t *cursor;                         // [(V >> RSEG_SHIFT) + 1] fill of every resolve segment's mailbox region
   uint4 *tmp_ent, *bucket, *corrections;
   uint8_t *bucket_line;                     // [creators] line (within its segment) of every delivered entry
   uint32_t *tmp_dest, *tmp_cursor;

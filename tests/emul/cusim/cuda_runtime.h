@@ -319,24 +319,12 @@ static inline unsigned long max(unsigned int a, unsigned long b) { return a > b 
 
 // ---------------------------------------------------------------- runtime API
 struct cudaDeviceProp {
-  int multiProcessorCount, l2CacheSize, persistingL2CacheMaxSize, accessPolicyMaxWindowSize;
+  int multiProcessorCount;
   char name[64];
 };
-enum cudaLimit { cudaLimitPersistingL2CacheSize, cudaLimitMaxL2FetchGranularity };
 enum cudaDeviceAttr { cudaDevAttrCooperativeLaunch, cudaDevAttrMultiProcessorCount };
 enum cudaFuncAttribute { cudaFuncAttributeMaxDynamicSharedMemorySize, cudaFuncAttributePreferredSharedMemoryCarveout };
 enum { cudaStreamNonBlocking = 1, cudaEventDisableTiming = 2, cudaIpcMemLazyEnablePeerAccess = 1 };
-enum cudaAccessProperty { cudaAccessPropertyNormal, cudaAccessPropertyStreaming, cudaAccessPropertyPersisting };
-struct cudaAccessPolicyWindow {
-  void *base_ptr;
-  size_t num_bytes;
-  float hitRatio;
-  cudaAccessProperty hitProp, missProp;
-};
-union cudaStreamAttrValue {
-  cudaAccessPolicyWindow accessPolicyWindow;
-};
-enum cudaStreamAttrID { cudaStreamAttributeAccessPolicyWindow };
 struct cudaIpcMemHandle_t { char reserved[64]; };
 
 static inline cudaError_t cudaGetDeviceCount(int *n) { *n = 1; return cudaSuccess; }
@@ -345,12 +333,9 @@ static inline cudaError_t cudaGetDevice(int *d) { *d = 0; return cudaSuccess; }
 static inline cudaError_t cudaGetDeviceProperties(cudaDeviceProp *p, int) {
   memset(p, 0, sizeof(*p));
   p->multiProcessorCount = 2;                 // small grids: the persistent kernels size themselves by this
-  p->l2CacheSize = 1 << 20;
   strcpy(p->name, "cusim");
   return cudaSuccess;
 }
-static inline cudaError_t cudaDeviceSetLimit(cudaLimit, size_t) { return cudaSuccess; }
-static inline cudaError_t cudaDeviceGetLimit(size_t *v, cudaLimit) { *v = 0; return cudaSuccess; }
 static inline cudaError_t cudaDeviceGetAttribute(int *v, cudaDeviceAttr a, int) {
   *v = a == cudaDevAttrMultiProcessorCount ? 2 : 1;     // cooperative launch: every block alive at once
   return cudaSuccess;
@@ -373,7 +358,6 @@ static inline cudaError_t cudaStreamDestroy(cudaStream_t s) { free(s); return cu
 static inline cudaError_t cudaStreamSynchronize(cudaStream_t) { return cudaSuccess; }
 static inline cudaError_t cudaDeviceSynchronize() { return cudaSuccess; }
 static inline cudaError_t cudaStreamWaitEvent(cudaStream_t, cudaEvent_t, unsigned = 0) { return cudaSuccess; }
-static inline cudaError_t cudaStreamSetAttribute(cudaStream_t, cudaStreamAttrID, const cudaStreamAttrValue *) { return cudaSuccess; }
 // events carry the host's clock: cudaEventElapsedTime is emulation time, useful only to see which
 // kernel the emulation spends its rendezvous on
 struct cusim_event { double t; };
