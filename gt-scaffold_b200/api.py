@@ -189,6 +189,38 @@ def shard_lines(inp, world: int, rank: int, mail_weight: float = MAIL_WEIGHT):
                      meta=dict(inp.meta, shard=(rank, world, lo, hi)), **kw)
 
 
+def _piece_root(text: bytes, s: int, e: int):
+    """First ' '-separated token of the fgets piece [s, e) (its last character dropped), or None."""
+    tok = text[s:e - 1].lstrip(b" ").split(b" ", 1)[0]
+    return tok or None
+
+
+def shard_text(text: bytes, world: int, rank: int, mail_weight: float = MAIL_WEIGHT):
+    """Rank `rank`'s chunk [lo, hi) of a .de / .astat text for gtsb_parse_*_host on a partitioned
+    context: cuts start at the byte fractions of chunk_fractions() and move forward to a line start;
+    they keep moving while the root of the line after the cut equals the root of the last fgets
+    piece (<= 1023 characters) before it, so that a run of one root's lines stays on one rank.  A
+    last line without '\n' is never cut off from the last rank.  mail_weight=0 for .astat text."""
+    n = len(text)
+    end = n if text.endswith(b"\n") else text.rfind(b"\n") + 1       # cuts lie in [0, end]
+    fr = chunk_fractions(world, mail_weight)
+    cuts = [0]
+    for r in range(1, world):
+        i = max(min(int(n * fr[r]), end), cuts[-1])
+        if i > 0 and text[i - 1:i] != b"\n":
+            i = text.find(b"\n", i) + 1 or end
+        while 0 < i < end:
+            s = text.rfind(b"\n", 0, i - 1) + 1                  # start of the line that ends at i
+            last = _piece_root(text, s + (i - 1 - s) // 1023 * 1023, i)
+            nxt = text.find(b"\n", i)
+            if last is None or last != _piece_root(text, i, min(i + 1023, nxt + 1)):
+                break
+            i = nxt + 1
+        cuts.append(i)
+    cuts.append(n)
+    return cuts[rank], cuts[rank + 1]
+
+
 class ScaffoldGraphB200:
     """A scaffold graph resident in B200 HBM."""
 
@@ -245,7 +277,9 @@ class ScaffoldGraphB200:
 
     def parse_de(self, text: bytes):
         """-> (irregular bits, nof_records).  irregular != 0: the text is outside the canonical
-        spelling, nothing was set, tokenise on the host."""
+        spelling, nothing was set, tokenise on the host.  On a partitioned context (dist_init) every
+        rank calls this together with its own chunk of the file (shard_text) and keeps the records of
+        its chunk; the bits are the OR over the ranks, and a refusal anywhere sets nothing anywhere."""
         R = C.c_uint64(0)
         irr = C.c_uint32(0)
         self._ck(self.L.gtsb_parse_de_host(self.h, text, C.c_uint64(len(text)), C.byref(R), C.byref(irr)))
@@ -254,7 +288,10 @@ class ScaffoldGraphB200:
 
     def parse_astat(self, text: bytes, astat, copy_num):
         """-> (irregular bits, astat, copy_num): copies of the inputs with the .astat text applied
-        (algorithms.c:118-149); irregular != 0: untouched, read the file on the host."""
+        (algorithms.c:118-149); irregular != 0: untouched, read the file on the host.  On a partitioned
+        context every rank calls this together with its own chunk of the file (shard_text with
+        mail_weight=0) and the full arrays; all ranks get the same values, the last line in file
+        order winning."""
         a = np.array(astat, np.float32)
         cn = np.array(copy_num, np.float32)
         irr = C.c_uint32(0)

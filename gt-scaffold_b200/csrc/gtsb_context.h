@@ -75,10 +75,11 @@ struct gtsb_context {
   // .de text on the device (gtsb_parse.cu)
   DevBuf p_names, p_name_off, p_slots, p_flags, p_text, p_chunk_cnt, p_chunk_off, p_line_end,
       p_line_cnt, p_line_off, num_pairs, p_last, p_astat, p_copy_num;
+  DevBuf p_key, p_win;          // partitioned `.astat`: (rank, offset) of the winning line, winners' values
   DevBuf f_state, f_sense, f_src, f_dst, f_dist, f_len, f_off, f_out;     // .dot lines (gtsb_format.cu)
   DevBuf s_root, s_recoff, s_end, s_dist, s_std, s_flags, s_len_r, s_off_r;   // .scaf records (gtsb_format.cu)
   DevBuf m_pairs, m_size, m_count, m_pmf, m_logp, m_L, m_c, m_n, m_g, m_slot_pair, m_gmax, m_mag, m_cand;   // distance MLE (gtsb_mle.cu)
-  uint64_t names_V = 0, names_mask = 0;
+  uint64_t names_V = 0, names_mask = 0, names_bytes = 0;
   bool have_names = false, names_dup = false, have_num_pairs = false;
 
   uint32_t *h_counters = nullptr;   // pinned
@@ -138,6 +139,20 @@ struct ProfScope {                      // routes KernelTimer to the context's p
 int dist_pipeline(gtsb_context *c, float cn_cutoff, float astat_cutoff, int use_cn, float pcutoff,
                   float cncutoff, int64_t ocutoff);
 void dist_release(gtsb_context *c);
+// `.de` / `.astat` text on every rank of a partitioned context (collective)
+int dist_parse_de(gtsb_context *c, const char *text, uint64_t n, uint64_t *nof_records, uint32_t *irregular);
+int dist_parse_astat(gtsb_context *c, const char *text, uint64_t n, float *astat, float *copy_num,
+                     uint32_t *irregular);
+
+// the stages of the text entry points (gtsb_parse.cu), shared by the single-device and the
+// partitioned calls
+int parse_preamble(gtsb_context *c, const char *what, const char *text, uint64_t n);
+int de_count(gtsb_context *c, const char *text, uint64_t n, uint64_t *nlines, uint32_t *total, uint32_t *irregular);
+int de_emit(gtsb_context *c, uint64_t nlines, uint32_t total);
+void keep_parsed_records(gtsb_context *c, uint64_t R);
+int astat_last(gtsb_context *c, const char *text, uint64_t n, const float *astat, const float *copy_num,
+               uint64_t *nlines, uint32_t *irregular);
+int astat_apply(gtsb_context *c, uint64_t nlines);
 
 }  // namespace gtsbi
 

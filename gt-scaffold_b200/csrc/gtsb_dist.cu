@@ -20,6 +20,8 @@
 //           fire status, once per fire round        allgatherv,     1 B/vertex
 //           final per-vertex facts vres             allgatherv,     4 B/vertex
 //           vertex states                           allreduce(max), 1 B/vertex
+//   .astat  key of the winning line (rank, offset)  allreduce(max), 8 B/vertex
+//           the winners' values (u32 bit patterns)  allreduce(sum), 8 B/vertex
 //
 // Both directed edges of a link are evaluated by their own rows' owners from
 // the same vertex-level facts, so the symmetric edge marks agree without any
@@ -333,6 +335,41 @@ __global__ void __launch_bounds__(256) k_digest_vertices(uint64_t V, const uint8
        v += (uint64_t) gridDim.x * blockDim.x)
     if (v < V) h += mix64(mix64(v) ^ vstate[v]);
   digest_add(h, acc);
+}
+
+// `.astat` text over the ranks: the last line in FILE order wins.  A vertex named on this rank has the
+// key (rank << 32 | offset + 1 of its last piece here), 0 elsewhere; the maximum over the ranks is the
+// winner's key (offsets are below 2^32: a chunk is smaller than 4 GiB).
+__global__ void k_dist_astat_keys(uint64_t V, uint32_t rank, const uint64_t *__restrict__ last,
+                                  uint64_t *__restrict__ key) {
+  const uint64_t v = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x;
+  if (v < V) key[v] = last[v] ? ((uint64_t) rank << 32 | last[v]) : 0ull;
+}
+
+// a local last line that a later line beat is forgotten, so that kp_astat<apply> writes winners only
+__global__ void k_dist_astat_winners(uint64_t V, uint32_t rank, const uint64_t *__restrict__ key,
+                                     uint64_t *__restrict__ last) {
+  const uint64_t v = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x;
+  if (v < V && last[v] && key[v] != ((uint64_t) rank << 32 | last[v])) last[v] = 0;
+}
+
+// the winner's two values as bit patterns, zero on every other rank: a sum over the ranks delivers them
+// bit for bit (-0 and NaN included)
+__global__ void k_dist_astat_pack(uint64_t V, const uint64_t *__restrict__ last, const float *__restrict__ astat,
+                                  const float *__restrict__ copy_num, uint32_t *__restrict__ win) {
+  const uint64_t v = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x;
+  if (v >= V) return;
+  win[v] = last[v] ? __float_as_uint(astat[v]) : 0u;
+  win[V + v] = last[v] ? __float_as_uint(copy_num[v]) : 0u;
+}
+
+__global__ void k_dist_astat_unpack(uint64_t V, const uint64_t *__restrict__ key, const uint32_t *__restrict__ win,
+                                    float *__restrict__ astat, float *__restrict__ copy_num) {
+  const uint64_t v = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x;
+  if (v < V && key[v]) {
+    astat[v] = __uint_as_float(win[v]);
+    copy_num[v] = __uint_as_float(win[V + v]);
+  }
 }
 
 // (re)open every rank's receive buffers; collective
@@ -1030,6 +1067,125 @@ int dist_pipeline(gtsb_context *c, float cn_cutoff, float astat_cutoff, int use_
     KernelTimer t_("nccl_allreduce_vstate", c->stream);
     NK(g_nccl.AllReduce(c->vstate.p, c->vstate.p, c->V, ncclUint8, ncclMax, D->comm, c->stream));
   }
+  CK(cudaGetLastError());
+  return 0;
+}
+
+// ---- `.de` / `.astat` text, every rank its own chunk of the file (collective)
+
+// the local checks that every text call makes before it reads its chunk
+int dist_text_checks(gtsb_context *c, const char *what, const char *text, uint64_t n) {
+  if (parse_preamble(c, what, text, n) != 0) return -1;
+  // the fgets pieces of the chunks are those of the whole file only if every chunk but the last
+  // ends a line
+  if (c->rank < c->world - 1 && n != 0 && text[n - 1] != '\n')
+    return fail(c, "%s: the chunk of rank %d does not end in '\\n' (only the last rank's may)", what, c->rank);
+  bool unused = false;
+  return injected_failure(c, "parse", unused);
+}
+
+// every rank's status, IRR_* bits and names set; *irregular = the OR of the bits
+int dist_text_agree(gtsb_context *c, int local_rc, const char *what, uint32_t irregular_mine, uint32_t *irregular) {
+  const uint32_t mine[4] = {irregular_mine, (uint32_t) c->names_V, (uint32_t) c->names_bytes,
+                            (uint32_t) (c->names_bytes >> 32)};
+  std::vector<uint32_t> all;
+  if (exchange(c, local_rc, what, mine, 4, all) != 0) return -1;
+  uint32_t irr = 0;
+  for (int r = 0; r < c->world; r++) {
+    irr |= all[(size_t) r * 4];
+    for (int i = 1; i < 4; i++)
+      if (all[(size_t) r * 4 + i] != mine[i])
+        return fail(c, "%s: the ranks hold different vertex name sets (rank %d: %u contigs, %llu header bytes; "
+                       "rank %d: %u, %llu)", what, c->rank, mine[1], (unsigned long long) c->names_bytes, r,
+                    all[(size_t) r * 4 + 1],
+                    (unsigned long long) all[(size_t) r * 4 + 2] | (unsigned long long) all[(size_t) r * 4 + 3] << 32);
+  }
+  *irregular = irr;
+  return 0;
+}
+
+int dist_parse_de(gtsb_context *c, const char *text, uint64_t n, uint64_t *nof_records, uint32_t *irregular_out) {
+  const char *what = "gtsb_parse_de_host";
+  ProfScope prof(c);
+  uint64_t nlines = 0;
+  uint32_t total = 0, irregular = 0;
+  const int rc = [&]() -> int {
+    if (nof_records == nullptr || irregular_out == nullptr) return fail(c, "%s: null argument", what);
+    if (dist_text_checks(c, what, text, n) != 0) return -1;
+    if (await_records(c) != 0) return -1;
+    if (c->names_dup) {
+      irregular = GTSB_IRR_DUP_NAME;
+      return 0;
+    }
+    return de_count(c, text, n, &nlines, &total, &irregular);
+  }();
+  c->have_records = false;
+  c->have_graph = false;
+  if (nof_records != nullptr) *nof_records = 0;
+  if (irregular_out != nullptr) *irregular_out = 0;
+  uint32_t irr = 0;
+  if (dist_text_agree(c, rc, what, irregular, &irr) != 0) return -1;
+  if (irr) {                           // a refusal anywhere: no rank keeps records, all read the file on the host
+    *irregular_out = irr;
+    return 0;
+  }
+  if (agree(c, de_emit(c, nlines, total), what) != 0) return -1;
+  keep_parsed_records(c, total);
+  *nof_records = total;
+  return 0;
+}
+
+int dist_parse_astat(gtsb_context *c, const char *text, uint64_t n, float *astat, float *copy_num,
+                     uint32_t *irregular_out) {
+  const char *what = "gtsb_parse_astat_host";
+  DistState *D = static_cast<DistState *>(c->dstate);
+  ProfScope prof(c);
+  cudaStream_t s = c->stream;
+  const uint64_t V = c->names_V;
+  uint64_t nlines = 0;
+  uint32_t irregular = 0;
+  const int rc = [&]() -> int {
+    if (irregular_out == nullptr) return fail(c, "%s: null argument", what);
+    if (dist_text_checks(c, what, text, n) != 0) return -1;
+    if (V && (astat == nullptr || copy_num == nullptr)) return fail(c, "%s: null argument", what);
+    if (c->names_dup) {
+      irregular = GTSB_IRR_DUP_NAME;
+      return 0;
+    }
+    ENSURE(c->p_key, (V + 1) * 8);
+    ENSURE(c->p_win, (V + 1) * 8);
+    return astat_last(c, text, n, astat, copy_num, &nlines, &irregular);
+  }();
+  if (irregular_out != nullptr) *irregular_out = 0;
+  uint32_t irr = 0;
+  if (dist_text_agree(c, rc, what, irregular, &irr) != 0) return -1;
+  if (irr) {                           // a refusal anywhere: no rank touches the arrays
+    *irregular_out = irr;
+    return 0;
+  }
+  uint64_t *last = c->p_last.as<uint64_t>(), *key = c->p_key.as<uint64_t>();
+  uint32_t *win = c->p_win.as<uint32_t>();
+  const uint32_t blocks = (uint32_t) ((V + 255) / 256), me = (uint32_t) c->rank;
+  if (V) {
+    KernelTimer t_("k_dist_astat(winners)+allreduce", s);
+    k_dist_astat_keys<<<blocks, 256, 0, s>>>(V, me, last, key);
+    NK(g_nccl.AllReduce(key, key, V, ncclUint64, ncclMax, D->comm, s));
+    k_dist_astat_winners<<<blocks, 256, 0, s>>>(V, me, key, last);
+    c->stats.kernel_launches += 2;
+  }
+  if (astat_apply(c, nlines) != 0) return -1;
+  if (V) {
+    KernelTimer t_("k_dist_astat(values)+allreduce", s);
+    k_dist_astat_pack<<<blocks, 256, 0, s>>>(V, last, c->p_astat.as<float>(), c->p_copy_num.as<float>(), win);
+    NK(g_nccl.AllReduce(win, win, 2 * V, ncclUint32, ncclSum, D->comm, s));
+    k_dist_astat_unpack<<<blocks, 256, 0, s>>>(V, key, win, c->p_astat.as<float>(), c->p_copy_num.as<float>());
+    c->stats.kernel_launches += 2;
+  }
+  if (V) {
+    CK(cudaMemcpyAsync(astat, c->p_astat.p, V * 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(copy_num, c->p_copy_num.p, V * 4, cudaMemcpyDeviceToHost, s));
+  }
+  CK(cudaStreamSynchronize(s));
   CK(cudaGetLastError());
   return 0;
 }

@@ -13,6 +13,9 @@
 //   kp_astat<false>   one thread per line: per contig, the offset of the last line naming it
 //   kp_astat<true>    that line writes the contig's a-statistic and copy number
 //
+// On a partitioned context every rank runs these passes on its chunk of the file; the agreement
+// between the ranks and the `.astat` winners across them are gtsb_dist.cu's (dist_parse_*).
+//
 // The walk is a byte loop per thread over its own line; neighbouring threads hold neighbouring
 // lines, so a warp's loads fall into one window of a few KB that L1 keeps.
 #include "gtsb_context.h"
@@ -112,6 +115,7 @@ int gtsb_set_vertex_names_host(gtsb_context *c, uint64_t V, const char *names, c
   // texts of this graph are left to the host (every parse call reports GTSB_IRR_DUP_NAME)
   c->names_dup = (irregular & IRR_DUP_NAME) != 0;
   c->names_V = V;
+  c->names_bytes = bytes;
   c->have_names = true;
   return 0;
 }
@@ -160,37 +164,23 @@ static int index_lines(gtsb_context *c, const char *text, uint64_t n, uint64_t *
   return 0;
 }
 
-static int parse_preamble(gtsb_context *c, const char *what, const char *text, uint64_t n) {
+}  // namespace gtsbparse
+
+namespace gtsbi {
+
+int parse_preamble(gtsb_context *c, const char *what, const char *text, uint64_t n) {
   if (!c->have_names) return fail(c, "%s: vertex names not set", what);
   if (n && text == nullptr) return fail(c, "%s: null argument", what);
-  if (c->world > 1) return fail(c, "%s: single-device contexts only", what);
   // line and record counts are 32-bit sums over the text: every line and every record takes
   // a byte at least, so below 4 GiB none of them can wrap
   if (n >= (1ull << 32)) return fail(c, "%s: text of 4 GiB or more", what);
   return 0;
 }
 
-}  // namespace gtsbparse
-
-extern "C" {
-
-int gtsb_parse_de_host(gtsb_context *c, const char *text, uint64_t n, uint64_t *nof_records,
-                       uint32_t *irregular_out) {
-  if (c == nullptr) return -1;
-  CK(cudaSetDevice(c->device));
-  if (nof_records == nullptr || irregular_out == nullptr) return fail(c, "gtsb_parse_de_host: null argument");
-  if (parse_preamble(c, "gtsb_parse_de_host", text, n) != 0) return -1;
-  if (await_records(c) != 0) return -1;
-  ProfScope prof(c);
+// line index, then records per line: *total records, *irregular = the text's IRR_* bits
+int de_count(gtsb_context *c, const char *text, uint64_t n, uint64_t *nlines_out, uint32_t *total_out,
+             uint32_t *irregular_out) {
   cudaStream_t s = c->stream;
-  *nof_records = 0;
-  *irregular_out = 0;
-  c->have_records = false;
-  c->have_graph = false;
-  if (c->names_dup) {
-    *irregular_out = IRR_DUP_NAME;
-    return 0;
-  }
   uint64_t nlines = 0;
   if (index_lines(c, text, n, &nlines) != 0) return -1;
   ENSURE(c->p_line_cnt, (nlines + 1) * 4);
@@ -199,8 +189,6 @@ int gtsb_parse_de_host(gtsb_context *c, const char *text, uint64_t n, uint64_t *
   const char *d_text = c->p_text.as<char>();
   const uint64_t *line_end = c->p_line_end.as<uint64_t>();
   uint32_t *flags = c->p_flags.as<uint32_t>();
-
-  // records per line, then the records
   const NameTable t{c->p_names.as<char>(), c->p_name_off.as<uint64_t>(), c->p_slots.as<uint64_t>(),
                     c->names_mask};
   Records out{};
@@ -219,10 +207,17 @@ int gtsb_parse_de_host(gtsb_context *c, const char *text, uint64_t n, uint64_t *
   CK(cudaMemcpyAsync(&irregular, flags, 4, cudaMemcpyDeviceToHost, s));
   CK(cudaStreamSynchronize(s));
   CK(cudaGetLastError());
-  if (irregular) {                     // nothing is kept: the caller parses this file on the host
-    *irregular_out = irregular;
-    return 0;
-  }
+  *nlines_out = nlines;
+  *total_out = total;
+  *irregular_out = irregular;
+  return 0;
+}
+
+// the records de_count counted, written into the context's record columns
+int de_emit(gtsb_context *c, uint64_t nlines, uint32_t total) {
+  cudaStream_t s = c->stream;
+  const NameTable t{c->p_names.as<char>(), c->p_name_off.as<uint64_t>(), c->p_slots.as<uint64_t>(),
+                    c->names_mask};
   const uint64_t R = total;
   DevBuf *bs[] = {&c->root, &c->ctg, &c->dist, &c->std_dev, &c->flags};
   for (DevBuf *b : bs)
@@ -233,40 +228,33 @@ int gtsb_parse_de_host(gtsb_context *c, const char *text, uint64_t n, uint64_t *
   ENSURE(c->std_dev, R * 4);
   ENSURE(c->flags, R);
   ENSURE(c->num_pairs, R * 4);
-  out = Records{c->root.as<uint32_t>(), c->ctg.as<uint32_t>(), c->dist.as<int32_t>(), c->std_dev.as<float>(),
-                c->num_pairs.as<uint32_t>(), c->flags.as<uint8_t>()};
+  const Records out{c->root.as<uint32_t>(), c->ctg.as<uint32_t>(), c->dist.as<int32_t>(), c->std_dev.as<float>(),
+                    c->num_pairs.as<uint32_t>(), c->flags.as<uint8_t>()};
   if (R) {
     GTSB_TIMED("kp_walk(emit)", s);
-    kp_walk<true><<<blocks_for(nlines, 128), 128, 0, s>>>(d_text, line_end, nlines, t, out, nullptr,
-                                                         c->p_line_off.as<uint32_t>(), flags);
+    kp_walk<true><<<blocks_for(nlines, 128), 128, 0, s>>>(c->p_text.as<char>(), c->p_line_end.as<uint64_t>(), nlines,
+                                                         t, out, nullptr, c->p_line_off.as<uint32_t>(),
+                                                         c->p_flags.as<uint32_t>());
     c->stats.kernel_launches++;
     CK(cudaGetLastError());
   }
+  return 0;
+}
+
+void keep_parsed_records(gtsb_context *c, uint64_t R) {
   c->R = R;
   c->have_records = true;
   c->have_root_column = true;
   c->have_lines = false;
   c->have_num_pairs = true;
   c->stats.nof_records = R;
-  *nof_records = R;
-  return 0;
 }
 
-int gtsb_parse_astat_host(gtsb_context *c, const char *text, uint64_t n, float *astat, float *copy_num,
-                          uint32_t *irregular_out) {
-  if (c == nullptr) return -1;
-  CK(cudaSetDevice(c->device));
-  if (irregular_out == nullptr) return fail(c, "gtsb_parse_astat_host: null argument");
-  if (parse_preamble(c, "gtsb_parse_astat_host", text, n) != 0) return -1;
-  const uint64_t V = c->names_V;
-  if (V && (astat == nullptr || copy_num == nullptr)) return fail(c, "gtsb_parse_astat_host: null argument");
-  ProfScope prof(c);
+// line index, the caller's values on the device, last[v] = offset + 1 of the last piece naming v
+int astat_last(gtsb_context *c, const char *text, uint64_t n, const float *astat, const float *copy_num,
+               uint64_t *nlines_out, uint32_t *irregular_out) {
   cudaStream_t s = c->stream;
-  *irregular_out = 0;
-  if (c->names_dup) {
-    *irregular_out = IRR_DUP_NAME;
-    return 0;
-  }
+  const uint64_t V = c->names_V;
   uint64_t nlines = 0;
   if (index_lines(c, text, n, &nlines) != 0) return -1;
   ENSURE(c->p_last, (V + 1) * 8);
@@ -291,17 +279,85 @@ int gtsb_parse_astat_host(gtsb_context *c, const char *text, uint64_t n, float *
   CK(cudaMemcpyAsync(&irregular, flags, 4, cudaMemcpyDeviceToHost, s));
   CK(cudaStreamSynchronize(s));
   CK(cudaGetLastError());
+  *nlines_out = nlines;
+  *irregular_out = irregular;
+  return 0;
+}
+
+// the piece at last[v] writes v's two values on the device
+int astat_apply(gtsb_context *c, uint64_t nlines) {
+  cudaStream_t s = c->stream;
+  if (nlines) {
+    const NameTable t{c->p_names.as<char>(), c->p_name_off.as<uint64_t>(), c->p_slots.as<uint64_t>(),
+                      c->names_mask};
+    GTSB_TIMED("kp_astat(apply)", s);
+    kp_astat<true><<<blocks_for(nlines, 128), 128, 0, s>>>(c->p_text.as<char>(), c->p_line_end.as<uint64_t>(),
+                                                          nlines, t, c->p_last.as<uint64_t>(),
+                                                          c->p_astat.as<float>(), c->p_copy_num.as<float>(),
+                                                          c->p_flags.as<uint32_t>());
+    c->stats.kernel_launches++;
+  }
+  return 0;
+}
+
+}  // namespace gtsbi
+
+extern "C" {
+
+int gtsb_parse_de_host(gtsb_context *c, const char *text, uint64_t n, uint64_t *nof_records,
+                       uint32_t *irregular_out) {
+  if (c == nullptr) return -1;
+  CK(cudaSetDevice(c->device));
+  if (c->world > 1) return dist_parse_de(c, text, n, nof_records, irregular_out);
+  if (nof_records == nullptr || irregular_out == nullptr) return fail(c, "gtsb_parse_de_host: null argument");
+  if (parse_preamble(c, "gtsb_parse_de_host", text, n) != 0) return -1;
+  if (await_records(c) != 0) return -1;
+  ProfScope prof(c);
+  *nof_records = 0;
+  *irregular_out = 0;
+  c->have_records = false;
+  c->have_graph = false;
+  if (c->names_dup) {
+    *irregular_out = IRR_DUP_NAME;
+    return 0;
+  }
+  uint64_t nlines = 0;
+  uint32_t total = 0, irregular = 0;
+  if (de_count(c, text, n, &nlines, &total, &irregular) != 0) return -1;
+  if (irregular) {                     // nothing is kept: the caller parses this file on the host
+    *irregular_out = irregular;
+    return 0;
+  }
+  if (de_emit(c, nlines, total) != 0) return -1;
+  keep_parsed_records(c, total);
+  *nof_records = total;
+  return 0;
+}
+
+int gtsb_parse_astat_host(gtsb_context *c, const char *text, uint64_t n, float *astat, float *copy_num,
+                          uint32_t *irregular_out) {
+  if (c == nullptr) return -1;
+  CK(cudaSetDevice(c->device));
+  if (c->world > 1) return dist_parse_astat(c, text, n, astat, copy_num, irregular_out);
+  if (irregular_out == nullptr) return fail(c, "gtsb_parse_astat_host: null argument");
+  if (parse_preamble(c, "gtsb_parse_astat_host", text, n) != 0) return -1;
+  const uint64_t V = c->names_V;
+  if (V && (astat == nullptr || copy_num == nullptr)) return fail(c, "gtsb_parse_astat_host: null argument");
+  ProfScope prof(c);
+  cudaStream_t s = c->stream;
+  *irregular_out = 0;
+  if (c->names_dup) {
+    *irregular_out = IRR_DUP_NAME;
+    return 0;
+  }
+  uint64_t nlines = 0;
+  uint32_t irregular = 0;
+  if (astat_last(c, text, n, astat, copy_num, &nlines, &irregular) != 0) return -1;
   if (irregular) {                     // nothing is touched: the caller reads this file on the host
     *irregular_out = irregular;
     return 0;
   }
-  if (nlines) {
-    GTSB_TIMED("kp_astat(apply)", s);
-    kp_astat<true><<<blocks_for(nlines, 128), 128, 0, s>>>(c->p_text.as<char>(), c->p_line_end.as<uint64_t>(),
-                                                          nlines, t, c->p_last.as<uint64_t>(),
-                                                          c->p_astat.as<float>(), c->p_copy_num.as<float>(), flags);
-    c->stats.kernel_launches++;
-  }
+  if (astat_apply(c, nlines) != 0) return -1;
   if (V) {
     CK(cudaMemcpyAsync(astat, c->p_astat.p, V * 4, cudaMemcpyDeviceToHost, s));
     CK(cudaMemcpyAsync(copy_num, c->p_copy_num.p, V * 4, cudaMemcpyDeviceToHost, s));

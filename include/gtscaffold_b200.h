@@ -134,7 +134,17 @@ int gtsb_set_states_host(gtsb_context *ctx, const uint8_t *vstate, const uint8_t
    (gtsb_build follows) and keeps their pair counts for gtsb_get_records.  It accepts
    the canonical spelling of records only (csrc/gtsb_parse_core.h); for any other text
    it returns 0 with *irregular != 0 (GTSB_IRR_* bits) and NO records set -- the caller
-   then tokenises on the host with the C library's sscanf, as the reference does. */
+   then tokenises on the host with the C library's sscanf, as the reference does.
+   Partitioned context (after gtsb_dist_init): a COLLECTIVE call, every rank passes its own chunk of
+   the file.  Chunks are consecutive byte ranges held by the ranks in file order; every chunk but the
+   last rank's ends right after a '\n' (else the call fails on every rank); chunks may be empty; the
+   4 GiB limit is per chunk.  Every rank must have set the same names (gtsb_set_vertex_names_host):
+   the call compares the contig count and the header bytes and fails on every rank if they differ.
+   Each rank keeps the records of its chunk, as gtsb_set_records_* would leave that rank's records
+   (gtsb_pipeline follows, with the partitioned build's restrictions -- a root whose lines land on two
+   ranks is refused there); *nof_records and gtsb_get_records are this rank's.  *irregular is the OR
+   over the ranks, the same on every rank: a refusal anywhere sets records nowhere.  Errors, also
+   allocation failures, come back from every rank. */
 #define GTSB_IRR_NUL      1u   /* NUL byte in the text */
 #define GTSB_IRR_TOKEN    2u   /* "header,..." token that is not a canonical record */
 #define GTSB_IRR_RANGE    4u   /* distance outside int32 / pair count outside uint32 */
@@ -150,7 +160,12 @@ int gtsb_parse_de_host(gtsb_context *ctx, const char *text, uint64_t text_bytes,
    contigs the text names are overwritten (last line wins, as the sequential loop has it),
    the others keep their value.  Canonical lines only (single tabs, plain decimals);
    *irregular != 0: nothing was touched, read the file on the host -- that includes every
-   text the reference would reject with "Invalid record". */
+   text the reference would reject with "Invalid record".
+   Partitioned context: a COLLECTIVE call with the chunk rules, name check and error handling of
+   gtsb_parse_de_host.  astat / copy_num hold all V values on every rank, in and out, and come back
+   identical on every rank: the last line in FILE order wins (a line on a later rank beats every line
+   on an earlier one), contigs no chunk names keep the caller's value.  *irregular is the OR over the
+   ranks; if it is not 0, no rank's arrays were touched. */
 int gtsb_parse_astat_host(gtsb_context *ctx, const char *text, uint64_t text_bytes, float *astat,
                           float *copy_num, uint32_t *irregular);
 /* the records held by the context, file order (NULL pointers are skipped); num_pairs
