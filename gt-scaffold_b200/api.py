@@ -38,6 +38,8 @@ EXPORTS = [
     "gtsb_set_states_host", "gtsb_get_edge_states",
     "gtsb_set_vertex_names_host", "gtsb_parse_de_host", "gtsb_get_records", "gtsb_parse_astat_host",
     "gtsb_dot_vertex_lines_host", "gtsb_dot_edge_lines_host", "gtsb_scaf_lines_host", "gtsb_result_digest", "gtsb_components", "gtsb_set_vertices_slice_host", "gtsb_mle_host",
+    "gtsb_de_stream_begin", "gtsb_astat_stream_begin", "gtsb_stream_feed", "gtsb_de_stream_end",
+    "gtsb_astat_stream_end", "gtsb_stream_set_slot",
 ]
 
 
@@ -107,6 +109,12 @@ def load_library():
     L.gtsb_parse_de_host.argtypes = [vp, C.c_char_p, u64, C.POINTER(u64), C.POINTER(C.c_uint32)]
     L.gtsb_get_records.argtypes = [vp] * 7
     L.gtsb_parse_astat_host.argtypes = [vp, C.c_char_p, u64, vp, vp, C.POINTER(C.c_uint32)]
+    L.gtsb_de_stream_begin.argtypes = [vp]
+    L.gtsb_astat_stream_begin.argtypes = [vp, vp, vp]
+    L.gtsb_stream_feed.argtypes = [vp, vp, u64, C.POINTER(C.c_uint32)]
+    L.gtsb_de_stream_end.argtypes = [vp, C.POINTER(u64), C.POINTER(C.c_uint32)]
+    L.gtsb_astat_stream_end.argtypes = [vp, vp, vp, C.POINTER(C.c_uint32)]
+    L.gtsb_stream_set_slot.argtypes = [vp, u64]
     L.gtsb_dot_vertex_lines_host.argtypes = [vp, i32, u64, u64, vp, C.c_char_p, u64, C.POINTER(u64)]
     L.gtsb_dot_edge_lines_host.argtypes = [vp, i32, u64, vp, vp, vp, vp, vp, C.c_char_p, u64, C.POINTER(u64)]
     L.gtsb_scaf_lines_host.argtypes = [vp, u64, vp, vp, vp, vp, vp, vp, C.c_char_p, u64, C.POINTER(u64)]
@@ -298,6 +306,46 @@ class ScaffoldGraphB200:
         self._ck(self.L.gtsb_parse_astat_host(self.h, text, C.c_uint64(len(text)), _ptr(a), _ptr(cn),
                                               C.byref(irr)))
         return int(irr.value), a, cn
+
+    def _feed(self, pieces):
+        """pieces -> gtsb_stream_feed until the stream is refused; -> the IRR_* bits so far"""
+        irr = C.c_uint32(0)
+        for piece in pieces:
+            b = np.frombuffer(piece, np.uint8)
+            self._ck(self.L.gtsb_stream_feed(self.h, _ptr(b) if len(b) else None, C.c_uint64(len(b)), C.byref(irr)))
+            if irr.value:
+                break
+        return irr
+
+    def parse_de_pieces(self, pieces):
+        """parse_de for a text given as consecutive pieces, cut anywhere (any iterable of bytes-like
+        objects; empty pieces are fine) -> (irregular bits, nof_records), the records those of the
+        whole text.  No size limit, and a file need not be in memory at once:
+
+            with open(path, "rb") as f:
+                irr, R = g.parse_de_pieces(iter(lambda: f.read(1 << 26), b""))
+
+        Single-device contexts only."""
+        self._ck(self.L.gtsb_de_stream_begin(self.h))
+        irr = self._feed(pieces)
+        R = C.c_uint64(0)
+        self._ck(self.L.gtsb_de_stream_end(self.h, C.byref(R), C.byref(irr)))
+        self.R = int(R.value)
+        return int(irr.value), int(R.value)
+
+    def parse_astat_pieces(self, pieces, astat, copy_num):
+        """parse_astat for a text given as consecutive pieces (see parse_de_pieces) -> (irregular
+        bits, astat, copy_num); irregular != 0: the copies are the inputs, untouched."""
+        a = np.array(astat, np.float32)
+        cn = np.array(copy_num, np.float32)
+        self._ck(self.L.gtsb_astat_stream_begin(self.h, _ptr(a), _ptr(cn)))
+        irr = self._feed(pieces)
+        self._ck(self.L.gtsb_astat_stream_end(self.h, _ptr(a), _ptr(cn), C.byref(irr)))
+        return int(irr.value), a, cn
+
+    def set_stream_slot(self, nbytes: int):
+        """Bytes of one staging slot of the *_pieces calls (default 64 MiB)."""
+        self._ck(self.L.gtsb_stream_set_slot(self.h, C.c_uint64(nbytes)))
 
     # ---- .dot text (graph.c:269-343)
     def dot_vertex_lines(self, vstate, first: int = 0, scaffold_only: bool = False, names_bytes: int = 0):

@@ -823,7 +823,8 @@ void gtsb_destroy(gtsb_context *c) {
   cudaStreamSynchronize(c->stream);
   if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
   dist_release(c);
-  DevBuf *bufs[] = {&c->vattr, &c->astat, &c->seq_len_in, &c->copy_num_in, &c->root, &c->ctg, &c->dist,
+  text_stream_release(c);
+  DevBuf *bufs[] ={&c->vattr, &c->astat, &c->seq_len_in, &c->copy_num_in, &c->root, &c->ctg, &c->dist,
                     &c->std_dev, &c->flags, &c->row_ptr, &c->dst, &c->edist, &c->estd, &c->eflags,
                     &c->eid, &c->win_rec, &c->estate, &c->vstate, &c->rep_pred, &c->cnt, &c->bptr,
                     &c->cursor, &c->deg, &c->krank, &c->scan_scratch, &c->entries, &c->bwin,

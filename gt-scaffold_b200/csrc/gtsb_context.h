@@ -35,6 +35,32 @@ struct Timer {
   cudaEvent_t a = nullptr, b = nullptr;
 };
 
+// `.de` / `.astat` text fed in pieces (gtsb_parse.cu, gtsb_*_stream_*).  Everything a stream keeps
+// between two feeds lives here, so that other calls on the context (which share p_flags and the
+// single call's line index) cannot disturb it.  The buffers stay allocated for the next stream.
+struct TextStream {
+  enum Kind { CLOSED = 0, DE = 1, ASTAT = 2 };
+  int kind = CLOSED;
+  uint64_t slot = 64ull << 20;      // bytes of one step (carry included)
+  char *host = nullptr;            // pinned: the step being filled, then 4 words the device reports into
+  uint64_t host_cap = 0;
+  uint64_t fill = 0;               // bytes in host[]
+  uint64_t file_off = 0;           // file offset of host[0]
+  uint32_t irregular = 0;          // IRR_* bits found so far; != 0: refused, no more device work
+  DevBuf text;                     // two device slots of `slot` bytes, steps alternate
+  int next = 0;                    // device slot of the next step
+  DevBuf line_end, line_off, flags;   // the line index of one step; flags[0] = IRR_* bits
+  // .de: the step whose records are counted but not yet written (emitted after the next sync)
+  bool pending = false;
+  int pending_slot = 0;
+  uint64_t pending_lines = 0;
+  uint64_t R = 0;                  // records written so far
+  DevBuf root, ctg, dist, std_dev, rflags, num_pairs;   // grow geometrically, earlier records kept
+  // .astat: 64-bit file offset + 1 of the winning piece per vertex, the values applied so far
+  DevBuf last, astat, copy_num;
+  cudaEvent_t ev_copied = nullptr, ev_free[2] = {nullptr, nullptr};
+};
+
 struct gtsb_context {
   int device = 0;
   int sm_count = 148;
@@ -81,6 +107,7 @@ struct gtsb_context {
   DevBuf m_pairs, m_size, m_count, m_pmf, m_logp, m_L, m_c, m_n, m_g, m_slot_pair, m_gmax, m_mag, m_cand;   // distance MLE (gtsb_mle.cu)
   uint64_t names_V = 0, names_mask = 0, names_bytes = 0;
   bool have_names = false, names_dup = false, have_num_pairs = false;
+  TextStream ts;
 
   uint32_t *h_counters = nullptr;   // pinned
   gtsb_stats stats{};
@@ -153,6 +180,8 @@ void keep_parsed_records(gtsb_context *c, uint64_t R);
 int astat_last(gtsb_context *c, const char *text, uint64_t n, const float *astat, const float *copy_num,
                uint64_t *nlines, uint32_t *irregular);
 int astat_apply(gtsb_context *c, uint64_t nlines);
+void text_stream_release(gtsb_context *c);      // gtsb_destroy
+void release(DevBuf &b);
 
 }  // namespace gtsbi
 

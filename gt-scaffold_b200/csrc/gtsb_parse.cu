@@ -16,6 +16,9 @@
 // On a partitioned context every rank runs these passes on its chunk of the file; the agreement
 // between the ranks and the `.astat` winners across them are gtsb_dist.cu's (dist_parse_*).
 //
+// Text fed in pieces (gtsb_*_stream_*, end of this file) runs the same passes step by step on a
+// fixed number of staging slots; `.astat` steps use kp_astat_at, whose offsets are file offsets.
+//
 // The walk is a byte loop per thread over its own line; neighbouring threads hold neighbouring
 // lines, so a warp's loads fall into one window of a few KB that L1 keeps.
 #include "gtsb_context.h"
@@ -72,6 +75,16 @@ __global__ void __launch_bounds__(128) kp_astat(const char *__restrict__ text, c
   walk_astat_line<APPLY>(text, l ? line_end[l - 1] : 0, line_end[l], t, last, astat, copy_num, irregular);
 }
 
+// kp_astat on one step of a stream: the step starts at file offset `base`
+template <bool APPLY>
+__global__ void __launch_bounds__(128) kp_astat_at(const char *__restrict__ text, const uint64_t *__restrict__ line_end,
+                                                   uint64_t nlines, uint64_t base, NameTable t, uint64_t *last,
+                                                   float *astat, float *copy_num, uint32_t *irregular) {
+  const uint64_t l = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x;
+  if (l >= nlines) return;
+  walk_astat_line_at<APPLY>(text, l ? line_end[l - 1] : 0, line_end[l], base, t, last, astat, copy_num, irregular);
+}
+
 inline uint32_t blocks_for(uint64_t n, uint32_t threads) { return (uint32_t) ((n + threads - 1) / threads); }
 
 }  // namespace gtsbparse
@@ -83,6 +96,8 @@ extern "C" {
 int gtsb_set_vertex_names_host(gtsb_context *c, uint64_t V, const char *names, const uint64_t *name_off) {
   if (c == nullptr) return -1;
   CK(cudaSetDevice(c->device));
+  if (c->ts.kind != TextStream::CLOSED)
+    return fail(c, "gtsb_set_vertex_names_host: a text stream is open (end it first)");
   c->names_V = 0;
   if (V > GTSB_MAX_VERTICES) return fail(c, "gtsb_set_vertex_names_host: too many contigs");
   if (V && (names == nullptr || name_off == nullptr)) return fail(c, "gtsb_set_vertex_names_host: null input");
@@ -387,6 +402,381 @@ int gtsb_get_records(gtsb_context *c, uint32_t *root, uint32_t *ctg, int32_t *di
     if (num_pairs) CK(cudaMemcpyAsync(num_pairs, c->num_pairs.p, R * 4, cudaMemcpyDeviceToHost, s));
   }
   CK(cudaStreamSynchronize(s));
+  return 0;
+}
+
+}  // extern "C"
+
+// ================================================================ text fed in pieces
+//
+// A step is a prefix of the bytes fed so far that ends where an fgets piece ends: after the last
+// '\n' of a full slot or, inside a physical line that runs past it, at line start + k * 1023.
+// walk_line and walk_astat_line cut a line into 1023-byte pieces from wherever they start, so a step
+// that starts at such a point holds exactly the pieces of the whole file; the bytes after the cut
+// (fewer than 1023) begin the next step.  The last step ends the file and may end without a '\n',
+// as index_lines allows.
+//
+// One step, on the context's stream:
+//   A  the copy (pinned slot -> device slot, on the copy stream), kp_chunk_newlines, scan
+//   -- the one host synchronisation: IRR_* bits so far, the step's '\n' count, and the record count
+//      of the step before --
+//   C  .de: kp_walk(emit) of the step before, into the record columns at the running offset
+//   B  kp_line_ends; .de: kp_walk(count) + scan (emitted by the next step's C);
+//      .astat: kp_astat_at(last line) + kp_astat_at(apply), so later steps overwrite earlier winners
+// The host fills the pinned slot again while C and B run, and the next copy runs beside them; two
+// device slots alternate, a copy waits for the kernels that read its slot.
+namespace gtsbparse {
+
+constexpr uint64_t STREAM_MIN_SLOT = 4096, STREAM_MAX_SLOT = 1ull << 30;
+constexpr uint64_t STREAM_MAX_RECORDS = 0x7FFFFFF7ull;      // 2 R < 0xFFFFFFF0, gtsb_build's limit
+
+static uint64_t slot_stride(uint64_t slot) { return (slot + 8 + 255) & ~255ull; }
+static uint64_t host_tail(uint64_t slot) { return (slot + 15) & ~15ull; }   // 32 B the device reports into
+
+// the bytes of b[0, n) that make a step
+static uint64_t step_cut(const char *b, uint64_t n) {
+  uint64_t ls = n;                                     // start of the last physical line
+  while (ls > 0 && b[ls - 1] != '\n') ls--;
+  return ls + (n - ls) / PIECE * PIECE;
+}
+
+static void stream_close(gtsb_context *c) {
+  TextStream &ts = c->ts;
+  ts.kind = TextStream::CLOSED;
+  ts.fill = ts.file_off = ts.R = 0;
+  ts.irregular = 0;
+  ts.pending = false;
+}
+
+// b holds `used` bytes: room for `need` (doubling), the bytes kept
+static int grow_keep(gtsb_context *c, DevBuf &b, uint64_t used, uint64_t need) {
+  if (b.p != nullptr && b.cap >= need) return 0;
+  uint64_t cap = b.cap ? b.cap : 1ull << 16;
+  while (cap < need) cap *= 2;
+  void *p = nullptr;
+  CK(cudaMalloc(&p, cap));
+  if (used) CK(cudaMemcpyAsync(p, b.p, used, cudaMemcpyDeviceToDevice, c->stream));
+  if (b.p != nullptr) {
+    CK(cudaStreamSynchronize(c->stream));
+    CK(cudaFree(b.p));
+  }
+  b.p = p;
+  b.cap = cap;
+  b.owned = true;
+  return 0;
+}
+
+// one step: the first n bytes of the pinned slot.  n == 0: only the synchronisation and the
+// pending emit (end of the stream).
+static int stream_step(gtsb_context *c, uint64_t n) {
+  TextStream &ts = c->ts;
+  cudaStream_t s = c->stream;
+  uint32_t *h = (uint32_t *) (ts.host + host_tail(ts.slot));     // h[0] bits, h[1] '\n', h[2] records
+  uint64_t *h_end = (uint64_t *) (h + 4);                         // end of an open last line
+  uint32_t *flags = ts.flags.as<uint32_t>();
+  const NameTable t{c->p_names.as<char>(), c->p_name_off.as<uint64_t>(), c->p_slots.as<uint64_t>(),
+                    c->names_mask};
+  const int slot = ts.next;
+  const char *d_text = ts.text.as<char>() + slot * slot_stride(ts.slot);
+  const uint64_t nchunks = (n + CHUNK - 1) / CHUNK;
+  h[1] = 0;
+  if (n) {                                                        // A
+    ts.next ^= 1;
+    CK(cudaStreamWaitEvent(c->copy_stream, ts.ev_free[slot], 0));
+    {
+      GTSB_TIMED("stream h2d", c->copy_stream);
+      CK(cudaMemcpyAsync((void *) d_text, ts.host, n, cudaMemcpyHostToDevice, c->copy_stream));
+    }
+    CK(cudaEventRecord(ts.ev_copied, c->copy_stream));
+    CK(cudaStreamWaitEvent(s, ts.ev_copied, 0));
+    ENSURE(c->p_chunk_cnt, nchunks + 1);
+    ENSURE(c->p_chunk_off, (nchunks + 2) * 4);
+    ENSURE(c->scan_scratch, scan_scratch_elems(nchunks) * 4);
+    {
+      GTSB_TIMED("kp_chunk_newlines", s);
+      kp_chunk_newlines<<<blocks_for(nchunks, 256), 256, 0, s>>>(d_text, n, nchunks, c->p_chunk_cnt.as<uint8_t>(),
+                                                                flags);
+    }
+    exclusive_scan<uint8_t>(c->p_chunk_cnt.as<uint8_t>(), nchunks, c->p_chunk_off.as<uint32_t>(),
+                            c->scan_scratch.as<uint32_t>(), s);
+    c->stats.kernel_launches += 4;
+    CK(cudaMemcpyAsync(h + 1, c->p_chunk_off.as<uint32_t>() + nchunks, 4, cudaMemcpyDeviceToHost, s));
+  }
+  CK(cudaMemcpyAsync(h, flags, 4, cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));           // the copy above has run: the pinned slot may be refilled
+  CK(cudaGetLastError());
+  ts.irregular |= h[0];
+  if (ts.irregular) return 0;             // refused: no more device work
+  if (ts.pending) {                                               // C
+    const uint64_t total = h[2], R = ts.R;
+    if (R + total > STREAM_MAX_RECORDS)
+      return fail(c, "gtsb_stream_feed: more than %llu records, the most gtsb_build takes",
+                  (unsigned long long) STREAM_MAX_RECORDS);
+    DevBuf *col[] = {&ts.root, &ts.ctg, &ts.dist, &ts.std_dev, &ts.num_pairs, &ts.rflags};
+    for (int k = 0; k < 6; k++) {
+      const uint64_t w = k < 5 ? 4 : 1;
+      if (grow_keep(c, *col[k], R * w, (R + total) * w) != 0) return -1;
+    }
+    if (total) {
+      const Records out{ts.root.as<uint32_t>() + R, ts.ctg.as<uint32_t>() + R, ts.dist.as<int32_t>() + R,
+                        ts.std_dev.as<float>() + R, ts.num_pairs.as<uint32_t>() + R, ts.rflags.as<uint8_t>() + R};
+      GTSB_TIMED("kp_walk(emit)", s);
+      kp_walk<true><<<blocks_for(ts.pending_lines, 128), 128, 0, s>>>(
+          ts.text.as<char>() + ts.pending_slot * slot_stride(ts.slot), ts.line_end.as<uint64_t>(), ts.pending_lines,
+          t, out, nullptr, ts.line_off.as<uint32_t>(), flags);
+      c->stats.kernel_launches++;
+    }
+    ts.R = R + total;
+    CK(cudaEventRecord(ts.ev_free[ts.pending_slot], s));
+    ts.pending = false;
+  }
+  if (n == 0) return 0;
+  const uint64_t newlines = h[1];                                 // B
+  const bool open_end = ts.host[n - 1] != '\n';
+  const uint64_t nlines = newlines + (open_end ? 1 : 0);
+  ENSURE(ts.line_end, (nlines + 1) * 8);
+  uint64_t *line_end = ts.line_end.as<uint64_t>();
+  if (newlines) {
+    GTSB_TIMED("kp_line_ends", s);
+    kp_line_ends<<<blocks_for(nchunks, 256), 256, 0, s>>>(d_text, n, nchunks, c->p_chunk_cnt.as<uint8_t>(),
+                                                          c->p_chunk_off.as<uint32_t>(), line_end);
+    c->stats.kernel_launches++;
+  }
+  if (open_end) {
+    *h_end = n;
+    CK(cudaMemcpyAsync(line_end + newlines, h_end, 8, cudaMemcpyHostToDevice, s));
+  }
+  if (ts.kind == TextStream::DE) {
+    ENSURE(c->p_line_cnt, (nlines + 1) * 4);
+    ENSURE(ts.line_off, (nlines + 2) * 4);
+    ENSURE(c->scan_scratch, scan_scratch_elems(nlines) * 4);
+    const Records none{};
+    {
+      GTSB_TIMED("kp_walk(count)", s);
+      kp_walk<false><<<blocks_for(nlines, 128), 128, 0, s>>>(d_text, line_end, nlines, t, none,
+                                                            c->p_line_cnt.as<uint32_t>(), nullptr, flags);
+    }
+    exclusive_scan<uint32_t>(c->p_line_cnt.as<uint32_t>(), nlines, ts.line_off.as<uint32_t>(),
+                             c->scan_scratch.as<uint32_t>(), s);
+    c->stats.kernel_launches += 4;
+    CK(cudaMemcpyAsync(h + 2, ts.line_off.as<uint32_t>() + nlines, 4, cudaMemcpyDeviceToHost, s));
+    ts.pending = true;
+    ts.pending_slot = slot;
+    ts.pending_lines = nlines;
+  } else {
+    {
+      GTSB_TIMED("kp_astat_at(last line)", s);
+      kp_astat_at<false><<<blocks_for(nlines, 128), 128, 0, s>>>(d_text, line_end, nlines, ts.file_off, t,
+                                                                ts.last.as<uint64_t>(), ts.astat.as<float>(),
+                                                                ts.copy_num.as<float>(), flags);
+    }
+    {
+      GTSB_TIMED("kp_astat_at(apply)", s);
+      kp_astat_at<true><<<blocks_for(nlines, 128), 128, 0, s>>>(d_text, line_end, nlines, ts.file_off, t,
+                                                               ts.last.as<uint64_t>(), ts.astat.as<float>(),
+                                                               ts.copy_num.as<float>(), flags);
+    }
+    c->stats.kernel_launches += 2;
+    CK(cudaEventRecord(ts.ev_free[slot], s));
+  }
+  return 0;
+}
+
+// what both begins share: a discarded open stream, the checks, the staging memory
+static int stream_prepare(gtsb_context *c, const char *what) {
+  TextStream &ts = c->ts;
+  stream_close(c);                                  // a new begin discards an open stream
+  if (c->world > 1)
+    return fail(c, "%s: a partitioned context reads text with the collective gtsb_parse_*_host calls", what);
+  if (!c->have_names) return fail(c, "%s: vertex names not set", what);
+  const uint64_t host_bytes = host_tail(ts.slot) + 32;
+  if (ts.host != nullptr && ts.host_cap != host_bytes) {
+    CK(cudaFreeHost(ts.host));
+    ts.host = nullptr;
+  }
+  if (ts.host == nullptr) {
+    CK(cudaMallocHost(&ts.host, host_bytes));
+    ts.host_cap = host_bytes;
+  }
+  ENSURE(ts.text, 2 * slot_stride(ts.slot));
+  ENSURE(ts.flags, 16);
+  for (cudaEvent_t *e : {&ts.ev_copied, &ts.ev_free[0], &ts.ev_free[1]})
+    if (*e == nullptr) CK(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+  CK(cudaMemsetAsync(ts.flags.p, 0, 16, c->stream));
+  ts.next = 0;
+  return 0;
+}
+
+// the remaining bytes as the last step, then the synchronisation that reads its results
+static int stream_finish(gtsb_context *c) {
+  TextStream &ts = c->ts;
+  if (ts.irregular == 0 && stream_step(c, ts.fill) != 0) return -1;
+  if (ts.irregular == 0 && stream_step(c, 0) != 0) return -1;
+  return 0;
+}
+
+static int stream_end_check(gtsb_context *c, const char *what, int kind) {
+  const int open = c->ts.kind;
+  if (open == kind) return 0;
+  stream_close(c);
+  if (open == TextStream::CLOSED) return fail(c, "%s: no open stream", what);
+  return fail(c, "%s: the open stream reads %s text", what, open == TextStream::DE ? ".de" : ".astat");
+}
+
+}  // namespace gtsbparse
+
+namespace gtsbi {
+
+void text_stream_release(gtsb_context *c) {
+  TextStream &ts = c->ts;
+  if (ts.host != nullptr) cudaFreeHost(ts.host);
+  ts.host = nullptr;
+  for (DevBuf *b : {&ts.text, &ts.line_end, &ts.line_off, &ts.flags, &ts.root, &ts.ctg, &ts.dist, &ts.std_dev,
+                    &ts.rflags, &ts.num_pairs, &ts.last, &ts.astat, &ts.copy_num})
+    release(*b);
+  for (cudaEvent_t e : {ts.ev_copied, ts.ev_free[0], ts.ev_free[1]})
+    if (e != nullptr) cudaEventDestroy(e);
+}
+
+}  // namespace gtsbi
+
+extern "C" {
+
+int gtsb_stream_set_slot(gtsb_context *c, uint64_t bytes) {
+  if (c == nullptr) return -1;
+  if (c->ts.kind != TextStream::CLOSED) return fail(c, "gtsb_stream_set_slot: a text stream is open");
+  if (bytes < STREAM_MIN_SLOT || bytes > STREAM_MAX_SLOT)
+    return fail(c, "gtsb_stream_set_slot: %llu bytes is outside [%llu, %llu]", (unsigned long long) bytes,
+                (unsigned long long) STREAM_MIN_SLOT, (unsigned long long) STREAM_MAX_SLOT);
+  c->ts.slot = bytes;
+  return 0;
+}
+
+int gtsb_de_stream_begin(gtsb_context *c) {
+  if (c == nullptr) return -1;
+  CK(cudaSetDevice(c->device));
+  if (stream_prepare(c, "gtsb_de_stream_begin") != 0) return -1;
+  if (await_records(c) != 0) return -1;
+  c->have_records = false;                          // as gtsb_parse_de_host: the old records are gone
+  c->have_graph = false;
+  c->ts.kind = TextStream::DE;
+  c->ts.irregular = c->names_dup ? IRR_DUP_NAME : 0;
+  return 0;
+}
+
+int gtsb_astat_stream_begin(gtsb_context *c, const float *astat, const float *copy_num) {
+  if (c == nullptr) return -1;
+  CK(cudaSetDevice(c->device));
+  if (stream_prepare(c, "gtsb_astat_stream_begin") != 0) return -1;
+  TextStream &ts = c->ts;
+  const uint64_t V = c->names_V;
+  if (V && (astat == nullptr || copy_num == nullptr)) return fail(c, "gtsb_astat_stream_begin: null argument");
+  cudaStream_t s = c->stream;
+  ENSURE(ts.last, (V + 1) * 8);
+  ENSURE(ts.astat, (V + 1) * 4);
+  ENSURE(ts.copy_num, (V + 1) * 4);
+  CK(cudaMemsetAsync(ts.last.p, 0, (V + 1) * 8, s));
+  if (V) {
+    CK(cudaMemcpyAsync(ts.astat.p, astat, V * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(ts.copy_num.p, copy_num, V * 4, cudaMemcpyHostToDevice, s));
+  }
+  ts.kind = TextStream::ASTAT;
+  ts.irregular = c->names_dup ? IRR_DUP_NAME : 0;
+  return 0;
+}
+
+int gtsb_stream_feed(gtsb_context *c, const char *bytes, uint64_t n, uint32_t *irregular) {
+  if (c == nullptr) return -1;
+  CK(cudaSetDevice(c->device));
+  TextStream &ts = c->ts;
+  if (ts.kind == TextStream::CLOSED) return fail(c, "gtsb_stream_feed: no open stream");
+  if (irregular == nullptr || (n && bytes == nullptr)) {
+    stream_close(c);
+    return fail(c, "gtsb_stream_feed: null argument");
+  }
+  ProfScope prof(c);
+  while (n && ts.irregular == 0) {
+    const uint64_t take = n < ts.slot - ts.fill ? n : ts.slot - ts.fill;
+    memcpy(ts.host + ts.fill, bytes, take);
+    ts.fill += take;
+    bytes += take;
+    n -= take;
+    if (ts.fill < ts.slot) break;
+    const uint64_t cut = step_cut(ts.host, ts.fill);
+    if (stream_step(c, cut) != 0) {
+      stream_close(c);
+      return -1;
+    }
+    memmove(ts.host, ts.host + cut, ts.fill - cut);
+    ts.file_off += cut;
+    ts.fill -= cut;
+  }
+  *irregular = ts.irregular;
+  return 0;
+}
+
+int gtsb_de_stream_end(gtsb_context *c, uint64_t *nof_records, uint32_t *irregular) {
+  if (c == nullptr) return -1;
+  CK(cudaSetDevice(c->device));
+  if (stream_end_check(c, "gtsb_de_stream_end", TextStream::DE) != 0) return -1;
+  TextStream &ts = c->ts;
+  if (nof_records == nullptr || irregular == nullptr) {
+    stream_close(c);
+    return fail(c, "gtsb_de_stream_end: null argument");
+  }
+  ProfScope prof(c);
+  *nof_records = 0;
+  *irregular = 0;
+  const int rc = stream_finish(c);
+  const uint32_t irr = ts.irregular;
+  const uint64_t R = ts.R;
+  stream_close(c);
+  if (rc != 0) return -1;
+  if (irr) {                                        // nothing is kept: the caller parses this file on the host
+    *irregular = irr;
+    return 0;
+  }
+  // the stream's columns become the context's records
+  DevBuf *mine[] = {&ts.root, &ts.ctg, &ts.dist, &ts.std_dev, &ts.rflags, &ts.num_pairs};
+  DevBuf *ctx[] = {&c->root, &c->ctg, &c->dist, &c->std_dev, &c->flags, &c->num_pairs};
+  for (int k = 0; k < 6; k++) {
+    if (mine[k]->p == nullptr) ENSURE(*mine[k], 16);
+    release(*ctx[k]);
+    *ctx[k] = *mine[k];
+    *mine[k] = DevBuf();
+  }
+  keep_parsed_records(c, R);
+  *nof_records = R;
+  return 0;
+}
+
+int gtsb_astat_stream_end(gtsb_context *c, float *astat, float *copy_num, uint32_t *irregular) {
+  if (c == nullptr) return -1;
+  CK(cudaSetDevice(c->device));
+  if (stream_end_check(c, "gtsb_astat_stream_end", TextStream::ASTAT) != 0) return -1;
+  TextStream &ts = c->ts;
+  const uint64_t V = c->names_V;
+  if (irregular == nullptr || (V && (astat == nullptr || copy_num == nullptr))) {
+    stream_close(c);
+    return fail(c, "gtsb_astat_stream_end: null argument");
+  }
+  ProfScope prof(c);
+  *irregular = 0;
+  const int rc = stream_finish(c);
+  const uint32_t irr = ts.irregular;
+  stream_close(c);
+  if (rc != 0) return -1;
+  if (irr) {                                        // nothing is touched: the caller reads this file on the host
+    *irregular = irr;
+    return 0;
+  }
+  cudaStream_t s = c->stream;
+  if (V) {
+    CK(cudaMemcpyAsync(astat, ts.astat.p, V * 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(copy_num, ts.copy_num.p, V * 4, cudaMemcpyDeviceToHost, s));
+  }
+  CK(cudaStreamSynchronize(s));
+  CK(cudaGetLastError());
   return 0;
 }
 

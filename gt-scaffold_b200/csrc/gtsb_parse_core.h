@@ -405,11 +405,12 @@ GTSB_HD void max64(uint64_t *addr, uint64_t val) {
 #endif
 }
 
-// One physical line [s, e).  APPLY = false: last[v] = max(piece offset + 1) over the pieces
-// naming v; APPLY = true: the piece that holds that maximum writes its values.
+// One physical line [s, e) of a text that starts at file offset `base`.  APPLY = false:
+// last[v] = max(file offset + 1) over the pieces naming v; APPLY = true: the piece that holds
+// that maximum writes its values.
 template <bool APPLY>
-GTSB_HD void walk_astat_line(const char *text, uint64_t s, uint64_t e, const NameTable &tab, uint64_t *last,
-                             float *astat, float *copy_num, uint32_t *irregular) {
+GTSB_HD void walk_astat_line_at(const char *text, uint64_t s, uint64_t e, uint64_t base, const NameTable &tab,
+                                uint64_t *last, float *astat, float *copy_num, uint32_t *irregular) {
   for (uint64_t p = s; p < e;) {
     const uint64_t piece_end = p + PIECE < e ? p + PIECE : e;
     AstatLine a;
@@ -418,14 +419,21 @@ GTSB_HD void walk_astat_line(const char *text, uint64_t s, uint64_t e, const Nam
       flag_or(irregular, bad);
     } else if (a.v != NOT_FOUND) {
       if (!APPLY) {
-        max64(last + a.v, p + 1);
-      } else if (last[a.v] == p + 1) {
+        max64(last + a.v, base + p + 1);
+      } else if (last[a.v] == base + p + 1) {
         astat[a.v] = a.astat;                                 // algorithms.c:140-141
         copy_num[a.v] = a.copy_num;
       }
     }
     p = piece_end;
   }
+}
+
+// the same for a whole text (offsets are file offsets)
+template <bool APPLY>
+GTSB_HD void walk_astat_line(const char *text, uint64_t s, uint64_t e, const NameTable &tab, uint64_t *last,
+                             float *astat, float *copy_num, uint32_t *irregular) {
+  walk_astat_line_at<APPLY>(text, s, e, 0, tab, last, astat, copy_num, irregular);
 }
 
 }  // namespace gtsbp

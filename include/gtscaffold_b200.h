@@ -18,6 +18,7 @@
  *
  *   gtsb_parse_de_host     <- the .de record loop (gt_scaffolder_parser.c:323-388)
  *   gtsb_parse_astat_host  <- the .astat line loop (gt_scaffolder_algorithms.c:118-149)
+ *   gtsb_*_stream_*        <- the same two loops for a file fed in pieces, of any size
  *   gtsb_dot_*_lines_host  <- gt_scaffolder_graph_print_generic / _print_scaffold
  *                             (gt_scaffolder_graph.c:269-343)
  *
@@ -168,8 +169,45 @@ int gtsb_parse_de_host(gtsb_context *ctx, const char *text, uint64_t text_bytes,
    ranks; if it is not 0, no rank's arrays were touched. */
 int gtsb_parse_astat_host(gtsb_context *ctx, const char *text, uint64_t text_bytes, float *astat,
                           float *copy_num, uint32_t *irregular);
+/* ---- the same two readings for text fed in pieces: no size limit, bounded memory, and the copy of
+   each piece overlapping the kernels of the piece before.  Single-device contexts only: begin on a
+   partitioned context (after gtsb_dist_init) fails, ranks keep using the collective calls above.
+
+     gtsb_de_stream_begin / gtsb_astat_stream_begin   open a stream (an open one is discarded)
+     gtsb_stream_feed     the next bytes of the file
+     gtsb_de_stream_end / gtsb_astat_stream_end       the result
+
+   Pieces are consecutive bytes of the file and may be cut anywhere -- inside a token, a line or a
+   1023-byte fgets piece; pieces may be empty.  feed returns once the bytes are copied: the caller
+   may reuse its buffer.  *irregular is the set of GTSB_IRR_* bits found so far; once it is not 0
+   the stream is refused and feed does no more device work.
+   For any text below 4 GiB cut in any way, .de end leaves exactly the records, pair counts and
+   gtsb_get_records results gtsb_parse_de_host leaves on the whole text, and .astat end returns
+   exactly its arrays; *irregular is not 0 exactly when the single call's is, its bits a subset of
+   the single call's.  Beyond 4 GiB the one limit is the record count gtsb_build takes (2 R <
+   2^32 - 16); a stream that passes it fails with a message.
+   .de begin drops the context's records, as gtsb_parse_de_host does; after a refusal or an error no
+   records are held.  .astat begin takes the initial values (one per vertex of the names set, NULL
+   for none); end writes astat / copy_num only when it succeeds with *irregular == 0.
+   Errors: feed or end without an open stream, end of the other kind, a null argument, a CUDA or
+   allocation error -- each closes the stream.  gtsb_set_vertex_names_host fails while a stream is
+   open.  Other calls on the context may run between feeds; the single-call entry points keep
+   their own buffers.
+   Memory: the stream copies through one pinned host slot and two device slots of 64 MiB
+   (gtsb_stream_set_slot), plus the line index of one slot (16 B per line) and, for .de, the
+   record columns (21 B per record, grown by doubling).  They stay allocated for the next stream
+   until gtsb_destroy. */
+int gtsb_de_stream_begin(gtsb_context *ctx);
+int gtsb_astat_stream_begin(gtsb_context *ctx, const float *astat, const float *copy_num);
+int gtsb_stream_feed(gtsb_context *ctx, const char *bytes, uint64_t n, uint32_t *irregular);
+int gtsb_de_stream_end(gtsb_context *ctx, uint64_t *nof_records, uint32_t *irregular);
+int gtsb_astat_stream_end(gtsb_context *ctx, float *astat, float *copy_num, uint32_t *irregular);
+/* bytes of one staging slot (default 64 MiB, 4096 .. 2^30); not while a stream is open.  A step
+   of the stream is at most one slot; smaller slots mean more steps (and more synchronisations). */
+int gtsb_stream_set_slot(gtsb_context *ctx, uint64_t bytes);
+
 /* the records held by the context, file order (NULL pointers are skipped); num_pairs
-   only after gtsb_parse_de_host */
+   only after gtsb_parse_de_host or gtsb_de_stream_end */
 int gtsb_get_records(gtsb_context *ctx, uint32_t *root, uint32_t *ctg, int32_t *dist,
                      float *std_dev, uint8_t *flags, uint32_t *num_pairs);
 

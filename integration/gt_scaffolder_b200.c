@@ -21,10 +21,14 @@
  * SURVEY.md section 2, rows 2-3).  The `.de` record loop (parser.c:323-388:
  * 1024-byte fgets, last character dropped, ' ' tokens, "%[^>,],%ld,%ld,%f"
  * records, ';' switches the direction) runs on the device for files in the
- * canonical spelling (gtsb_parse_de_host); a file the device refuses -- or
- * every file with GTSB_TOKENISER=host in the environment -- is tokenised by
- * read_de_records below with the C library's sscanf.  The `.astat` tokeniser
- * (algorithms.c:118-149) is host C.  All graph work happens on the GPU; there
+ * canonical spelling; a file the device refuses -- or every file with
+ * GTSB_TOKENISER=host in the environment -- is tokenised by read_de_records
+ * below with the C library's sscanf.  The `.astat` line loop
+ * (algorithms.c:118-149) runs on the device the same way (device_astat), with
+ * the reference's host loop for a file the device refuses.  Both files are
+ * read in blocks of B200_BLOCK bytes and fed to the device as they are read
+ * (gtsb_stream_feed), so neither is ever whole in host memory and there is no
+ * size limit.  All graph work happens on the GPU; there
  * is no CPU fallback -- a missing device or a CUDA error is reported the
  * reference's way (-1 + GtError) or, for the void filter, printed and aborted.
  */
@@ -46,6 +50,7 @@
 #include "gtscaffold_b200.h"
 
 #define B200_LINE 1024            /* the reference's BUFSIZE, parser.c:30 */
+#define B200_BLOCK (64u << 20)    /* bytes of text read and fed to the device at a time */
 
 /* ------------------------------------------------------------------ context */
 
@@ -258,24 +263,29 @@ static int read_de_records(const char *filename, const GtScaffolderGraph *graph,
   return 0;
 }
 
-/* whole file into memory; NULL if it cannot be read that way */
-static char *slurp(const char *filename, uint64_t *bytes)
+/* the file in blocks into an open text stream until it ends or the device refuses it.
+   1: fed to the end (or refused, *irregular != 0); 0: it cannot be read that way, the caller
+   leaves the file to the host loop (which reports the problem); -1: a device error. */
+static int feed_file(gtsb_context *c, const char *filename, uint32_t *irregular)
 {
   FILE *fp = fopen(filename, "rb");
-  char *text = NULL;
-  long size;
+  char *block;
+  size_t n;
+  int rc = 1;
   if (fp == NULL)
-    return NULL;
-  if (fseek(fp, 0, SEEK_END) == 0 && (size = ftell(fp)) >= 0 && fseek(fp, 0, SEEK_SET) == 0) {
-    text = gt_malloc((size_t) size + 1);
-    if (fread(text, 1, (size_t) size, fp) != (size_t) size) {
-      gt_free(text);
-      text = NULL;
+    return 0;
+  block = gt_malloc(B200_BLOCK);
+  while (*irregular == 0 && (n = fread(block, 1, B200_BLOCK, fp)) > 0) {
+    if (gtsb_stream_feed(c, block, n, irregular) != 0) {
+      rc = -1;
+      break;
     }
-    *bytes = (uint64_t) size;
   }
+  if (rc == 1 && ferror(fp))
+    rc = 0;
+  gt_free(block);
   fclose(fp);
-  return text;
+  return rc;
 }
 
 /* the vertices' headers, id order -> the device's gt_scaffolder_graph_get_vertex */
@@ -306,34 +316,31 @@ static int device_vertex_names(gtsb_context *c, const GtScaffolderGraph *graph)
 static int device_de_records(gtsb_context *c, const char *filename, const GtScaffolderGraph *graph,
                              B200Records *recs, bool *on_device, GtError *err)
 {
-  uint64_t nof_records = 0, bytes = 0, r;
+  uint64_t nof_records = 0, r;
   uint32_t irregular = 0, *pairs = NULL;
-  char *text = slurp(filename, &bytes);
-  int had_err = 0;
+  int had_err = 0, fed = 0;
 
   *on_device = false;
-  if (text == NULL)
-    return 0;                                   /* let the host tokeniser report it */
-  if (device_vertex_names(c, graph) != 0 ||
-      gtsb_parse_de_host(c, text, bytes, &nof_records, &irregular) != 0) {
+  if (device_vertex_names(c, graph) != 0 || gtsb_de_stream_begin(c) != 0 ||
+      (fed = feed_file(c, filename, &irregular)) < 0 ||
+      gtsb_de_stream_end(c, &nof_records, &irregular) != 0) {
+    gt_error_set(err, "%s", gtsb_error(c));
+    return -1;
+  }
+  if (fed == 0 || irregular != 0)
+    return 0;                                   /* the host tokeniser reads it (and reports) */
+  pairs = gt_malloc((nof_records + 1) * sizeof (*pairs));
+  if (gtsb_get_records(c, NULL, NULL, NULL, NULL, NULL, pairs) != 0) {
     gt_error_set(err, "%s", gtsb_error(c));
     had_err = -1;
-  }
-  if (had_err == 0 && irregular == 0) {
-    pairs = gt_malloc((nof_records + 1) * sizeof (*pairs));
-    if (gtsb_get_records(c, NULL, NULL, NULL, NULL, NULL, pairs) != 0) {
-      gt_error_set(err, "%s", gtsb_error(c));
-      had_err = -1;
-    } else {
-      recs->num_pairs = gt_malloc((nof_records + 1) * sizeof (*recs->num_pairs));
-      for (r = 0; r < nof_records; r++)
-        recs->num_pairs[r] = pairs[r];
-      recs->n = recs->cap = nof_records;
-      *on_device = true;
-    }
+  } else {
+    recs->num_pairs = gt_malloc((nof_records + 1) * sizeof (*recs->num_pairs));
+    for (r = 0; r < nof_records; r++)
+      recs->num_pairs[r] = pairs[r];
+    recs->n = recs->cap = nof_records;
+    *on_device = true;
   }
   gt_free(pairs);
-  gt_free(text);
   return had_err;
 }
 
@@ -344,27 +351,24 @@ static int device_de_records(gtsb_context *c, const char *filename, const GtScaf
 static int device_astat(gtsb_context *c, const char *filename, GtScaffolderGraph *graph, bool *on_device,
                         GtError *err)
 {
-  uint64_t bytes = 0;
   uint32_t irregular = 0;
-  char *text = slurp(filename, &bytes);
   float *astat, *copy_num;
   GtUword i;
-  int had_err = 0;
+  int had_err = 0, fed = 0;
 
   *on_device = false;
-  if (text == NULL)
-    return 0;
   astat = gt_malloc((graph->nof_vertices + 1) * sizeof (*astat));
   copy_num = gt_malloc((graph->nof_vertices + 1) * sizeof (*copy_num));
   for (i = 0; i < graph->nof_vertices; i++) {
     astat[i] = graph->vertices[i].astat;
     copy_num[i] = graph->vertices[i].copy_num;
   }
-  if (device_vertex_names(c, graph) != 0 ||
-      gtsb_parse_astat_host(c, text, bytes, astat, copy_num, &irregular) != 0) {
+  if (device_vertex_names(c, graph) != 0 || gtsb_astat_stream_begin(c, astat, copy_num) != 0 ||
+      (fed = feed_file(c, filename, &irregular)) < 0 ||
+      gtsb_astat_stream_end(c, astat, copy_num, &irregular) != 0) {
     gt_error_set(err, "%s", gtsb_error(c));
     had_err = -1;
-  } else if (irregular == 0) {
+  } else if (fed == 1 && irregular == 0) {
     for (i = 0; i < graph->nof_vertices; i++) {
       graph->vertices[i].astat = astat[i];
       graph->vertices[i].copy_num = copy_num[i];
@@ -373,7 +377,6 @@ static int device_astat(gtsb_context *c, const char *filename, GtScaffolderGraph
   }
   gt_free(astat);
   gt_free(copy_num);
-  gt_free(text);
   return had_err;
 }
 
