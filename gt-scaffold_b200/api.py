@@ -39,7 +39,7 @@ EXPORTS = [
     "gtsb_set_vertex_names_host", "gtsb_parse_de_host", "gtsb_get_records", "gtsb_parse_astat_host",
     "gtsb_dot_vertex_lines_host", "gtsb_dot_edge_lines_host", "gtsb_scaf_lines_host", "gtsb_result_digest", "gtsb_components", "gtsb_set_vertices_slice_host", "gtsb_mle_host",
     "gtsb_de_stream_begin", "gtsb_astat_stream_begin", "gtsb_stream_feed", "gtsb_de_stream_end",
-    "gtsb_astat_stream_end", "gtsb_stream_set_slot",
+    "gtsb_astat_stream_end", "gtsb_stream_set_slot", "gtsb_dist_any_input",
 ]
 
 
@@ -99,6 +99,7 @@ def load_library():
     L.gtsb_ambig_thresholds.argtypes = [f32, C.POINTER(f32), C.POINTER(f32), C.POINTER(i32)]
     L.gtsb_dist_unique_id.argtypes = [vp]
     L.gtsb_dist_init.argtypes = [vp, i32, i32, vp]
+    L.gtsb_dist_any_input.argtypes = [vp, i32]
     L.gtsb_get_edges.argtypes = [vp, C.POINTER(u64)] + [vp] * 7
     L.gtsb_set_record_lines_host.argtypes = [vp, u64, vp, vp, u64, vp, vp, vp, vp]
     L.gtsb_set_record_lines_device.argtypes = [vp, u64, vp, vp, u64, vp, vp, vp, vp]
@@ -192,6 +193,17 @@ def shard_lines(inp, world: int, rank: int, mail_weight: float = MAIL_WEIGHT):
         cuts.append(max(i, cuts[-1]))
     cuts.append(R)
     lo, hi = cuts[rank], cuts[rank + 1]
+    kw = {k: getattr(inp, k)[lo:hi] for k in ("root", "ctg", "dist", "std_dev", "num_pairs", "flags")}
+    return type(inp)(inp.seq_len, inp.astat, inp.copy_num, name=inp.name,
+                     meta=dict(inp.meta, shard=(rank, world, lo, hi)), **kw)
+
+
+def shard_records(inp, world: int, rank: int):
+    """Rank `rank`'s share of the records cut by count alone: a contiguous slice, ranks in file
+    order, lines split wherever the cut falls.  Only a partitioned graph with dist_any_input on
+    takes such slices.  Vertex attributes are not sharded."""
+    R = np.asarray(inp.root).shape[0]
+    lo, hi = R * rank // world, R * (rank + 1) // world
     kw = {k: getattr(inp, k)[lo:hi] for k in ("root", "ctg", "dist", "std_dev", "num_pairs", "flags")}
     return type(inp)(inp.seq_len, inp.astat, inp.copy_num, name=inp.name,
                      meta=dict(inp.meta, shard=(rank, world, lo, hi)), **kw)
@@ -447,6 +459,13 @@ class ScaffoldGraphB200:
         """Join the ranks that hold one partitioned graph (NCCL over NVLink)."""
         self._ck(self.L.gtsb_dist_init(self.h, rank, world, unique_id))
         self.rank, self.world = rank, world
+
+    def dist_any_input(self, on: bool = True):
+        """Let pipeline() on a partitioned graph take any record input: what the line-ordered
+        partitioned build refuses is rebuilt by the general build spread over the ranks, and every
+        rank may then hold any contiguous slice of the records (shard_records).  Every rank must
+        pass the same value."""
+        self._ck(self.L.gtsb_dist_any_input(self.h, int(on)))
 
     # ---- the hot path
     def build(self):

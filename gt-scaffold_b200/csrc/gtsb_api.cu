@@ -1321,7 +1321,7 @@ int gtsb_get_stats(gtsb_context *c, gtsb_stats *st) {
     if (c->h_counters[CNT_RING_ROUNDS] >= c->V + 2 && c->V) return fail(c, "gtsb_filter: fire rounds did not converge");
   }
   c->stats.nof_vertices = c->V;
-  c->stats.line_ordered_build = c->line_layout ? 1u : 0u;
+  c->stats.line_ordered_build = c->line_layout && !c->id_rows ? 1u : 0u;
   c->stats.fallback_reason = c->fallback_reason;
   *st = c->stats;
   return 0;

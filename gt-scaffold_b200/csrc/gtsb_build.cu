@@ -473,10 +473,14 @@ static inline uint32_t grid_for(uint64_t n, int threads, int max_blocks) {
   return (uint32_t) b;
 }
 
-void launch_build_count(const BuildArgs &a, cudaStream_t s) {
-  { KernelTimer t_("k_count_halfedges", s);
+void launch_count_halfedges(const BuildArgs &a, cudaStream_t s) {
+  KernelTimer t_("k_count_halfedges", s);
   k_count_halfedges<<<grid_for(a.R, 256, a.sm_count * 16), 256, 0, s>>>(a.R, a.V, a.root, a.ctg,
-                                                                         a.cnt, a.counters + CNT_ERROR); }
+                                                                         a.cnt, a.counters + CNT_ERROR);
+}
+
+void launch_build_count(const BuildArgs &a, cudaStream_t s) {
+  launch_count_halfedges(a, s);
   exclusive_scan<uint32_t>(a.cnt, a.V, a.bptr, a.scan_scratch, s);
 }
 
@@ -484,6 +488,10 @@ void launch_build_scatter_resolve(const BuildArgs &a, cudaStream_t s) {
   { KernelTimer t_("k_scatter_halfedges", s);
   k_scatter_halfedges<<<grid_for(a.R, 256, a.sm_count * 16), 256, 0, s>>>(
       a.R, a.V, a.root, a.ctg, a.dist, a.std_dev, a.flags, a.bptr, a.cursor, a.entries); }
+  launch_build_resolve(a, s);
+}
+
+void launch_build_resolve(const BuildArgs &a, cudaStream_t s) {
   // A graph with hubs (a.hubs: the line-ordered build met a line longer than it takes): a thread
   // takes buckets of up to 16 entries, a warp those of 17 .. 128 (k_resolve_mid), a block the rest --
   // a warp of the thread path lasts as long as its largest bucket's quadratic sort.  Otherwise a

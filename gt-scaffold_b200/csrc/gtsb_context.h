@@ -133,6 +133,8 @@ struct gtsb_context {
   void *dstate = nullptr;            // DistState of gtsb_dist.cu
   uint32_t row_base = 0;            // global position of local row 0
   uint64_t Vloc = 0;                // rows held by this rank (== V when world == 1)
+  int dist_any_input = 0;           // gtsb_dist_any_input: input the line-ordered build refuses takes the general build
+  bool id_rows = false;             // the rows came from the partitioned general build: positions are vertex ids
 
   // cached ambiguous-order thresholds
   bool ambig_valid = false;

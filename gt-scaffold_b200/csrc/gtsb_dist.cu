@@ -23,6 +23,16 @@
 //   .astat  key of the winning line (rank, offset)  allreduce(max), 8 B/vertex
 //           the winners' values (u32 bit patterns)  allreduce(sum), 8 B/vertex
 //
+// With gtsb_dist_any_input on, input the line-ordered build refuses (its FB_* reason mask is
+// agreed at the exchange where it shows) is rebuilt by the general build of gtsb_build.cu spread
+// over the ranks (dist_general): rank r owns the buckets of a range of vertex ids, balanced by
+// half-edges, and positions are the ids themselves.  What crosses NVLink there:
+//
+//   general half-edges per vertex                   allreduce(sum), 4 B/vertex
+//           half-edges (DIRECT to the root's owner, remote stores into the owner's receive
+//             TWIN to the ctg's owner)                buffers (CUDA IPC), 16 + 4 B/half-edge
+//           creating records                         allreduce(sum) of disjoint bits, R_total / 8 B
+//
 // Both directed edges of a link are evaluated by their own rows' owners from
 // the same vertex-level facts, so the symmetric edge marks agree without any
 // edge exchange.  NCCL is loaded with dlopen when gtsb_dist_init is called;
@@ -91,6 +101,7 @@ struct DistState {
   cudaStream_t side = nullptr;
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   DevBuf small, bounds, rank_cnt, rx_ent, rx_dest, corr_all, prop_all, stage, stage2, peer_tab, handles, mail_hist;
+  DevBuf deg_prefix, creators;     // general build: prefix of the global half-edge counts; creator bits, popcounts, prefix
   uint32_t *h_small = nullptr;     // pinned, world * SMALL_N words
   // every rank's receive buffers, opened through CUDA IPC (peer memory over NVLink)
   void *peer_ptr[MAX_RANKS][2] = {};
@@ -372,6 +383,216 @@ __global__ void k_dist_astat_unpack(uint64_t V, const uint64_t *__restrict__ key
   }
 }
 
+// ---- the general build over the ranks (dist_general)
+
+// owner of vertex v: the last rank whose range starts at or before v (an empty range starts where
+// the next one does)
+__device__ __forceinline__ uint32_t owner_of(const uint32_t *lo, int N, uint32_t v) {
+  int a = 0, b = N - 1;
+  while (a < b) {
+    const int m = (a + b + 1) >> 1;
+    if (lo[m] <= v) a = m;
+    else b = m - 1;
+  }
+  return (uint32_t) a;
+}
+
+// owner ranges: rank r starts at the first vertex with at least r/N of all half-edges before it
+__global__ void k_dist_owner_bounds(uint32_t Vg, const uint32_t *__restrict__ prefix, int N, uint32_t *__restrict__ lo) {
+  const int r = threadIdx.x;
+  if (r > N) return;
+  if (r == 0 || r == N) {
+    lo[r] = r == 0 ? 0u : Vg;
+    return;
+  }
+  const uint64_t target = (uint64_t) prefix[Vg] * (uint64_t) r / (uint64_t) N;
+  uint32_t a = 0, b = Vg;                          // first v in [0, Vg] with prefix[v] >= target
+  while (a < b) {
+    const uint32_t m = a + (b - a) / 2;
+    if (prefix[m] < target) a = m + 1;
+    else b = m;
+  }
+  lo[r] = a;
+}
+
+__global__ void k_dist_iota(uint32_t n, uint32_t *__restrict__ a, uint32_t *__restrict__ b) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) a[i] = b[i] = i;
+}
+
+// half-edges this rank sends to every rank (records are checked: ids in range, no self link)
+__global__ void __launch_bounds__(256) k_dist_route_count(uint64_t R, const uint32_t *__restrict__ root,
+                                                           const uint32_t *__restrict__ ctg,
+                                                           const uint32_t *__restrict__ bounds, int N,
+                                                           uint32_t *__restrict__ rank_cnt) {
+  __shared__ uint32_t s_lo[MAX_RANKS + 1], s_cnt[MAX_RANKS];
+  for (int i = threadIdx.x; i <= N; i += blockDim.x) {
+    s_lo[i] = bounds[i];
+    if (i < N) s_cnt[i] = 0;
+  }
+  __syncthreads();
+  for (uint64_t i = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x; i < R; i += (uint64_t) gridDim.x * blockDim.x) {
+    atomicAdd(&s_cnt[owner_of(s_lo, N, root[i])], 1u);
+    atomicAdd(&s_cnt[owner_of(s_lo, N, ctg[i])], 1u);
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < N; i += blockDim.x)
+    if (s_cnt[i]) atomicAdd(&rank_cnt[i], s_cnt[i]);
+}
+
+// every record's two half-edges, built as k_scatter_halfedges builds them (x = the global record
+// index), stored with their owner's local vertex straight into the owner's receive buffers (peer
+// memory over NVLink): entry `at` of this rank's share for rank d goes to index base[d] + at.  One
+// cursor per destination, advanced once per warp and destination, so that runs leave contiguous.
+__global__ void __launch_bounds__(256) k_dist_route_send(
+    uint64_t R, uint32_t rec_base, const uint32_t *__restrict__ root, const uint32_t *__restrict__ ctg,
+    const int32_t *__restrict__ dist, const float *__restrict__ std_dev, const uint8_t *__restrict__ flags,
+    const uint32_t *__restrict__ bounds, int N, uint32_t *__restrict__ cursor, uint4 *const *__restrict__ peer_ent,
+    uint32_t *const *__restrict__ peer_dest, const long long *__restrict__ base) {
+  __shared__ uint32_t s_lo[MAX_RANKS + 1];
+  for (int i = threadIdx.x; i <= N; i += blockDim.x) s_lo[i] = bounds[i];
+  __syncthreads();
+  const uint32_t lane = lane_id();
+  const uint64_t stride = (uint64_t) gridDim.x * blockDim.x;
+  for (uint64_t i0 = (uint64_t) blockIdx.x * blockDim.x + (threadIdx.x & ~31u); i0 < R; i0 += stride) {   // warp-uniform
+    const uint64_t i = i0 + lane;
+    const bool valid = i < R;
+    uint32_t r = 0, c = 0, fb = 0;
+    uint4 e = make_uint4(0u, 0u, 0u, 0u);
+    if (valid) {
+      r = root[i];
+      c = ctg[i];
+      const uint32_t f = flags[i];
+      fb = ((f & F_SENSE) ? E_SENSE : 0u) | ((f & F_SAME) ? E_SAME : 0u);
+      e.x = rec_base + (uint32_t) i;
+      e.z = (uint32_t) dist[i];
+      e.w = __float_as_uint(std_dev[i]);
+    }
+    for (int half = 0; half < 2; half++) {
+      const uint32_t v = half ? c : r;
+      e.y = half ? (r | fb | E_TWIN) : (c | fb);     // DIRECT r -> c lives in r's bucket, TWIN in c's
+      const uint32_t d = valid ? owner_of(s_lo, N, v) : 0u;
+      unsigned todo = __ballot_sync(0xffffffffu, valid);
+      while (todo) {
+        const uint32_t dl = __shfl_sync(0xffffffffu, d, __ffs(todo) - 1);
+        const unsigned same = __ballot_sync(0xffffffffu, valid && d == dl);
+        uint32_t at = 0;
+        if (lane == (uint32_t) (__ffs(same) - 1)) at = atomicAdd(&cursor[dl], (uint32_t) __popc(same));
+        at = __shfl_sync(0xffffffffu, at, __ffs(same) - 1);
+        if (valid && d == dl) {
+          const uint64_t k = (uint64_t) base[dl] + at + __popc(same & ((1u << lane) - 1u));
+          peer_ent[dl][k] = e;
+          peer_dest[dl][k] = v - s_lo[dl];
+        }
+        todo &= ~same;
+      }
+    }
+  }
+}
+
+// received half-edges into the buckets of the local vertices (order inside a bucket is free: the
+// resolve kernels sort)
+__global__ void __launch_bounds__(256) k_dist_bucket_scatter(uint64_t n, const uint4 *__restrict__ rx_ent,
+                                                              const uint32_t *__restrict__ rx_dest,
+                                                              const uint32_t *__restrict__ bptr,
+                                                              uint32_t *__restrict__ cursor, uint4 *__restrict__ entries) {
+  for (uint64_t j = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x; j < n; j += (uint64_t) gridDim.x * blockDim.x) {
+    const uint32_t d = rx_dest[j];
+    entries[bptr[d] + atomicAdd(&cursor[d], 1u)] = rx_ent[j];
+  }
+}
+
+// creator flags (one byte per global record) -> bits; each creator is flagged on one rank only
+// (the owner of its root's bucket), so a sum over the ranks is their OR
+__global__ void __launch_bounds__(256) k_dist_pack_creators(uint64_t R, const uint8_t *__restrict__ flag,
+                                                             uint32_t *__restrict__ words) {
+  const uint64_t stride = (uint64_t) gridDim.x * blockDim.x;
+  for (uint64_t i = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x; i < ((R + 31ull) & ~31ull); i += stride) {
+    const unsigned w = __ballot_sync(0xffffffffu, i < R && flag[i] != 0);
+    if (lane_id() == 0) words[i >> 5] = w;
+  }
+}
+
+__global__ void k_dist_popc(uint64_t W, const uint32_t *__restrict__ words, uint32_t *__restrict__ out) {
+  for (uint64_t w = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x; w < W; w += (uint64_t) gridDim.x * blockDim.x)
+    out[w] = (uint32_t) __popc(words[w]);
+}
+
+// k_emit_csr with the edge id from the creator bits: k = creating records before record x
+__device__ __forceinline__ void dist_emit_slot(const uint4 e, uint32_t slot, const uint32_t *__restrict__ words,
+                                               const uint32_t *__restrict__ wprefix, uint32_t *__restrict__ dst,
+                                               int32_t *__restrict__ dist, float *__restrict__ std_dev,
+                                               uint8_t *__restrict__ flags, uint32_t *__restrict__ eid) {
+  dst[slot] = e.y & E_OTHER_MASK;
+  dist[slot] = (int32_t) e.z;
+  std_dev[slot] = __uint_as_float(e.w);
+  flags[slot] = (uint8_t) (((e.y & E_SENSE) ? F_SENSE : 0u) | ((e.y & E_SAME) ? F_SAME : 0u) |
+                           ((e.y & E_RSENSE) ? F_RSENSE : 0u) | ((e.y & E_RSAME) ? F_RSAME : 0u));
+  const uint32_t k = wprefix[e.x >> 5] + (uint32_t) __popc(words[e.x >> 5] & ((1u << (e.x & 31u)) - 1u));
+  eid[slot] = 2u * k + ((e.y & E_TWIN) ? 1u : 0u);
+}
+
+__global__ void __launch_bounds__(256) k_dist_emit_csr(uint32_t V, const uint32_t *__restrict__ bptr,
+                                                        const uint32_t *__restrict__ row_ptr,
+                                                        const uint4 *__restrict__ entries,
+                                                        const uint32_t *__restrict__ words,
+                                                        const uint32_t *__restrict__ wprefix, uint32_t *__restrict__ dst,
+                                                        int32_t *__restrict__ dist, float *__restrict__ std_dev,
+                                                        uint8_t *__restrict__ flags, uint32_t *__restrict__ eid) {
+  const uint32_t v = blockIdx.x * blockDim.x + threadIdx.x;
+  uint32_t b0 = 0, r0 = 0, d = 0;
+  if (v < V) {
+    b0 = bptr[v];
+    r0 = row_ptr[v];
+    d = row_ptr[v + 1] - r0;
+  }
+  const bool big = d > BIG_ROW;
+  if (!big)
+    for (uint32_t k = 0; k < d; k++) dist_emit_slot(entries[b0 + k], r0 + k, words, wprefix, dst, dist, std_dev, flags, eid);
+  unsigned todo = __ballot_sync(0xffffffffu, big);   // big rows: the whole warp copies
+  while (todo) {
+    const int l = __ffs(todo) - 1;
+    todo &= todo - 1;
+    const uint32_t bb = __shfl_sync(0xffffffffu, b0, l), rr = __shfl_sync(0xffffffffu, r0, l),
+                   dd = __shfl_sync(0xffffffffu, d, l);
+    for (uint32_t k = lane_id(); k < dd; k += 32)
+      dist_emit_slot(entries[bb + k], rr + k, words, wprefix, dst, dist, std_dev, flags, eid);
+  }
+}
+
+// k4_fill_srcp for rows that start at position row_base: srcp and the big-row list hold global
+// positions, F_LT compares ids (= positions here)
+__global__ void __launch_bounds__(256) k_dist_fill_srcp(GraphArgs g, uint32_t *__restrict__ srcp,
+                                                         uint32_t *__restrict__ big_rows) {
+  const uint32_t pl = blockIdx.x * blockDim.x + threadIdx.x;
+  const uint32_t p = g.row_base + pl;
+  uint32_t r0 = 0, d = 0;
+  if (pl < g.V) {
+    r0 = g.row_ptr[pl];
+    d = g.row_ptr[pl + 1] - r0;
+  }
+  const bool big = d > BIG_ROW;
+  if (!big)
+    for (uint32_t k = 0; k < d; k++) {
+      srcp[r0 + k] = p;
+      g.flags[r0 + k] = (uint8_t) ((g.flags[r0 + k] & 0x0Fu) | (g.dst[r0 + k] < p ? F_LT : 0u));
+    }
+  const uint32_t wmax = __reduce_max_sync(0xffffffffu, d);
+  if (lane_id() == 0 && wmax) atomicMax(&g.counters[CNT_MAX_DEG], wmax);
+  warp_append(big, p, big_rows, &g.counters[CNT_BIG_ROWS]);
+  unsigned todo = __ballot_sync(0xffffffffu, big);
+  while (todo) {
+    const int l = __ffs(todo) - 1;
+    todo &= todo - 1;
+    const uint32_t pp = __shfl_sync(0xffffffffu, p, l), rr = __shfl_sync(0xffffffffu, r0, l),
+                   dd = __shfl_sync(0xffffffffu, d, l);
+    for (uint32_t k = lane_id(); k < dd; k += 32) {
+      srcp[rr + k] = pp | S_BIG;
+      g.flags[rr + k] = (uint8_t) ((g.flags[rr + k] & 0x0Fu) | (g.dst[rr + k] < pp ? F_LT : 0u));
+    }
+  }
+}
+
 // (re)open every rank's receive buffers; collective
 int open_peer_buffers(gtsb_context *c) {
   DistState *D = static_cast<DistState *>(c->dstate);
@@ -422,13 +643,14 @@ void dist_release(gtsb_context *c) {
     for (int k = 0; k < 2; k++)
       if (r != c->rank && D->peer_ptr[r][k] != nullptr) cudaIpcCloseMemHandle(D->peer_ptr[r][k]);
   for (DevBuf *b : {&D->small, &D->bounds, &D->rank_cnt, &D->rx_ent, &D->rx_dest, &D->corr_all, &D->prop_all, &D->stage,
-                    &D->stage2, &D->peer_tab, &D->handles, &D->mail_hist})
+                    &D->stage2, &D->peer_tab, &D->handles, &D->mail_hist, &D->deg_prefix, &D->creators})
     if (b->owned && b->p != nullptr) cudaFree(b->p);
   if (D->h_small != nullptr) cudaFreeHost(D->h_small);
   delete D;
   c->dstate = nullptr;
   c->world = 1;
   c->rank = 0;
+  c->id_rows = false;
 }
 
 namespace detail {
@@ -467,6 +689,8 @@ struct Plan {                     // what the ranks agreed on while building
   bool facts_on_side = false;     // vinfo was computed and gathered on the side stream
   std::vector<uint64_t> vlo;      // [N+1] vertex-attribute slices by id (gtsb_set_vertices_slice_host)
   bool gather_attributes = false;
+  bool any_input = false;         // gtsb_dist_any_input, agreed at the build setup
+  uint32_t reason = 0;            // FB_* bits of any rank that made the line-ordered attempt give way
 };
 
 // contig ids by position and the packed per-neighbour facts of the pairs pass: both depend on
@@ -498,7 +722,7 @@ int dist_side_facts(gtsb_context *c, DistState *D, Plan &P) {
     if (allgatherv(c, "nccl_allgather_vattr", c->vattr.p, sizeof(VAttr), P.vlo, side) != 0) return -1;
     if (allgatherv(c, "nccl_allgather_vattr", c->astat.p, 4, P.vlo, side) != 0) return -1;
   }
-  if (allgatherv(c, "nccl_allgather_vid", c->vid.p, 4, P.lo, side) != 0) return -1;
+  if (!c->id_rows && allgatherv(c, "nccl_allgather_vid", c->vid.p, 4, P.lo, side) != 0) return -1;
   FilterArgs fa{};
   c->line_layout = true;
   fa.g = graph_args(c);
@@ -513,7 +737,7 @@ int dist_side_facts(gtsb_context *c, DistState *D, Plan &P) {
   return 0;
 }
 
-// lines, positions, contig ids by position
+// lines, positions, contig ids by position.  1: the general build takes over (P.reason)
 int dist_positions(gtsb_context *c, DistState *D, Build2Args &a, Plan &P, int setup_rc) {
   const int N = c->world, me = c->rank;
   const bool last = me == N - 1;
@@ -532,18 +756,26 @@ int dist_positions(gtsb_context *c, DistState *D, Build2Args &a, Plan &P, int se
     CK(cudaMemcpyAsync(&L, a.tile_off + ntiles, 4, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
   }
-  // with the line count: which slice of the vertex attributes this rank uploaded (all of them: 0, Vg)
-  const uint32_t setup_mine[3] = {L, c->vertices_sliced ? (uint32_t) c->vslice_first : 0u,
-                                  c->vertices_sliced ? (uint32_t) c->vslice_count : (uint32_t) Vg};
-  if (exchange(c, setup_rc, "build setup", setup_mine, 3, all) != 0) return -1;
+  // with the line count: which slice of the vertex attributes this rank uploaded (all of them: 0, Vg),
+  // and the build switches (bit 0: gtsb_dist_any_input, bit 1: with gtsb_force_general_build)
+  const uint32_t mode = c->dist_any_input ? 1u | (c->force_general ? 2u : 0u) : 0u;
+  const uint32_t setup_mine[4] = {L, c->vertices_sliced ? (uint32_t) c->vslice_first : 0u,
+                                  c->vertices_sliced ? (uint32_t) c->vslice_count : (uint32_t) Vg, mode};
+  if (exchange(c, setup_rc, "build setup", setup_mine, 4, all) != 0) return -1;
+  for (int r = 0; r < N; r++)
+    if (all[(size_t) r * 4 + 3] != mode)
+      return fail(c, "gtsb_pipeline: the ranks disagree on gtsb_dist_any_input / gtsb_force_general_build "
+                     "(rank %d: %u, rank %d: %u; bit 0 = any input, bit 1 = forced general build)",
+                  me, mode, r, all[(size_t) r * 4 + 3]);
+  P.any_input = (mode & 1u) != 0;
   P.lo.assign(N + 1, 0);
-  for (int r = 0; r < N; r++) P.lo[r + 1] = P.lo[r] + all[(size_t) r * 3];
+  for (int r = 0; r < N; r++) P.lo[r + 1] = P.lo[r] + all[(size_t) r * 4];
   {
     bool whole = true, tiled = true;
     uint64_t at = 0;
     P.vlo.assign(N + 1, 0);
     for (int r = 0; r < N; r++) {
-      const uint64_t f = all[(size_t) r * 3 + 1], n = all[(size_t) r * 3 + 2];
+      const uint64_t f = all[(size_t) r * 4 + 1], n = all[(size_t) r * 4 + 2];
       whole &= f == 0 && n == Vg;
       tiled &= f == at;
       at = f + n;
@@ -556,6 +788,11 @@ int dist_positions(gtsb_context *c, DistState *D, Build2Args &a, Plan &P, int se
   }
   P.L = L;
   P.L_total = P.lo[N];
+  if (mode & 2u) return 1;
+  if (P.L_total > Vg && P.any_input) {
+    P.reason = FB_MULTIRUN;
+    return 1;
+  }
   if (P.L_total > Vg) return fail(c, "more lines than contigs: a contig heads more than one line");
   P.lo[N] = Vg;                                               // the last rank also holds the lineless contigs
   P.own_lo = (uint32_t) P.lo[me];
@@ -596,6 +833,36 @@ int dist_positions(gtsb_context *c, DistState *D, Build2Args &a, Plan &P, int se
   return 0;
 }
 
+// windows over my rows; the graph is complete
+int dist_windows(gtsb_context *c, const Plan &P) {
+  const int N = c->world;
+  // window tables: sized by the largest share of rows / slots any rank holds (uniform growth)
+  uint64_t rows_max = 0;
+  for (int r = 0; r < N; r++) rows_max = P.lo[r + 1] - P.lo[r] > rows_max ? P.lo[r + 1] - P.lo[r] : rows_max;
+  bool grew = c->wcount.cap < ((rows_max + 63) / 64 + 2) * 4 || c->win_start.cap < ((rows_max < P.E_max + 1 ? rows_max : P.E_max + 1) + 2) * 4;
+  const int rc = injected_failure(c, "windows", grew) != 0 ? -1 : ensure_windows(c, rows_max, P.E_max + 1);
+  if (grew && agree(c, rc, "windows") != 0) return -1;
+  if (!grew && rc != 0) return -1;
+  c->line_layout = true;
+  c->csr_exported = false;
+  c->have_graph = true;
+  {
+    GraphArgs g{};
+    g.V = P.Vloc;
+    g.row_ptr = c->row_ptr.as<uint32_t>();
+    g.counters = c->counters.as<uint32_t>();
+    c->stats.kernel_launches += launch_pack_windows(g, c->wcount.as<uint32_t>(), c->woff.as<uint32_t>(),
+                                                    c->win_start.as<uint32_t>(), c->scan_scratch.as<uint32_t>(), c->stream);
+  }
+  if (read_counters(c) != 0) return -1;
+  c->n_windows = P.Vloc ? c->h_counters[CNT_WINDOWS] : 0;
+  c->stats.nof_edges = c->E;
+  c->stats.big_rows = c->n_big_rows;
+  c->stats.max_degree = c->max_deg;
+  return 0;
+}
+
+// the line-ordered build over the ranks.  1: it gave way to the general build (any input, P.reason)
 int dist_build(gtsb_context *c, DistState *D, Plan &P, int inputs_rc) {
   const int N = c->world, me = c->rank;
   const bool last = me == N - 1;
@@ -679,7 +946,7 @@ int dist_build(gtsb_context *c, DistState *D, Plan &P, int inputs_rc) {
   a.rank_cnt = D->rank_cnt.as<uint32_t>();
 
   rc = dist_positions(c, D, a, P, setup_rc);      // exchanges the setup status with the line counts
-  if (rc != 0) return -1;
+  if (rc != 0) return rc;
   tr.mark(me, "positions");
   if (dist_side_facts(c, D, P) != 0) return -1;
 
@@ -691,18 +958,22 @@ int dist_build(gtsb_context *c, DistState *D, Plan &P, int inputs_rc) {
     if (read_counters(c) != 0) return -1;
     if (c->h_counters[CNT_ERROR] & 1u) return fail(c, "gtsb_pipeline: a record names a vertex id >= nof_vertices");
     if (c->h_counters[CNT_ERROR] & 2u) return fail(c, "gtsb_pipeline: self link (root == ctg) is not supported");
-    if (c->h_counters[CNT_FALLBACK])
+    if (c->h_counters[CNT_FALLBACK] && !P.any_input)
       return fail(c, "gtsb_pipeline: input outside what the rank-partitioned build accepts (reason mask %u: "
                      "1 = a contig heads several lines, 2 = line longer than %u records, 4 = oversized segment, "
                      "8 = a link listed only on the later line); a single device rebuilds such input with its "
                      "general path, the partitioned build has none", c->h_counters[CNT_FALLBACK], MAX_LINE_RECS);
+    mine[N + 1] = c->h_counters[CNT_FALLBACK];
     CK(cudaMemcpyAsync(&mine[1], a.rank_cnt, N * 4, cudaMemcpyDeviceToHost, s));
     CK(cudaMemcpyAsync(&mine[0], a.k0 + P.Vloc, 4, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     return 0;
   }();
-  if (exchange(c, rc, "classify", mine, N + 1, all) != 0) return -1;
-  const int W = N + 1;
+  // any input: the reason masks travel with the counts, so that every rank gives way here
+  if (exchange(c, rc, "classify", mine, N + (P.any_input ? 2 : 1), all) != 0) return -1;
+  const int W = N + (P.any_input ? 2 : 1);
+  for (int r = 0; r < N && P.any_input; r++) P.reason |= all[(size_t) r * W + N + 1];
+  if (P.reason) return 1;
   uint64_t k_base = 0, n_creators = 0, creators_max = 0;
   for (int r = 0; r < N; r++) {
     if (r < me) k_base += all[(size_t) r * W];
@@ -815,7 +1086,7 @@ int dist_build(gtsb_context *c, DistState *D, Plan &P, int inputs_rc) {
   rc = [&]() -> int {
     if (read_counters(c) != 0) return -1;
     if (c->h_counters[CNT_ERROR] & 8u) return fail(c, "gtsb_pipeline: mail for a row of another rank (internal)");
-    if (c->h_counters[CNT_FALLBACK])
+    if (c->h_counters[CNT_FALLBACK] && !P.any_input)
       return fail(c, "gtsb_pipeline: input outside what the rank-partitioned build accepts (reason mask %u: "
                      "1 = a contig heads several lines, 2 = line longer than %u records, 4 = oversized segment, "
                      "8 = a link listed only on the later line); a single device rebuilds such input with its "
@@ -830,14 +1101,17 @@ int dist_build(gtsb_context *c, DistState *D, Plan &P, int inputs_rc) {
   // ---- reverse-flag corrections may belong to rows of other ranks
   const uint32_t my_corr = c->h_counters[CNT_CORRECTIONS] < a.corrections_cap ? c->h_counters[CNT_CORRECTIONS]
                                                                                 : a.corrections_cap;
-  const uint32_t rows_mine[3] = {my_corr, c->n_big_rows, c->max_deg};
-  if (exchange(c, rc, "rows", rows_mine, 3, all) != 0) return -1;
+  const uint32_t rows_mine[4] = {my_corr, c->n_big_rows, c->max_deg, c->h_counters[CNT_FALLBACK]};
+  const int RW = P.any_input ? 4 : 3;
+  if (exchange(c, rc, "rows", rows_mine, RW, all) != 0) return -1;
+  for (int r = 0; r < N && P.any_input; r++) P.reason |= all[(size_t) r * RW + 3];
+  if (P.reason) return 1;
   std::vector<uint64_t> c_off(N + 1, 0);
   P.big_rows_max = P.deg_max = 0;
   for (int r = 0; r < N; r++) {
-    c_off[r + 1] = c_off[r] + all[(size_t) r * 3];
-    P.big_rows_max = all[(size_t) r * 3 + 1] > P.big_rows_max ? all[(size_t) r * 3 + 1] : P.big_rows_max;
-    P.deg_max = all[(size_t) r * 3 + 2] > P.deg_max ? all[(size_t) r * 3 + 2] : P.deg_max;
+    c_off[r + 1] = c_off[r] + all[(size_t) r * RW];
+    P.big_rows_max = all[(size_t) r * RW + 1] > P.big_rows_max ? all[(size_t) r * RW + 1] : P.big_rows_max;
+    P.deg_max = all[(size_t) r * RW + 2] > P.deg_max ? all[(size_t) r * RW + 2] : P.deg_max;
   }
   if (c_off[N]) {
     bool grew = false;
@@ -854,33 +1128,272 @@ int dist_build(gtsb_context *c, DistState *D, Plan &P, int inputs_rc) {
     c->stats.kernel_launches += launch_b2_apply_corrections(a, D->corr_all.as<uint4>(), (uint32_t) c_off[N], s);
   }
 
-  // ---- windows over my rows
-  {
-    // window tables: sized by the largest share of rows / slots any rank holds (uniform growth)
-    uint64_t rows_max = 0;
-    for (int r = 0; r < N; r++) rows_max = P.lo[r + 1] - P.lo[r] > rows_max ? P.lo[r + 1] - P.lo[r] : rows_max;
-    bool grew = c->wcount.cap < ((rows_max + 63) / 64 + 2) * 4 || c->win_start.cap < ((rows_max < P.E_max + 1 ? rows_max : P.E_max + 1) + 2) * 4;
-    rc = injected_failure(c, "windows", grew) != 0 ? -1 : ensure_windows(c, rows_max, P.E_max + 1);
-    if (grew && agree(c, rc, "windows") != 0) return -1;
-    if (!grew && rc != 0) return -1;
+  if (dist_windows(c, P) != 0) return -1;
+  tr.mark(me, "corrections+windows");
+  return 0;
+}
+
+// The general (sort-based) build of gtsb_build.cu over the ranks, for any record input: rank r owns
+// the buckets of the vertex ids [lo[r], lo[r+1]) -- ranges cut by the global half-edge counts, so
+// that every bucket, a hub's included, is whole on one rank -- and its rows are those vertices in id
+// order (positions are ids).  Every half-edge travels to its bucket's owner, the buckets resolve
+// with the single device's kernels, and the one global fact, the rank of each creating record among
+// all creating records, comes from the OR of the ranks' creator bits.  The records are any
+// contiguous slices in file order, ranks in order; the line-ordered attempt read them only.
+int dist_general(gtsb_context *c, DistState *D, Plan &P) {
+  const int N = c->world, me = c->rank;
+  const uint64_t Vg = c->V, R = c->R;
+  cudaStream_t s = c->stream;
+  uint32_t *cnt = c->counters.as<uint32_t>();
+  std::vector<uint32_t> all;
+  Trace tr(s);
+  c->fallback_reason = P.reason;
+  c->id_rows = true;
+  c->have_graph = false;
+  // the attempt's neighbour facts may still be on their way (side stream) into vid / vinfo
+  if (P.facts_on_side) CK(cudaStreamWaitEvent(s, D->ev_join, 0));
+  P.facts_on_side = false;
+
+  // ---- half-edges per vertex over all ranks' records, and the global record numbering
+  BuildArgs b{};
+  b.R = R;
+  b.V = (uint32_t) Vg;
+  b.sm_count = c->sm_count;
+  int rc = [&]() -> int {
+    bool unused = false;
+    if (injected_failure(c, "general", unused) != 0) return -1;
+    ENSURE(c->cnt, (Vg + 1) * 4);
+    ENSURE(D->deg_prefix, (Vg + 1) * 4);
+    if (ensure_root_column(c) != 0) return -1;
+    CK(cudaMemsetAsync(c->counters.p, 0, CNT_NUM * 4, s));
+    CK(cudaMemsetAsync(c->cnt.p, 0, (Vg + 1) * 4, s));
+    CK(cudaMemsetAsync(c->vstate.p, 0, Vg ? Vg : 1, s));
+    b.root = c->root.as<uint32_t>();
+    b.ctg = c->ctg.as<uint32_t>();
+    b.cnt = c->cnt.as<uint32_t>();
+    b.counters = cnt;
+    if (R) launch_count_halfedges(b, s);
+    c->stats.kernel_launches += R ? 1 : 0;
+    if (read_counters(c) != 0) return -1;
+    if (c->h_counters[CNT_ERROR] & 1u) return fail(c, "gtsb_pipeline: a record names a vertex id >= nof_vertices");
+    if (c->h_counters[CNT_ERROR] & 2u) return fail(c, "gtsb_pipeline: self link (root == ctg) is not supported");
+    return 0;
+  }();
+  const uint32_t r_mine = (uint32_t) R;           // below 2^31: checked at the setup
+  if (exchange(c, rc, "general build: records", &r_mine, 1, all) != 0) return -1;
+  uint64_t R_total = 0, rec_base = 0;
+  for (int r = 0; r < N; r++) {
+    if (r < me) rec_base += all[r];
+    R_total += all[r];
   }
-  c->line_layout = true;
-  c->csr_exported = false;
-  c->have_graph = true;
+  if (2 * R_total >= 0xFFFFFFF0ull) return fail(c, "too many records");
   {
-    GraphArgs g{};
-    g.V = P.Vloc;
-    g.row_ptr = c->row_ptr.as<uint32_t>();
-    g.counters = cnt;
-    c->stats.kernel_launches += launch_pack_windows(g, c->wcount.as<uint32_t>(), c->woff.as<uint32_t>(),
-                                                    c->win_start.as<uint32_t>(), c->scan_scratch.as<uint32_t>(), s);
+    KernelTimer t_("nccl_allreduce_degrees", s);
+    NK(g_nccl.AllReduce(c->cnt.p, c->cnt.p, Vg, ncclUint32, ncclSum, D->comm, s));
+  }
+  uint32_t *prefix = D->deg_prefix.as<uint32_t>();
+  exclusive_scan<uint32_t>(c->cnt.as<uint32_t>(), Vg, prefix, c->scan_scratch.as<uint32_t>(), s);
+  k_dist_owner_bounds<<<1, MAX_RANKS + 1, 0, s>>>((uint32_t) Vg, prefix, N, D->bounds.as<uint32_t>());
+  uint32_t hb[MAX_RANKS + 1];
+  CK(cudaMemcpyAsync(hb, D->bounds.p, (N + 1) * 4, cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
+  P.lo.assign(N + 1, 0);
+  for (int r = 0; r <= N; r++) P.lo[r] = hb[r];
+  P.own_lo = hb[me];
+  P.Vloc = hb[me + 1] - hb[me];
+  c->row_base = P.own_lo;
+  c->Vloc = P.Vloc;
+  if (Vg) {
+    k_dist_iota<<<(uint32_t) ((Vg + 255) / 256), 256, 0, s>>>((uint32_t) Vg, c->vid.as<uint32_t>(), c->pos.as<uint32_t>());
+    c->stats.kernel_launches += 1;
+  }
+  c->stats.kernel_launches += 4;
+  tr.mark(me, "general: owners");
+  if (dist_side_facts(c, D, P) != 0) return -1;
+
+  // ---- half-edges per destination rank
+  CK(cudaMemsetAsync(D->rank_cnt.p, 0, (MAX_RANKS + 2) * 4, s));
+  const uint32_t rblocks = (uint32_t) ((R + 255) / 256 < (uint64_t) c->sm_count * 8 ? (R + 255) / 256 : c->sm_count * 8);
+  if (R) {
+    KernelTimer t_("k_dist_route_count", s);
+    k_dist_route_count<<<rblocks, 256, 0, s>>>(R, b.root, b.ctg, D->bounds.as<uint32_t>(), N, D->rank_cnt.as<uint32_t>());
+    c->stats.kernel_launches += 1;
+  }
+  uint32_t mine[MAX_RANKS];
+  CK(cudaMemcpyAsync(mine, D->rank_cnt.p, N * 4, cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
+  if (exchange(c, 0, "general build: routes", mine, N, all) != 0) return -1;
+  uint64_t M = 0, M_max = 0;
+  std::vector<long long> base(N, 0);
+  for (int r = 0; r < N; r++) {
+    uint64_t Mr = 0;
+    for (int h = 0; h < N; h++) {
+      if (h < me) base[r] += all[(size_t) h * N + r];
+      Mr += all[(size_t) h * N + r];
+    }
+    if (r == me) M = Mr;
+    M_max = Mr > M_max ? Mr : M_max;
+  }
+  const uint64_t W = (R_total + 31) / 32;           // words of creator bits
+
+  // ---- receive buffers and the build's work arrays.  The shared buffers are sized from numbers
+  // every rank holds (the line-ordered build decides on their growth locally); the exchange that
+  // ends the block is due in any case
+  bool rx_grew = false;
+  rc = [&]() -> int {
+    bool unused = false;
+    if (injected_failure(c, "general_receive", unused) != 0) return -1;
+    if (ensure_u(c, D->rx_ent, (M_max + M_max / 8 + 16) * sizeof(uint4), rx_grew) != 0) return -1;
+    if (ensure_u(c, D->rx_dest, (M_max + M_max / 8 + 16) * 4, rx_grew) != 0) return -1;
+    ENSURE(D->peer_tab, MAX_RANKS * 24);
+    const uint64_t max_rows = M_max / 2 + 1;           // slots <= groups <= half-edges received
+    if ((c->srcp.cap < 2 * max_rows * 4 + 256 || c->estate.cap < 2 * max_rows) && ensure_rows(c, max_rows) != 0) return -1;
+    ENSURE(c->entries, (M + 1) * sizeof(uint4));
+    ENSURE(c->bptr, (P.Vloc + 2) * 4);
+    ENSURE(c->cursor, (P.Vloc + 2) * 4);
+    ENSURE(c->deg, (P.Vloc + 2) * 4);
+    ENSURE(c->row_ptr, (P.Vloc + 2) * 4);
+    ENSURE(c->big_rows, (P.Vloc + 2) * 4);
+    ENSURE(c->large_list, (P.Vloc + 2) * sizeof(uint2));
+    ENSURE(c->creator_flag, R_total + 1);
+    ENSURE(D->creators, (3 * W + 3) * 4);           // words, their popcounts, the prefix of those (W + 1 each)
+    const uint64_t scan_n = Vg > W ? Vg : W;
+    ENSURE(c->scan_scratch, scan_scratch_elems(scan_n > R ? scan_n : R) * 4);
+    return 0;
+  }();
+  const uint32_t grew_mine = rx_grew ? 1u : 0u;
+  if (exchange(c, rc, "general build: receive buffers", &grew_mine, 1, all) != 0) return -1;
+  bool reopen = !D->peers_open;
+  for (int r = 0; r < N; r++) reopen |= all[r] != 0;
+  if (reopen && open_peer_buffers(c) != 0) return -1;
+  {
+    char tab[MAX_RANKS * 24];
+    void **pe = reinterpret_cast<void **>(tab), **pd = pe + MAX_RANKS;
+    long long *ps = reinterpret_cast<long long *>(pd + MAX_RANKS);
+    for (int r = 0; r < N; r++) {
+      pe[r] = D->peer_ptr[r][0];
+      pd[r] = D->peer_ptr[r][1];
+      ps[r] = base[r];
+    }
+    CK(cudaMemcpyAsync(D->peer_tab.p, tab, sizeof tab, cudaMemcpyHostToDevice, s));
+    CK(cudaStreamSynchronize(s));                                      // tab lives on this stack frame
+  }
+
+  // ---- every half-edge to its bucket's owner.  The exchanges above ordered every rank behind every
+  // rank's earlier reads of its receive buffers.
+  if (await_records(c) != 0) return -1;          // dist/std_dev/flags may still be on their way (copy stream)
+  CK(cudaMemsetAsync(D->rank_cnt.p, 0, (MAX_RANKS + 2) * 4, s));
+  if (R) {
+    KernelTimer t_("k_dist_route_send", s);
+    k_dist_route_send<<<rblocks, 256, 0, s>>>(
+        R, (uint32_t) rec_base, b.root, b.ctg, c->dist.as<int32_t>(), c->std_dev.as<float>(), c->flags.as<uint8_t>(),
+        D->bounds.as<uint32_t>(), N, D->rank_cnt.as<uint32_t>(), reinterpret_cast<uint4 *const *>(D->peer_tab.p),
+        reinterpret_cast<uint32_t *const *>(D->peer_tab.as<char>() + MAX_RANKS * 8),
+        reinterpret_cast<const long long *>(D->peer_tab.as<char>() + MAX_RANKS * 16));
+    c->stats.kernel_launches += 1;
+  }
+  {
+    // all half-edges have landed once every rank's send kernel is complete: a stream-ordered barrier
+    KernelTimer t_("nccl_barrier_mail", s);
+    NK(g_nccl.AllReduce(D->small.p, D->small.p, 1, ncclUint32, ncclSum, D->comm, s));
+  }
+  tr.mark(me, "general: routes");
+
+  // ---- buckets of my vertices (their sizes are the reduced counts), resolution
+  b.R = R_total;
+  b.V = P.Vloc;
+  b.bptr = c->bptr.as<uint32_t>();
+  b.cursor = c->cursor.as<uint32_t>();
+  b.deg = c->deg.as<uint32_t>();
+  b.scan_scratch = c->scan_scratch.as<uint32_t>();
+  b.entries = c->entries.as<uint4>();
+  b.creator_flag = c->creator_flag.as<uint8_t>();
+  b.large_list = c->large_list.as<uint2>();
+  b.hubs = (P.reason & FB_LONGLINE) ? 1 : 0;
+  exclusive_scan<uint32_t>(c->cnt.as<uint32_t>() + P.own_lo, P.Vloc, b.bptr, b.scan_scratch, s);
+  CK(cudaMemsetAsync(b.cursor, 0, (P.Vloc + 1) * 4, s));
+  CK(cudaMemsetAsync(c->counters.p, 0, CNT_NUM * 4, s));
+  CK(cudaMemsetAsync(b.creator_flag, 0, R_total + 1, s));
+  if (M) {
+    KernelTimer t_("k_dist_bucket_scatter", s);
+    const uint32_t blocks = (uint32_t) ((M + 255) / 256 < (uint64_t) c->sm_count * 8 ? (M + 255) / 256 : c->sm_count * 8);
+    k_dist_bucket_scatter<<<blocks, 256, 0, s>>>(M, D->rx_ent.as<uint4>(), D->rx_dest.as<uint32_t>(), b.bptr, b.cursor,
+                                                 b.entries);
+    c->stats.kernel_launches += 1;
+  }
+  launch_build_resolve(b, s);
+  c->stats.kernel_launches += 3 + (P.Vloc ? 2 : 0);
+  uint32_t nlarge = 0;
+  rc = [&]() -> int {
+    if (read_counters(c) != 0) return -1;
+    if (c->h_counters[CNT_ERROR] & 16u)
+      return fail(c, "gtsb_pipeline: the hub buckets of rank %d need more than 2^32 scratch entries in the general "
+                     "build (about 5e8 records of hub vertices on one rank); use more ranks or split the input", me);
+    nlarge = c->h_counters[CNT_LARGE_BUCKETS];
+    if (nlarge) {
+      const uint64_t pad = c->h_counters[CNT_LARGE_PAD];
+      ENSURE(c->lscratch, pad * sizeof(uint4));
+      ENSURE(c->ltag, pad * 4);
+    }
+    return 0;
+  }();
+  if (exchange(c, rc, "general build: hub buckets", &nlarge, 1, all) != 0) return -1;
+  c->stats.large_buckets = 0;
+  for (int r = 0; r < N; r++) c->stats.large_buckets += all[r];
+  if (nlarge) {
+    launch_build_resolve_large(b, c->lscratch.as<uint4>(), c->ltag.as<uint32_t>(), nlarge, s);
+    c->stats.kernel_launches += 1;
+  }
+  tr.mark(me, "general: resolve");
+
+  // ---- edge ids: the rank of a creating record among all of them, from the OR of the creator bits
+  uint32_t *words = D->creators.as<uint32_t>(), *popc = words + W + 1, *wprefix = popc + W + 1;
+  if (W) {
+    KernelTimer t_("k_dist_creators+allreduce", s);
+    const uint32_t blocks = (uint32_t) ((W + 7) / 8 < (uint64_t) c->sm_count * 8 ? (W + 7) / 8 : c->sm_count * 8);
+    k_dist_pack_creators<<<blocks, 256, 0, s>>>(R_total, b.creator_flag, words);
+    NK(g_nccl.AllReduce(words, words, W, ncclUint32, ncclSum, D->comm, s));
+    k_dist_popc<<<blocks, 256, 0, s>>>(W, words, popc);
+    c->stats.kernel_launches += 2;
+  }
+  exclusive_scan<uint32_t>(popc, W, wprefix, b.scan_scratch, s);
+
+  // ---- rows
+  exclusive_scan<uint32_t>(b.deg, P.Vloc, c->row_ptr.as<uint32_t>(), b.scan_scratch, s);
+  if (P.Vloc) {
+    KernelTimer t_("k_dist_emit_csr", s);
+    k_dist_emit_csr<<<(P.Vloc + 255) / 256, 256, 0, s>>>(P.Vloc, b.bptr, c->row_ptr.as<uint32_t>(), b.entries, words,
+                                                         wprefix, c->dst.as<uint32_t>(), c->edist.as<int32_t>(),
+                                                         c->estd.as<float>(), c->eflags.as<uint8_t>(), c->eid.as<uint32_t>());
+    c->stats.kernel_launches += 1;
+  }
+  c->stats.kernel_launches += 6;
+  uint32_t e32 = 0;
+  CK(cudaMemcpyAsync(&e32, c->row_ptr.as<uint32_t>() + P.Vloc, 4, cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
+  c->E = e32;
+  CK(cudaMemsetAsync(c->estate.p, 0, c->E ? c->E : 1, s));      // GIS_UNVISITED, graph.c:162
+  c->line_layout = true;                          // vid / pos: identity
+  if (P.Vloc) {
+    GraphArgs g = graph_args(c);
+    KernelTimer t_("k_dist_fill_srcp", s);
+    k_dist_fill_srcp<<<(P.Vloc + 255) / 256, 256, 0, s>>>(g, c->srcp.as<uint32_t>(), c->big_rows.as<uint32_t>());
+    c->stats.kernel_launches += 1;
   }
   if (read_counters(c) != 0) return -1;
-  c->n_windows = P.Vloc ? c->h_counters[CNT_WINDOWS] : 0;
-  c->stats.nof_edges = c->E;
-  c->stats.big_rows = c->n_big_rows;
-  c->stats.max_degree = c->max_deg;
-  tr.mark(me, "corrections+windows");
+  c->n_big_rows = c->h_counters[CNT_BIG_ROWS];
+  c->max_deg = c->h_counters[CNT_MAX_DEG];
+  const uint32_t rows_mine[3] = {(uint32_t) c->E, c->n_big_rows, c->max_deg};
+  if (exchange(c, 0, "general build: rows", rows_mine, 3, all) != 0) return -1;
+  P.E_max = 0;
+  P.big_rows_max = P.deg_max = 0;
+  for (int r = 0; r < N; r++) {
+    P.E_max = all[(size_t) r * 3] > P.E_max ? all[(size_t) r * 3] : P.E_max;
+    P.big_rows_max = all[(size_t) r * 3 + 1] > P.big_rows_max ? all[(size_t) r * 3 + 1] : P.big_rows_max;
+    P.deg_max = all[(size_t) r * 3 + 2] > P.deg_max ? all[(size_t) r * 3 + 2] : P.deg_max;
+  }
+  if (dist_windows(c, P) != 0) return -1;
+  tr.mark(me, "general: rows+windows");
   return 0;
 }
 
@@ -1057,9 +1570,14 @@ int dist_pipeline(gtsb_context *c, float cn_cutoff, float astat_cutoff, int use_
   P.cn_cutoff = cn_cutoff;
   P.astat_cutoff = astat_cutoff;
   P.use_cn = use_cn;
+  c->fallback_reason = 0;
+  c->id_rows = false;
+  c->stats.large_buckets = 0;
   {
     KernelTimer t_("PHASE_build", c->stream);
-    if (dist_build(c, D, P, rc) != 0) return -1;
+    const int b = dist_build(c, D, P, rc);
+    if (b < 0) return -1;
+    if (b > 0 && dist_general(c, D, P) != 0) return -1;
   }
   KernelTimer t_("PHASE_filter", c->stream);
   if (dist_filter(c, D, P, cn_cutoff, astat_cutoff, use_cn, cncutoff, ocutoff) != 0) return -1;
@@ -1234,6 +1752,12 @@ int gtsb_dist_init(gtsb_context *c, int rank, int world, const void *id128) {
   }
   ENSURE(D->small, (size_t) MAX_RANKS * SMALL_N * 4);
   CK(cudaMallocHost(&D->h_small, (size_t) MAX_RANKS * SMALL_N * 4));
+  return 0;
+}
+
+int gtsb_dist_any_input(gtsb_context *c, int on) {
+  if (c == nullptr) return -1;
+  c->dist_any_input = on != 0 ? 1 : 0;
   return 0;
 }
 

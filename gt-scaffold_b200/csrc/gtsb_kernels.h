@@ -172,7 +172,11 @@ struct BuildArgs {
 };
 
 void launch_build_count(const BuildArgs &a, cudaStream_t s);
+void launch_count_halfedges(const BuildArgs &a, cudaStream_t s);   // launch_build_count without the scan
 void launch_build_scatter_resolve(const BuildArgs &a, cudaStream_t s);
+// the resolution of buckets that are already filled (bptr, entries): launch_build_scatter_resolve
+// without the scatter; buckets above the thread / warp paths are queued for launch_build_resolve_large
+void launch_build_resolve(const BuildArgs &a, cudaStream_t s);
 void launch_build_resolve_large(const BuildArgs &a, uint4 *scratch, uint32_t *scratch_tag,
                                 uint32_t nlarge, cudaStream_t s);
 void launch_build_emit(const BuildArgs &a, cudaStream_t s);

@@ -69,7 +69,8 @@ int gtsb_set_stream(gtsb_context *ctx, void *cuda_stream);
 /* also record, per edge, which record's attributes it carries (needed to fill
    GtScaffolderGraphEdge.num_pairs); costs 8 B/edge of extra traffic */
 int gtsb_want_win_rec(gtsb_context *ctx, int on);
-/* testing aid: always take the general (any-input) build path */
+/* testing aid: always take the general (any-input) build path.  A partitioned context (after
+   gtsb_dist_init) follows it only while gtsb_dist_any_input is on, and ignores it otherwise. */
 int gtsb_force_general_build(gtsb_context *ctx, int on);
 
 /* ---- inputs.  *_host variants copy from host memory (H2D on the context's
@@ -256,13 +257,25 @@ int gtsb_pipeline(gtsb_context *ctx, float copy_num_cutoff, float astat_cutoff, 
    edges stay with their rank (gtsb_get_edges).  The exchanges are NCCL over
    NVLink; the 128-byte id from rank 0 has to reach every rank by the caller's
    own means (MPI, torch.distributed, a file).
-   The partitioned build is the line-ordered one only: a contig heading lines on two ranks, a
-   line of more than 64 records, or a link listed only on the later of its two lines fails
+   By default the partitioned build is the line-ordered one only: a contig heading lines on two
+   ranks, a line of more than 64 records, or a link listed only on the later of its two lines fails
    gtsb_pipeline on EVERY rank with the reason mask in the message (a single device rebuilds such
-   input with its general sort-based path; the partitioned build has none).  An error on one
+   input with its general sort-based path).  gtsb_dist_any_input lifts this.  An error on one
    rank -- also an allocation failure -- reaches all ranks at the next agreed exchange. */
 int gtsb_dist_unique_id(void *id128);
 int gtsb_dist_init(gtsb_context *ctx, int rank, int world, const void *id128);
+/* Any record input on a partitioned graph (default off).  With it on, gtsb_pipeline still tries the
+   line-ordered partitioned build first; where that build would fail with a reason mask, every rank
+   rebuilds the same records with the general (sort-based) build spread over the ranks, and the
+   filter runs as before.  The records may then be ANY contiguous slices of the file's records,
+   ranks in file order: lines may be split between ranks and slices may be empty.  The results are
+   the single device's: edges by eid through gtsb_get_edges, vertex states complete on every rank,
+   digests that add up to the one-device digest.  gtsb_get_stats reports line_ordered_build = 0, the
+   reason mask agreed by the ranks (0 under gtsb_force_general_build, which now skips the
+   line-ordered attempt) and the large buckets of all ranks.  Every rank must pass the same value
+   (and the same gtsb_force_general_build); if they differ, gtsb_pipeline fails on every rank.  On
+   one device the switch has no effect: gtsb_build takes any input. */
+int gtsb_dist_any_input(gtsb_context *ctx, int on);
 /* this device's edges with the reference's vertex ids: eid = index into
    graph->edges[] (creation order; within a vertex, adjacency order = eid order) */
 int gtsb_get_edges(gtsb_context *ctx, uint64_t *nof_edges, uint32_t *eid, uint32_t *src, uint32_t *dst,
