@@ -40,6 +40,7 @@ EXPORTS = [
     "gtsb_dot_vertex_lines_host", "gtsb_dot_edge_lines_host", "gtsb_scaf_lines_host", "gtsb_result_digest", "gtsb_components", "gtsb_set_vertices_slice_host", "gtsb_mle_host",
     "gtsb_de_stream_begin", "gtsb_astat_stream_begin", "gtsb_stream_feed", "gtsb_de_stream_end",
     "gtsb_astat_stream_end", "gtsb_stream_set_slot", "gtsb_dist_any_input",
+    "gtsb_dist_de_stream_begin", "gtsb_dist_astat_stream_begin",
 ]
 
 
@@ -112,6 +113,8 @@ def load_library():
     L.gtsb_parse_astat_host.argtypes = [vp, C.c_char_p, u64, vp, vp, C.POINTER(C.c_uint32)]
     L.gtsb_de_stream_begin.argtypes = [vp]
     L.gtsb_astat_stream_begin.argtypes = [vp, vp, vp]
+    L.gtsb_dist_de_stream_begin.argtypes = [vp]
+    L.gtsb_dist_astat_stream_begin.argtypes = [vp, vp, vp]
     L.gtsb_stream_feed.argtypes = [vp, vp, u64, C.POINTER(C.c_uint32)]
     L.gtsb_de_stream_end.argtypes = [vp, C.POINTER(u64), C.POINTER(C.c_uint32)]
     L.gtsb_astat_stream_end.argtypes = [vp, vp, vp, C.POINTER(C.c_uint32)]
@@ -209,10 +212,57 @@ def shard_records(inp, world: int, rank: int):
                      meta=dict(inp.meta, shard=(rank, world, lo, hi)), **kw)
 
 
-def _piece_root(text: bytes, s: int, e: int):
-    """First ' '-separated token of the fgets piece [s, e) (its last character dropped), or None."""
-    tok = text[s:e - 1].lstrip(b" ").split(b" ", 1)[0]
+def _piece_root(piece: bytes):
+    """First ' '-separated token of an fgets piece without its last character, or None."""
+    tok = piece.lstrip(b" ").split(b" ", 1)[0]
     return tok or None
+
+
+_SCAN = 1 << 16          # bytes the cut search reads at a time
+
+
+def _find_nl(read, n: int, i: int) -> int:
+    """offset of the first '\n' at or after i, or -1"""
+    while i < n:
+        blk = read(i, min(n, i + _SCAN))
+        k = blk.find(b"\n")
+        if k >= 0:
+            return i + k
+        i += len(blk)
+    return -1
+
+
+def _rfind_nl(read, j: int) -> int:
+    """offset of the last '\n' before j, or -1"""
+    while j > 0:
+        a = max(0, j - _SCAN)
+        k = read(a, j).rfind(b"\n")
+        if k >= 0:
+            return a + k
+        j = a
+    return -1
+
+
+def _shard(read, n: int, world: int, rank: int, mail_weight: float):
+    """The cut search of shard_text over a byte-range reader: read(a, b) -> bytes [a, b) of the n-byte
+    text.  It reads only bytes near the cuts and the tail of the text."""
+    end = _rfind_nl(read, n) + 1                                  # cuts lie in [0, end]
+    fr = chunk_fractions(world, mail_weight)
+    cuts = [0]
+    for r in range(1, world):
+        i = max(min(int(n * fr[r]), end), cuts[-1])
+        if i > 0 and read(i - 1, i) != b"\n":
+            i = _find_nl(read, n, i) + 1 or end
+        while 0 < i < end:
+            s = _rfind_nl(read, i - 1) + 1                        # start of the line that ends at i
+            last = _piece_root(read(s + (i - 1 - s) // 1023 * 1023, i - 1))
+            nxt = _find_nl(read, n, i)
+            if last is None or last != _piece_root(read(i, min(i + 1023, nxt + 1) - 1)):
+                break
+            i = nxt + 1
+        cuts.append(i)
+    cuts.append(n)
+    return cuts[rank], cuts[rank + 1]
 
 
 def shard_text(text: bytes, world: int, rank: int, mail_weight: float = MAIL_WEIGHT):
@@ -221,24 +271,32 @@ def shard_text(text: bytes, world: int, rank: int, mail_weight: float = MAIL_WEI
     they keep moving while the root of the line after the cut equals the root of the last fgets
     piece (<= 1023 characters) before it, so that a run of one root's lines stays on one rank.  A
     last line without '\n' is never cut off from the last rank.  mail_weight=0 for .astat text."""
-    n = len(text)
-    end = n if text.endswith(b"\n") else text.rfind(b"\n") + 1       # cuts lie in [0, end]
-    fr = chunk_fractions(world, mail_weight)
-    cuts = [0]
-    for r in range(1, world):
-        i = max(min(int(n * fr[r]), end), cuts[-1])
-        if i > 0 and text[i - 1:i] != b"\n":
-            i = text.find(b"\n", i) + 1 or end
-        while 0 < i < end:
-            s = text.rfind(b"\n", 0, i - 1) + 1                  # start of the line that ends at i
-            last = _piece_root(text, s + (i - 1 - s) // 1023 * 1023, i)
-            nxt = text.find(b"\n", i)
-            if last is None or last != _piece_root(text, i, min(i + 1023, nxt + 1)):
-                break
-            i = nxt + 1
-        cuts.append(i)
-    cuts.append(n)
-    return cuts[rank], cuts[rank + 1]
+    return _shard(lambda a, b: text[a:b], len(text), world, rank, mail_weight)
+
+
+def shard_file(path, world: int, rank: int, mail_weight: float = MAIL_WEIGHT):
+    """shard_text(open(path, "rb").read(), world, rank, mail_weight) without reading the file: only
+    the bytes around the cuts and the file's tail are read.  Every rank finds its own [lo, hi)."""
+    with open(path, "rb") as f:
+        n = f.seek(0, os.SEEK_END)
+
+        def read(a, b):
+            f.seek(a)
+            return f.read(b - a)
+
+        return _shard(read, n, world, rank, mail_weight)
+
+
+def read_pieces(path, lo: int, hi: int, piece: int = 1 << 26):
+    """The bytes [lo, hi) of a file, `piece` bytes at a time (for parse_*_pieces)."""
+    with open(path, "rb") as f:
+        f.seek(lo)
+        while lo < hi:
+            b = f.read(min(piece, hi - lo))
+            if not b:
+                raise EOFError(f"{path}: ends at {lo}, before {hi}")
+            lo += len(b)
+            yield b
 
 
 class ScaffoldGraphB200:
@@ -319,15 +377,31 @@ class ScaffoldGraphB200:
                                               C.byref(irr)))
         return int(irr.value), a, cn
 
-    def _feed(self, pieces):
-        """pieces -> gtsb_stream_feed until the stream is refused; -> the IRR_* bits so far"""
+    def _stream(self, begin, pieces, end):
+        """begin(), pieces -> gtsb_stream_feed until the stream is refused, end(irr).  On a partitioned
+        context every rank must reach the collective end: a failed begin or feed leaves the stream
+        failed (the end then fails on every rank), and an exception of `pieces` fails the stream with
+        a null feed before the end."""
+        dist = getattr(self, "world", 1) > 1
         irr = C.c_uint32(0)
-        for piece in pieces:
-            b = np.frombuffer(piece, np.uint8)
-            self._ck(self.L.gtsb_stream_feed(self.h, _ptr(b) if len(b) else None, C.c_uint64(len(b)), C.byref(irr)))
-            if irr.value:
-                break
-        return irr
+        rc = begin()
+        if not dist:
+            self._ck(rc)
+        try:
+            for piece in pieces if rc == 0 else ():
+                b = np.frombuffer(piece, np.uint8)
+                rc = self.L.gtsb_stream_feed(self.h, _ptr(b) if len(b) else None, C.c_uint64(len(b)), C.byref(irr))
+                if rc != 0 and not dist:
+                    self._ck(rc)
+                if rc != 0 or irr.value:
+                    break
+        except BaseException:
+            if dist:
+                self.L.gtsb_stream_feed(self.h, None, C.c_uint64(1), C.byref(irr))
+                end(irr)
+            raise
+        self._ck(end(irr))
+        return int(irr.value)
 
     def parse_de_pieces(self, pieces):
         """parse_de for a text given as consecutive pieces, cut anywhere (any iterable of bytes-like
@@ -337,23 +411,31 @@ class ScaffoldGraphB200:
             with open(path, "rb") as f:
                 irr, R = g.parse_de_pieces(iter(lambda: f.read(1 << 26), b""))
 
-        Single-device contexts only."""
-        self._ck(self.L.gtsb_de_stream_begin(self.h))
-        irr = self._feed(pieces)
+        On a partitioned context (dist_init) every rank streams its own chunk and the end is
+        collective, as parse_de on chunks; no rank needs the whole file:
+
+            lo, hi = shard_file(path, world, rank)
+            irr, R = g.parse_de_pieces(read_pieces(path, lo, hi))"""
         R = C.c_uint64(0)
-        self._ck(self.L.gtsb_de_stream_end(self.h, C.byref(R), C.byref(irr)))
+        dist = getattr(self, "world", 1) > 1
+        begin = self.L.gtsb_dist_de_stream_begin if dist else self.L.gtsb_de_stream_begin
+        irr = self._stream(lambda: begin(self.h), pieces,
+                           lambda irr: self.L.gtsb_de_stream_end(self.h, C.byref(R), C.byref(irr)))
         self.R = int(R.value)
-        return int(irr.value), int(R.value)
+        return irr, int(R.value)
 
     def parse_astat_pieces(self, pieces, astat, copy_num):
         """parse_astat for a text given as consecutive pieces (see parse_de_pieces) -> (irregular
-        bits, astat, copy_num); irregular != 0: the copies are the inputs, untouched."""
+        bits, astat, copy_num); irregular != 0: the copies are the inputs, untouched.  On a partitioned
+        context every rank streams its own chunk (shard_file with mail_weight=0) with the full arrays;
+        all ranks get the same values, the last line in file order winning."""
         a = np.array(astat, np.float32)
         cn = np.array(copy_num, np.float32)
-        self._ck(self.L.gtsb_astat_stream_begin(self.h, _ptr(a), _ptr(cn)))
-        irr = self._feed(pieces)
-        self._ck(self.L.gtsb_astat_stream_end(self.h, _ptr(a), _ptr(cn), C.byref(irr)))
-        return int(irr.value), a, cn
+        dist = getattr(self, "world", 1) > 1
+        begin = self.L.gtsb_dist_astat_stream_begin if dist else self.L.gtsb_astat_stream_begin
+        irr = self._stream(lambda: begin(self.h, _ptr(a), _ptr(cn)), pieces,
+                           lambda irr: self.L.gtsb_astat_stream_end(self.h, _ptr(a), _ptr(cn), C.byref(irr)))
+        return irr, a, cn
 
     def set_stream_slot(self, nbytes: int):
         """Bytes of one staging slot of the *_pieces calls (default 64 MiB)."""

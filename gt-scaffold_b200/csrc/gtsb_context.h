@@ -47,6 +47,12 @@ struct TextStream {
   uint64_t fill = 0;               // bytes in host[]
   uint64_t file_off = 0;           // file offset of host[0]
   uint32_t irregular = 0;          // IRR_* bits found so far; != 0: refused, no more device work
+  uint64_t fed = 0;                // bytes fed so far
+  char last_byte = 0;              // the last of them
+  // opened by gtsb_dist_*_stream_begin: the end is collective.  An error there leaves the stream
+  // failed instead of closing it, with this rank's message; the end reports it on every rank.
+  bool partitioned = false, failed = false;
+  std::string fail_msg;
   DevBuf text;                     // two device slots of `slot` bytes, steps alternate
   int next = 0;                    // device slot of the next step
   DevBuf line_end, line_off, flags;   // the line index of one step; flags[0] = IRR_* bits
@@ -184,6 +190,13 @@ int astat_last(gtsb_context *c, const char *text, uint64_t n, const float *astat
 int astat_apply(gtsb_context *c, uint64_t nlines);
 void text_stream_release(gtsb_context *c);      // gtsb_destroy
 void release(DevBuf &b);
+// the ends of a stream (gtsb_parse.cu), shared by the single-device and the partitioned ones
+int stream_end_local(gtsb_context *c, const char *what, int kind);
+void stream_close(gtsb_context *c);
+void adopt_stream_records(gtsb_context *c, uint64_t R);
+// a partitioned stream's end (gtsb_dist.cu, collective)
+int dist_de_stream_end(gtsb_context *c, uint64_t *nof_records, uint32_t *irregular);
+int dist_astat_stream_end(gtsb_context *c, float *astat, float *copy_num, uint32_t *irregular);
 
 }  // namespace gtsbi
 

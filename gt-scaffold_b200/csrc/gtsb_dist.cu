@@ -22,6 +22,7 @@
 //           vertex states                           allreduce(max), 1 B/vertex
 //   .astat  key of the winning line (rank, offset)  allreduce(max), 8 B/vertex
 //           the winners' values (u32 bit patterns)  allreduce(sum), 8 B/vertex
+//             (the same for a partitioned stream's end; its feeds exchange nothing)
 //
 // With gtsb_dist_any_input on, input the line-ordered build refuses (its FB_* reason mask is
 // agreed at the exchange where it shows) is rebuilt by the general build of gtsb_build.cu spread
@@ -349,19 +350,21 @@ __global__ void __launch_bounds__(256) k_digest_vertices(uint64_t V, const uint8
 }
 
 // `.astat` text over the ranks: the last line in FILE order wins.  A vertex named on this rank has the
-// key (rank << 32 | offset + 1 of its last piece here), 0 elsewhere; the maximum over the ranks is the
-// winner's key (offsets are below 2^32: a chunk is smaller than 4 GiB).
+// key (rank << 56 | offset + 1 of its last piece here), 0 elsewhere; the maximum over the ranks is the
+// winner's key.  Offsets are below 2^56: a single call's chunk is smaller than 4 GiB, a stream's end
+// refuses a chunk of 2^56 bytes or more.
+constexpr int ASTAT_KEY_SHIFT = 56;
 __global__ void k_dist_astat_keys(uint64_t V, uint32_t rank, const uint64_t *__restrict__ last,
                                   uint64_t *__restrict__ key) {
   const uint64_t v = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x;
-  if (v < V) key[v] = last[v] ? ((uint64_t) rank << 32 | last[v]) : 0ull;
+  if (v < V) key[v] = last[v] ? ((uint64_t) rank << ASTAT_KEY_SHIFT | last[v]) : 0ull;
 }
 
 // a local last line that a later line beat is forgotten, so that kp_astat<apply> writes winners only
 __global__ void k_dist_astat_winners(uint64_t V, uint32_t rank, const uint64_t *__restrict__ key,
                                      uint64_t *__restrict__ last) {
   const uint64_t v = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x;
-  if (v < V && last[v] && key[v] != ((uint64_t) rank << 32 | last[v])) last[v] = 0;
+  if (v < V && last[v] && key[v] != ((uint64_t) rank << ASTAT_KEY_SHIFT | last[v])) last[v] = 0;
 }
 
 // the winner's two values as bit patterns, zero on every other rank: a sum over the ranks delivers them
@@ -1653,12 +1656,47 @@ int dist_parse_de(gtsb_context *c, const char *text, uint64_t n, uint64_t *nof_r
   return 0;
 }
 
+// `.astat` over the ranks, once they agree, on this rank's last[] (offset + 1 of its last piece
+// naming v, 0 for none) and values: keys -> allreduce(max) -> winners -> apply -> pack ->
+// allreduce(sum) -> unpack, then the values to the host arrays, identical on every rank.  apply_lines:
+// the lines of the single call, whose kp_astat<apply> writes the pieces this rank won; a stream has
+// applied each step's last pieces as it went, its winners' values are in place (0 lines).
+int astat_over_ranks(gtsb_context *c, uint64_t *last, float *d_astat, float *d_copy_num, uint64_t apply_lines,
+                     float *astat, float *copy_num) {
+  DistState *D = static_cast<DistState *>(c->dstate);
+  cudaStream_t s = c->stream;
+  const uint64_t V = c->names_V;
+  uint64_t *key = c->p_key.as<uint64_t>();
+  uint32_t *win = c->p_win.as<uint32_t>();
+  const uint32_t blocks = (uint32_t) ((V + 255) / 256), me = (uint32_t) c->rank;
+  if (V) {
+    KernelTimer t_("k_dist_astat(winners)+allreduce", s);
+    k_dist_astat_keys<<<blocks, 256, 0, s>>>(V, me, last, key);
+    NK(g_nccl.AllReduce(key, key, V, ncclUint64, ncclMax, D->comm, s));
+    k_dist_astat_winners<<<blocks, 256, 0, s>>>(V, me, key, last);
+    c->stats.kernel_launches += 2;
+  }
+  if (astat_apply(c, apply_lines) != 0) return -1;
+  if (V) {
+    KernelTimer t_("k_dist_astat(values)+allreduce", s);
+    k_dist_astat_pack<<<blocks, 256, 0, s>>>(V, last, d_astat, d_copy_num, win);
+    NK(g_nccl.AllReduce(win, win, 2 * V, ncclUint32, ncclSum, D->comm, s));
+    k_dist_astat_unpack<<<blocks, 256, 0, s>>>(V, key, win, d_astat, d_copy_num);
+    c->stats.kernel_launches += 2;
+  }
+  if (V) {
+    CK(cudaMemcpyAsync(astat, d_astat, V * 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(copy_num, d_copy_num, V * 4, cudaMemcpyDeviceToHost, s));
+  }
+  CK(cudaStreamSynchronize(s));
+  CK(cudaGetLastError());
+  return 0;
+}
+
 int dist_parse_astat(gtsb_context *c, const char *text, uint64_t n, float *astat, float *copy_num,
                      uint32_t *irregular_out) {
   const char *what = "gtsb_parse_astat_host";
-  DistState *D = static_cast<DistState *>(c->dstate);
   ProfScope prof(c);
-  cudaStream_t s = c->stream;
   const uint64_t V = c->names_V;
   uint64_t nlines = 0;
   uint32_t irregular = 0;
@@ -1681,31 +1719,65 @@ int dist_parse_astat(gtsb_context *c, const char *text, uint64_t n, float *astat
     *irregular_out = irr;
     return 0;
   }
-  uint64_t *last = c->p_last.as<uint64_t>(), *key = c->p_key.as<uint64_t>();
-  uint32_t *win = c->p_win.as<uint32_t>();
-  const uint32_t blocks = (uint32_t) ((V + 255) / 256), me = (uint32_t) c->rank;
-  if (V) {
-    KernelTimer t_("k_dist_astat(winners)+allreduce", s);
-    k_dist_astat_keys<<<blocks, 256, 0, s>>>(V, me, last, key);
-    NK(g_nccl.AllReduce(key, key, V, ncclUint64, ncclMax, D->comm, s));
-    k_dist_astat_winners<<<blocks, 256, 0, s>>>(V, me, key, last);
-    c->stats.kernel_launches += 2;
+  return astat_over_ranks(c, c->p_last.as<uint64_t>(), c->p_astat.as<float>(), c->p_copy_num.as<float>(), nlines,
+                          astat, copy_num);
+}
+
+// ---- `.de` / `.astat` text fed in pieces, every rank its own chunk (gtsb_dist_*_stream_begin):
+// feeding is local, the end is collective and agrees as the single calls do
+
+int dist_de_stream_end(gtsb_context *c, uint64_t *nof_records, uint32_t *irregular_out) {
+  const char *what = "gtsb_de_stream_end";
+  ProfScope prof(c);
+  const int rc = [&]() -> int {
+    if (nof_records == nullptr || irregular_out == nullptr) return fail(c, "%s: null argument", what);
+    if (stream_end_local(c, what, TextStream::DE) != 0) return -1;
+    bool unused = false;
+    return injected_failure(c, "stream", unused);
+  }();
+  const uint32_t irregular = c->ts.irregular;
+  const uint64_t R = c->ts.R;
+  stream_close(c);
+  if (nof_records != nullptr) *nof_records = 0;
+  if (irregular_out != nullptr) *irregular_out = 0;
+  uint32_t irr = 0;
+  if (dist_text_agree(c, rc, what, irregular, &irr) != 0) return -1;
+  if (irr) {                           // a refusal anywhere: no rank keeps records (begin dropped the old ones)
+    *irregular_out = irr;
+    return 0;
   }
-  if (astat_apply(c, nlines) != 0) return -1;
-  if (V) {
-    KernelTimer t_("k_dist_astat(values)+allreduce", s);
-    k_dist_astat_pack<<<blocks, 256, 0, s>>>(V, last, c->p_astat.as<float>(), c->p_copy_num.as<float>(), win);
-    NK(g_nccl.AllReduce(win, win, 2 * V, ncclUint32, ncclSum, D->comm, s));
-    k_dist_astat_unpack<<<blocks, 256, 0, s>>>(V, key, win, c->p_astat.as<float>(), c->p_copy_num.as<float>());
-    c->stats.kernel_launches += 2;
-  }
-  if (V) {
-    CK(cudaMemcpyAsync(astat, c->p_astat.p, V * 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(copy_num, c->p_copy_num.p, V * 4, cudaMemcpyDeviceToHost, s));
-  }
-  CK(cudaStreamSynchronize(s));
-  CK(cudaGetLastError());
+  adopt_stream_records(c, R);
+  *nof_records = R;
   return 0;
+}
+
+int dist_astat_stream_end(gtsb_context *c, float *astat, float *copy_num, uint32_t *irregular_out) {
+  const char *what = "gtsb_astat_stream_end";
+  const uint64_t V = c->names_V;
+  ProfScope prof(c);
+  const int rc = [&]() -> int {
+    if (irregular_out == nullptr || (V && (astat == nullptr || copy_num == nullptr)))
+      return fail(c, "%s: null argument", what);
+    if (stream_end_local(c, what, TextStream::ASTAT) != 0) return -1;
+    if (c->ts.fed >> ASTAT_KEY_SHIFT) return fail(c, "%s: a chunk of 2^%d bytes or more", what, ASTAT_KEY_SHIFT);
+    ENSURE(c->p_key, (V + 1) * 8);
+    ENSURE(c->p_win, (V + 1) * 8);
+    bool unused = false;
+    return injected_failure(c, "stream", unused);
+  }();
+  const uint32_t irregular = c->ts.irregular;
+  stream_close(c);
+  if (irregular_out != nullptr) *irregular_out = 0;
+  uint32_t irr = 0;
+  if (dist_text_agree(c, rc, what, irregular, &irr) != 0) return -1;
+  if (irr) {                           // a refusal anywhere: no rank touches the arrays
+    *irregular_out = irr;
+    return 0;
+  }
+  // the stream's steps have applied this rank's last pieces already: nothing left to apply
+  TextStream &ts = c->ts;
+  return astat_over_ranks(c, ts.last.as<uint64_t>(), ts.astat.as<float>(), ts.copy_num.as<float>(), 0, astat,
+                          copy_num);
 }
 
 }  // namespace gtsbi

@@ -425,6 +425,24 @@ int gtsb_get_records(gtsb_context *c, uint32_t *root, uint32_t *ctg, int32_t *di
 //      .astat: kp_astat_at(last line) + kp_astat_at(apply), so later steps overwrite earlier winners
 // The host fills the pinned slot again while C and B run, and the next copy runs beside them; two
 // device slots alternate, a copy waits for the kernels that read its slot.
+//
+// On a partitioned context (gtsb_dist_*_stream_begin) every rank streams its own chunk the same way;
+// only the end is collective (gtsb_dist.cu, dist_*_stream_end).
+namespace gtsbi {
+
+void stream_close(gtsb_context *c) {
+  TextStream &ts = c->ts;
+  ts.kind = TextStream::CLOSED;
+  ts.fill = ts.file_off = ts.R = ts.fed = 0;
+  ts.last_byte = 0;
+  ts.irregular = 0;
+  ts.pending = false;
+  ts.partitioned = ts.failed = false;
+  ts.fail_msg.clear();
+}
+
+}  // namespace gtsbi
+
 namespace gtsbparse {
 
 constexpr uint64_t STREAM_MIN_SLOT = 4096, STREAM_MAX_SLOT = 1ull << 30;
@@ -440,12 +458,17 @@ static uint64_t step_cut(const char *b, uint64_t n) {
   return ls + (n - ls) / PIECE * PIECE;
 }
 
-static void stream_close(gtsb_context *c) {
+// an error in a stream: a single-device stream closes; a partitioned one keeps this rank's message
+// and fails every later feed, and its end still joins the other ranks' to report it everywhere
+static int stream_error(gtsb_context *c) {
   TextStream &ts = c->ts;
-  ts.kind = TextStream::CLOSED;
-  ts.fill = ts.file_off = ts.R = 0;
-  ts.irregular = 0;
-  ts.pending = false;
+  if (!ts.partitioned) {
+    stream_close(c);
+    return -1;
+  }
+  ts.failed = true;
+  ts.fail_msg = c->err;
+  return -1;
 }
 
 // b holds `used` bytes: room for `need` (doubling), the bytes kept
@@ -582,12 +605,16 @@ static int stream_step(gtsb_context *c, uint64_t n) {
   return 0;
 }
 
-// what both begins share: a discarded open stream, the checks, the staging memory
-static int stream_prepare(gtsb_context *c, const char *what) {
+// what every begin shares: a discarded open stream, the checks, the staging memory.  plain: for a
+// partitioned begin, the name of the single-device one; nullptr for that one itself.
+static int stream_prepare(gtsb_context *c, const char *what, const char *plain) {
   TextStream &ts = c->ts;
   stream_close(c);                                  // a new begin discards an open stream
-  if (c->world > 1)
-    return fail(c, "%s: a partitioned context reads text with the collective gtsb_parse_*_host calls", what);
+  if (plain == nullptr && c->world > 1)
+    return fail(c, "%s: a partitioned context reads text with the collective gtsb_parse_*_host calls or "
+                   "gtsb_dist_*_stream_begin", what);
+  if (plain != nullptr && c->world == 1)
+    return fail(c, "%s: not a partitioned context (one device reads text in pieces with %s)", what, plain);
   if (!c->have_names) return fail(c, "%s: vertex names not set", what);
   const uint64_t host_bytes = host_tail(ts.slot) + 32;
   if (ts.host != nullptr && ts.host_cap != host_bytes) {
@@ -607,12 +634,43 @@ static int stream_prepare(gtsb_context *c, const char *what) {
   return 0;
 }
 
-// the remaining bytes as the last step, then the synchronisation that reads its results
-static int stream_finish(gtsb_context *c) {
-  TextStream &ts = c->ts;
-  if (ts.irregular == 0 && stream_step(c, ts.fill) != 0) return -1;
-  if (ts.irregular == 0 && stream_step(c, 0) != 0) return -1;
+static int de_begin(gtsb_context *c, const char *what, const char *plain) {
+  if (stream_prepare(c, what, plain) != 0) return -1;
+  if (await_records(c) != 0) return -1;
+  c->have_records = false;                          // as gtsb_parse_de_host: the old records are gone
+  c->have_graph = false;
+  c->ts.kind = TextStream::DE;
+  c->ts.irregular = c->names_dup ? IRR_DUP_NAME : 0;
   return 0;
+}
+
+static int astat_begin(gtsb_context *c, const char *what, const char *plain, const float *astat,
+                       const float *copy_num) {
+  if (stream_prepare(c, what, plain) != 0) return -1;
+  TextStream &ts = c->ts;
+  const uint64_t V = c->names_V;
+  if (V && (astat == nullptr || copy_num == nullptr)) return fail(c, "%s: null argument", what);
+  cudaStream_t s = c->stream;
+  ENSURE(ts.last, (V + 1) * 8);
+  ENSURE(ts.astat, (V + 1) * 4);
+  ENSURE(ts.copy_num, (V + 1) * 4);
+  CK(cudaMemsetAsync(ts.last.p, 0, (V + 1) * 8, s));
+  if (V) {
+    CK(cudaMemcpyAsync(ts.astat.p, astat, V * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(ts.copy_num.p, copy_num, V * 4, cudaMemcpyHostToDevice, s));
+  }
+  ts.kind = TextStream::ASTAT;
+  ts.irregular = c->names_dup ? IRR_DUP_NAME : 0;
+  return 0;
+}
+
+// a partitioned begin is local.  One that fails still leaves a stream open, failed, so that this
+// rank's end joins the other ranks' and the failure reaches all of them.
+static int dist_begun(gtsb_context *c, int rc, int kind) {
+  if (c->world == 1) return rc;                     // refused: nothing is open
+  c->ts.kind = kind;
+  c->ts.partitioned = true;
+  return rc == 0 ? 0 : stream_error(c);
 }
 
 static int stream_end_check(gtsb_context *c, const char *what, int kind) {
@@ -626,6 +684,42 @@ static int stream_end_check(gtsb_context *c, const char *what, int kind) {
 }  // namespace gtsbparse
 
 namespace gtsbi {
+
+// what every end does on its own device: a partitioned stream's failure and chunk rule, then the
+// remaining bytes as the last step and the synchronisation that reads its results (ts.irregular and
+// ts.R are the stream's), and record columns that exist, so that adopting them cannot fail
+int stream_end_local(gtsb_context *c, const char *what, int kind) {
+  TextStream &ts = c->ts;
+  if (ts.kind != kind)
+    return fail(c, "%s: the open stream reads %s text", what, ts.kind == TextStream::DE ? ".de" : ".astat");
+  if (ts.failed) {
+    c->err = ts.fail_msg;
+    return -1;
+  }
+  // as dist_text_checks: the fgets pieces of the chunks are those of the whole file only if every
+  // chunk but the last ends a line.  A refused stream is exempt: its caller may stop feeding.
+  if (c->rank < c->world - 1 && ts.irregular == 0 && ts.fed != 0 && ts.last_byte != '\n')
+    return fail(c, "%s: the chunk of rank %d does not end in '\\n' (only the last rank's may)", what, c->rank);
+  if (ts.irregular == 0 && stream_step(c, ts.fill) != 0) return -1;
+  if (ts.irregular == 0 && stream_step(c, 0) != 0) return -1;
+  if (kind == TextStream::DE)
+    for (DevBuf *b : {&ts.root, &ts.ctg, &ts.dist, &ts.std_dev, &ts.rflags, &ts.num_pairs})
+      if (b->p == nullptr) ENSURE(*b, 16);
+  return 0;
+}
+
+// the stream's columns become the context's records
+void adopt_stream_records(gtsb_context *c, uint64_t R) {
+  TextStream &ts = c->ts;
+  DevBuf *mine[] = {&ts.root, &ts.ctg, &ts.dist, &ts.std_dev, &ts.rflags, &ts.num_pairs};
+  DevBuf *ctx[] = {&c->root, &c->ctg, &c->dist, &c->std_dev, &c->flags, &c->num_pairs};
+  for (int k = 0; k < 6; k++) {
+    release(*ctx[k]);
+    *ctx[k] = *mine[k];
+    *mine[k] = DevBuf();
+  }
+  keep_parsed_records(c, R);
+}
 
 void text_stream_release(gtsb_context *c) {
   TextStream &ts = c->ts;
@@ -655,34 +749,26 @@ int gtsb_stream_set_slot(gtsb_context *c, uint64_t bytes) {
 int gtsb_de_stream_begin(gtsb_context *c) {
   if (c == nullptr) return -1;
   CK(cudaSetDevice(c->device));
-  if (stream_prepare(c, "gtsb_de_stream_begin") != 0) return -1;
-  if (await_records(c) != 0) return -1;
-  c->have_records = false;                          // as gtsb_parse_de_host: the old records are gone
-  c->have_graph = false;
-  c->ts.kind = TextStream::DE;
-  c->ts.irregular = c->names_dup ? IRR_DUP_NAME : 0;
-  return 0;
+  return de_begin(c, "gtsb_de_stream_begin", nullptr);
 }
 
 int gtsb_astat_stream_begin(gtsb_context *c, const float *astat, const float *copy_num) {
   if (c == nullptr) return -1;
   CK(cudaSetDevice(c->device));
-  if (stream_prepare(c, "gtsb_astat_stream_begin") != 0) return -1;
-  TextStream &ts = c->ts;
-  const uint64_t V = c->names_V;
-  if (V && (astat == nullptr || copy_num == nullptr)) return fail(c, "gtsb_astat_stream_begin: null argument");
-  cudaStream_t s = c->stream;
-  ENSURE(ts.last, (V + 1) * 8);
-  ENSURE(ts.astat, (V + 1) * 4);
-  ENSURE(ts.copy_num, (V + 1) * 4);
-  CK(cudaMemsetAsync(ts.last.p, 0, (V + 1) * 8, s));
-  if (V) {
-    CK(cudaMemcpyAsync(ts.astat.p, astat, V * 4, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(ts.copy_num.p, copy_num, V * 4, cudaMemcpyHostToDevice, s));
-  }
-  ts.kind = TextStream::ASTAT;
-  ts.irregular = c->names_dup ? IRR_DUP_NAME : 0;
-  return 0;
+  return astat_begin(c, "gtsb_astat_stream_begin", nullptr, astat, copy_num);
+}
+
+int gtsb_dist_de_stream_begin(gtsb_context *c) {
+  if (c == nullptr) return -1;
+  CK(cudaSetDevice(c->device));
+  return dist_begun(c, de_begin(c, "gtsb_dist_de_stream_begin", "gtsb_de_stream_begin"), TextStream::DE);
+}
+
+int gtsb_dist_astat_stream_begin(gtsb_context *c, const float *astat, const float *copy_num) {
+  if (c == nullptr) return -1;
+  CK(cudaSetDevice(c->device));
+  return dist_begun(c, astat_begin(c, "gtsb_dist_astat_stream_begin", "gtsb_astat_stream_begin", astat, copy_num),
+                    TextStream::ASTAT);
 }
 
 int gtsb_stream_feed(gtsb_context *c, const char *bytes, uint64_t n, uint32_t *irregular) {
@@ -690,9 +776,17 @@ int gtsb_stream_feed(gtsb_context *c, const char *bytes, uint64_t n, uint32_t *i
   CK(cudaSetDevice(c->device));
   TextStream &ts = c->ts;
   if (ts.kind == TextStream::CLOSED) return fail(c, "gtsb_stream_feed: no open stream");
+  if (ts.failed) {                                  // a partitioned stream after an error: no device work
+    c->err = ts.fail_msg;
+    return -1;
+  }
   if (irregular == nullptr || (n && bytes == nullptr)) {
-    stream_close(c);
-    return fail(c, "gtsb_stream_feed: null argument");
+    fail(c, "gtsb_stream_feed: null argument");
+    return stream_error(c);
+  }
+  if (n) {
+    ts.fed += n;
+    ts.last_byte = bytes[n - 1];
   }
   ProfScope prof(c);
   while (n && ts.irregular == 0) {
@@ -703,10 +797,7 @@ int gtsb_stream_feed(gtsb_context *c, const char *bytes, uint64_t n, uint32_t *i
     n -= take;
     if (ts.fill < ts.slot) break;
     const uint64_t cut = step_cut(ts.host, ts.fill);
-    if (stream_step(c, cut) != 0) {
-      stream_close(c);
-      return -1;
-    }
+    if (stream_step(c, cut) != 0) return stream_error(c);
     memmove(ts.host, ts.host + cut, ts.fill - cut);
     ts.file_off += cut;
     ts.fill -= cut;
@@ -718,6 +809,7 @@ int gtsb_stream_feed(gtsb_context *c, const char *bytes, uint64_t n, uint32_t *i
 int gtsb_de_stream_end(gtsb_context *c, uint64_t *nof_records, uint32_t *irregular) {
   if (c == nullptr) return -1;
   CK(cudaSetDevice(c->device));
+  if (c->ts.partitioned) return dist_de_stream_end(c, nof_records, irregular);
   if (stream_end_check(c, "gtsb_de_stream_end", TextStream::DE) != 0) return -1;
   TextStream &ts = c->ts;
   if (nof_records == nullptr || irregular == nullptr) {
@@ -727,7 +819,7 @@ int gtsb_de_stream_end(gtsb_context *c, uint64_t *nof_records, uint32_t *irregul
   ProfScope prof(c);
   *nof_records = 0;
   *irregular = 0;
-  const int rc = stream_finish(c);
+  const int rc = stream_end_local(c, "gtsb_de_stream_end", TextStream::DE);
   const uint32_t irr = ts.irregular;
   const uint64_t R = ts.R;
   stream_close(c);
@@ -736,16 +828,7 @@ int gtsb_de_stream_end(gtsb_context *c, uint64_t *nof_records, uint32_t *irregul
     *irregular = irr;
     return 0;
   }
-  // the stream's columns become the context's records
-  DevBuf *mine[] = {&ts.root, &ts.ctg, &ts.dist, &ts.std_dev, &ts.rflags, &ts.num_pairs};
-  DevBuf *ctx[] = {&c->root, &c->ctg, &c->dist, &c->std_dev, &c->flags, &c->num_pairs};
-  for (int k = 0; k < 6; k++) {
-    if (mine[k]->p == nullptr) ENSURE(*mine[k], 16);
-    release(*ctx[k]);
-    *ctx[k] = *mine[k];
-    *mine[k] = DevBuf();
-  }
-  keep_parsed_records(c, R);
+  adopt_stream_records(c, R);
   *nof_records = R;
   return 0;
 }
@@ -753,6 +836,7 @@ int gtsb_de_stream_end(gtsb_context *c, uint64_t *nof_records, uint32_t *irregul
 int gtsb_astat_stream_end(gtsb_context *c, float *astat, float *copy_num, uint32_t *irregular) {
   if (c == nullptr) return -1;
   CK(cudaSetDevice(c->device));
+  if (c->ts.partitioned) return dist_astat_stream_end(c, astat, copy_num, irregular);
   if (stream_end_check(c, "gtsb_astat_stream_end", TextStream::ASTAT) != 0) return -1;
   TextStream &ts = c->ts;
   const uint64_t V = c->names_V;
@@ -762,7 +846,7 @@ int gtsb_astat_stream_end(gtsb_context *c, float *astat, float *copy_num, uint32
   }
   ProfScope prof(c);
   *irregular = 0;
-  const int rc = stream_finish(c);
+  const int rc = stream_end_local(c, "gtsb_astat_stream_end", TextStream::ASTAT);
   const uint32_t irr = ts.irregular;
   stream_close(c);
   if (rc != 0) return -1;

@@ -171,8 +171,10 @@ int gtsb_parse_de_host(gtsb_context *ctx, const char *text, uint64_t text_bytes,
 int gtsb_parse_astat_host(gtsb_context *ctx, const char *text, uint64_t text_bytes, float *astat,
                           float *copy_num, uint32_t *irregular);
 /* ---- the same two readings for text fed in pieces: no size limit, bounded memory, and the copy of
-   each piece overlapping the kernels of the piece before.  Single-device contexts only: begin on a
-   partitioned context (after gtsb_dist_init) fails, ranks keep using the collective calls above.
+   each piece overlapping the kernels of the piece before.  gtsb_de_stream_begin /
+   gtsb_astat_stream_begin take single-device contexts only: on a partitioned context (after
+   gtsb_dist_init) they fail, and ranks use the collective calls above or the partitioned stream
+   below.
 
      gtsb_de_stream_begin / gtsb_astat_stream_begin   open a stream (an open one is discarded)
      gtsb_stream_feed     the next bytes of the file
@@ -191,7 +193,7 @@ int gtsb_parse_astat_host(gtsb_context *ctx, const char *text, uint64_t text_byt
    records are held.  .astat begin takes the initial values (one per vertex of the names set, NULL
    for none); end writes astat / copy_num only when it succeeds with *irregular == 0.
    Errors: feed or end without an open stream, end of the other kind, a null argument, a CUDA or
-   allocation error -- each closes the stream.  gtsb_set_vertex_names_host fails while a stream is
+   allocation error -- each closes a single-device stream.  gtsb_set_vertex_names_host fails while a stream is
    open.  Other calls on the context may run between feeds; the single-call entry points keep
    their own buffers.
    Memory: the stream copies through one pinned host slot and two device slots of 64 MiB
@@ -206,6 +208,28 @@ int gtsb_astat_stream_end(gtsb_context *ctx, float *astat, float *copy_num, uint
 /* bytes of one staging slot (default 64 MiB, 4096 .. 2^30); not while a stream is open.  A step
    of the stream is at most one slot; smaller slots mean more steps (and more synchronisations). */
 int gtsb_stream_set_slot(gtsb_context *ctx, uint64_t bytes);
+/* The partitioned stream: every rank of a partitioned context streams its own chunk of the file,
+   with the chunk rules of gtsb_parse_de_host (consecutive byte ranges in rank order, every chunk but
+   the last rank's ends right after a '\n' or is empty; no 4 GiB limit).
+     gtsb_dist_de_stream_begin / gtsb_dist_astat_stream_begin   LOCAL: open a stream on this rank
+       (on a single-device context they fail, that context uses gtsb_*_stream_begin)
+     gtsb_stream_feed     LOCAL: this rank's next bytes; *irregular = this rank's bits so far.  Ranks
+       may feed different numbers of pieces; nothing is exchanged while feeding.
+     gtsb_de_stream_end / gtsb_astat_stream_end   COLLECTIVE on such a stream: every rank calls it
+       after feeding its chunk, or after feed reported *irregular != 0 (the rest of a refused chunk
+       need not be fed, and the chunk rule is not checked then).  One status exchange carries each rank's error state, IRR_* bits and
+       name-set size.  The results are those of gtsb_parse_de_host / gtsb_parse_astat_host on the same
+       chunks: .de, this rank keeps its chunk's records (gtsb_pipeline follows, the line-ordered build
+       or gtsb_dist_any_input); .astat, the arrays come back identical on every rank, the last line in
+       file order winning.  *irregular is the OR over the ranks; a refusal anywhere keeps no records
+       on any rank and touches no arrays.  An .astat chunk must be below 2^56 bytes.
+   Errors on a partitioned stream do not close it: a failed begin, a null argument, a CUDA or
+   allocation error or the record limit leave it failed, holding this rank's message; later feeds
+   return -1 and do no device work, and the end still joins the exchange, so that it returns -1 on
+   every rank (this rank's message here, "rank k failed" elsewhere).  The next stream works on all
+   ranks.  An end without an open stream fails on this rank alone, as on one device. */
+int gtsb_dist_de_stream_begin(gtsb_context *ctx);
+int gtsb_dist_astat_stream_begin(gtsb_context *ctx, const float *astat, const float *copy_num);
 
 /* the records held by the context, file order (NULL pointers are skipped); num_pairs
    only after gtsb_parse_de_host or gtsb_de_stream_end */
