@@ -47,7 +47,9 @@ enum {
 enum : uint32_t {
   FB_MULTIRUN = 1,        // a root contig heads more than one line
   FB_LONGLINE = 2,        // a line longer than MAX_LINE_RECS records
-  FB_SEGMENT = 4,         // a segment does not fit the staging buffers
+  FB_SEGMENT = 4,         // a segment does not fit the staging buffers, or k2_resolve posted more reverse-flag
+                          // corrections than their list holds (R / 8 + 4096): no reason of its own, since the
+                          // partitioned ranks agree on this mask
   FB_DOWN_ORPHAN = 8      // a link listed only on the later of the two lines
 };
 
