@@ -646,7 +646,7 @@ int do_filter(gtsb_context *c, float pcutoff, float cncutoff, int64_t ocutoff, b
   // phase 1: who proposes whom (+ the static overlap answer of every small row)
   launch_vertex_facts(a, fused ? 1 : 0, cn_cutoff, astat_cutoff, use_cn, s);
   launch_pairs(a, s);
-  c->stats.kernel_launches += (V ? 1 : 0) + (E ? 1 : 0) + (E && c->n_big_rows ? 1 : 0);
+  c->stats.kernel_launches += (V ? 1 : 0) + (E ? 2 : 0) + (E && c->n_big_rows ? 1 : 0);
   if (read_counters(c) != 0) return -1;
   if (c->h_counters[CNT_ERROR] & 4u) return fail(c, "gtsb_filter: a contig is longer than 2^31-1");
   if (c->h_counters[CNT_OVERFLOW] && a.proposals_cap < E + 1) {
@@ -658,7 +658,7 @@ int do_filter(gtsb_context *c, float pcutoff, float cncutoff, int64_t ocutoff, b
     CK(cudaMemsetAsync(cnt + CNT_OVERFLOW, 0, 4, s));
     CK(cudaMemsetAsync(c->gbits.p, 0, V + 1, s));
     launch_pairs(a, s);
-    c->stats.kernel_launches += (E ? 1 : 0) + (E && c->n_big_rows ? 1 : 0);
+    c->stats.kernel_launches += (E ? 2 : 0) + (E && c->n_big_rows ? 1 : 0);
     if (read_counters(c) != 0) return -1;
   }
   if (c->h_counters[CNT_OVERFLOW]) return fail(c, "gtsb_filter: proposal list overflow");
@@ -692,7 +692,7 @@ int do_filter(gtsb_context *c, float pcutoff, float cncutoff, int64_t ocutoff, b
   uint32_t *n_dense = coop ? cnt + CNT_RING0 : cnt + CNT_WORK_B;
   CK(cudaMemsetAsync(n_dense, 0, 4, s));
   launch_fire_init(a, n_dense, s);
-  c->stats.kernel_launches += (V ? 2 : 0) + (V && c->n_big_rows ? 1 : 0);
+  c->stats.kernel_launches += (V ? 1 : 0) + (V && c->n_big_rows ? 1 : 0);
   c->stats.fire_rounds = 0;
   c->fire_ring_pending = false;
   uint32_t *win = a.work_b, *wout = a.work_a;

@@ -74,21 +74,37 @@ struct AmbigParams {
 // Fast path: compare squares in f32 outside a guard band that is wider than the
 // worst-case rounding of both formulations; inside the band fall back to the
 // literal double expression (IEEE div/sqrt => bit-exact with the host).
-__device__ __forceinline__ bool ambiguous_order(int32_t dist1, float s1, int32_t dist2, float s2,
-                                                const AmbigParams &ap) {
+//   ambiguous_order_fast: 1 / 0 where the fast path decides, -1 where only the
+//                         double expression can (the inside of the band, extreme operands)
+//   ambiguous_order:      the decision
+// A caller whose registers are scarce can take the rare -1 cases apart: the
+// double division and square root need many registers.
+__device__ __forceinline__ int ambiguous_order_fast(int32_t dist1, float s1, int32_t dist2, float s2,
+                                                    const AmbigParams &ap) {
   const float expval = __ll2float_rn((long long) dist1 - (long long) dist2);
   const float variance = __fmul_rn(2.0f, __fadd_rn(__fmul_rn(s1, s1), __fmul_rn(s2, s2)));
   const float x = __fsub_rn(0.0f, expval);          // numerator, exact negation
   const bool neg = x < 0.0f;
   const float t = neg ? ap.t_neg : ap.t_pos;
-  if (!(t >= 0.0f)) return false;                   // never ambiguous on this side
+  if (!(t >= 0.0f)) return 0;                       // never ambiguous on this side
   if (t < 3.0e38f && variance > 1.0e-30f && variance < 1.0e30f && fabsf(x) < 1.0e15f) {
     const float lhs = __fmul_rn(x, x);
     const float rhs = __fmul_rn(neg ? ap.c_neg : ap.c_pos, variance);
     const float band = __fmul_rn(rhs, 1.0e-5f);
-    if (lhs < __fsub_rn(rhs, band)) return true;
-    if (lhs > __fadd_rn(rhs, band)) return false;
+    if (lhs < __fsub_rn(rhs, band)) return 1;
+    if (lhs > __fadd_rn(rhs, band)) return 0;
   }
+  return -1;
+}
+
+__device__ __forceinline__ bool ambiguous_order(int32_t dist1, float s1, int32_t dist2, float s2,
+                                                const AmbigParams &ap) {
+  const int fast = ambiguous_order_fast(dist1, s1, dist2, s2, ap);
+  if (fast >= 0) return fast != 0;
+  const float expval = __ll2float_rn((long long) dist1 - (long long) dist2);
+  const float variance = __fmul_rn(2.0f, __fadd_rn(__fmul_rn(s1, s1), __fmul_rn(s2, s2)));
+  const float x = __fsub_rn(0.0f, expval);
+  const bool neg = x < 0.0f;
   const double q = __ddiv_rn((double) x, __dsqrt_rn((double) variance));
   const float interval = __double2float_rn(q);
   if (interval != interval) return false;           // NaN: p_wrong > cutoff is false

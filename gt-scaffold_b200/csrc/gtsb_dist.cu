@@ -1444,7 +1444,7 @@ int dist_filter(gtsb_context *c, DistState *D, const Plan &P, float cn_cutoff, f
   // phase 1: the neighbour facts were computed and gathered under the build (dist_side_facts)
   if (P.facts_on_side) CK(cudaStreamWaitEvent(s, D->ev_join, 0));
   launch_pairs(a, s);
-  c->stats.kernel_launches += 1 + (c->n_big_rows ? 1 : 0);
+  c->stats.kernel_launches += 2 + (c->n_big_rows ? 1 : 0);
   rc = [&]() -> int {
     if (read_counters(c) != 0) return -1;
     if (c->h_counters[CNT_ERROR] & 4u) return fail(c, "gtsb_filter: a contig is longer than 2^31-1");
@@ -1497,7 +1497,7 @@ int dist_filter(gtsb_context *c, DistState *D, const Plan &P, float cn_cutoff, f
   // phase 2
   CK(cudaMemsetAsync(cnt + CNT_WORK_B, 0, 4, s));
   launch_fire_init(a, cnt + CNT_WORK_B, s);
-  c->stats.kernel_launches += 2 + (c->n_big_rows ? 1 : 0);
+  c->stats.kernel_launches += 1 + (c->n_big_rows ? 1 : 0);
   if (allgatherv(c, "nccl_allgather_fstat", c->fstat.p, 1, P.lo) != 0) return -1;
   c->stats.fire_rounds = 0;
   if (ocutoff >= 0) {

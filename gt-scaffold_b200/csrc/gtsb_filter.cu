@@ -271,11 +271,10 @@ __device__ __forceinline__ uint32_t nth_set_bit(uint32_t m, uint32_t r) {
 template <typename Body>
 __device__ __forceinline__ void for_each_pair(uint32_t P, Body body) {
   const uint32_t lane = lane_id();
-  const uint32_t c = __popc(P);
-  const uint32_t incl = warp_incl_scan_u32(c);
-  const uint32_t total = __shfl_sync(FULL, incl, 31);
-  const uint32_t excl = incl - c;
-  for (uint32_t q0 = 0; q0 < total; q0 += 32u) {
+  const uint32_t incl = warp_incl_scan_u32(__popc(P));   // the total and each lane's start are read back by shuffle
+  for (uint32_t q0 = 0;; q0 += 32u) {
+    const uint32_t total = __shfl_sync(FULL, incl, 31);
+    if (q0 >= total) break;
     const uint32_t q = q0 + lane;
     const bool live = q < total;
     uint32_t i = 0;                                // number of lanes with incl <= q = owner of pair q
@@ -285,8 +284,8 @@ __device__ __forceinline__ void for_each_pair(uint32_t P, Body body) {
       if (t <= q) i += step;
     }
     i &= 31u;
-    const uint32_t r = q - __shfl_sync(FULL, excl, i);
     const uint32_t Pi = __shfl_sync(FULL, P, i);
+    const uint32_t r = q - (__shfl_sync(FULL, incl, i) - __popc(Pi));
     const uint32_t j = live ? nth_set_bit(Pi, r) : 0u;
     body(live, i, j);
   }
@@ -428,32 +427,23 @@ void launch_validate_csr(const GraphArgs &g, unsigned long long *sums, uint32_t 
 
 // ------------------------------------------------------------------ phase 1 + static overlap
 
-struct SlotFacts {
-  int32_t dist;
-  float std_dev, cn;
-  uint32_t len;
-};
-
-__device__ __forceinline__ SlotFacts shfl_facts(const SlotFacts &f, uint32_t src_lane) {
-  SlotFacts r;
-  r.dist = __shfl_sync(FULL, f.dist, src_lane);
-  r.std_dev = __shfl_sync(FULL, f.std_dev, src_lane);
-  r.cn = __shfl_sync(FULL, f.cn, src_lane);
-  r.len = __shfl_sync(FULL, f.len, src_lane);
-  return r;
-}
-
 // Proposals of check_mark_polymorphic (algorithms.c:283-295) and, in the same
 // sweep over the pairs, G0[v,s] = "some same-direction pair of edges that are
 // unmarked on entry overlaps by more than ocutoff" (algorithms.c:301-324 before
 // any mark of this filter run is taken into account; k4_fire_init repairs the
 // rows next to polymorphic vertices).  gbits must be zero on entry.
 struct PairsState {
-  uint32_t start, n, sp, dst, fl, own_y;
+  uint32_t sp, dst, own_y;   // sp = NONE beyond the window's end
+  uint32_t fe;               // flags | estate << 8
   uint2 vi;
-  SlotFacts me;
-  uint8_t es;
+  int32_t dist;
+  float std_dev;
 };
+
+// the window of a PairsState, from its srcp column alone
+__device__ __forceinline__ Window pairs_window(const PairsState &t) {
+  return open_window(0u, (uint32_t) __popc(__ballot_sync(FULL, t.sp != NONE)), t.sp);
+}
 
 // Most pairs need no evaluation.  All that phase 2 needs from a (row, direction) is whether SOME
 // pair of unmarked edges overlaps by more than ocutoff, and most groups have such a pair among
@@ -465,84 +455,133 @@ struct PairsState {
 // covers the rounding of the float sum; the exact test decides).
 // (Dealing out every pair took the same 1.59 ms at C3 with 11 % more instructions; walking ALL
 // pairs per slot, lane i stepping through its partners, measured slower: 1.86 ms.)
-__global__ void __launch_bounds__(32 * WARPS, 8) k4_pairs3(FilterArgs a) {
+//
+// The pass runs at 8 blocks per SM (6, with more registers, measured slower), so at 32 registers,
+// and holds nothing in local memory: step B keeps only what its tests read live (the window's row
+// masks are opened again after it).  The ambiguous-order test decides on its f32 fast path here; a
+// window with a pair that only the double expression can decide (inside the guard band, extreme
+// operands: rare) writes its gbits, leaves its proposals, and is listed (first row | (slots - 1) <<
+// 27 in work_a, CNT_PAIRS_EXACT).  EXACT = true runs the same code over the listed windows with the
+// double expression, whose division and square root need more registers than 32, and appends their
+// proposals.
+template <bool EXACT>
+__global__ void __launch_bounds__(32 * WARPS, EXACT ? 1 : 8) k4_pairs3(FilterArgs a) {
   const GraphArgs &g = a.g;
   const uint32_t lane = lane_id();
   const float half = __fmul_rn(a.cncutoff, 0.5f);
   const float low_bound = half + fabsf(half) * 1e-6f + 1e-30f;
-  for_each_window<1>(g,
-    [&](uint32_t start, uint32_t n) {
-      PairsState t;
-      t.start = start;
-      t.n = n;
-      const bool valid = lane < n;
-      const uint32_t s = start + lane;
-      t.sp = valid ? __ldcs(g.srcp + s) : NONE;
-      t.dst = valid ? __ldcs(g.dst + s) : 0u;
-      t.fl = valid ? __ldcs(g.flags + s) : 0u;
-      t.me.dist = valid ? __ldcs(g.dist + s) : 0;
-      t.me.std_dev = valid ? __ldcs(g.std_dev + s) : 0.f;
-      t.es = (valid && !a.fused_repeats) ? __ldcs(g.estate + s) : (uint8_t) 0;
-      return t;
-    },
-    [&](PairsState &t) {
-      const bool valid = lane < t.n;
-      t.own_y = valid ? a.vinfo[t.sp & S_POS].y : VI_MARKED;
-      t.vi = valid ? a.vinfo[t.dst] : make_uint2(0u, 0u);
-    },
-    [&](PairsState &t) {
-      const Window W = open_window(t.start, t.n, t.sp);
-      const bool act = W.valid && !(t.own_y & VI_MARKED) && (W.ve - W.vb) >= 2u;
+  auto stageA = [&](uint32_t start, uint32_t n) {
+    PairsState t;
+    const bool valid = lane < n;
+    const uint32_t s = start + lane;
+    t.sp = valid ? __ldcs(g.srcp + s) : NONE;
+    t.dst = valid ? __ldcs(g.dst + s) : 0u;
+    t.fe = valid ? (uint32_t) __ldcs(g.flags + s) : 0u;
+    if (valid && !a.fused_repeats) t.fe |= (uint32_t) __ldcs(g.estate + s) << 8;
+    t.dist = valid ? __ldcs(g.dist + s) : 0;
+    t.std_dev = valid ? __ldcs(g.std_dev + s) : 0.f;
+    return t;
+  };
+  auto stageB = [&](PairsState &t) {
+    const bool valid = t.sp != NONE;
+    t.own_y = valid ? a.vinfo[t.sp & S_POS].y : VI_MARKED;
+    t.vi = valid ? a.vinfo[t.dst] : make_uint2(0u, 0u);
+  };
+  auto stageC = [&](PairsState &t) {
+    const float cn = __uint_as_float(t.vi.x);
+    const uint32_t len = t.vi.y & ~VI_MARKED;
+    const bool wm = (t.vi.y & VI_MARKED) != 0;
+    const bool sense = (t.fe & F_SENSE) != 0;
+    bool act;
+    uint32_t OK, P, fire_mask;
+    {
+      const Window W = pairs_window(t);
+      act = W.valid && !(t.own_y & VI_MARKED) && (W.ve - W.vb) >= 2u;
       if (!__any_sync(FULL, act)) return;
-      SlotFacts me = t.me;
-      me.cn = __uint_as_float(t.vi.x);
-      me.len = t.vi.y & ~VI_MARKED;
-      const bool wm = (t.vi.y & VI_MARKED) != 0;
-      const bool ok = act && (a.fused_repeats ? !wm : !edge_state_marked(t.es)) && a.ocutoff >= 0;
-      const bool sense = (t.fl & F_SENSE) != 0;
-      const bool low = act && !(me.cn > low_bound);
+      const bool ok = act && (a.fused_repeats ? !wm : !edge_state_marked((uint8_t) (t.fe >> 8))) && a.ocutoff >= 0;
+      const bool low = act && !(cn > low_bound);
       const uint32_t A = __ballot_sync(FULL, act), S = __ballot_sync(FULL, act && sense);
-      const uint32_t OK = __ballot_sync(FULL, ok), LOW = __ballot_sync(FULL, low);
+      OK = __ballot_sync(FULL, ok);
+      const uint32_t LOW = __ballot_sync(FULL, low);
       const uint32_t higher = lane == 31u ? 0u : FULL << (lane + 1u);
       const uint32_t grp = act ? (W.rowmask & (sense ? S : (A & ~S))) : 0u;     // my row and direction
       // step A: the next unmarked slot of the group
       const uint32_t cand = ok ? (grp & OK & higher) : 0u;
       const uint32_t nxt = cand ? (uint32_t) __ffs(cand) - 1u : lane;
-      const int32_t d2 = __shfl_sync(FULL, me.dist, nxt);
-      const uint32_t l2 = __shfl_sync(FULL, me.len, nxt);
-      uint32_t fire_mask = __ballot_sync(FULL, cand != 0u && interval_overlap(me.dist, me.len, d2, l2) > a.ocutoff);
+      const int32_t d2 = __shfl_sync(FULL, t.dist, nxt);
+      const uint32_t l2 = __shfl_sync(FULL, len, nxt);
+      fire_mask = __ballot_sync(FULL, cand != 0u && interval_overlap(t.dist, len, d2, l2) > a.ocutoff);
       const bool fired = (fire_mask & grp) != 0u;
       // step B: what is left
-      uint32_t P = 0;
+      P = 0;
       if (act) {
         uint32_t rest = LOW;
         if (low) rest = FULL;
         else if (ok && !fired) rest |= OK & ~(cand ? 1u << nxt : 0u);
         P = grp & higher & rest;
       }
-      uint32_t prop_mask = 0;
-      if (__any_sync(FULL, P != 0u)) {
-        for_each_pair(P, [&](bool live, uint32_t i, uint32_t j) {
-          const SlotFacts e1 = shfl_facts(me, i), e2 = shfl_facts(me, j);   // e1 = earlier adjacency slot
-          uint32_t hit = 0, fire = 0;
-          if (live) {
-            // check_mark_polymorphic, algorithms.c:232-238
-            if (__fadd_rn(e1.cn, e2.cn) < a.cncutoff &&
-                ambiguous_order(e1.dist, e1.std_dev, e2.dist, e2.std_dev, a.ambig))
-              hit = 1u << (e1.cn < e2.cn ? i : j);
-            if (((OK >> i) & (OK >> j) & 1u) && interval_overlap(e1.dist, e1.len, e2.dist, e2.len) > a.ocutoff)
-              fire = 1u << i;
-          }
-          prop_mask |= __reduce_or_sync(FULL, hit);
-          fire_mask |= __reduce_or_sync(FULL, fire);
-        });
-      }
-      // proposals (target must be unmarked, algorithms.c:242)
-      warp_append2(act && ((prop_mask >> lane) & 1u) && !wm, make_uint2(W.row, t.dst), a.proposals,
-                   a.proposals_cap, &g.counters[CNT_PROPOSALS], &g.counters[CNT_OVERFLOW]);
+    }
+    uint32_t prop_mask = 0;
+    bool exact = false;                          // a pair of mine needs the double expression
+    if (__any_sync(FULL, P != 0u)) {
+      // operands move by shuffle, each only for the test that reads it (slot i = the earlier adjacency slot)
+      for_each_pair(P, [&](bool live, uint32_t i, uint32_t j) {
+        const int32_t d1 = __shfl_sync(FULL, t.dist, i), d2 = __shfl_sync(FULL, t.dist, j);
+        const uint32_t l1 = __shfl_sync(FULL, len, i), l2 = __shfl_sync(FULL, len, j);
+        const bool fire = live && ((OK >> i) & (OK >> j) & 1u) && interval_overlap(d1, l1, d2, l2) > a.ocutoff;
+        fire_mask |= __reduce_or_sync(FULL, fire ? 1u << i : 0u);
+        // check_mark_polymorphic, algorithms.c:232-238; std_dev only for pairs that pass the copy-number test
+        const float c1 = __shfl_sync(FULL, cn, i), c2 = __shfl_sync(FULL, cn, j);
+        const bool cpair = live && __fadd_rn(c1, c2) < a.cncutoff;
+        if (__any_sync(FULL, cpair)) {
+          const float s1 = __shfl_sync(FULL, t.std_dev, i), s2 = __shfl_sync(FULL, t.std_dev, j);
+          int amb = 0;
+          if (cpair) amb = EXACT ? (int) ambiguous_order(d1, s1, d2, s2, a.ambig) : ambiguous_order_fast(d1, s1, d2, s2, a.ambig);
+          exact |= amb < 0;
+          prop_mask |= __reduce_or_sync(FULL, amb > 0 ? 1u << (c1 < c2 ? i : j) : 0u);
+        }
+      });
+    }
+    {
+      const Window W = pairs_window(t);
+      const uint32_t S = __ballot_sync(FULL, act && sense);
       const uint32_t g1 = fire_mask & W.rowmask & S, g0 = fire_mask & W.rowmask & ~S;
       if (W.head && act && (g0 | g1)) a.gbits[W.row] = (uint8_t) ((g0 ? 1u : 0u) | (g1 ? 2u : 0u));
-    });
+    }
+    if (__any_sync(FULL, exact)) {               // never with EXACT: the window's proposals wait for that pass
+      const uint32_t n = (uint32_t) __popc(__ballot_sync(FULL, t.sp != NONE));
+      if (lane == 0) a.work_a[atomicAdd(&g.counters[CNT_PAIRS_EXACT], 1u)] = (t.sp & S_POS) | ((n - 1u) << 27);
+      return;
+    }
+    // proposals (target must be unmarked, algorithms.c:242)
+    warp_append2(act && ((prop_mask >> lane) & 1u) && !wm, make_uint2(t.sp & S_POS, t.dst), a.proposals,
+                 a.proposals_cap, &g.counters[CNT_PROPOSALS], &g.counters[CNT_OVERFLOW]);
+  };
+  if (!EXACT) {
+    // for_each_window<1>, but with the end of a batch's last window read only when that window is
+    // reached: one register less across the stages, the one this pass needs to stay out of local memory
+    const uint32_t nwin = g.n_windows, nbatch = (nwin + 31u) / 32u;
+    for (uint32_t b = blockIdx.x * WARPS + (threadIdx.x >> 5); b < nbatch; b += gridDim.x * WARPS) {
+      const uint32_t w0 = b * 32u;
+      const uint32_t ws = w0 + lane <= nwin ? __ldcs(g.win_start + w0 + lane) : 0u;
+      for (uint32_t k = 0; k < 32u && w0 + k < nwin; k++) {
+        const uint32_t start = __shfl_sync(FULL, ws, k);
+        const uint32_t end = k < 31u ? __shfl_sync(FULL, ws, k + 1u) : __ldcs(g.win_start + w0 + 32u);
+        if (end - start > 32u) continue;           // a row of more than BIG_ROW slots
+        PairsState t = stageA(start, end - start);
+        stageB(t);
+        stageC(t);
+      }
+    }
+    return;
+  }
+  const uint32_t n_listed = g.counters[CNT_PAIRS_EXACT];
+  for (uint32_t x = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; x < n_listed; x += (gridDim.x * blockDim.x) >> 5) {
+    const uint32_t e = a.work_a[x], p = e & ((1u << 27) - 1u);
+    PairsState t = stageA(g.row_ptr[p - g.row_base], (e >> 27) + 1u);
+    stageB(t);
+    stageC(t);
+  }
 }
 
 // block per big row; per-block scratch: copy_num[max_deg] f32, low[max_deg] u32, mark[max_deg] u8.
@@ -787,7 +826,9 @@ void launch_pairs(const FilterArgs &a, cudaStream_t s) {
   if (a.g.E == 0) return;
   {
     KernelTimer t_("k4_pairs", s);
-    k4_pairs3<<<host_flat_grid(a.g.n_windows), 32 * WARPS, 0, s>>>(a);
+    cudaMemsetAsync(&a.g.counters[CNT_PAIRS_EXACT], 0, 4, s);
+    k4_pairs3<false><<<host_flat_grid(a.g.n_windows), 32 * WARPS, 0, s>>>(a);
+    k4_pairs3<true><<<a.g.sm_count, 32 * WARPS, 0, s>>>(a);
   }
   if (a.g.n_big_rows) {
     KernelTimer t_("k4_pairs_big", s);
@@ -917,18 +958,22 @@ __device__ __forceinline__ bool slot_unmarked(const FilterArgs &a, uint32_t s, u
 
 // G[v,s]: max overlap over same-direction pairs that are unmarked when v is
 // reached, not yet counting the fires of smaller neighbours (algorithms.c:301-320).
-// Streaming pass by position: rows away from every polymorphic vertex keep the
-// pairs pass's static answer; the others are listed for k4_fire_redo.
-__global__ void __launch_bounds__(256) k4_fire_init(FilterArgs a, uint32_t *__restrict__ redo_list,
-                                                     uint32_t *__restrict__ n_redo) {
+// Streaming pass by position, thread per row: rows away from every polymorphic vertex keep the
+// pairs pass's static answer.  A row next to one (k4_dirty) is recomputed by its warp straight
+// away, one such row at a time: lanes are its slots (coalesced slot columns, vinfo / poly_cur
+// gathered in parallel), and "some unmarked same-direction pair overlaps by more than ocutoff" is
+// found as in k4_pairs3 -- every slot against the next unmarked slot of its direction, then the
+// remaining pairs of a direction without a hit dealt out to the lanes.
+__global__ void __launch_bounds__(256) k4_fire_init(FilterArgs a) {
   const GraphArgs &g = a.g;
-  __shared__ uint32_t s_q[8][WarpQueue::QCAP];
-  WarpQueue q{s_q[threadIdx.x >> 5], 0u};
+  const uint32_t lane = lane_id();
   const uint32_t pl = blockIdx.x * blockDim.x + threadIdx.x;
   const uint32_t p = g.row_base + pl;
   bool redo = false;
+  uint32_t r0 = 0, d = 0;
   if (pl < g.V) {
-    const uint32_t d = g.row_ptr[pl + 1] - g.row_ptr[pl];
+    r0 = g.row_ptr[pl];
+    d = g.row_ptr[pl + 1] - r0;
     if (d <= BIG_ROW) {
       const uint32_t v_id = id_at(g, p);
       const bool active = !(a.vinfo[p].y & VI_MARKED) && !(a.poly_cur[p] < v_id);
@@ -943,73 +988,46 @@ __global__ void __launch_bounds__(256) k4_fire_init(FilterArgs a, uint32_t *__re
       }
     }
   }
-  q.push(redo, p, redo_list, n_redo);
-  q.flush(redo_list, n_redo);
-}
-
-// thread per listed row (active, at most BIG_ROW slots, next to a polymorphic vertex)
-__global__ void __launch_bounds__(128) k4_fire_redo(FilterArgs a, const uint32_t *__restrict__ redo_list,
-                                                     const uint32_t *__restrict__ n_redo) {
-  const GraphArgs &g = a.g;
-  const uint32_t n = *n_redo;
-  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    const uint32_t p = redo_list[i];
-    const uint32_t r0 = g.row_ptr[p - g.row_base], d = g.row_ptr[p - g.row_base + 1] - r0;
-    const uint32_t v_id = id_at(g, p);
-    int32_t dist[BIG_ROW];
-    uint32_t len[BIG_ROW];
-    uint32_t sense_mask = 0, ok_mask = 0;
-    for (uint32_t k0 = 0; k0 < d; k0 += 8) {       // 8 slots at a time: their loads and gathers overlap
-      uint32_t w[8], fl[8], pt[8];
-      uint2 vi[8];
-      int32_t di[8];
-      uint8_t es[8];
-#pragma unroll
-      for (int j = 0; j < 8; j++) {
-        const bool in = k0 + j < d;
-        const uint32_t s = r0 + k0 + j;
-        w[j] = in ? g.dst[s] : 0u;
-        di[j] = in ? g.dist[s] : 0;
-        fl[j] = in ? g.flags[s] : 0u;
-        es[j] = (in && !a.fused_repeats) ? g.estate[s] : (uint8_t) 0;
-      }
-#pragma unroll
-      for (int j = 0; j < 8; j++) {
-        const bool in = k0 + j < d;
-        vi[j] = in ? a.vinfo[w[j]] : make_uint2(0u, 0u);
-        pt[j] = in ? a.poly_cur[w[j]] : 0u;
-      }
-#pragma unroll
-      for (int j = 0; j < 8; j++) {
-        if (k0 + j >= d) break;
-        const uint32_t k = k0 + j;
-        dist[k] = di[j];
-        len[k] = vi[j].y & ~VI_MARKED;
-        if (fl[j] & F_SENSE) sense_mask |= 1u << k;
-        const bool ok0 = a.fused_repeats ? !(vi[j].y & VI_MARKED) : !edge_state_marked(es[j]);
-        if (ok0 && !(pt[j] <= v_id)) ok_mask |= 1u << k;      // U(e), see slot_unmarked
-      }
+  unsigned todo = __ballot_sync(FULL, redo);
+  while (todo) {
+    const int l = __ffs(todo) - 1;
+    todo &= todo - 1;
+    const uint32_t rp = __shfl_sync(FULL, p, l), rr = __shfl_sync(FULL, r0, l), dd = __shfl_sync(FULL, d, l);
+    const uint32_t v_id = id_at(g, rp);
+    const bool in = lane < dd;
+    const uint32_t s = rr + lane;
+    const uint32_t w = in ? g.dst[s] : 0u;
+    const int32_t dist = in ? g.dist[s] : 0;
+    const uint32_t fl = in ? g.flags[s] : 0u;
+    const uint8_t es = (in && !a.fused_repeats) ? g.estate[s] : (uint8_t) 0;
+    const uint2 vi = in ? a.vinfo[w] : make_uint2(0u, 0u);
+    const uint32_t pt = in ? a.poly_cur[w] : 0u;
+    const uint32_t len = vi.y & ~VI_MARKED;
+    const bool ok0 = a.fused_repeats ? !(vi.y & VI_MARKED) : !edge_state_marked(es);
+    const bool ok = in && ok0 && !(pt <= v_id);                 // U(e), see slot_unmarked
+    const bool sense = (fl & F_SENSE) != 0;
+    const uint32_t OK = __ballot_sync(FULL, ok), S = __ballot_sync(FULL, in && sense);
+    const uint32_t higher = lane == 31u ? 0u : FULL << (lane + 1u);
+    const uint32_t cand = ok ? (OK & (sense ? S : ~S) & higher) : 0u;     // later unmarked slots, my direction
+    // the next one
+    const uint32_t nxt = cand ? (uint32_t) __ffs(cand) - 1u : lane;
+    const int32_t d2 = __shfl_sync(FULL, dist, nxt);
+    const uint32_t l2 = __shfl_sync(FULL, len, nxt);
+    uint32_t fire_mask = __ballot_sync(FULL, cand != 0u && interval_overlap(dist, len, d2, l2) > a.ocutoff);
+    // the others, in a direction without a hit yet
+    const bool fired = (fire_mask & (sense ? S : ~S)) != 0u;
+    const uint32_t P = fired ? 0u : cand & ~(1u << nxt);
+    if (__any_sync(FULL, P != 0u))
+      for_each_pair(P, [&](bool live, uint32_t i, uint32_t j) {
+        const int32_t e1 = __shfl_sync(FULL, dist, i), e2 = __shfl_sync(FULL, dist, j);
+        const uint32_t m1 = __shfl_sync(FULL, len, i), m2 = __shfl_sync(FULL, len, j);
+        fire_mask |= __reduce_or_sync(FULL, live && interval_overlap(e1, m1, e2, m2) > a.ocutoff ? 1u << i : 0u);
+      });
+    const uint32_t gb = ((fire_mask & ~S) ? 1u : 0u) | ((fire_mask & S) ? 2u : 0u);
+    if (lane == 0) {
+      a.gbits[rp] = (uint8_t) gb;
+      a.fstat[rp] = (uint8_t) (FS_DECIDED_ALL & ~(gb << 2));
     }
-    // only "some pair overlaps by more than ocutoff" matters per direction: stop at the first hit
-    uint32_t gb = 0;
-    for (uint32_t x = 0; x + 1 < d && gb != 3u; x++) {
-      if (!((ok_mask >> x) & 1u)) continue;
-      const uint32_t sx = (sense_mask >> x) & 1u;
-      if ((gb >> sx) & 1u) continue;
-      // partners: later slots of the same direction that are still unmarked
-      uint32_t cand = ok_mask & (sx ? sense_mask : ~sense_mask) & (x == 31u ? 0u : (0xFFFFFFFFu << (x + 1u)));
-      if (d < 32u) cand &= (1u << d) - 1u;
-      while (cand) {
-        const uint32_t y = (uint32_t) __ffs(cand) - 1u;
-        cand &= cand - 1u;
-        if (interval_overlap(dist[x], len[x], dist[y], len[y]) > a.ocutoff) {
-          gb |= 1u << sx;
-          break;
-        }
-      }
-    }
-    a.gbits[p] = (uint8_t) gb;
-    a.fstat[p] = (uint8_t) (FS_DECIDED_ALL & ~(gb << 2));
   }
 }
 
@@ -1076,9 +1094,8 @@ __global__ void __launch_bounds__(512) k4_fire_init_big(FilterArgs a, uint32_t *
 void launch_fire_init(const FilterArgs &a, uint32_t *n_work_b, cudaStream_t s) {
   if (a.g.V == 0) return;
   {
-    KernelTimer t_("k4_fire_init(2 kernels)", s);
-    k4_fire_init<<<(a.g.V + 255) / 256, 256, 0, s>>>(a, a.work_a, &a.g.counters[CNT_WORK_A]);
-    k4_fire_redo<<<a.g.sm_count * 16, 128, 0, s>>>(a, a.work_a, &a.g.counters[CNT_WORK_A]);
+    KernelTimer t_("k4_fire_init", s);
+    k4_fire_init<<<(a.g.V + 255) / 256, 256, 0, s>>>(a);
   }
   if (a.g.n_big_rows) {
     KernelTimer t_("k4_fire_init_big", s);

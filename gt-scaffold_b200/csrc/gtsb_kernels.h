@@ -40,6 +40,7 @@ enum {
   CNT_RING0, CNT_RING1, CNT_RING2, CNT_RING_ROUNDS,   // worklist lengths / round count of k_fire_rounds_all
   CNT_HUB_ITEMS,          // work items (hub row, chunk of its low-copy-number slots) of the split pairs pass
   CNT_MID_BUCKETS,        // buckets of the general build a warp sorts in shared memory (k_resolve_mid)
+  CNT_PAIRS_EXACT,        // windows the pairs pass leaves to its double-precision sweep (listed in work_a)
   CNT_NUM
 };
 
