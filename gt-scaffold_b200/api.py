@@ -604,7 +604,9 @@ class ScaffoldGraphB200:
         return dist, used
 
     def components(self):
-        """(label[V], terminal[V]) of the current graph and states, see gtsb_components."""
+        """(label[V], terminal[V]) of the current graph and states, see gtsb_components.  On a
+        partitioned context this is collective: every rank calls it and gets the arrays of all V
+        contigs, the same on every rank."""
         lab, term = np.zeros(self.V, np.uint32), np.zeros(self.V, np.uint8)
         self._ck(self.L.gtsb_components(self.h, _ptr(lab), _ptr(term)))
         return lab, term

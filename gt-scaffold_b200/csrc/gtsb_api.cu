@@ -1204,7 +1204,7 @@ int gtsb_components(gtsb_context *c, uint32_t *label, uint8_t *terminal) {
   if (c == nullptr) return -1;
   CK(cudaSetDevice(c->device));
   if (!c->have_graph) return fail(c, "gtsb_components: no graph (call gtsb_build or gtsb_set_graph_host)");
-  if (c->world > 1) return fail(c, "gtsb_components: single-device graphs only");
+  if (c->world > 1) return dist_components(c, label, terminal);
   ProfScope ps_(c);
   if (await_vertices(c) != 0) return -1;
   const uint64_t V = c->V;
@@ -1217,7 +1217,7 @@ int gtsb_components(gtsb_context *c, uint32_t *label, uint8_t *terminal) {
   const GraphArgs g = graph_args(c);
   uint32_t *lab = c->poly_cur.as<uint32_t>();
   uint32_t *cnt = c->counters.as<uint32_t>();
-  launch_cc_init(g, lab, c->gbits.as<uint8_t>(), s);
+  launch_cc_init(g, g.V, lab, c->gbits.as<uint8_t>(), s);
   c->stats.kernel_launches += 1;
   uint32_t rounds = 0;
   for (;;) {

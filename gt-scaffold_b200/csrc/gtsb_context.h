@@ -174,6 +174,8 @@ struct ProfScope {                      // routes KernelTimer to the context's p
 int dist_pipeline(gtsb_context *c, float cn_cutoff, float astat_cutoff, int use_cn, float pcutoff,
                   float cncutoff, int64_t ocutoff);
 void dist_release(gtsb_context *c);
+// gtsb_components on a partitioned graph (collective)
+int dist_components(gtsb_context *c, uint32_t *label, uint8_t *terminal);
 // `.de` / `.astat` text on every rank of a partitioned context (collective)
 int dist_parse_de(gtsb_context *c, const char *text, uint64_t n, uint64_t *nof_records, uint32_t *irregular);
 int dist_parse_astat(gtsb_context *c, const char *text, uint64_t n, float *astat, float *copy_num,

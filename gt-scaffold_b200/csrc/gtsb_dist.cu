@@ -20,6 +20,8 @@
 //           fire status, once per fire round        allgatherv,     1 B/vertex
 //           final per-vertex facts vres             allgatherv,     4 B/vertex
 //           vertex states                           allreduce(max), 1 B/vertex
+//   components  labels by position, once per batch  allreduce(min), 4 B/vertex
+//           terminal flags of the ranks' rows       allgatherv,     1 B/vertex (once)
 //   .astat  key of the winning line (rank, offset)  allreduce(max), 8 B/vertex
 //           the winners' values (u32 bit patterns)  allreduce(sum), 8 B/vertex
 //             (the same for a partitioned stream's end; its feeds exchange nothing)
@@ -1590,6 +1592,97 @@ int dist_pipeline(gtsb_context *c, float cn_cutoff, float astat_cutoff, int use_
   }
   CK(cudaGetLastError());
   return 0;
+}
+
+// ---- components and terminals (gtsb_components, collective)
+//
+// Every rank holds the labels of ALL positions (4 B/vertex, like poly_cur), equal on every rank at
+// the start (from the complete vstate).  A batch runs CC_ROUNDS_PER_BATCH rounds on the rank's own
+// copy -- hooking over its own slots, pointer jumping over every position -- and then merges the
+// copies with allreduce(min).  The copies of other ranks' labels a rank works with are stale, and
+// that is safe: at all times every label is the id of an ancestor of its vertex (u ->* v), since
+// hooking passes an ancestor of v across a usable v -> w, jumping passes the label of an ancestor,
+// and the min of ancestors is one; and labels only decrease.  When no rank moves a label in a batch,
+// the merged labels (the same on every rank) are a fixed point over the edges of all ranks: no usable
+// v -> w anywhere has lab[v] < lab[w].  Take the smallest ancestor u of w and a path u -> x1 -> ...
+// -> w: lab[u] = u, and every step carries a label <= u forward, so lab[w] <= u; lab[w] names an
+// ancestor, so lab[w] >= u.  Hence lab[w] = u, whatever the ranks did in between.  By the same path
+// argument the batch after the b-th has settled every vertex b hops from its smallest ancestor, so
+// more than Vg + 2 batches means the labels do not converge.
+// Terminal flags are a property of a row: every rank sets its own rows' and they are gathered once.
+constexpr int CC_ROUNDS_PER_BATCH = 4;
+
+int dist_components(gtsb_context *c, uint32_t *label, uint8_t *terminal) {
+  ProfScope ps_(c);
+  DistState *D = static_cast<DistState *>(c->dstate);
+  const int N = c->world;
+  const uint64_t Vg = c->V;
+  cudaStream_t s = c->stream;
+  uint32_t *changed = c->counters.as<uint32_t>() + CNT_POLY_CHANGED;
+  std::vector<uint32_t> all;
+  // the filter's work arrays, free between its calls.  The exchange after them (status and every rank's
+  // rows) is unconditional, so an allocation that fails on one rank stops every rank there.
+  int rc = [&]() -> int {
+    bool unused = false;
+    if (injected_failure(c, "components", unused) != 0) return -1;
+    if (await_vertices(c) != 0) return -1;
+    ENSURE(c->poly_cur, (Vg + 1) * 4);          // labels by position
+    ENSURE(c->poly_new, (Vg + 1) * 4);          // labels by id
+    ENSURE(c->gbits, Vg + 1);                   // terminal flags by position
+    ENSURE(c->fstat, Vg + 1);                   // ... by id
+    return 0;
+  }();
+  const uint32_t rows_mine[2] = {c->row_base, (uint32_t) c->Vloc};
+  if (exchange(c, rc, "gtsb_components", rows_mine, 2, all) != 0) return -1;
+  std::vector<uint64_t> lo(N + 1, 0);
+  for (int r = 0; r < N; r++) {
+    if (all[(size_t) r * 2] != lo[r])
+      return fail(c, "gtsb_components: the ranks' rows do not tile the positions (rank %d starts at %u, not %llu)", r,
+                  all[(size_t) r * 2], (unsigned long long) lo[r]);
+    lo[r + 1] = lo[r] + all[(size_t) r * 2 + 1];
+  }
+  if (lo[N] != Vg)
+    return fail(c, "gtsb_components: the ranks hold %llu rows of %llu vertices", (unsigned long long) lo[N],
+                (unsigned long long) Vg);
+
+  GraphArgs g = graph_args(c);
+  g.V = (uint32_t) Vg;                          // labels, jumping and the output span every position
+  uint32_t *lab = c->poly_cur.as<uint32_t>();
+  uint8_t *term = c->gbits.as<uint8_t>();
+  launch_cc_init(g, (uint32_t) c->Vloc, lab, term, s);
+  c->stats.kernel_launches += 1;
+  if (allgatherv(c, "nccl_allgather_cc_terminal", term, 1, lo) != 0) return -1;
+  for (uint64_t batches = 1;; batches++) {
+    rc = [&]() -> int {
+      CK(cudaMemsetAsync(changed, 0, 4, s));
+      for (int k = 0; k < CC_ROUNDS_PER_BATCH; k++) launch_cc_round(g, lab, changed, s);
+      c->stats.kernel_launches += 2 * CC_ROUNDS_PER_BATCH;
+      return 0;
+    }();
+    {
+      KernelTimer t_("nccl_allreduce_cc_labels", s);
+      NK(g_nccl.AllReduce(lab, lab, Vg, ncclUint32, ncclMin, D->comm, s));
+      NK(g_nccl.AllReduce(changed, changed, 1, ncclUint32, ncclMax, D->comm, s));     // any rank moved a label
+    }
+    if (rc == 0)
+      rc = [&]() -> int {
+        CK(cudaMemcpyAsync(c->h_counters + CNT_POLY_CHANGED, changed, 4, cudaMemcpyDeviceToHost, s));
+        return 0;
+      }();
+    if (agree(c, rc, "gtsb_components") != 0) return -1;        // the host synchronisation of the batch
+    if (!c->h_counters[CNT_POLY_CHANGED]) break;
+    if (batches > Vg + 2) return fail(c, "gtsb_components: labels did not converge");
+  }
+  launch_cc_out(g, lab, term, c->poly_new.as<uint32_t>(), c->fstat.as<uint8_t>(), s);
+  c->stats.kernel_launches += 1;
+  rc = [&]() -> int {
+    if (label != nullptr && Vg) CK(cudaMemcpyAsync(label, c->poly_new.p, Vg * 4, cudaMemcpyDeviceToHost, s));
+    if (terminal != nullptr && Vg) CK(cudaMemcpyAsync(terminal, c->fstat.p, Vg, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    CK(cudaGetLastError());
+    return 0;
+  }();
+  return agree(c, rc, "gtsb_components");       // every rank returns the same outcome
 }
 
 // ---- `.de` / `.astat` text, every rank its own chunk of the file (collective)

@@ -1319,14 +1319,21 @@ int launch_fire_rounds_all(const FilterArgs &a, uint32_t *ring, uint32_t max_rou
 // computed by min-label hooking over the usable edges plus pointer jumping
 // (label(v) <- label(label(v)): the label of an ancestor is an ancestor's), a few passes over the
 // slots.  gt_scaffolder_graph_isterminal (:346-373) is "the unmarked edges do not point both ways".
+//
+// g.V counts every position (on a rank of a partitioned graph: all of them, with that rank's
+// row_base and slots), `rows` the rows held here: labels cover all positions, terminal flags the
+// rows held only.
 
-__global__ void __launch_bounds__(256) k_cc_init(GraphArgs g, uint32_t *__restrict__ lab, uint8_t *__restrict__ term) {
+__global__ void __launch_bounds__(256) k_cc_init(GraphArgs g, uint32_t rows, uint32_t *__restrict__ lab,
+                                                 uint8_t *__restrict__ term) {
   const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
   if (p >= g.V) return;
   const uint32_t v = id_at(g, p);
   lab[p] = vertex_state_marked(g.vstate[v]) ? NONE : v;
+  const uint32_t r = p - g.row_base;
+  if (r >= rows) return;
   uint32_t dirs = 0;
-  for (uint32_t s = g.row_ptr[p]; s < g.row_ptr[p + 1]; s++)
+  for (uint32_t s = g.row_ptr[r]; s < g.row_ptr[r + 1]; s++)
     if (!edge_state_marked(g.estate[s])) dirs |= (g.flags[s] & F_SENSE) ? 2u : 1u;
   term[p] = dirs == 3u ? 0 : 1;
 }
@@ -1369,10 +1376,10 @@ __global__ void __launch_bounds__(256) k_cc_out(GraphArgs g, const uint32_t *__r
   term_by_id[v] = term[p];
 }
 
-void launch_cc_init(const GraphArgs &g, uint32_t *lab, uint8_t *term, cudaStream_t s) {
+void launch_cc_init(const GraphArgs &g, uint32_t rows, uint32_t *lab, uint8_t *term, cudaStream_t s) {
   if (g.V == 0) return;
   KernelTimer t_("k_cc_init", s);
-  k_cc_init<<<(g.V + 255) / 256, 256, 0, s>>>(g, lab, term);
+  k_cc_init<<<(g.V + 255) / 256, 256, 0, s>>>(g, rows, lab, term);
 }
 
 void launch_cc_round(const GraphArgs &g, uint32_t *lab, uint32_t *changed, cudaStream_t s) {

@@ -265,8 +265,9 @@ constexpr int POLY_SWEEPS_PER_SYNC = 4;
 void launch_vres(const FilterArgs &a, cudaStream_t s);          // final per-vertex facts (+ POLYMORPHIC vertex marks)
 void launch_finalize(const FilterArgs &a, cudaStream_t s);      // final edge states; needs every neighbour's vres
 // components of gt_scaffolder_calc_cc_and_terminals: lab/term by position; one round = hooking + pointer
-// jumping, *changed is raised when a label moved
-void launch_cc_init(const GraphArgs &g, uint32_t *lab, uint8_t *term, cudaStream_t s);
+// jumping, *changed is raised when a label moved.  g.V = every position (a rank of a partitioned graph
+// passes all Vg, with its row_base and slots); launch_cc_init flags the `rows` rows held from row_base
+void launch_cc_init(const GraphArgs &g, uint32_t rows, uint32_t *lab, uint8_t *term, cudaStream_t s);
 void launch_cc_round(const GraphArgs &g, uint32_t *lab, uint32_t *changed, cudaStream_t s);
 void launch_cc_out(const GraphArgs &g, const uint32_t *lab, const uint8_t *term, uint32_t *label_by_id,
                    uint8_t *term_by_id, cudaStream_t s);

@@ -325,7 +325,14 @@ int gtsb_mle_host(gtsb_context *ctx, uint64_t nof_pairs, const uint64_t *frag_of
    from which v is reached along unmarked edges between unmarked vertices (v itself included) --
    the root of the reference's component of v; 0xFFFFFFFF for a marked vertex.  terminal[v] =
    gt_scaffolder_graph_isterminal (:346-373): the unmarked edges of v do not point both ways.
-   Single-device graphs. */
+   On a partitioned context (gtsb_dist_init) after a successful gtsb_pipeline the call is
+   COLLECTIVE: every rank calls it and gets label[V] and terminal[V] of all V contigs, by id, the
+   same on every rank and equal to what one device returns for the same records, cutoffs and states
+   (both partitioned builds).  Refusals (no graph: before any pipeline, or after a failed step) fail
+   locally, on every rank alike, before any exchange.  A CUDA, NCCL or allocation failure on one
+   rank fails the call on every rank at the next exchange, with that rank's message there and
+   "rank k failed" elsewhere; the graph is then released on every rank, as after any failed
+   partitioned step, and a new gtsb_pipeline works on all ranks. */
 int gtsb_components(gtsb_context *ctx, uint32_t *label, uint8_t *terminal);
 
 /* order-independent digests of the result, for comparing runs too large to fetch: out[0] = edges
