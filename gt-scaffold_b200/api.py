@@ -41,6 +41,7 @@ EXPORTS = [
     "gtsb_de_stream_begin", "gtsb_astat_stream_begin", "gtsb_stream_feed", "gtsb_de_stream_end",
     "gtsb_astat_stream_end", "gtsb_stream_set_slot", "gtsb_dist_any_input",
     "gtsb_dist_de_stream_begin", "gtsb_dist_astat_stream_begin",
+    "gtsb_dot_write_begin", "gtsb_dot_write_next", "gtsb_dot_write_end",
 ]
 
 
@@ -126,6 +127,9 @@ def load_library():
     L.gtsb_components.argtypes = [vp, vp, vp]
     L.gtsb_set_vertices_slice_host.argtypes = [vp, u64, u64, u64, vp, vp, vp]
     L.gtsb_mle_host.argtypes = [vp, u64, vp, vp, vp, vp, vp, vp, vp, u64, C.c_double, i32, C.c_int64, C.c_int64, vp, vp]
+    L.gtsb_dot_write_begin.argtypes = [vp, i32, u64, C.POINTER(u64)]
+    L.gtsb_dot_write_next.argtypes = [vp, C.POINTER(vp), C.POINTER(u64), C.POINTER(u64)]
+    L.gtsb_dot_write_end.argtypes = [vp, i32]
     _lib = L
     return L
 
@@ -387,6 +391,9 @@ class ScaffoldGraphB200:
         rc = begin()
         if not dist:
             self._ck(rc)
+        # a partitioned begin may be refused without opening a stream (a .dot write is open); the end
+        # then reports only "no open stream", so the begin's own message is the one raised
+        first = self.L.gtsb_error(self.h).decode() if rc != 0 else None
         try:
             for piece in pieces if rc == 0 else ():
                 b = np.frombuffer(piece, np.uint8)
@@ -400,7 +407,10 @@ class ScaffoldGraphB200:
                 self.L.gtsb_stream_feed(self.h, None, C.c_uint64(1), C.byref(irr))
                 end(irr)
             raise
-        self._ck(end(irr))
+        rc = end(irr)
+        if rc != 0 and first is not None:
+            raise RuntimeError(first)
+        self._ck(rc)
         return int(irr.value)
 
     def parse_de_pieces(self, pieces):
@@ -464,6 +474,35 @@ class ScaffoldGraphB200:
         self._ck(self.L.gtsb_dot_edge_lines_host(self.h, int(scaffold_only), len(a[0]), *[_ptr(x) for x in a],
                                                  out, cap, C.byref(n)))
         return out.raw[:n.value]
+
+    def write_dot(self, path, scaffold_only: bool = False, piece_bytes: int = 0) -> int:
+        """Write the `.dot` file of the resident graph (gt_scaffolder_graph_print, or _print_scaffold
+        with scaffold_only) to `path`, formatted on the device; -> its size in bytes.  On a partitioned
+        context every rank calls this with the same path and arguments and writes its own byte ranges
+        of the one file (see gtsb_dot_write_begin); on one device it is the same call."""
+        n = C.c_uint64(0)
+        self._ck(self.L.gtsb_dot_write_begin(self.h, int(scaffold_only), C.c_uint64(piece_bytes), C.byref(n)))
+        try:
+            # no O_TRUNC: the ranks open the file in any order; every write lies below the size set here
+            fd = os.open(path, os.O_WRONLY | os.O_CREAT, 0o644)
+            try:
+                os.ftruncate(fd, n.value)
+                ptr, off, nb = C.c_void_p(), C.c_uint64(), C.c_uint64()
+                while True:
+                    self._ck(self.L.gtsb_dot_write_next(self.h, C.byref(ptr), C.byref(off), C.byref(nb)))
+                    if nb.value == 0:
+                        break
+                    view = memoryview((C.c_char * nb.value).from_address(ptr.value)).cast("B")
+                    done = 0
+                    while done < nb.value:
+                        done += os.pwrite(fd, view[done:], off.value + done)
+            finally:
+                os.close(fd)
+        except BaseException:
+            self.L.gtsb_dot_write_end(self.h, 1)
+            raise
+        self._ck(self.L.gtsb_dot_write_end(self.h, 0))
+        return int(n.value)
 
     def scaf_lines(self, rec_root, rec_edge_off, edge_end, edge_dist, edge_std_dev, edge_flags, cap: int):
         """The `.scaf` text of gt_scaffolder_graph_write_scaffold (algorithms.c:1000-1042) for records

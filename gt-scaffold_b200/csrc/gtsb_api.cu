@@ -824,6 +824,7 @@ void gtsb_destroy(gtsb_context *c) {
   if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
   dist_release(c);
   text_stream_release(c);
+  dot_release(c);
   DevBuf *bufs[] ={&c->vattr, &c->astat, &c->seq_len_in, &c->copy_num_in, &c->root, &c->ctg, &c->dist,
                     &c->std_dev, &c->flags, &c->row_ptr, &c->dst, &c->edist, &c->estd, &c->eflags,
                     &c->eid, &c->win_rec, &c->estate, &c->vstate, &c->rep_pred, &c->cnt, &c->bptr,
@@ -881,6 +882,7 @@ int gtsb_want_win_rec(gtsb_context *c, int on) {
 int gtsb_set_vertices_host(gtsb_context *c, uint64_t V, const uint32_t *seq_len, const float *astat,
                            const float *copy_num) {
   if (c == nullptr) return -1;
+  if (dot_refuse_open(c, "gtsb_set_vertices_host") != 0) return -1;          // kf_dot_put reads vstate
   CK(cudaSetDevice(c->device));
   if (!c->seq_len_in.owned) c->seq_len_in = DevBuf();
   if (!c->copy_num_in.owned) c->copy_num_in = DevBuf();
@@ -900,6 +902,7 @@ int gtsb_set_vertices_host(gtsb_context *c, uint64_t V, const uint32_t *seq_len,
 int gtsb_set_vertices_slice_host(gtsb_context *c, uint64_t V, uint64_t first, uint64_t count, const uint32_t *seq_len,
                                  const float *astat, const float *copy_num) {
   if (c == nullptr) return -1;
+  if (dot_refuse_open(c, "gtsb_set_vertices_slice_host") != 0) return -1;          // kf_dot_put reads vstate
   CK(cudaSetDevice(c->device));
   if (c->world <= 1) return fail(c, "gtsb_set_vertices_slice_host: only for a graph partitioned over ranks (gtsb_dist_init)");
   if (first + count > V) return fail(c, "gtsb_set_vertices_slice_host: slice outside the vertices");
@@ -925,6 +928,7 @@ int gtsb_set_vertices_slice_host(gtsb_context *c, uint64_t V, uint64_t first, ui
 int gtsb_set_vertices_device(gtsb_context *c, uint64_t V, const uint32_t *seq_len, const float *astat,
                              const float *copy_num) {
   if (c == nullptr) return -1;
+  if (dot_refuse_open(c, "gtsb_set_vertices_device") != 0) return -1;          // kf_dot_put reads vstate
   CK(cudaSetDevice(c->device));
   if (c->vertices_pending) CK(cudaStreamSynchronize(c->copy_stream));
   adopt(c->seq_len_in, seq_len);
@@ -958,6 +962,7 @@ int gtsb_update_vertices_host(gtsb_context *c, uint64_t V, const uint32_t *seq_l
 
 int gtsb_set_states_host(gtsb_context *c, const uint8_t *vstate, const uint8_t *estate_by_eid) {
   if (c == nullptr) return -1;
+  if (dot_refuse_open(c, "gtsb_set_states_host") != 0) return -1;
   CK(cudaSetDevice(c->device));
   if (!c->have_graph) return fail(c, "gtsb_set_states_host: no graph");
   if (c->world > 1) return fail(c, "gtsb_set_states_host: single-device graphs only");
@@ -1099,6 +1104,7 @@ int gtsb_set_graph_host(gtsb_context *c, uint64_t V, uint64_t E, const uint32_t 
                         const uint8_t *flags, const uint32_t *seq_len, const float *astat,
                         const float *copy_num, const uint8_t *vstate, const uint8_t *estate) {
   if (c == nullptr) return -1;
+  if (dot_refuse_open(c, "gtsb_set_graph_host") != 0) return -1;
   if (E >= 0xFFFFFFF0ull) return fail(c, "too many edges");
   if (row_ptr == nullptr || (E && (dst == nullptr || dist == nullptr || std_dev == nullptr || flags == nullptr ||
                                    estate == nullptr)) || (V && vstate == nullptr))
@@ -1164,6 +1170,7 @@ int gtsb_set_graph_host(gtsb_context *c, uint64_t V, uint64_t E, const uint32_t 
 
 int gtsb_build(gtsb_context *c) {
   if (c == nullptr) return -1;
+  if (dot_refuse_open(c, "gtsb_build") != 0) return -1;
   if (c->world > 1) return fail(c, "a rank-partitioned graph runs through gtsb_pipeline only");
   CK(cudaSetDevice(c->device));
   if (timer_begin(c, c->t_build) != 0) return -1;
@@ -1173,6 +1180,7 @@ int gtsb_build(gtsb_context *c) {
 
 int gtsb_mark_repeats(gtsb_context *c, float cn_cutoff, float astat_cutoff, int use_cn) {
   if (c == nullptr) return -1;
+  if (dot_refuse_open(c, "gtsb_mark_repeats") != 0) return -1;
   if (c->world > 1) return fail(c, "a rank-partitioned graph runs through gtsb_pipeline only");
   CK(cudaSetDevice(c->device));
   if (timer_begin(c, c->t_rep) != 0) return -1;
@@ -1182,6 +1190,7 @@ int gtsb_mark_repeats(gtsb_context *c, float cn_cutoff, float astat_cutoff, int 
 
 int gtsb_filter(gtsb_context *c, float pcutoff, float cncutoff, int64_t ocutoff) {
   if (c == nullptr) return -1;
+  if (dot_refuse_open(c, "gtsb_filter") != 0) return -1;
   if (c->world > 1) return fail(c, "a rank-partitioned graph runs through gtsb_pipeline only");
   CK(cudaSetDevice(c->device));
   if (timer_begin(c, c->t_filter) != 0) return -1;
@@ -1192,6 +1201,7 @@ int gtsb_filter(gtsb_context *c, float pcutoff, float cncutoff, int64_t ocutoff)
 int gtsb_pipeline(gtsb_context *c, float cn_cutoff, float astat_cutoff, int use_cn, float pcutoff,
                   float cncutoff, int64_t ocutoff) {
   if (c == nullptr) return -1;
+  if (dot_refuse_open(c, "gtsb_pipeline") != 0) return -1;
   CK(cudaSetDevice(c->device));
   if (c->world > 1) return dist_pipeline(c, cn_cutoff, astat_cutoff, use_cn, pcutoff, cncutoff, ocutoff);
   if (do_build(c) != 0) return -1;

@@ -67,6 +67,33 @@ struct TextStream {
   cudaEvent_t ev_copied = nullptr, ev_free[2] = {nullptr, nullptr};
 };
 
+// `.dot` of the resident graph written in pieces (gtsb_format.cu, gtsb_dot_write_*).  A rank's text
+// is two byte ranges of the file: part 0 = ["digraph {\n" on rank 0] + the vertex lines of its ids,
+// part 1 = the edge lines of its eids + ["}\n" on the last rank].  Items are the lines of both parts
+// in that order; len[] holds their lengths, pieces are cut from it one at a time.
+struct DotWrite {
+  bool open = false, failed = false;
+  int scaffold_only = 0;
+  uint64_t piece = 0;              // bytes of a piece at most
+  uint64_t hdr = 0, v_lo = 0, nv = 0, e_lo = 0, ne = 0, trl = 0;   // the items
+  uint64_t part_end[2] = {0, 0};   // item after the last of each part
+  uint64_t part_bytes[2] = {0, 0}, part_off[2] = {0, 0};   // bytes and file offset of each part
+  uint64_t file_bytes = 0;
+  uint32_t longest = 1;            // bytes of the longest line of this rank
+  int part = 0;                    // part of the next piece to cut (of the piece in flight, if any)
+  uint64_t item = 0;               // its first item
+  uint64_t done[2] = {0, 0};       // bytes of each part cut so far
+  int slot = 0;                    // slot of the last piece cut
+  bool in_flight = false;          // a piece is on its way to the host slot `slot`
+  const uint4 *ent = nullptr;      // edges of this rank's eids: the receive buffer of the route
+  DevBuf own_ent, len;             // one device's route buffer, the line lengths: per write
+  DevBuf list, out, info;          // two slots each: the piece's non-empty lines {item, offset}, its text,
+                                   // its counts (after the two byte sums of the lengths)
+  char *host = nullptr;            // pinned: two slots of `piece` bytes, then the sums and the counts
+  uint64_t host_cap = 0;
+  cudaEvent_t ev[2] = {nullptr, nullptr};
+};
+
 struct gtsb_context {
   int device = 0;
   int sm_count = 148;
@@ -114,6 +141,7 @@ struct gtsb_context {
   uint64_t names_V = 0, names_mask = 0, names_bytes = 0;
   bool have_names = false, names_dup = false, have_num_pairs = false;
   TextStream ts;
+  DotWrite dot;
 
   uint32_t *h_counters = nullptr;   // pinned
   gtsb_stats stats{};
@@ -199,6 +227,22 @@ void adopt_stream_records(gtsb_context *c, uint64_t R);
 // a partitioned stream's end (gtsb_dist.cu, collective)
 int dist_de_stream_end(gtsb_context *c, uint64_t *nof_records, uint32_t *irregular);
 int dist_astat_stream_end(gtsb_context *c, float *astat, float *copy_num, uint32_t *irregular);
+
+// the `.dot` write (gtsb_format.cu), its steps shared by one device and the ranks (gtsb_dist.cu)
+int dot_checks(gtsb_context *c, uint64_t piece_bytes, uint64_t *file_bytes);   // local refusals
+int dot_slots(gtsb_context *c, int scaffold_only, uint64_t piece_bytes);       // piece buffers
+void dot_ranges(gtsb_context *c, uint64_t E, int N, int r);                    // this rank's ids and eids
+int dot_route(gtsb_context *c, uint64_t E, uint4 *const *targets);            // edges to their eid owner
+int dot_lengths(gtsb_context *c, uint64_t part_bytes[2]);                     // + the first piece
+int dot_enqueue(gtsb_context *c);
+void dot_place(gtsb_context *c, const std::vector<uint64_t> &part0, const std::vector<uint64_t> &part1);
+void dot_close(gtsb_context *c);
+void dot_abandon(gtsb_context *c);      // a failed partitioned step released what an open write reads
+void dot_release(gtsb_context *c);                                            // gtsb_destroy
+int dot_refuse_open(gtsb_context *c, const char *what);    // calls that change the graph or the names
+int dot_end_local(gtsb_context *c, int status);
+int dist_dot_begin(gtsb_context *c, int scaffold_only, uint64_t piece_bytes, uint64_t *file_bytes);
+int dist_dot_end(gtsb_context *c, int status);
 
 }  // namespace gtsbi
 

@@ -22,6 +22,9 @@
 //           vertex states                           allreduce(max), 1 B/vertex
 //   components  labels by position, once per batch  allreduce(min), 4 B/vertex
 //           terminal flags of the ranks' rows       allgatherv,     1 B/vertex (once)
+//   .dot    edges to the owner of their eid          remote stores into the owner's receive buffer
+//                                                   (CUDA IPC), 16 B/edge; edge counts and byte
+//                                                   totals in the small status exchanges
 //   .astat  key of the winning line (rank, offset)  allreduce(max), 8 B/vertex
 //           the winners' values (u32 bit patterns)  allreduce(sum), 8 B/vertex
 //             (the same for a partitioned stream's end; its feeds exchange nothing)
@@ -126,6 +129,7 @@ void dist_reset_buffers(gtsb_context *c) {
   DistState *D = static_cast<DistState *>(c->dstate);
   cudaStreamSynchronize(c->stream);
   if (D->side != nullptr) cudaStreamSynchronize(D->side);
+  dot_abandon(c);                        // an open `.dot` write reads the receive buffer and the graph
   for (int r = 0; r < c->world; r++)
     for (int k = 0; k < 2; k++) {
       if (r != c->rank && D->peer_ptr[r][k] != nullptr) cudaIpcCloseMemHandle(D->peer_ptr[r][k]);
@@ -226,11 +230,34 @@ int injected_failure(gtsb_context *c, const char *place, bool &grew) {
   return fail(c, "injected failure at '%s' on rank %d (GTSB_FAIL_AT)", place, c->rank);
 }
 
+// after a failed step that did not touch the graph (the `.dot` write; collective): only the receive
+// buffers, whose capacities must stay rank-uniform, are given back, and the graph is kept
+void release_receive_buffers(gtsb_context *c) {
+  DistState *D = static_cast<DistState *>(c->dstate);
+  cudaStreamSynchronize(c->stream);
+  dot_abandon(c);                        // the receive buffer holds an open write's edges
+  for (int r = 0; r < c->world; r++)
+    for (int k = 0; k < 2; k++) {
+      if (r != c->rank && D->peer_ptr[r][k] != nullptr) cudaIpcCloseMemHandle(D->peer_ptr[r][k]);
+      D->peer_ptr[r][k] = nullptr;
+    }
+  D->peers_open = false;
+  // nobody frees a receive buffer a peer still has mapped
+  if (g_nccl.AllReduce(D->small.p, D->small.p, 1, ncclUint32, ncclSum, D->comm, c->stream) == ncclSuccess)
+    cudaStreamSynchronize(c->stream);
+  for (DevBuf *b : {&D->rx_ent, &D->rx_dest}) {
+    if (b->owned && b->p != nullptr) cudaFree(b->p);
+    *b = DevBuf();
+  }
+  cudaGetLastError();
+}
+
 // Every rank contributes n words and its own status; any rank in trouble stops
 // every rank at the same place (the collectives that follow must be entered by
 // all ranks or by none).  out = world x n matrix.  One host synchronisation.
+// keep_graph: a failure releases the receive buffers only (release_receive_buffers).
 int exchange(gtsb_context *c, int local_rc, const char *where, const uint32_t *mine, int n,
-             std::vector<uint32_t> &out) {
+             std::vector<uint32_t> &out, bool keep_graph = false) {
   uint32_t buf[SMALL_N];
   buf[0] = local_rc != 0 ? 1u : 0u;
   for (int i = 0; i < n; i++) buf[1 + i] = mine[i];
@@ -247,7 +274,10 @@ int exchange(gtsb_context *c, int local_rc, const char *where, const uint32_t *m
     // grown, and rank-uniform capacities are what lets a step decide locally whether an agreement
     // is due: give all of them back, so that the next call starts from equal (empty) buffers.
     const std::string msg = c->err;
-    dist_reset_buffers(c);
+    if (keep_graph)
+      release_receive_buffers(c);
+    else
+      dist_reset_buffers(c);
     c->err = msg;
     return local_rc == 0 ? fail(c, "%s: rank %d failed (see its message)", where, bad) : -1;
   }
@@ -638,6 +668,7 @@ namespace gtsbi {
 void dist_release(gtsb_context *c) {
   DistState *D = static_cast<DistState *>(c->dstate);
   if (D == nullptr) return;
+  dot_abandon(c);
   if (D->side != nullptr) cudaStreamSynchronize(D->side);
   if (D->comm2 != nullptr && g_nccl.CommDestroy != nullptr) g_nccl.CommDestroy(D->comm2);
   if (D->comm != nullptr && g_nccl.CommDestroy != nullptr) g_nccl.CommDestroy(D->comm);
@@ -1873,6 +1904,81 @@ int dist_astat_stream_end(gtsb_context *c, float *astat, float *copy_num, uint32
                           copy_num);
 }
 
+// ---- the `.dot` of the graph, every rank writing its own byte ranges (gtsb_dot_write_*, collective
+// begin and end).  Rank r formats the vertex lines of ids [V r/N, V (r+1)/N) and the edge lines of
+// eids [E r/N, E (r+1)/N).  Every rank stores its slots' edges into the receive buffer of their eid's
+// owner (remote stores, 16 B per edge), after one exchange of the edge counts and one of the
+// buffers' growth; the exchange of the two byte totals per rank after the lengths gives every rank
+// its file offsets.  A failure anywhere fails begin on every rank and keeps the graph.
+int dist_dot_begin(gtsb_context *c, int scaffold_only, uint64_t piece_bytes, uint64_t *file_bytes) {
+  const char *what = "gtsb_dot_write_begin";
+  ProfScope prof(c);
+  DistState *D = static_cast<DistState *>(c->dstate);
+  const int N = c->world, me = c->rank;
+  std::vector<uint32_t> all;
+  int rc = [&]() -> int {
+    bool unused = false;
+    if (injected_failure(c, "dot", unused) != 0) return -1;
+    return dot_slots(c, scaffold_only, piece_bytes);
+  }();
+  const uint32_t mine[4] = {(uint32_t) c->E, (uint32_t) (c->E >> 32), (uint32_t) c->names_V,
+                            (uint32_t) (scaffold_only != 0)};
+  if (exchange(c, rc, what, mine, 4, all, true) != 0) return -1;
+  uint64_t E = 0;
+  for (int r = 0; r < N; r++) {
+    E += all[(size_t) r * 4] | (uint64_t) all[(size_t) r * 4 + 1] << 32;
+    if (all[(size_t) r * 4 + 2] != mine[2] || all[(size_t) r * 4 + 3] != mine[3])
+      return fail(c, "%s: the ranks differ in names set or scaffold_only (rank %d: %u contigs, %u; rank %d: %u, %u)",
+                  what, me, mine[2], mine[3], r, all[(size_t) r * 4 + 2], all[(size_t) r * 4 + 3]);
+  }
+  if (E > 0xFFFFFFFFull) return fail(c, "%s: %llu edges, eids are 32-bit", what, (unsigned long long) E);
+  dot_ranges(c, E, N, me);
+
+  // every rank's receive buffer holds the largest range: rank-uniform sizes, grown on every rank or none
+  bool grew = false;
+  rc = [&]() -> int {
+    if (ensure_u(c, D->rx_ent, (E / N + 16) * sizeof(uint4), grew) != 0) return -1;
+    return ensure_u(c, D->rx_dest, 16, grew);
+  }();
+  const uint32_t grew_mine = grew ? 1u : 0u;
+  if (exchange(c, rc, what, &grew_mine, 1, all, true) != 0) return -1;
+  bool reopen = !D->peers_open;
+  for (int r = 0; r < N; r++) reopen |= all[r] != 0;
+  if (reopen && open_peer_buffers(c) != 0) return -1;
+  uint4 *targets[MAX_RANKS];
+  for (int r = 0; r < N; r++) targets[r] = static_cast<uint4 *>(D->peer_ptr[r][0]);
+  c->dot.ent = D->rx_ent.as<uint4>();
+  rc = dot_route(c, E, targets);
+  {
+    // all edges have landed once every rank's route kernel is complete: a stream-ordered barrier
+    KernelTimer t_("nccl_barrier_dot", c->stream);
+    NK(g_nccl.AllReduce(D->small.p, D->small.p, 1, ncclUint32, ncclSum, D->comm, c->stream));
+  }
+  uint64_t parts[2] = {0, 0};
+  if (rc == 0) rc = dot_lengths(c, parts);
+  const uint32_t totals[4] = {(uint32_t) parts[0], (uint32_t) (parts[0] >> 32), (uint32_t) parts[1],
+                              (uint32_t) (parts[1] >> 32)};
+  if (exchange(c, rc, what, totals, 4, all, true) != 0) {
+    dot_close(c);
+    return -1;
+  }
+  std::vector<uint64_t> part0(N), part1(N);
+  for (int r = 0; r < N; r++) {
+    part0[r] = all[(size_t) r * 4] | (uint64_t) all[(size_t) r * 4 + 1] << 32;
+    part1[r] = all[(size_t) r * 4 + 2] | (uint64_t) all[(size_t) r * 4 + 3] << 32;
+  }
+  dot_place(c, part0, part1);
+  *file_bytes = c->dot.file_bytes;
+  return 0;
+}
+
+// one status exchange: any rank's failure (its own or its caller's) fails the end on every rank
+int dist_dot_end(gtsb_context *c, int status) {
+  const int rc = dot_end_local(c, status);
+  std::vector<uint32_t> none;
+  return exchange(c, rc, "gtsb_dot_write_end", nullptr, 0, none, true);
+}
+
 }  // namespace gtsbi
 
 // =============================================================== C ABI
@@ -1895,6 +2001,7 @@ int gtsb_dist_unique_id(void *id128) {
 int gtsb_dist_init(gtsb_context *c, int rank, int world, const void *id128) {
   if (c == nullptr) return -1;
   if (world < 1 || world > MAX_RANKS || rank < 0 || rank >= world) return fail(c, "gtsb_dist_init: bad rank/world");
+  if (dot_refuse_open(c, "gtsb_dist_init") != 0) return -1;
   if (world == 1) return 0;
   const char *err = load_nccl();
   if (err != nullptr) return fail(c, "gtsb_dist_init: %s", err);

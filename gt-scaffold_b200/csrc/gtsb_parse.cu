@@ -98,6 +98,7 @@ int gtsb_set_vertex_names_host(gtsb_context *c, uint64_t V, const char *names, c
   CK(cudaSetDevice(c->device));
   if (c->ts.kind != TextStream::CLOSED)
     return fail(c, "gtsb_set_vertex_names_host: a text stream is open (end it first)");
+  if (dot_refuse_open(c, "gtsb_set_vertex_names_host") != 0) return -1;
   c->names_V = 0;
   if (V > GTSB_MAX_VERTICES) return fail(c, "gtsb_set_vertex_names_host: too many contigs");
   if (V && (names == nullptr || name_off == nullptr)) return fail(c, "gtsb_set_vertex_names_host: null input");
@@ -323,6 +324,7 @@ int gtsb_parse_de_host(gtsb_context *c, const char *text, uint64_t n, uint64_t *
                        uint32_t *irregular_out) {
   if (c == nullptr) return -1;
   CK(cudaSetDevice(c->device));
+  if (dot_refuse_open(c, "gtsb_parse_de_host") != 0) return -1;
   if (c->world > 1) return dist_parse_de(c, text, n, nof_records, irregular_out);
   if (nof_records == nullptr || irregular_out == nullptr) return fail(c, "gtsb_parse_de_host: null argument");
   if (parse_preamble(c, "gtsb_parse_de_host", text, n) != 0) return -1;
@@ -610,6 +612,7 @@ static int stream_step(gtsb_context *c, uint64_t n) {
 static int stream_prepare(gtsb_context *c, const char *what, const char *plain) {
   TextStream &ts = c->ts;
   stream_close(c);                                  // a new begin discards an open stream
+  if (dot_refuse_open(c, what) != 0) return -1;
   if (plain == nullptr && c->world > 1)
     return fail(c, "%s: a partitioned context reads text with the collective gtsb_parse_*_host calls or "
                    "gtsb_dist_*_stream_begin", what);
@@ -761,12 +764,15 @@ int gtsb_astat_stream_begin(gtsb_context *c, const float *astat, const float *co
 int gtsb_dist_de_stream_begin(gtsb_context *c) {
   if (c == nullptr) return -1;
   CK(cudaSetDevice(c->device));
+  // refused before a stream is opened: a failed partitioned stream's end would release the graph
+  if (dot_refuse_open(c, "gtsb_dist_de_stream_begin") != 0) return -1;
   return dist_begun(c, de_begin(c, "gtsb_dist_de_stream_begin", "gtsb_de_stream_begin"), TextStream::DE);
 }
 
 int gtsb_dist_astat_stream_begin(gtsb_context *c, const float *astat, const float *copy_num) {
   if (c == nullptr) return -1;
   CK(cudaSetDevice(c->device));
+  if (dot_refuse_open(c, "gtsb_dist_astat_stream_begin") != 0) return -1;
   return dist_begun(c, astat_begin(c, "gtsb_dist_astat_stream_begin", "gtsb_astat_stream_begin", astat, copy_num),
                     TextStream::ASTAT);
 }

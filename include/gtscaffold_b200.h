@@ -249,6 +249,50 @@ int gtsb_dot_edge_lines_host(gtsb_context *ctx, int scaffold_only, uint64_t coun
                              const uint32_t *dst, const int32_t *dist, const uint8_t *estate,
                              const uint8_t *sense, char *out, uint64_t cap, uint64_t *bytes);
 
+/* ---- the `.dot` file of the resident graph, of any size, formatted on the device and handed out in
+   pieces that the caller writes at their file offsets (pwrite).  The file is exactly what
+   gt_scaffolder_graph_print writes (gt_scaffolder_graph_print_scaffold when scaffold_only != 0):
+   "digraph {\n", one line per vertex in id order (its vstate, the names set), one line per edge in
+   graph->edges[] (eid) order, "}\n" -- the text of gtsb_dot_vertex_lines_host over all vertices and
+   gtsb_dot_edge_lines_host over all edges in eid order between the two, with no size limit.
+
+     gtsb_dot_write_begin  COLLECTIVE on a partitioned context (every rank calls it with the same
+       arguments), local on one device.  *file_bytes = the file's size, the same on every rank.
+       piece_bytes: the most bytes of one piece, 0 for 64 MiB, else 4096 .. 2^30.
+     gtsb_dot_write_next   LOCAL: the next piece of this rank's text, whole lines, at most piece_bytes,
+       at file offset *file_offset; *bytes == 0 when this rank has nothing left.  *piece points into
+       pinned memory owned by the context and stays valid until the next call on ctx.
+     gtsb_dot_write_end    COLLECTIVE on a partitioned context: status = the caller's own result of
+       writing the pieces (0 = ok).  Returns -1 on every rank if any rank passes a non-zero status,
+       failed in next or did not take all its pieces.
+
+   Rank r of N formats the vertex lines of ids [V r/N, V (r+1)/N) and the edge lines of eids
+   [E r/N, E (r+1)/N) (E: the edges of all ranks); rank 0 also the header and the last rank the
+   trailer.  The pieces of all ranks tile [0, *file_bytes) exactly once; the file is byte-identical to
+   what one device writes for the same records, cutoffs and states.  One device is the N = 1 case.
+   Every edge travels once to the rank that owns its eid (16 B, remote stores on a partitioned graph);
+   each rank's two byte totals are exchanged once.  While the caller writes one piece, the next one is
+   formatted and copied to the host.
+   Memory: 16 B per edge of this rank's eid range (on a partitioned graph in the build's receive
+   buffer, which the build keeps anyway) and 4 B per line of its ranges, both given back at end; two
+   device and two pinned host slots of piece_bytes and 8 B per 14 bytes of a slot for the offsets of
+   its lines, which stay allocated for the next write until gtsb_destroy.
+   Refused locally (on every rank alike): no graph, no names set or one whose size is not V, a graph
+   without edge ids, a bad piece_bytes; a line longer than a piece fails begin.  A begin while a write
+   is open discards it.  While a write is open, gtsb_pipeline, gtsb_build, gtsb_mark_repeats,
+   gtsb_filter, gtsb_set_states_host, gtsb_set_graph_host, gtsb_set_vertices_*,
+   gtsb_set_vertex_names_host, gtsb_parse_de_host, gtsb_dist_init and the stream begins fail with a
+   message and change nothing (a refused gtsb_dist_*_stream_begin opens no stream).  A CUDA, NCCL or
+   allocation failure on one rank fails begin on every rank, with that rank's message there and
+   "rank k failed" elsewhere.  The writer does not change the graph: after any failure of begin, next
+   or end, the graph and its states are kept on every rank, and the next begin, gtsb_pipeline and
+   gtsb_components work.  If another collective call fails while a write is open on a partitioned
+   graph (which releases the graph on every rank), the write is left failed: next fails without device
+   work and end returns -1 on every rank. */
+int gtsb_dot_write_begin(gtsb_context *ctx, int scaffold_only, uint64_t piece_bytes, uint64_t *file_bytes);
+int gtsb_dot_write_next(gtsb_context *ctx, const char **piece, uint64_t *file_offset, uint64_t *bytes);
+int gtsb_dot_write_end(gtsb_context *ctx, int status);
+
 /* ---- `.scaf` text: what gt_scaffolder_graph_write_scaffold prints (gt_scaffolder_algorithms.c:
    1000-1042), one line per scaffold record -- the root's header, then per edge
    "\t<end header>,<dist %ld>,<std_dev %f>,<sense %d>,<same %d>," -- with the "%f" produced by
@@ -278,7 +322,8 @@ int gtsb_pipeline(gtsb_context *ctx, float copy_num_cutoff, float astat_cutoff, 
    gtsb_set_vertices_*; gtsb_pipeline then builds and filters the global graph,
    each rank holding the rows of the contigs that head its lines (contigs
    without a line: last rank).  Vertex states come back complete on every rank;
-   edges stay with their rank (gtsb_get_edges).  The exchanges are NCCL over
+   edges stay with their rank (gtsb_get_edges); the ranks write the graph's `.dot` file together
+   (gtsb_dot_write_*).  The exchanges are NCCL over
    NVLink; the 128-byte id from rank 0 has to reach every rank by the caller's
    own means (MPI, torch.distributed, a file).
    By default the partitioned build is the line-ordered one only: a contig heading lines on two
