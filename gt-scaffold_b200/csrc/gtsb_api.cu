@@ -836,9 +836,8 @@ void gtsb_destroy(gtsb_context *c) {
                     &c->tmp_ent, &c->tmp_dest, &c->tmp_cursor, &c->bucket, &c->bucket_line, &c->line_root, &c->line_start,
                     &c->corrections, &c->lineless_flag, &c->lineless_rank, &c->x_row_ptr, &c->x_dst,
                     &c->x_dist, &c->x_std, &c->x_flags, &c->x_eid, &c->x_estate, &c->x_deg, &c->x_win,
-                    &c->p_names, &c->p_name_off, &c->p_slots, &c->p_flags, &c->p_text, &c->p_chunk_cnt,
-                    &c->p_chunk_off, &c->p_line_end, &c->p_line_cnt, &c->p_line_off, &c->num_pairs,
-                    &c->p_last, &c->p_astat, &c->p_copy_num, &c->p_key, &c->p_win, &c->f_state, &c->f_sense, &c->f_src, &c->f_dst,
+                    &c->p_names, &c->p_name_off, &c->p_slots, &c->p_flags, &c->p_chunk_cnt,
+                    &c->p_chunk_off, &c->p_line_cnt, &c->num_pairs, &c->p_key, &c->p_win, &c->f_state, &c->f_sense, &c->f_src, &c->f_dst,
                     &c->f_dist, &c->f_len, &c->f_off, &c->f_out, &c->vsum, &c->s_root, &c->s_recoff, &c->s_end, &c->s_dist,
                     &c->s_std, &c->s_flags, &c->s_len_r, &c->s_off_r, &c->m_pairs, &c->m_size, &c->m_count, &c->m_pmf,
                     &c->m_logp, &c->m_L, &c->m_c, &c->m_n, &c->m_g, &c->m_slot_pair, &c->m_gmax, &c->m_mag, &c->m_cand};

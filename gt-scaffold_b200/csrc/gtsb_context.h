@@ -35,13 +35,14 @@ struct Timer {
   cudaEvent_t a = nullptr, b = nullptr;
 };
 
-// `.de` / `.astat` text fed in pieces (gtsb_parse.cu, gtsb_*_stream_*).  Everything a stream keeps
-// between two feeds lives here, so that other calls on the context (which share p_flags and the
-// single call's line index) cannot disturb it.  The buffers stay allocated for the next stream.
+// `.de` / `.astat` text read in steps (gtsb_parse.cu): fed in pieces (gtsb_*_stream_*, the context's
+// `ts`) or whole (gtsb_parse_*_host, the context's `whole`, a single step).  Everything a stream keeps
+// between two feeds lives here, so that other calls on the context, the whole-text calls included,
+// cannot disturb it.  The buffers stay allocated for the next read.
 struct TextStream {
   enum Kind { CLOSED = 0, DE = 1, ASTAT = 2 };
   int kind = CLOSED;
-  uint64_t slot = 64ull << 20;      // bytes of one step (carry included)
+  uint64_t slot = 64ull << 20;      // bytes of one step (carry included); 0: whole text, not staged
   char *host = nullptr;            // pinned: the step being filled, then 4 words the device reports into
   uint64_t host_cap = 0;
   uint64_t fill = 0;               // bytes in host[]
@@ -132,15 +133,14 @@ struct gtsb_context {
   DevBuf hub_cn, hub_low, hub_mark, hub_nlow, hub_items;   // split pairs pass of the hub rows
   uint32_t n_big_rows = 0, max_deg = 0;
   // .de text on the device (gtsb_parse.cu)
-  DevBuf p_names, p_name_off, p_slots, p_flags, p_text, p_chunk_cnt, p_chunk_off, p_line_end,
-      p_line_cnt, p_line_off, num_pairs, p_last, p_astat, p_copy_num;
+  DevBuf p_names, p_name_off, p_slots, p_flags, p_chunk_cnt, p_chunk_off, p_line_cnt, num_pairs;
   DevBuf p_key, p_win;          // partitioned `.astat`: (rank, offset) of the winning line, winners' values
   DevBuf f_state, f_sense, f_src, f_dst, f_dist, f_len, f_off, f_out;     // .dot lines (gtsb_format.cu)
   DevBuf s_root, s_recoff, s_end, s_dist, s_std, s_flags, s_len_r, s_off_r;   // .scaf records (gtsb_format.cu)
   DevBuf m_pairs, m_size, m_count, m_pmf, m_logp, m_L, m_c, m_n, m_g, m_slot_pair, m_gmax, m_mag, m_cand;   // distance MLE (gtsb_mle.cu)
   uint64_t names_V = 0, names_mask = 0, names_bytes = 0;
   bool have_names = false, names_dup = false, have_num_pairs = false;
-  TextStream ts;
+  TextStream ts, whole;
   DotWrite dot;
 
   uint32_t *h_counters = nullptr;   // pinned
@@ -204,29 +204,18 @@ int dist_pipeline(gtsb_context *c, float cn_cutoff, float astat_cutoff, int use_
 void dist_release(gtsb_context *c);
 // gtsb_components on a partitioned graph (collective)
 int dist_components(gtsb_context *c, uint32_t *label, uint8_t *terminal);
-// `.de` / `.astat` text on every rank of a partitioned context (collective)
-int dist_parse_de(gtsb_context *c, const char *text, uint64_t n, uint64_t *nof_records, uint32_t *irregular);
-int dist_parse_astat(gtsb_context *c, const char *text, uint64_t n, float *astat, float *copy_num,
-                     uint32_t *irregular);
-
-// the stages of the text entry points (gtsb_parse.cu), shared by the single-device and the
-// partitioned calls
-int parse_preamble(gtsb_context *c, const char *what, const char *text, uint64_t n);
-int de_count(gtsb_context *c, const char *text, uint64_t n, uint64_t *nlines, uint32_t *total, uint32_t *irregular);
-int de_emit(gtsb_context *c, uint64_t nlines, uint32_t total);
-void keep_parsed_records(gtsb_context *c, uint64_t R);
-int astat_last(gtsb_context *c, const char *text, uint64_t n, const float *astat, const float *copy_num,
-               uint64_t *nlines, uint32_t *irregular);
-int astat_apply(gtsb_context *c, uint64_t nlines);
 void text_stream_release(gtsb_context *c);      // gtsb_destroy
 void release(DevBuf &b);
-// the ends of a stream (gtsb_parse.cu), shared by the single-device and the partitioned ones
-int stream_end_local(gtsb_context *c, const char *what, int kind);
-void stream_close(gtsb_context *c);
-void adopt_stream_records(gtsb_context *c, uint64_t R);
-// a partitioned stream's end (gtsb_dist.cu, collective)
-int dist_de_stream_end(gtsb_context *c, uint64_t *nof_records, uint32_t *irregular);
-int dist_astat_stream_end(gtsb_context *c, float *astat, float *copy_num, uint32_t *irregular);
+// the end of a text read (gtsb_parse.cu), shared by one device and the ranks: src = the host bytes
+// of the last step
+int stream_end_local(gtsb_context *c, TextStream &ts, const char *src, const char *what, int kind);
+void stream_close(TextStream &ts);
+void adopt_stream_records(gtsb_context *c, TextStream &ts, uint64_t R);
+void release_stream_records(TextStream &ts);
+// the end of a partitioned text read, stream or whole text (gtsb_dist.cu, collective).  rc: this
+// rank's status so far; stage: the GTSB_FAIL_AT place
+int dist_text_end(gtsb_context *c, TextStream &ts, const char *src, const char *what, int kind, const char *stage,
+                  int rc, uint64_t *nof_records, float *astat, float *copy_num, uint32_t *irregular);
 
 // the `.dot` write (gtsb_format.cu), its steps shared by one device and the ranks (gtsb_dist.cu)
 int dot_checks(gtsb_context *c, uint64_t piece_bytes, uint64_t *file_bytes);   // local refusals

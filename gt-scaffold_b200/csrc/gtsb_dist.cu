@@ -392,7 +392,7 @@ __global__ void k_dist_astat_keys(uint64_t V, uint32_t rank, const uint64_t *__r
   if (v < V) key[v] = last[v] ? ((uint64_t) rank << ASTAT_KEY_SHIFT | last[v]) : 0ull;
 }
 
-// a local last line that a later line beat is forgotten, so that kp_astat<apply> writes winners only
+// a local last line that a later line beat is forgotten, so that only the winners' values are packed
 __global__ void k_dist_astat_winners(uint64_t V, uint32_t rank, const uint64_t *__restrict__ key,
                                      uint64_t *__restrict__ last) {
   const uint64_t v = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x;
@@ -1716,18 +1716,8 @@ int dist_components(gtsb_context *c, uint32_t *label, uint8_t *terminal) {
   return agree(c, rc, "gtsb_components");       // every rank returns the same outcome
 }
 
-// ---- `.de` / `.astat` text, every rank its own chunk of the file (collective)
-
-// the local checks that every text call makes before it reads its chunk
-int dist_text_checks(gtsb_context *c, const char *what, const char *text, uint64_t n) {
-  if (parse_preamble(c, what, text, n) != 0) return -1;
-  // the fgets pieces of the chunks are those of the whole file only if every chunk but the last
-  // ends a line
-  if (c->rank < c->world - 1 && n != 0 && text[n - 1] != '\n')
-    return fail(c, "%s: the chunk of rank %d does not end in '\\n' (only the last rank's may)", what, c->rank);
-  bool unused = false;
-  return injected_failure(c, "parse", unused);
-}
+// ---- `.de` / `.astat` text, every rank its own chunk of the file: a collective gtsb_parse_*_host, or a
+// stream whose begin and feeds are local (gtsb_dist_*_stream_begin).  Both end here.
 
 // every rank's status, IRR_* bits and names set; *irregular = the OR of the bits
 int dist_text_agree(gtsb_context *c, int local_rc, const char *what, uint32_t irregular_mine, uint32_t *irregular) {
@@ -1749,44 +1739,11 @@ int dist_text_agree(gtsb_context *c, int local_rc, const char *what, uint32_t ir
   return 0;
 }
 
-int dist_parse_de(gtsb_context *c, const char *text, uint64_t n, uint64_t *nof_records, uint32_t *irregular_out) {
-  const char *what = "gtsb_parse_de_host";
-  ProfScope prof(c);
-  uint64_t nlines = 0;
-  uint32_t total = 0, irregular = 0;
-  const int rc = [&]() -> int {
-    if (nof_records == nullptr || irregular_out == nullptr) return fail(c, "%s: null argument", what);
-    if (dist_text_checks(c, what, text, n) != 0) return -1;
-    if (await_records(c) != 0) return -1;
-    if (c->names_dup) {
-      irregular = GTSB_IRR_DUP_NAME;
-      return 0;
-    }
-    return de_count(c, text, n, &nlines, &total, &irregular);
-  }();
-  c->have_records = false;
-  c->have_graph = false;
-  if (nof_records != nullptr) *nof_records = 0;
-  if (irregular_out != nullptr) *irregular_out = 0;
-  uint32_t irr = 0;
-  if (dist_text_agree(c, rc, what, irregular, &irr) != 0) return -1;
-  if (irr) {                           // a refusal anywhere: no rank keeps records, all read the file on the host
-    *irregular_out = irr;
-    return 0;
-  }
-  if (agree(c, de_emit(c, nlines, total), what) != 0) return -1;
-  keep_parsed_records(c, total);
-  *nof_records = total;
-  return 0;
-}
-
 // `.astat` over the ranks, once they agree, on this rank's last[] (offset + 1 of its last piece
-// naming v, 0 for none) and values: keys -> allreduce(max) -> winners -> apply -> pack ->
-// allreduce(sum) -> unpack, then the values to the host arrays, identical on every rank.  apply_lines:
-// the lines of the single call, whose kp_astat<apply> writes the pieces this rank won; a stream has
-// applied each step's last pieces as it went, its winners' values are in place (0 lines).
-int astat_over_ranks(gtsb_context *c, uint64_t *last, float *d_astat, float *d_copy_num, uint64_t apply_lines,
-                     float *astat, float *copy_num) {
+// naming v, 0 for none) and values, its own last pieces applied: keys -> allreduce(max) -> winners ->
+// pack -> allreduce(sum) -> unpack, then the values to the host arrays, identical on every rank
+int astat_over_ranks(gtsb_context *c, uint64_t *last, float *d_astat, float *d_copy_num, float *astat,
+                     float *copy_num) {
   DistState *D = static_cast<DistState *>(c->dstate);
   cudaStream_t s = c->stream;
   const uint64_t V = c->names_V;
@@ -1800,7 +1757,6 @@ int astat_over_ranks(gtsb_context *c, uint64_t *last, float *d_astat, float *d_c
     k_dist_astat_winners<<<blocks, 256, 0, s>>>(V, me, key, last);
     c->stats.kernel_launches += 2;
   }
-  if (astat_apply(c, apply_lines) != 0) return -1;
   if (V) {
     KernelTimer t_("k_dist_astat(values)+allreduce", s);
     k_dist_astat_pack<<<blocks, 256, 0, s>>>(V, last, d_astat, d_copy_num, win);
@@ -1817,91 +1773,41 @@ int astat_over_ranks(gtsb_context *c, uint64_t *last, float *d_astat, float *d_c
   return 0;
 }
 
-int dist_parse_astat(gtsb_context *c, const char *text, uint64_t n, float *astat, float *copy_num,
-                     uint32_t *irregular_out) {
-  const char *what = "gtsb_parse_astat_host";
-  ProfScope prof(c);
+// this rank's last steps (if rc, its status so far, is 0), then the agreement of the ranks; .de keeps
+// the records of this rank's chunk, .astat returns the values of the whole file
+int dist_text_end(gtsb_context *c, TextStream &ts, const char *src, const char *what, int kind, const char *stage,
+                  int rc, uint64_t *nof_records, float *astat, float *copy_num, uint32_t *irregular_out) {
   const uint64_t V = c->names_V;
-  uint64_t nlines = 0;
-  uint32_t irregular = 0;
-  const int rc = [&]() -> int {
-    if (irregular_out == nullptr) return fail(c, "%s: null argument", what);
-    if (dist_text_checks(c, what, text, n) != 0) return -1;
-    if (V && (astat == nullptr || copy_num == nullptr)) return fail(c, "%s: null argument", what);
-    if (c->names_dup) {
-      irregular = GTSB_IRR_DUP_NAME;
-      return 0;
-    }
-    ENSURE(c->p_key, (V + 1) * 8);
-    ENSURE(c->p_win, (V + 1) * 8);
-    return astat_last(c, text, n, astat, copy_num, &nlines, &irregular);
-  }();
-  if (irregular_out != nullptr) *irregular_out = 0;
-  uint32_t irr = 0;
-  if (dist_text_agree(c, rc, what, irregular, &irr) != 0) return -1;
-  if (irr) {                           // a refusal anywhere: no rank touches the arrays
-    *irregular_out = irr;
-    return 0;
-  }
-  return astat_over_ranks(c, c->p_last.as<uint64_t>(), c->p_astat.as<float>(), c->p_copy_num.as<float>(), nlines,
-                          astat, copy_num);
-}
-
-// ---- `.de` / `.astat` text fed in pieces, every rank its own chunk (gtsb_dist_*_stream_begin):
-// feeding is local, the end is collective and agrees as the single calls do
-
-int dist_de_stream_end(gtsb_context *c, uint64_t *nof_records, uint32_t *irregular_out) {
-  const char *what = "gtsb_de_stream_end";
-  ProfScope prof(c);
-  const int rc = [&]() -> int {
-    if (nof_records == nullptr || irregular_out == nullptr) return fail(c, "%s: null argument", what);
-    if (stream_end_local(c, what, TextStream::DE) != 0) return -1;
-    bool unused = false;
-    return injected_failure(c, "stream", unused);
-  }();
-  const uint32_t irregular = c->ts.irregular;
-  const uint64_t R = c->ts.R;
-  stream_close(c);
+  if (rc == 0)
+    rc = [&]() -> int {
+      if (stream_end_local(c, ts, src, what, kind) != 0) return -1;
+      if (kind == TextStream::ASTAT) {
+        if (ts.fed >> ASTAT_KEY_SHIFT) return fail(c, "%s: a chunk of 2^%d bytes or more", what, ASTAT_KEY_SHIFT);
+        ENSURE(c->p_key, (V + 1) * 8);
+        ENSURE(c->p_win, (V + 1) * 8);
+      }
+      bool unused = false;
+      return injected_failure(c, stage, unused);
+    }();
+  const uint32_t irregular = ts.irregular;
+  const uint64_t R = ts.R;
+  stream_close(ts);
   if (nof_records != nullptr) *nof_records = 0;
   if (irregular_out != nullptr) *irregular_out = 0;
   uint32_t irr = 0;
-  if (dist_text_agree(c, rc, what, irregular, &irr) != 0) return -1;
-  if (irr) {                           // a refusal anywhere: no rank keeps records (begin dropped the old ones)
+  rc = dist_text_agree(c, rc, what, irregular, &irr);
+  if (kind == TextStream::DE && (rc != 0 || irr)) release_stream_records(ts);
+  if (rc != 0) return -1;
+  if (irr) {                           // a refusal anywhere: no rank keeps records or touches the arrays
     *irregular_out = irr;
     return 0;
   }
-  adopt_stream_records(c, R);
+  if (kind == TextStream::ASTAT)
+    return astat_over_ranks(c, ts.last.as<uint64_t>(), ts.astat.as<float>(), ts.copy_num.as<float>(), astat,
+                            copy_num);
+  adopt_stream_records(c, ts, R);
   *nof_records = R;
   return 0;
-}
-
-int dist_astat_stream_end(gtsb_context *c, float *astat, float *copy_num, uint32_t *irregular_out) {
-  const char *what = "gtsb_astat_stream_end";
-  const uint64_t V = c->names_V;
-  ProfScope prof(c);
-  const int rc = [&]() -> int {
-    if (irregular_out == nullptr || (V && (astat == nullptr || copy_num == nullptr)))
-      return fail(c, "%s: null argument", what);
-    if (stream_end_local(c, what, TextStream::ASTAT) != 0) return -1;
-    if (c->ts.fed >> ASTAT_KEY_SHIFT) return fail(c, "%s: a chunk of 2^%d bytes or more", what, ASTAT_KEY_SHIFT);
-    ENSURE(c->p_key, (V + 1) * 8);
-    ENSURE(c->p_win, (V + 1) * 8);
-    bool unused = false;
-    return injected_failure(c, "stream", unused);
-  }();
-  const uint32_t irregular = c->ts.irregular;
-  stream_close(c);
-  if (irregular_out != nullptr) *irregular_out = 0;
-  uint32_t irr = 0;
-  if (dist_text_agree(c, rc, what, irregular, &irr) != 0) return -1;
-  if (irr) {                           // a refusal anywhere: no rank touches the arrays
-    *irregular_out = irr;
-    return 0;
-  }
-  // the stream's steps have applied this rank's last pieces already: nothing left to apply
-  TextStream &ts = c->ts;
-  return astat_over_ranks(c, ts.last.as<uint64_t>(), ts.astat.as<float>(), ts.copy_num.as<float>(), 0, astat,
-                          copy_num);
 }
 
 // ---- the `.dot` of the graph, every rank writing its own byte ranges (gtsb_dot_write_*, collective

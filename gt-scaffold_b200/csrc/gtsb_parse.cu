@@ -10,14 +10,13 @@
 //   exclusive_scan    first record index of every line
 //   kp_walk<true>     the same walk, records written in file order
 // and, for `.astat` text (algorithms.c:118-149), on the same line index
-//   kp_astat<false>   one thread per line: per contig, the offset of the last line naming it
-//   kp_astat<true>    that line writes the contig's a-statistic and copy number
+//   kp_astat_at<false> one thread per line: per contig, the file offset of the last line naming it
+//   kp_astat_at<true>  that line writes the contig's a-statistic and copy number
 //
-// On a partitioned context every rank runs these passes on its chunk of the file; the agreement
-// between the ranks and the `.astat` winners across them are gtsb_dist.cu's (dist_parse_*).
-//
-// Text fed in pieces (gtsb_*_stream_*, end of this file) runs the same passes step by step on a
-// fixed number of staging slots; `.astat` steps use kp_astat_at, whose offsets are file offsets.
+// The passes run step by step (stream_step, below): text fed in pieces (gtsb_*_stream_*) is a step
+// per staging slot; a whole-text call (gtsb_parse_*_host) is one step.  On a partitioned context
+// every rank runs them on its chunk of the file; the agreement between the ranks and the `.astat`
+// winners across them are gtsb_dist.cu's (dist_text_end).
 //
 // The walk is a byte loop per thread over its own line; neighbouring threads hold neighbouring
 // lines, so a warp's loads fall into one window of a few KB that L1 keeps.
@@ -66,16 +65,7 @@ __global__ void __launch_bounds__(128) kp_walk(const char *__restrict__ text, co
   }
 }
 
-template <bool APPLY>
-__global__ void __launch_bounds__(128) kp_astat(const char *__restrict__ text, const uint64_t *__restrict__ line_end,
-                                                uint64_t nlines, NameTable t, uint64_t *last, float *astat,
-                                                float *copy_num, uint32_t *irregular) {
-  const uint64_t l = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x;
-  if (l >= nlines) return;
-  walk_astat_line<APPLY>(text, l ? line_end[l - 1] : 0, line_end[l], t, last, astat, copy_num, irregular);
-}
-
-// kp_astat on one step of a stream: the step starts at file offset `base`
+// one step of `.astat` text: the step starts at file offset `base`
 template <bool APPLY>
 __global__ void __launch_bounds__(128) kp_astat_at(const char *__restrict__ text, const uint64_t *__restrict__ line_end,
                                                    uint64_t nlines, uint64_t base, NameTable t, uint64_t *last,
@@ -136,254 +126,6 @@ int gtsb_set_vertex_names_host(gtsb_context *c, uint64_t V, const char *names, c
   return 0;
 }
 
-}  // extern "C"
-
-namespace gtsbparse {
-
-// text -> device, physical lines indexed: c->p_line_end[l] = offset one past line l
-static int index_lines(gtsb_context *c, const char *text, uint64_t n, uint64_t *nlines_out) {
-  cudaStream_t s = c->stream;
-  const uint64_t nchunks = (n + CHUNK - 1) / CHUNK;
-  ENSURE(c->p_text, n + 8);
-  ENSURE(c->p_chunk_cnt, nchunks + 1);
-  ENSURE(c->p_chunk_off, (nchunks + 2) * 4);
-  ENSURE(c->scan_scratch, scan_scratch_elems(nchunks) * 4);
-  uint32_t *flags = c->p_flags.as<uint32_t>();
-  CK(cudaMemsetAsync(flags, 0, 16, s));
-  if (n) CK(cudaMemcpyAsync(c->p_text.p, text, n, cudaMemcpyHostToDevice, s));
-  const char *d_text = c->p_text.as<char>();
-  uint32_t newlines = 0;
-  if (nchunks) {
-    {
-      GTSB_TIMED("kp_chunk_newlines", s);
-      kp_chunk_newlines<<<blocks_for(nchunks, 256), 256, 0, s>>>(d_text, n, nchunks, c->p_chunk_cnt.as<uint8_t>(),
-                                                                flags);
-    }
-    exclusive_scan<uint8_t>(c->p_chunk_cnt.as<uint8_t>(), nchunks, c->p_chunk_off.as<uint32_t>(),
-                            c->scan_scratch.as<uint32_t>(), s);
-    c->stats.kernel_launches += 4;
-    CK(cudaMemcpyAsync(&newlines, c->p_chunk_off.as<uint32_t>() + nchunks, 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-  }
-  const bool open_end = n != 0 && text[n - 1] != '\n';       // last line without '\n'
-  const uint64_t nlines = (uint64_t) newlines + (open_end ? 1 : 0);
-  ENSURE(c->p_line_end, (nlines + 1) * 8);
-  uint64_t *line_end = c->p_line_end.as<uint64_t>();
-  if (newlines) {
-    GTSB_TIMED("kp_line_ends", s);
-    kp_line_ends<<<blocks_for(nchunks, 256), 256, 0, s>>>(d_text, n, nchunks, c->p_chunk_cnt.as<uint8_t>(),
-                                                          c->p_chunk_off.as<uint32_t>(), line_end);
-    c->stats.kernel_launches++;
-  }
-  if (open_end) CK(cudaMemcpyAsync(line_end + newlines, &n, 8, cudaMemcpyHostToDevice, s));
-  *nlines_out = nlines;
-  return 0;
-}
-
-}  // namespace gtsbparse
-
-namespace gtsbi {
-
-int parse_preamble(gtsb_context *c, const char *what, const char *text, uint64_t n) {
-  if (!c->have_names) return fail(c, "%s: vertex names not set", what);
-  if (n && text == nullptr) return fail(c, "%s: null argument", what);
-  // line and record counts are 32-bit sums over the text: every line and every record takes
-  // a byte at least, so below 4 GiB none of them can wrap
-  if (n >= (1ull << 32)) return fail(c, "%s: text of 4 GiB or more", what);
-  return 0;
-}
-
-// line index, then records per line: *total records, *irregular = the text's IRR_* bits
-int de_count(gtsb_context *c, const char *text, uint64_t n, uint64_t *nlines_out, uint32_t *total_out,
-             uint32_t *irregular_out) {
-  cudaStream_t s = c->stream;
-  uint64_t nlines = 0;
-  if (index_lines(c, text, n, &nlines) != 0) return -1;
-  ENSURE(c->p_line_cnt, (nlines + 1) * 4);
-  ENSURE(c->p_line_off, (nlines + 2) * 4);
-  ENSURE(c->scan_scratch, scan_scratch_elems(nlines) * 4);
-  const char *d_text = c->p_text.as<char>();
-  const uint64_t *line_end = c->p_line_end.as<uint64_t>();
-  uint32_t *flags = c->p_flags.as<uint32_t>();
-  const NameTable t{c->p_names.as<char>(), c->p_name_off.as<uint64_t>(), c->p_slots.as<uint64_t>(),
-                    c->names_mask};
-  Records out{};
-  uint32_t total = 0, irregular = 0;
-  if (nlines) {
-    {
-      GTSB_TIMED("kp_walk(count)", s);
-      kp_walk<false><<<blocks_for(nlines, 128), 128, 0, s>>>(d_text, line_end, nlines, t, out,
-                                                            c->p_line_cnt.as<uint32_t>(), nullptr, flags);
-    }
-    exclusive_scan<uint32_t>(c->p_line_cnt.as<uint32_t>(), nlines, c->p_line_off.as<uint32_t>(),
-                             c->scan_scratch.as<uint32_t>(), s);
-    c->stats.kernel_launches += 4;
-    CK(cudaMemcpyAsync(&total, c->p_line_off.as<uint32_t>() + nlines, 4, cudaMemcpyDeviceToHost, s));
-  }
-  CK(cudaMemcpyAsync(&irregular, flags, 4, cudaMemcpyDeviceToHost, s));
-  CK(cudaStreamSynchronize(s));
-  CK(cudaGetLastError());
-  *nlines_out = nlines;
-  *total_out = total;
-  *irregular_out = irregular;
-  return 0;
-}
-
-// the records de_count counted, written into the context's record columns
-int de_emit(gtsb_context *c, uint64_t nlines, uint32_t total) {
-  cudaStream_t s = c->stream;
-  const NameTable t{c->p_names.as<char>(), c->p_name_off.as<uint64_t>(), c->p_slots.as<uint64_t>(),
-                    c->names_mask};
-  const uint64_t R = total;
-  DevBuf *bs[] = {&c->root, &c->ctg, &c->dist, &c->std_dev, &c->flags};
-  for (DevBuf *b : bs)
-    if (!b->owned) *b = DevBuf();
-  ENSURE(c->root, R * 4);
-  ENSURE(c->ctg, R * 4);
-  ENSURE(c->dist, R * 4);
-  ENSURE(c->std_dev, R * 4);
-  ENSURE(c->flags, R);
-  ENSURE(c->num_pairs, R * 4);
-  const Records out{c->root.as<uint32_t>(), c->ctg.as<uint32_t>(), c->dist.as<int32_t>(), c->std_dev.as<float>(),
-                    c->num_pairs.as<uint32_t>(), c->flags.as<uint8_t>()};
-  if (R) {
-    GTSB_TIMED("kp_walk(emit)", s);
-    kp_walk<true><<<blocks_for(nlines, 128), 128, 0, s>>>(c->p_text.as<char>(), c->p_line_end.as<uint64_t>(), nlines,
-                                                         t, out, nullptr, c->p_line_off.as<uint32_t>(),
-                                                         c->p_flags.as<uint32_t>());
-    c->stats.kernel_launches++;
-    CK(cudaGetLastError());
-  }
-  return 0;
-}
-
-void keep_parsed_records(gtsb_context *c, uint64_t R) {
-  c->R = R;
-  c->have_records = true;
-  c->have_root_column = true;
-  c->have_lines = false;
-  c->have_num_pairs = true;
-  c->stats.nof_records = R;
-}
-
-// line index, the caller's values on the device, last[v] = offset + 1 of the last piece naming v
-int astat_last(gtsb_context *c, const char *text, uint64_t n, const float *astat, const float *copy_num,
-               uint64_t *nlines_out, uint32_t *irregular_out) {
-  cudaStream_t s = c->stream;
-  const uint64_t V = c->names_V;
-  uint64_t nlines = 0;
-  if (index_lines(c, text, n, &nlines) != 0) return -1;
-  ENSURE(c->p_last, (V + 1) * 8);
-  ENSURE(c->p_astat, (V + 1) * 4);
-  ENSURE(c->p_copy_num, (V + 1) * 4);
-  CK(cudaMemsetAsync(c->p_last.p, 0, (V + 1) * 8, s));
-  if (V) {
-    CK(cudaMemcpyAsync(c->p_astat.p, astat, V * 4, cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(c->p_copy_num.p, copy_num, V * 4, cudaMemcpyHostToDevice, s));
-  }
-  const NameTable t{c->p_names.as<char>(), c->p_name_off.as<uint64_t>(), c->p_slots.as<uint64_t>(),
-                    c->names_mask};
-  uint32_t *flags = c->p_flags.as<uint32_t>();
-  uint32_t irregular = 0;
-  if (nlines) {
-    GTSB_TIMED("kp_astat(last line)", s);
-    kp_astat<false><<<blocks_for(nlines, 128), 128, 0, s>>>(c->p_text.as<char>(), c->p_line_end.as<uint64_t>(),
-                                                           nlines, t, c->p_last.as<uint64_t>(),
-                                                           c->p_astat.as<float>(), c->p_copy_num.as<float>(), flags);
-    c->stats.kernel_launches++;
-  }
-  CK(cudaMemcpyAsync(&irregular, flags, 4, cudaMemcpyDeviceToHost, s));
-  CK(cudaStreamSynchronize(s));
-  CK(cudaGetLastError());
-  *nlines_out = nlines;
-  *irregular_out = irregular;
-  return 0;
-}
-
-// the piece at last[v] writes v's two values on the device
-int astat_apply(gtsb_context *c, uint64_t nlines) {
-  cudaStream_t s = c->stream;
-  if (nlines) {
-    const NameTable t{c->p_names.as<char>(), c->p_name_off.as<uint64_t>(), c->p_slots.as<uint64_t>(),
-                      c->names_mask};
-    GTSB_TIMED("kp_astat(apply)", s);
-    kp_astat<true><<<blocks_for(nlines, 128), 128, 0, s>>>(c->p_text.as<char>(), c->p_line_end.as<uint64_t>(),
-                                                          nlines, t, c->p_last.as<uint64_t>(),
-                                                          c->p_astat.as<float>(), c->p_copy_num.as<float>(),
-                                                          c->p_flags.as<uint32_t>());
-    c->stats.kernel_launches++;
-  }
-  return 0;
-}
-
-}  // namespace gtsbi
-
-extern "C" {
-
-int gtsb_parse_de_host(gtsb_context *c, const char *text, uint64_t n, uint64_t *nof_records,
-                       uint32_t *irregular_out) {
-  if (c == nullptr) return -1;
-  CK(cudaSetDevice(c->device));
-  if (dot_refuse_open(c, "gtsb_parse_de_host") != 0) return -1;
-  if (c->world > 1) return dist_parse_de(c, text, n, nof_records, irregular_out);
-  if (nof_records == nullptr || irregular_out == nullptr) return fail(c, "gtsb_parse_de_host: null argument");
-  if (parse_preamble(c, "gtsb_parse_de_host", text, n) != 0) return -1;
-  if (await_records(c) != 0) return -1;
-  ProfScope prof(c);
-  *nof_records = 0;
-  *irregular_out = 0;
-  c->have_records = false;
-  c->have_graph = false;
-  if (c->names_dup) {
-    *irregular_out = IRR_DUP_NAME;
-    return 0;
-  }
-  uint64_t nlines = 0;
-  uint32_t total = 0, irregular = 0;
-  if (de_count(c, text, n, &nlines, &total, &irregular) != 0) return -1;
-  if (irregular) {                     // nothing is kept: the caller parses this file on the host
-    *irregular_out = irregular;
-    return 0;
-  }
-  if (de_emit(c, nlines, total) != 0) return -1;
-  keep_parsed_records(c, total);
-  *nof_records = total;
-  return 0;
-}
-
-int gtsb_parse_astat_host(gtsb_context *c, const char *text, uint64_t n, float *astat, float *copy_num,
-                          uint32_t *irregular_out) {
-  if (c == nullptr) return -1;
-  CK(cudaSetDevice(c->device));
-  if (c->world > 1) return dist_parse_astat(c, text, n, astat, copy_num, irregular_out);
-  if (irregular_out == nullptr) return fail(c, "gtsb_parse_astat_host: null argument");
-  if (parse_preamble(c, "gtsb_parse_astat_host", text, n) != 0) return -1;
-  const uint64_t V = c->names_V;
-  if (V && (astat == nullptr || copy_num == nullptr)) return fail(c, "gtsb_parse_astat_host: null argument");
-  ProfScope prof(c);
-  cudaStream_t s = c->stream;
-  *irregular_out = 0;
-  if (c->names_dup) {
-    *irregular_out = IRR_DUP_NAME;
-    return 0;
-  }
-  uint64_t nlines = 0;
-  uint32_t irregular = 0;
-  if (astat_last(c, text, n, astat, copy_num, &nlines, &irregular) != 0) return -1;
-  if (irregular) {                     // nothing is touched: the caller reads this file on the host
-    *irregular_out = irregular;
-    return 0;
-  }
-  if (astat_apply(c, nlines) != 0) return -1;
-  if (V) {
-    CK(cudaMemcpyAsync(astat, c->p_astat.p, V * 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(copy_num, c->p_copy_num.p, V * 4, cudaMemcpyDeviceToHost, s));
-  }
-  CK(cudaStreamSynchronize(s));
-  CK(cudaGetLastError());
-  return 0;
-}
-
 int gtsb_get_records(gtsb_context *c, uint32_t *root, uint32_t *ctg, int32_t *dist, float *std_dev,
                      uint8_t *flags, uint32_t *num_pairs) {
   if (c == nullptr) return -1;
@@ -409,17 +151,21 @@ int gtsb_get_records(gtsb_context *c, uint32_t *root, uint32_t *ctg, int32_t *di
 
 }  // extern "C"
 
-// ================================================================ text fed in pieces
+// ================================================================ the text reader
 //
-// A step is a prefix of the bytes fed so far that ends where an fgets piece ends: after the last
-// '\n' of a full slot or, inside a physical line that runs past it, at line start + k * 1023.
-// walk_line and walk_astat_line cut a line into 1023-byte pieces from wherever they start, so a step
-// that starts at such a point holds exactly the pieces of the whole file; the bytes after the cut
-// (fewer than 1023) begin the next step.  The last step ends the file and may end without a '\n',
-// as index_lines allows.
+// Text is read in steps of a TextStream, fed in one of two ways:
+// - a stream (gtsb_*_stream_*, c->ts) copies the bytes fed into a pinned slot.  A step is a prefix
+//   of the bytes fed so far that ends where an fgets piece ends: after the last '\n' of a full slot
+//   or, inside a physical line that runs past it, at line start + k * 1023.  walk_line and
+//   walk_astat_line cut a line into 1023-byte pieces from wherever they start, so a step that starts
+//   at such a point holds exactly the pieces of the whole file; the bytes after the cut (fewer than
+//   1023) begin the next step.  The last step ends the file and may end without a '\n'.
+// - a whole-text call (gtsb_parse_*_host, c->whole) is that last step alone: the caller's bytes,
+//   copied from pageable memory into one device buffer.
+// Both end with a step of 0 bytes, which emits what the step before counted.
 //
 // One step, on the context's stream:
-//   A  the copy (pinned slot -> device slot, on the copy stream), kp_chunk_newlines, scan
+//   A  the copy (host bytes -> device slot, on the copy stream), kp_chunk_newlines, scan
 //   -- the one host synchronisation: IRR_* bits so far, the step's '\n' count, and the record count
 //      of the step before --
 //   C  .de: kp_walk(emit) of the step before, into the record columns at the running offset
@@ -428,12 +174,11 @@ int gtsb_get_records(gtsb_context *c, uint32_t *root, uint32_t *ctg, int32_t *di
 // The host fills the pinned slot again while C and B run, and the next copy runs beside them; two
 // device slots alternate, a copy waits for the kernels that read its slot.
 //
-// On a partitioned context (gtsb_dist_*_stream_begin) every rank streams its own chunk the same way;
-// only the end is collective (gtsb_dist.cu, dist_*_stream_end).
+// On a partitioned context (gtsb_dist_*_stream_begin, or a collective gtsb_parse_*_host) every rank
+// reads its own chunk the same way; only the end is collective (gtsb_dist.cu, dist_text_end).
 namespace gtsbi {
 
-void stream_close(gtsb_context *c) {
-  TextStream &ts = c->ts;
+void stream_close(TextStream &ts) {
   ts.kind = TextStream::CLOSED;
   ts.fill = ts.file_off = ts.R = ts.fed = 0;
   ts.last_byte = 0;
@@ -465,7 +210,7 @@ static uint64_t step_cut(const char *b, uint64_t n) {
 static int stream_error(gtsb_context *c) {
   TextStream &ts = c->ts;
   if (!ts.partitioned) {
-    stream_close(c);
+    stream_close(ts);
     return -1;
   }
   ts.failed = true;
@@ -473,9 +218,11 @@ static int stream_error(gtsb_context *c) {
   return -1;
 }
 
-// b holds `used` bytes: room for `need` (doubling), the bytes kept
+// b holds `used` bytes: room for `need` (doubling), the bytes kept.  Nothing to keep: exactly `need`,
+// as a whole-text call needs no room to grow.
 static int grow_keep(gtsb_context *c, DevBuf &b, uint64_t used, uint64_t need) {
-  if (b.p != nullptr && b.cap >= need) return 0;
+  if (used == 0) return ensure(c, b, need);
+  if (b.cap >= need) return 0;
   uint64_t cap = b.cap ? b.cap : 1ull << 16;
   while (cap < need) cap *= 2;
   void *p = nullptr;
@@ -491,10 +238,9 @@ static int grow_keep(gtsb_context *c, DevBuf &b, uint64_t used, uint64_t need) {
   return 0;
 }
 
-// one step: the first n bytes of the pinned slot.  n == 0: only the synchronisation and the
-// pending emit (end of the stream).
-static int stream_step(gtsb_context *c, uint64_t n) {
-  TextStream &ts = c->ts;
+// one step of ts: the n bytes at src (host memory).  n == 0: only the synchronisation and the
+// pending emit (end of the text).
+static int stream_step(gtsb_context *c, TextStream &ts, const char *src, uint64_t n) {
   cudaStream_t s = c->stream;
   uint32_t *h = (uint32_t *) (ts.host + host_tail(ts.slot));     // h[0] bits, h[1] '\n', h[2] records
   uint64_t *h_end = (uint64_t *) (h + 4);                         // end of an open last line
@@ -510,7 +256,7 @@ static int stream_step(gtsb_context *c, uint64_t n) {
     CK(cudaStreamWaitEvent(c->copy_stream, ts.ev_free[slot], 0));
     {
       GTSB_TIMED("stream h2d", c->copy_stream);
-      CK(cudaMemcpyAsync((void *) d_text, ts.host, n, cudaMemcpyHostToDevice, c->copy_stream));
+      CK(cudaMemcpyAsync((void *) d_text, src, n, cudaMemcpyHostToDevice, c->copy_stream));
     }
     CK(cudaEventRecord(ts.ev_copied, c->copy_stream));
     CK(cudaStreamWaitEvent(s, ts.ev_copied, 0));
@@ -528,11 +274,13 @@ static int stream_step(gtsb_context *c, uint64_t n) {
     CK(cudaMemcpyAsync(h + 1, c->p_chunk_off.as<uint32_t>() + nchunks, 4, cudaMemcpyDeviceToHost, s));
   }
   CK(cudaMemcpyAsync(h, flags, 4, cudaMemcpyDeviceToHost, s));
-  CK(cudaStreamSynchronize(s));           // the copy above has run: the pinned slot may be refilled
+  CK(cudaStreamSynchronize(s));           // the copy above has run: the host bytes may be refilled
   CK(cudaGetLastError());
   ts.irregular |= h[0];
-  if (ts.irregular) return 0;             // refused: no more device work
-  if (ts.pending) {                                               // C
+  // refused: no more device work.  A whole text (slot 0) is one step; it finishes its walks, so that
+  // it reports their bits too.
+  if (ts.irregular && ts.slot != 0) return 0;
+  if (ts.pending && ts.irregular == 0) {                          // C
     const uint64_t total = h[2], R = ts.R;
     if (R + total > STREAM_MAX_RECORDS)
       return fail(c, "gtsb_stream_feed: more than %llu records, the most gtsb_build takes",
@@ -557,7 +305,7 @@ static int stream_step(gtsb_context *c, uint64_t n) {
   }
   if (n == 0) return 0;
   const uint64_t newlines = h[1];                                 // B
-  const bool open_end = ts.host[n - 1] != '\n';
+  const bool open_end = src[n - 1] != '\n';
   const uint64_t nlines = newlines + (open_end ? 1 : 0);
   ENSURE(ts.line_end, (nlines + 1) * 8);
   uint64_t *line_end = ts.line_end.as<uint64_t>();
@@ -607,18 +355,10 @@ static int stream_step(gtsb_context *c, uint64_t n) {
   return 0;
 }
 
-// what every begin shares: a discarded open stream, the checks, the staging memory.  plain: for a
-// partitioned begin, the name of the single-device one; nullptr for that one itself.
-static int stream_prepare(gtsb_context *c, const char *what, const char *plain) {
-  TextStream &ts = c->ts;
-  stream_close(c);                                  // a new begin discards an open stream
-  if (dot_refuse_open(c, what) != 0) return -1;
-  if (plain == nullptr && c->world > 1)
-    return fail(c, "%s: a partitioned context reads text with the collective gtsb_parse_*_host calls or "
-                   "gtsb_dist_*_stream_begin", what);
-  if (plain != nullptr && c->world == 1)
-    return fail(c, "%s: not a partitioned context (one device reads text in pieces with %s)", what, plain);
-  if (!c->have_names) return fail(c, "%s: vertex names not set", what);
+
+// a stream's staging memory, its flags cleared: pinned, ts.slot bytes for the step being filled (none
+// for c->whole) and the 32 B the device reports into; text_bytes of device slots
+static int stream_memory(gtsb_context *c, TextStream &ts, uint64_t text_bytes) {
   const uint64_t host_bytes = host_tail(ts.slot) + 32;
   if (ts.host != nullptr && ts.host_cap != host_bytes) {
     CK(cudaFreeHost(ts.host));
@@ -628,7 +368,7 @@ static int stream_prepare(gtsb_context *c, const char *what, const char *plain) 
     CK(cudaMallocHost(&ts.host, host_bytes));
     ts.host_cap = host_bytes;
   }
-  ENSURE(ts.text, 2 * slot_stride(ts.slot));
+  ENSURE(ts.text, text_bytes);
   ENSURE(ts.flags, 16);
   for (cudaEvent_t *e : {&ts.ev_copied, &ts.ev_free[0], &ts.ev_free[1]})
     if (*e == nullptr) CK(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
@@ -637,20 +377,28 @@ static int stream_prepare(gtsb_context *c, const char *what, const char *plain) 
   return 0;
 }
 
-static int de_begin(gtsb_context *c, const char *what, const char *plain) {
-  if (stream_prepare(c, what, plain) != 0) return -1;
+// a .de read drops the context's records and grows its own into their columns, so that the context
+// holds one set of columns; columns the caller uploaded are dropped, and what an earlier read left in
+// ts (a stream closed by an error) is released
+static int de_open(gtsb_context *c, TextStream &ts) {
   if (await_records(c) != 0) return -1;
-  c->have_records = false;                          // as gtsb_parse_de_host: the old records are gone
+  c->have_records = false;
   c->have_graph = false;
-  c->ts.kind = TextStream::DE;
-  c->ts.irregular = c->names_dup ? IRR_DUP_NAME : 0;
+  DevBuf *mine[] = {&ts.root, &ts.ctg, &ts.dist, &ts.std_dev, &ts.rflags, &ts.num_pairs};
+  DevBuf *ctx[] = {&c->root, &c->ctg, &c->dist, &c->std_dev, &c->flags, &c->num_pairs};
+  for (int k = 0; k < 6; k++) {
+    release(*mine[k]);
+    if (ctx[k]->owned) *mine[k] = *ctx[k];
+    *ctx[k] = DevBuf();
+  }
+  ts.kind = TextStream::DE;
+  ts.irregular = c->names_dup ? IRR_DUP_NAME : 0;
   return 0;
 }
 
-static int astat_begin(gtsb_context *c, const char *what, const char *plain, const float *astat,
-                       const float *copy_num) {
-  if (stream_prepare(c, what, plain) != 0) return -1;
-  TextStream &ts = c->ts;
+// an .astat read applies its lines to the caller's values on the device
+static int astat_open(gtsb_context *c, TextStream &ts, const char *what, const float *astat,
+                      const float *copy_num) {
   const uint64_t V = c->names_V;
   if (V && (astat == nullptr || copy_num == nullptr)) return fail(c, "%s: null argument", what);
   cudaStream_t s = c->stream;
@@ -667,6 +415,31 @@ static int astat_begin(gtsb_context *c, const char *what, const char *plain, con
   return 0;
 }
 
+// what every begin shares: a discarded open stream, the checks, the staging memory.  plain: for a
+// partitioned begin, the name of the single-device one; nullptr for that one itself.
+static int stream_prepare(gtsb_context *c, const char *what, const char *plain) {
+  stream_close(c->ts);                              // a new begin discards an open stream
+  if (dot_refuse_open(c, what) != 0) return -1;
+  if (plain == nullptr && c->world > 1)
+    return fail(c, "%s: a partitioned context reads text with the collective gtsb_parse_*_host calls or "
+                   "gtsb_dist_*_stream_begin", what);
+  if (plain != nullptr && c->world == 1)
+    return fail(c, "%s: not a partitioned context (one device reads text in pieces with %s)", what, plain);
+  if (!c->have_names) return fail(c, "%s: vertex names not set", what);
+  return stream_memory(c, c->ts, 2 * slot_stride(c->ts.slot));
+}
+
+static int de_begin(gtsb_context *c, const char *what, const char *plain) {
+  if (stream_prepare(c, what, plain) != 0) return -1;
+  return de_open(c, c->ts);
+}
+
+static int astat_begin(gtsb_context *c, const char *what, const char *plain, const float *astat,
+                       const float *copy_num) {
+  if (stream_prepare(c, what, plain) != 0) return -1;
+  return astat_open(c, c->ts, what, astat, copy_num);
+}
+
 // a partitioned begin is local.  One that fails still leaves a stream open, failed, so that this
 // rank's end joins the other ranks' and the failure reaches all of them.
 static int dist_begun(gtsb_context *c, int rc, int kind) {
@@ -679,9 +452,30 @@ static int dist_begun(gtsb_context *c, int rc, int kind) {
 static int stream_end_check(gtsb_context *c, const char *what, int kind) {
   const int open = c->ts.kind;
   if (open == kind) return 0;
-  stream_close(c);
+  stream_close(c->ts);
   if (open == TextStream::CLOSED) return fail(c, "%s: no open stream", what);
   return fail(c, "%s: the open stream reads %s text", what, open == TextStream::DE ? ".de" : ".astat");
+}
+
+// a whole-text call's checks, then c->whole open on the caller's n bytes, its one step: they go from
+// pageable memory straight into a device buffer of n + 8 bytes
+static int whole_open(gtsb_context *c, const char *what, int kind, const char *text, uint64_t n,
+                      const float *astat, const float *copy_num) {
+  if (!c->have_names) return fail(c, "%s: vertex names not set", what);
+  if (n && text == nullptr) return fail(c, "%s: null argument", what);
+  // line and record counts are 32-bit sums over a step: every line and every record takes a byte at
+  // least, so below 4 GiB none of them can wrap
+  if (n >= (1ull << 32)) return fail(c, "%s: text of 4 GiB or more", what);
+  // the fgets pieces of a partitioned file's chunks are those of the whole file only if every chunk
+  // but the last ends a line
+  if (c->rank < c->world - 1 && n != 0 && text[n - 1] != '\n')
+    return fail(c, "%s: the chunk of rank %d does not end in '\\n' (only the last rank's may)", what, c->rank);
+  TextStream &ts = c->whole;
+  stream_close(ts);
+  ts.slot = 0;
+  if (stream_memory(c, ts, n + 8) != 0) return -1;
+  ts.fill = n;
+  return kind == TextStream::DE ? de_open(c, ts) : astat_open(c, ts, what, astat, copy_num);
 }
 
 }  // namespace gtsbparse
@@ -689,31 +483,30 @@ static int stream_end_check(gtsb_context *c, const char *what, int kind) {
 namespace gtsbi {
 
 // what every end does on its own device: a partitioned stream's failure and chunk rule, then the
-// remaining bytes as the last step and the synchronisation that reads its results (ts.irregular and
-// ts.R are the stream's), and record columns that exist, so that adopting them cannot fail
-int stream_end_local(gtsb_context *c, const char *what, int kind) {
-  TextStream &ts = c->ts;
+// remaining bytes (at src) as the last step and the synchronisation that reads its results
+// (ts.irregular and ts.R are the read's), and record columns that exist, so that adopting them
+// cannot fail
+int stream_end_local(gtsb_context *c, TextStream &ts, const char *src, const char *what, int kind) {
   if (ts.kind != kind)
     return fail(c, "%s: the open stream reads %s text", what, ts.kind == TextStream::DE ? ".de" : ".astat");
   if (ts.failed) {
     c->err = ts.fail_msg;
     return -1;
   }
-  // as dist_text_checks: the fgets pieces of the chunks are those of the whole file only if every
-  // chunk but the last ends a line.  A refused stream is exempt: its caller may stop feeding.
+  // the chunk rule of whole_open, from the last byte fed.  A refused stream is exempt: its caller may
+  // stop feeding.
   if (c->rank < c->world - 1 && ts.irregular == 0 && ts.fed != 0 && ts.last_byte != '\n')
     return fail(c, "%s: the chunk of rank %d does not end in '\\n' (only the last rank's may)", what, c->rank);
-  if (ts.irregular == 0 && stream_step(c, ts.fill) != 0) return -1;
-  if (ts.irregular == 0 && stream_step(c, 0) != 0) return -1;
+  if (ts.irregular == 0 && stream_step(c, ts, src, ts.fill) != 0) return -1;
+  if ((ts.irregular == 0 || ts.slot == 0) && stream_step(c, ts, src, 0) != 0) return -1;
   if (kind == TextStream::DE)
     for (DevBuf *b : {&ts.root, &ts.ctg, &ts.dist, &ts.std_dev, &ts.rflags, &ts.num_pairs})
       if (b->p == nullptr) ENSURE(*b, 16);
   return 0;
 }
 
-// the stream's columns become the context's records
-void adopt_stream_records(gtsb_context *c, uint64_t R) {
-  TextStream &ts = c->ts;
+// ts's columns become the context's records
+void adopt_stream_records(gtsb_context *c, TextStream &ts, uint64_t R) {
   DevBuf *mine[] = {&ts.root, &ts.ctg, &ts.dist, &ts.std_dev, &ts.rflags, &ts.num_pairs};
   DevBuf *ctx[] = {&c->root, &c->ctg, &c->dist, &c->std_dev, &c->flags, &c->num_pairs};
   for (int k = 0; k < 6; k++) {
@@ -721,23 +514,106 @@ void adopt_stream_records(gtsb_context *c, uint64_t R) {
     *ctx[k] = *mine[k];
     *mine[k] = DevBuf();
   }
-  keep_parsed_records(c, R);
+  c->R = R;
+  c->have_records = true;
+  c->have_root_column = true;
+  c->have_lines = false;
+  c->have_num_pairs = true;
+  c->stats.nof_records = R;
+}
+
+// a .de read that keeps no records: its columns are given back to the device
+void release_stream_records(TextStream &ts) {
+  for (DevBuf *b : {&ts.root, &ts.ctg, &ts.dist, &ts.std_dev, &ts.rflags, &ts.num_pairs}) release(*b);
 }
 
 void text_stream_release(gtsb_context *c) {
-  TextStream &ts = c->ts;
-  if (ts.host != nullptr) cudaFreeHost(ts.host);
-  ts.host = nullptr;
-  for (DevBuf *b : {&ts.text, &ts.line_end, &ts.line_off, &ts.flags, &ts.root, &ts.ctg, &ts.dist, &ts.std_dev,
-                    &ts.rflags, &ts.num_pairs, &ts.last, &ts.astat, &ts.copy_num})
-    release(*b);
-  for (cudaEvent_t e : {ts.ev_copied, ts.ev_free[0], ts.ev_free[1]})
-    if (e != nullptr) cudaEventDestroy(e);
+  for (TextStream *ts : {&c->ts, &c->whole}) {
+    if (ts->host != nullptr) cudaFreeHost(ts->host);
+    ts->host = nullptr;
+    release_stream_records(*ts);
+    for (DevBuf *b : {&ts->text, &ts->line_end, &ts->line_off, &ts->flags, &ts->last, &ts->astat, &ts->copy_num})
+      release(*b);
+    for (cudaEvent_t e : {ts->ev_copied, ts->ev_free[0], ts->ev_free[1]})
+      if (e != nullptr) cudaEventDestroy(e);
+  }
 }
 
 }  // namespace gtsbi
 
+namespace gtsbparse {
+
+// the end of a read on one device: its last steps, then the records kept or the .astat values
+// returned (nof_records: .de, astat and copy_num: .astat)
+static int text_end(gtsb_context *c, TextStream &ts, const char *src, const char *what, int kind,
+                    uint64_t *nof_records, float *astat, float *copy_num, uint32_t *irregular) {
+  if (nof_records != nullptr) *nof_records = 0;
+  *irregular = 0;
+  const int rc = stream_end_local(c, ts, src, what, kind);
+  const uint32_t irr = ts.irregular;
+  const uint64_t R = ts.R;
+  stream_close(ts);
+  if (kind == TextStream::DE && (rc != 0 || irr)) release_stream_records(ts);
+  if (rc != 0) return -1;
+  if (irr) {                     // nothing is kept or touched: the caller reads this file on the host
+    *irregular = irr;
+    return 0;
+  }
+  if (kind == TextStream::DE) {
+    adopt_stream_records(c, ts, R);
+    *nof_records = R;
+    return 0;
+  }
+  const uint64_t V = c->names_V;
+  cudaStream_t s = c->stream;
+  if (V) {
+    CK(cudaMemcpyAsync(astat, ts.astat.p, V * 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(copy_num, ts.copy_num.p, V * 4, cudaMemcpyDeviceToHost, s));
+  }
+  CK(cudaStreamSynchronize(s));
+  CK(cudaGetLastError());
+  return 0;
+}
+
+}  // namespace gtsbparse
+
 extern "C" {
+
+int gtsb_parse_de_host(gtsb_context *c, const char *text, uint64_t n, uint64_t *nof_records,
+                       uint32_t *irregular_out) {
+  const char *what = "gtsb_parse_de_host";
+  if (c == nullptr) return -1;
+  CK(cudaSetDevice(c->device));
+  if (dot_refuse_open(c, what) != 0) return -1;
+  const bool null_arg = nof_records == nullptr || irregular_out == nullptr;
+  ProfScope prof(c);
+  if (c->world > 1) {
+    const int rc = null_arg ? fail(c, "%s: null argument", what)
+                            : whole_open(c, what, TextStream::DE, text, n, nullptr, nullptr);
+    c->have_records = false;           // also after an error, on every rank
+    c->have_graph = false;
+    return dist_text_end(c, c->whole, text, what, TextStream::DE, "parse", rc, nof_records, nullptr, nullptr,
+                         irregular_out);
+  }
+  if (null_arg) return fail(c, "%s: null argument", what);
+  if (whole_open(c, what, TextStream::DE, text, n, nullptr, nullptr) != 0) return -1;
+  return text_end(c, c->whole, text, what, TextStream::DE, nof_records, nullptr, nullptr, irregular_out);
+}
+
+int gtsb_parse_astat_host(gtsb_context *c, const char *text, uint64_t n, float *astat, float *copy_num,
+                          uint32_t *irregular_out) {
+  const char *what = "gtsb_parse_astat_host";
+  if (c == nullptr) return -1;
+  CK(cudaSetDevice(c->device));
+  ProfScope prof(c);
+  const int rc = irregular_out == nullptr ? fail(c, "%s: null argument", what)
+                                          : whole_open(c, what, TextStream::ASTAT, text, n, astat, copy_num);
+  if (c->world > 1)
+    return dist_text_end(c, c->whole, text, what, TextStream::ASTAT, "parse", rc, nullptr, astat, copy_num,
+                         irregular_out);
+  if (rc != 0) return -1;
+  return text_end(c, c->whole, text, what, TextStream::ASTAT, nullptr, astat, copy_num, irregular_out);
+}
 
 int gtsb_stream_set_slot(gtsb_context *c, uint64_t bytes) {
   if (c == nullptr) return -1;
@@ -803,7 +679,7 @@ int gtsb_stream_feed(gtsb_context *c, const char *bytes, uint64_t n, uint32_t *i
     n -= take;
     if (ts.fill < ts.slot) break;
     const uint64_t cut = step_cut(ts.host, ts.fill);
-    if (stream_step(c, cut) != 0) return stream_error(c);
+    if (stream_step(c, ts, ts.host, cut) != 0) return stream_error(c);
     memmove(ts.host, ts.host + cut, ts.fill - cut);
     ts.file_off += cut;
     ts.fill -= cut;
@@ -813,61 +689,42 @@ int gtsb_stream_feed(gtsb_context *c, const char *bytes, uint64_t n, uint32_t *i
 }
 
 int gtsb_de_stream_end(gtsb_context *c, uint64_t *nof_records, uint32_t *irregular) {
+  const char *what = "gtsb_de_stream_end";
   if (c == nullptr) return -1;
   CK(cudaSetDevice(c->device));
-  if (c->ts.partitioned) return dist_de_stream_end(c, nof_records, irregular);
-  if (stream_end_check(c, "gtsb_de_stream_end", TextStream::DE) != 0) return -1;
-  TextStream &ts = c->ts;
-  if (nof_records == nullptr || irregular == nullptr) {
-    stream_close(c);
-    return fail(c, "gtsb_de_stream_end: null argument");
+  const bool null_arg = nof_records == nullptr || irregular == nullptr;
+  if (c->ts.partitioned) {
+    ProfScope prof(c);
+    return dist_text_end(c, c->ts, c->ts.host, what, TextStream::DE, "stream",
+                         null_arg ? fail(c, "%s: null argument", what) : 0, nof_records, nullptr, nullptr, irregular);
+  }
+  if (stream_end_check(c, what, TextStream::DE) != 0) return -1;
+  if (null_arg) {
+    stream_close(c->ts);
+    return fail(c, "%s: null argument", what);
   }
   ProfScope prof(c);
-  *nof_records = 0;
-  *irregular = 0;
-  const int rc = stream_end_local(c, "gtsb_de_stream_end", TextStream::DE);
-  const uint32_t irr = ts.irregular;
-  const uint64_t R = ts.R;
-  stream_close(c);
-  if (rc != 0) return -1;
-  if (irr) {                                        // nothing is kept: the caller parses this file on the host
-    *irregular = irr;
-    return 0;
-  }
-  adopt_stream_records(c, R);
-  *nof_records = R;
-  return 0;
+  return text_end(c, c->ts, c->ts.host, what, TextStream::DE, nof_records, nullptr, nullptr, irregular);
 }
 
 int gtsb_astat_stream_end(gtsb_context *c, float *astat, float *copy_num, uint32_t *irregular) {
+  const char *what = "gtsb_astat_stream_end";
   if (c == nullptr) return -1;
   CK(cudaSetDevice(c->device));
-  if (c->ts.partitioned) return dist_astat_stream_end(c, astat, copy_num, irregular);
-  if (stream_end_check(c, "gtsb_astat_stream_end", TextStream::ASTAT) != 0) return -1;
-  TextStream &ts = c->ts;
   const uint64_t V = c->names_V;
-  if (irregular == nullptr || (V && (astat == nullptr || copy_num == nullptr))) {
-    stream_close(c);
-    return fail(c, "gtsb_astat_stream_end: null argument");
+  const bool null_arg = irregular == nullptr || (V && (astat == nullptr || copy_num == nullptr));
+  if (c->ts.partitioned) {
+    ProfScope prof(c);
+    return dist_text_end(c, c->ts, c->ts.host, what, TextStream::ASTAT, "stream",
+                         null_arg ? fail(c, "%s: null argument", what) : 0, nullptr, astat, copy_num, irregular);
+  }
+  if (stream_end_check(c, what, TextStream::ASTAT) != 0) return -1;
+  if (null_arg) {
+    stream_close(c->ts);
+    return fail(c, "%s: null argument", what);
   }
   ProfScope prof(c);
-  *irregular = 0;
-  const int rc = stream_end_local(c, "gtsb_astat_stream_end", TextStream::ASTAT);
-  const uint32_t irr = ts.irregular;
-  stream_close(c);
-  if (rc != 0) return -1;
-  if (irr) {                                        // nothing is touched: the caller reads this file on the host
-    *irregular = irr;
-    return 0;
-  }
-  cudaStream_t s = c->stream;
-  if (V) {
-    CK(cudaMemcpyAsync(astat, ts.astat.p, V * 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(copy_num, ts.copy_num.p, V * 4, cudaMemcpyDeviceToHost, s));
-  }
-  CK(cudaStreamSynchronize(s));
-  CK(cudaGetLastError());
-  return 0;
+  return text_end(c, c->ts, c->ts.host, what, TextStream::ASTAT, nullptr, astat, copy_num, irregular);
 }
 
 }  // extern "C"

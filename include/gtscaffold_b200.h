@@ -171,10 +171,11 @@ int gtsb_parse_de_host(gtsb_context *ctx, const char *text, uint64_t text_bytes,
 int gtsb_parse_astat_host(gtsb_context *ctx, const char *text, uint64_t text_bytes, float *astat,
                           float *copy_num, uint32_t *irregular);
 /* ---- the same two readings for text fed in pieces: no size limit, bounded memory, and the copy of
-   each piece overlapping the kernels of the piece before.  gtsb_de_stream_begin /
-   gtsb_astat_stream_begin take single-device contexts only: on a partitioned context (after
-   gtsb_dist_init) they fail, and ranks use the collective calls above or the partitioned stream
-   below.
+   each piece overlapping the kernels of the piece before.  The single calls above are this reading
+   with the whole text as its one step, copied from the caller's memory without a pinned slot.
+   gtsb_de_stream_begin / gtsb_astat_stream_begin take single-device contexts only: on a partitioned
+   context (after gtsb_dist_init) they fail, and ranks use the collective calls above or the
+   partitioned stream below.
 
      gtsb_de_stream_begin / gtsb_astat_stream_begin   open a stream (an open one is discarded)
      gtsb_stream_feed     the next bytes of the file
@@ -194,8 +195,8 @@ int gtsb_parse_astat_host(gtsb_context *ctx, const char *text, uint64_t text_byt
    for none); end writes astat / copy_num only when it succeeds with *irregular == 0.
    Errors: feed or end without an open stream, end of the other kind, a null argument, a CUDA or
    allocation error -- each closes a single-device stream.  gtsb_set_vertex_names_host fails while a stream is
-   open.  Other calls on the context may run between feeds; the single-call entry points keep
-   their own buffers.
+   open.  Other calls on the context may run between feeds; the single calls read through a stream of
+   their own and leave an open one as it was.
    Memory: the stream copies through one pinned host slot and two device slots of 64 MiB
    (gtsb_stream_set_slot), plus the line index of one slot (16 B per line) and, for .de, the
    record columns (21 B per record, grown by doubling).  They stay allocated for the next stream

@@ -343,19 +343,30 @@ static inline cudaError_t cudaDeviceGetAttribute(int *v, cudaDeviceAttr a, int) 
 static inline cudaError_t cudaGetLastError() { return cudaSuccess; }
 static inline const char *cudaGetErrorString(cudaError_t) { return "cusim error"; }
 static inline const char *cudaGetErrorName(cudaError_t) { return "cusimError"; }
-static inline cudaError_t cudaMalloc(void **p, size_t n) { *p = calloc(n ? n : 1, 1); return *p ? cudaSuccess : cudaErrorMemoryAllocation; }
+// counted for the tests: allocations not yet freed (cusim_live_allocs), host synchronisations (cusim_stream_syncs)
+namespace cusim { extern long long live_allocs; extern unsigned long long stream_syncs; }
+static inline cudaError_t cudaMalloc(void **p, size_t n) {
+  *p = calloc(n ? n : 1, 1);
+  if (*p == nullptr) return cudaErrorMemoryAllocation;
+  __atomic_add_fetch(&cusim::live_allocs, 1, __ATOMIC_RELAXED);
+  return cudaSuccess;
+}
 template <typename P> static inline cudaError_t cudaMalloc(P **p, size_t n) { return cudaMalloc((void **) p, n); }
-static inline cudaError_t cudaFree(void *p) { free(p); return cudaSuccess; }
+static inline cudaError_t cudaFree(void *p) {
+  if (p != nullptr) __atomic_sub_fetch(&cusim::live_allocs, 1, __ATOMIC_RELAXED);
+  free(p);
+  return cudaSuccess;
+}
 static inline cudaError_t cudaMallocHost(void **p, size_t n) { return cudaMalloc(p, n); }
 template <typename P> static inline cudaError_t cudaMallocHost(P **p, size_t n) { return cudaMalloc((void **) p, n); }
-static inline cudaError_t cudaFreeHost(void *p) { free(p); return cudaSuccess; }
+static inline cudaError_t cudaFreeHost(void *p) { return cudaFree(p); }
 static inline cudaError_t cudaMemcpy(void *d, const void *s, size_t n, cudaMemcpyKind) { if (n) memmove(d, s, n); return cudaSuccess; }
 static inline cudaError_t cudaMemcpyAsync(void *d, const void *s, size_t n, cudaMemcpyKind, cudaStream_t = nullptr) { if (n) memmove(d, s, n); return cudaSuccess; }
 static inline cudaError_t cudaMemset(void *d, int v, size_t n) { if (n) memset(d, v, n); return cudaSuccess; }
 static inline cudaError_t cudaMemsetAsync(void *d, int v, size_t n, cudaStream_t = nullptr) { if (n) memset(d, v, n); return cudaSuccess; }
 static inline cudaError_t cudaStreamCreateWithFlags(cudaStream_t *s, unsigned) { *s = (cudaStream_t) malloc(8); return cudaSuccess; }
 static inline cudaError_t cudaStreamDestroy(cudaStream_t s) { free(s); return cudaSuccess; }
-static inline cudaError_t cudaStreamSynchronize(cudaStream_t) { return cudaSuccess; }
+static inline cudaError_t cudaStreamSynchronize(cudaStream_t) { __atomic_add_fetch(&cusim::stream_syncs, 1, __ATOMIC_RELAXED); return cudaSuccess; }
 static inline cudaError_t cudaDeviceSynchronize() { return cudaSuccess; }
 static inline cudaError_t cudaStreamWaitEvent(cudaStream_t, cudaEvent_t, unsigned = 0) { return cudaSuccess; }
 // events carry the host's clock: cudaEventElapsedTime is emulation time, useful only to see which

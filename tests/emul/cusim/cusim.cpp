@@ -294,7 +294,19 @@ void run_grid_coop(dim3 grid, dim3 blk, size_t smem, const std::function<void()>
   body = nullptr;
 }
 
+long long live_allocs = 0;
+unsigned long long stream_syncs = 0;
+
 }  // namespace cusim
+
+// device and pinned allocations not yet freed, and host synchronisations (cudaStreamSynchronize) so
+// far, of all contexts
+extern "C" long long cusim_live_allocs() {
+  return __atomic_load_n(&cusim::live_allocs, __ATOMIC_RELAXED);
+}
+extern "C" unsigned long long cusim_stream_syncs() {
+  return __atomic_load_n(&cusim::stream_syncs, __ATOMIC_RELAXED);
+}
 
 // the order of the threads' turns from now on (see CUSIM_ORDER)
 extern "C" void cusim_set_order(uint64_t mode) {

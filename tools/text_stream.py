@@ -9,8 +9,7 @@ The text is the seeded C3-shaped graph formatted as canonical .de text (tests/or
   * the stream (parse_*_pieces) fed 16, 64 and 256 MiB pieces, memoryview slices of the same bytes;
   * call time: host clock around the call and a device synchronisation, the best of --reps;
     kernel time and copy time: per-label CUDA events of a separate profiled call (gtsb_set_profile;
-    the stream's copy is "stream h2d", the single call's copy has no label, so its copy time is that
-    of torch copying the same pageable bytes to the device);
+    the copy of the text is "stream h2d" in both, the single call's straight from pageable memory);
   * text GB/s = bytes / call time, and whether the result equals the single call's;
   * a run past 4 GiB: the .de text repeated until it passes 2^32 bytes, in pieces of 37 MiB + 13 B,
     and the .astat text repeated until it does, then a different text that must win.
@@ -86,7 +85,6 @@ def main():
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
-    import torch
     import oracle_lib as O
     pkg = importlib.import_module("gt-scaffold_b200")
     name, power = gpu_name_and_power_limit(0)
@@ -107,24 +105,12 @@ def main():
     z = np.zeros(V, np.float32)
     rows = []
 
-    def pageable_copy_ms(t):
-        src = torch.frombuffer(bytearray(t), dtype=torch.uint8)
-        dst = torch.empty(len(t), dtype=torch.uint8, device="cuda")
-        ts = []
-        for _ in range(args.reps):
-            torch.cuda.synchronize()
-            t0 = time.perf_counter()
-            dst.copy_(src)
-            torch.cuda.synchronize()
-            ts.append((time.perf_counter() - t0) * 1e3)
-        return min(ts)
-
     # ---- .de
     g.parse_de(text)                                                # warm-up: allocations
     single = g.records()
     ms, _ = best_ms(lambda: g.parse_de(text), g, args.reps)
-    k, _, kern = profiled(lambda: g.parse_de(text), g)
-    rows.append(row("de single", len(text), ms, k, pageable_copy_ms(text), True, kern))
+    k, cp, kern = profiled(lambda: g.parse_de(text), g)
+    rows.append(row("de single", len(text), ms, k, cp, True, kern))
     for feed in (16 * MiB, 64 * MiB, 256 * MiB):
         run = lambda: g.parse_de_pieces(pieces_of(text, feed))       # noqa: E731
         run()
@@ -147,8 +133,8 @@ def main():
     # ---- .astat
     _, ea, ec = g.parse_astat(atext, z, z)
     ms, _ = best_ms(lambda: g.parse_astat(atext, z, z), g, args.reps)
-    k, _, kern = profiled(lambda: g.parse_astat(atext, z, z), g)
-    rows.append(row("astat single", len(atext), ms, k, pageable_copy_ms(atext), True, kern))
+    k, cp, kern = profiled(lambda: g.parse_astat(atext, z, z), g)
+    rows.append(row("astat single", len(atext), ms, k, cp, True, kern))
     for feed in (16 * MiB, 64 * MiB, 256 * MiB):
         run = lambda: g.parse_astat_pieces(pieces_of(atext, feed), z, z)     # noqa: E731
         run()
