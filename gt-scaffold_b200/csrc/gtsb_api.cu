@@ -40,6 +40,7 @@ int ensure(gtsb_context *c, DevBuf &b, size_t bytes) {
   b.p = nullptr;
   b.owned = true;
   b.cap = 0;
+  c->n_allocs++;
   // grow with some headroom so that repeated calls at one size never realloc
   CK(cudaMalloc(&b.p, bytes));
   b.cap = bytes;
@@ -556,185 +557,6 @@ int do_mark_repeats(gtsb_context *c, float cn_cutoff, float astat_cutoff, int us
   return 0;
 }
 
-// work arrays of the filter: per-vertex ones for Vg vertices, proposals for E slots
-uint64_t proposal_capacity(uint64_t E) { return E / 4 + 65536 < E + 1 ? E / 4 + 65536 : E + 1; }
-
-int ensure_filter_buffers(gtsb_context *c, uint64_t V, uint64_t E, FilterArgs &a) {
-  // proposals are rare (a pair needs two low copy numbers and an ambiguous order); room for E / 4,
-  // the single-device filter reruns the pairs pass with room for all E when that overflows
-  const uint64_t prop_cap = proposal_capacity(E) > c->proposals.cap / sizeof(uint2) ? proposal_capacity(E)
-                                                                                    : c->proposals.cap / sizeof(uint2);
-  ENSURE(c->proposals, prop_cap * sizeof(uint2));
-  ENSURE(c->poly_cur, (V + 1) * 4);
-  ENSURE(c->poly_new, (V + 1) * 4);
-  ENSURE(c->gbits, V + 1);
-  ENSURE(c->fstat, V + 1);
-  ENSURE(c->work_a, (V + 1) * 4);
-  ENSURE(c->work_b, (V + 1) * 4);
-  ENSURE(c->vinfo, (V + 1) * sizeof(uint2));
-  ENSURE(c->vres, (V + 1) * 4);
-  ENSURE(c->vsum, V + 1);
-  ENSURE(c->dirty, V + 1);
-  a.big_blocks = (uint32_t) c->sm_count * 2;
-  if (c->n_big_rows) {
-    if (a.big_blocks > c->n_big_rows) a.big_blocks = c->n_big_rows;
-    ENSURE(c->big_scratch, (size_t) a.big_blocks * c->max_deg * BIG_SCRATCH_STRIDE);
-  }
-  static const int split_hubs = [] {
-    const char *e = getenv("GTSB_HUBS");                 // 0: a block per hub row, as in round 1 (dev switch)
-    return (e != nullptr && atoi(e) == 0) ? 0 : 1;
-  }();
-  if (split_hubs && c->world == 1 && c->n_big_rows && c->max_deg > HUB_ROW) {
-    const uint64_t cap = E / HUB_LCH + c->n_big_rows + 1;
-    ENSURE(c->hub_cn, (E + 1) * 4);
-    ENSURE(c->hub_low, (E + 1) * 4);
-    ENSURE(c->hub_mark, E + 1);
-    ENSURE(c->hub_nlow, ((uint64_t) c->n_big_rows + 1) * 4);
-    ENSURE(c->hub_items, cap * sizeof(uint2));
-    a.hub_cn = c->hub_cn.as<float>();
-    a.hub_low = c->hub_low.as<uint32_t>();
-    a.hub_mark = c->hub_mark.as<uint8_t>();
-    a.hub_nlow = c->hub_nlow.as<uint32_t>();
-    a.hub_items = c->hub_items.as<uint2>();
-    a.hub_items_cap = (uint32_t) (cap > 0xFFFFFFFFull ? 0xFFFFFFFFull : cap);
-  }
-  a.g = graph_args(c);
-  a.proposals = c->proposals.as<uint2>();
-  a.proposals_cap = (uint32_t) (prop_cap > E + 1 ? E + 1 : prop_cap);
-  a.poly_cur = c->poly_cur.as<uint32_t>();
-  a.poly_new = c->poly_new.as<uint32_t>();
-  a.gbits = c->gbits.as<uint8_t>();
-  a.fstat = c->fstat.as<uint8_t>();
-  a.dirty = c->dirty.as<uint8_t>();
-  a.rep_pred = c->rep_pred.as<uint8_t>();
-  a.work_a = c->work_a.as<uint32_t>();
-  a.work_b = c->work_b.as<uint32_t>();
-  a.big_scratch = c->big_scratch.as<uint8_t>();
-  a.vinfo = c->vinfo.as<uint2>();
-  a.vres = c->vres.as<uint32_t>();
-  a.vsum = c->vsum.as<uint8_t>();
-  return 0;
-}
-
-// fused = the three stages back to back on a fresh graph (gtsb_pipeline): the
-// repeat predicate is evaluated inside the vertex-facts pass and the REPEAT edge
-// marks (pred(v) || pred(w)) are derived by the final pass instead of being
-// stored first and overwritten later
-int do_filter(gtsb_context *c, float pcutoff, float cncutoff, int64_t ocutoff, bool fused = false,
-              float cn_cutoff = 0.f, float astat_cutoff = 0.f, int use_cn = 0) {
-  ProfScope ps_(c);
-  if (!c->have_graph) return fail(c, "gtsb_filter: no graph (call gtsb_build or gtsb_set_graph_host)");
-  if (await_vertices(c) != 0) return -1;
-  if (get_ambig(c, pcutoff) != 0) return -1;
-  c->csr_exported = false;
-  const uint64_t V = c->V, E = c->E;
-  cudaStream_t s = c->stream;
-  FilterArgs a{};
-  if (ensure_filter_buffers(c, V, E, a) != 0) return -1;
-  a.ambig = c->ambig;
-  a.cncutoff = cncutoff;
-  a.ocutoff = ocutoff;
-  a.fused_repeats = fused ? 1 : 0;
-
-  uint32_t *cnt = c->counters.as<uint32_t>();
-  CK(cudaMemsetAsync(cnt + CNT_PROPOSALS, 0, (CNT_NUM - CNT_PROPOSALS) * 4, s));
-  CK(cudaMemsetAsync(c->poly_cur.p, 0xFF, (V + 1) * 4, s));
-  CK(cudaMemsetAsync(c->poly_new.p, 0xFF, (V + 1) * 4, s));
-  CK(cudaMemsetAsync(c->dirty.p, 0, V + 1, s));
-  CK(cudaMemsetAsync(c->gbits.p, 0, V + 1, s));
-  CK(cudaMemsetAsync(c->fstat.p, 0x0C, V + 1, s));      // rows without slots: decided, nothing fires
-  // phase 1: who proposes whom (+ the static overlap answer of every small row)
-  launch_vertex_facts(a, fused ? 1 : 0, cn_cutoff, astat_cutoff, use_cn, s);
-  launch_pairs(a, s);
-  c->stats.kernel_launches += (V ? 1 : 0) + (E ? 2 : 0) + (E && c->n_big_rows ? 1 : 0);
-  if (read_counters(c) != 0) return -1;
-  if (c->h_counters[CNT_ERROR] & 4u) return fail(c, "gtsb_filter: a contig is longer than 2^31-1");
-  if (c->h_counters[CNT_OVERFLOW] && a.proposals_cap < E + 1) {
-    // more proposals than the list was sized for: once more with room for every slot
-    ENSURE(c->proposals, (E + 1) * sizeof(uint2));
-    a.proposals = c->proposals.as<uint2>();
-    a.proposals_cap = (uint32_t) (E + 1);
-    CK(cudaMemsetAsync(cnt + CNT_PROPOSALS, 0, 4, s));
-    CK(cudaMemsetAsync(cnt + CNT_OVERFLOW, 0, 4, s));
-    CK(cudaMemsetAsync(c->gbits.p, 0, V + 1, s));
-    launch_pairs(a, s);
-    c->stats.kernel_launches += (E ? 2 : 0) + (E && c->n_big_rows ? 1 : 0);
-    if (read_counters(c) != 0) return -1;
-  }
-  if (c->h_counters[CNT_OVERFLOW]) return fail(c, "gtsb_filter: proposal list overflow");
-  const uint32_t nprop = c->h_counters[CNT_PROPOSALS];
-  c->stats.proposals = nprop;
-  c->stats.poly_sweeps = 0;
-  if (nprop) {
-    for (;;) {
-      // a few sweeps per host synchronisation; converged when the last one changed nothing
-      for (int k = 0; k < POLY_SWEEPS_PER_SYNC; k++) {
-        CK(cudaMemsetAsync(cnt + CNT_POLY_CHANGED, 0, 4, s));
-        launch_poly_sweep(a, nprop, s);
-        c->stats.kernel_launches += 3;
-        c->stats.poly_sweeps++;
-      }
-      if (read_counters(c) != 0) return -1;
-      if (!c->h_counters[CNT_POLY_CHANGED]) break;
-      if (c->stats.poly_sweeps > V + 2) return fail(c, "gtsb_filter: polyTime sweeps did not converge");
-    }
-    launch_dirty(a, nprop, s);
-    c->stats.kernel_launches += 1;
-  }
-  // phase 2: fire candidates (static answer, recomputed next to polymorphic
-  // vertices), then the order-respecting fire fixpoint
-  static const int coop = [] {
-    const char *e = getenv("GTSB_FIRE");                 // 1: one launch per fire round (dev switch)
-    return (e != nullptr && atoi(e) == 1) ? 0 : 1;
-  }();
-  // the worklist that fire_init_big and the dense round fill: its length lives in ring[0] when
-  // the cooperative rounds kernel follows (the counters were cleared above)
-  uint32_t *n_dense = coop ? cnt + CNT_RING0 : cnt + CNT_WORK_B;
-  CK(cudaMemsetAsync(n_dense, 0, 4, s));
-  launch_fire_init(a, n_dense, s);
-  c->stats.kernel_launches += (V ? 1 : 0) + (V && c->n_big_rows ? 1 : 0);
-  c->stats.fire_rounds = 0;
-  c->fire_ring_pending = false;
-  uint32_t *win = a.work_b, *wout = a.work_a;
-  int in_idx = CNT_WORK_B, out_idx = CNT_WORK_A;
-  uint32_t n_in = 0;
-  bool rounds_done = false;
-  if (ocutoff >= 0 && V) {
-    launch_fire_dense(a, a.work_b, n_dense, s);
-    c->stats.kernel_launches += E ? 1 : 0;
-    c->stats.fire_rounds++;
-    if (coop && launch_fire_rounds_all(a, cnt + CNT_RING0, (uint32_t) (V + 2), s) == 0) {
-      c->stats.kernel_launches += 1;
-      rounds_done = true;                              // the round count is read with the final counters
-      c->fire_ring_pending = true;
-    } else {
-      if (coop) CK(cudaMemcpyAsync(cnt + CNT_WORK_B, cnt + CNT_RING0, 4, cudaMemcpyDeviceToDevice, s));
-      if (read_counters(c) != 0) return -1;
-      n_in = c->h_counters[CNT_WORK_B];
-    }
-  }
-  while (n_in && !rounds_done) {
-    // worklists only shrink: n_in bounds the next rounds' lists, so a few rounds are queued per sync
-    for (int k = 0; k < FIRE_ROUNDS_PER_SYNC; k++) {
-      CK(cudaMemsetAsync(cnt + out_idx, 0, 4, s));
-      launch_fire_round(a, win, cnt + in_idx, n_in, wout, cnt + out_idx, s);
-      c->stats.kernel_launches += 1;
-      c->stats.fire_rounds++;
-      uint32_t *t = win; win = wout; wout = t;
-      int ti = in_idx; in_idx = out_idx; out_idx = ti;
-    }
-    if (read_counters(c) != 0) return -1;
-    const uint32_t n_next = c->h_counters[in_idx];
-    if (n_next >= n_in && c->stats.fire_rounds > V + 2) return fail(c, "gtsb_filter: fire rounds did not converge");
-    n_in = n_next;
-  }
-  launch_vres(a, s);
-  launch_finalize(a, s);
-  c->stats.kernel_launches += (V ? 1 : 0) + (E ? 1 : 0) + (E && c->n_big_rows ? 1 : 0);
-  CK(cudaGetLastError());
-  return 0;
-}
-
 // plain CSR (vertex order) copy of a line-layout graph, made on demand
 int export_csr(gtsb_context *c) {
   if (!c->line_layout || c->csr_exported) return 0;
@@ -1193,7 +1015,7 @@ int gtsb_filter(gtsb_context *c, float pcutoff, float cncutoff, int64_t ocutoff)
   if (c->world > 1) return fail(c, "a rank-partitioned graph runs through gtsb_pipeline only");
   CK(cudaSetDevice(c->device));
   if (timer_begin(c, c->t_filter) != 0) return -1;
-  if (do_filter(c, pcutoff, cncutoff, ocutoff) != 0) return -1;
+  if (run_filter(c, pcutoff, cncutoff, ocutoff, false, 0.f, 0.f, 0) != 0) return -1;
   return timer_end(c, c->t_filter, &c->stats.ms_filter);
 }
 
@@ -1204,7 +1026,7 @@ int gtsb_pipeline(gtsb_context *c, float cn_cutoff, float astat_cutoff, int use_
   CK(cudaSetDevice(c->device));
   if (c->world > 1) return dist_pipeline(c, cn_cutoff, astat_cutoff, use_cn, pcutoff, cncutoff, ocutoff);
   if (do_build(c) != 0) return -1;
-  return do_filter(c, pcutoff, cncutoff, ocutoff, true, cn_cutoff, astat_cutoff, use_cn);
+  return run_filter(c, pcutoff, cncutoff, ocutoff, true, cn_cutoff, astat_cutoff, use_cn);
 }
 
 uint64_t gtsb_nof_edges(const gtsb_context *c) { return c ? c->E : 0; }

@@ -144,6 +144,9 @@ struct gtsb_context {
   DotWrite dot;
 
   uint32_t *h_counters = nullptr;   // pinned
+  // allocations ensure() attempted.  Buffer sizes of a partitioned step come from numbers every
+  // rank holds, so a step that allocates on one rank allocates on all: such a step ends in an agreement.
+  uint64_t n_allocs = 0;
   gtsb_stats stats{};
   Timer t_build, t_rep, t_filter;
 
@@ -186,8 +189,6 @@ gtsb::GraphArgs graph_args(gtsb_context *c);
 int get_ambig(gtsb_context *c, float pcutoff);
 int ensure_windows(gtsb_context *c, uint64_t V, uint64_t max_edges);
 int ensure_rows(gtsb_context *c, uint64_t R);
-uint64_t proposal_capacity(uint64_t E);
-int ensure_filter_buffers(gtsb_context *c, uint64_t Vg, uint64_t E, gtsb::FilterArgs &a);
 int await_vertices(gtsb_context *c);      // the main stream waits for late copies (no host sync)
 int await_records(gtsb_context *c);
 int ensure_root_column(gtsb_context *c);
@@ -198,6 +199,12 @@ struct ProfScope {                      // routes KernelTimer to the context's p
   ~ProfScope();
 };
 
+// the filter of every context (gtsb_dist.cu), here on one device: gtsb_filter, and gtsb_pipeline with
+// fused = true, the three stages back to back on a fresh graph: the repeat predicate (these cutoffs) is
+// evaluated inside the vertex-facts pass and the REPEAT edge marks (pred(v) || pred(w)) are derived by
+// the final pass instead of being stored first and overwritten later
+int run_filter(gtsb_context *c, float pcutoff, float cncutoff, int64_t ocutoff, bool fused, float cn_cutoff,
+               float astat_cutoff, int use_cn);
 // rank-partitioned pipeline (gtsb_dist.cu)
 int dist_pipeline(gtsb_context *c, float cn_cutoff, float astat_cutoff, int use_cn, float pcutoff,
                   float cncutoff, int64_t ocutoff);

@@ -43,6 +43,10 @@
 // the same vertex-level facts, so the symmetric edge marks agree without any
 // edge exchange.  NCCL is loaded with dlopen when gtsb_dist_init is called;
 // single-device use never touches it.
+//
+// A single device is the partition of one rank: the filter of every context is run_filter, and at
+// one rank the exchanges it makes (exchange, agree, allgatherv, allreduce and the fire-round
+// updates) do nothing but return the local status.
 #include <dlfcn.h>
 #include <nccl.h>
 #include <stdlib.h>
@@ -174,6 +178,7 @@ int agree(gtsb_context *c, int local_rc, const char *where);
 // ~4x slower on 8 GPUs) and are copied to their places afterwards.
 int allgatherv(gtsb_context *c, const char *what, void *buf, size_t es, const std::vector<uint64_t> &lo,
                bool on_side = false) {
+  if (c->world == 1) return 0;
   DistState *D = static_cast<DistState *>(c->dstate);
   cudaStream_t st = on_side ? D->side : c->stream;
   ncclComm_t comm = on_side ? D->comm2 : D->comm;
@@ -222,7 +227,7 @@ int ensure_u(gtsb_context *c, DevBuf &b, size_t bytes, bool &grew) {
 // growth step is rank-uniform
 int injected_failure(gtsb_context *c, const char *place, bool &grew) {
   const char *e = getenv("GTSB_FAIL_AT");
-  if (e == nullptr) return 0;
+  if (e == nullptr || c->world == 1) return 0;
   const char *colon = strchr(e, ':');
   if (colon == nullptr || strcmp(colon + 1, place) != 0) return 0;
   grew = true;
@@ -258,6 +263,10 @@ void release_receive_buffers(gtsb_context *c) {
 // keep_graph: a failure releases the receive buffers only (release_receive_buffers).
 int exchange(gtsb_context *c, int local_rc, const char *where, const uint32_t *mine, int n,
              std::vector<uint32_t> &out, bool keep_graph = false) {
+  if (c->world == 1) {                   // one rank: its own words, its own status and message
+    out.assign(mine, mine + n);
+    return local_rc != 0 ? -1 : 0;
+  }
   uint32_t buf[SMALL_N];
   buf[0] = local_rc != 0 ? 1u : 0u;
   for (int i = 0; i < n; i++) buf[1 + i] = mine[i];
@@ -287,6 +296,15 @@ int exchange(gtsb_context *c, int local_rc, const char *where, const uint32_t *m
 int agree(gtsb_context *c, int local_rc, const char *where) {
   std::vector<uint32_t> none;
   return exchange(c, local_rc, where, nullptr, 0, none);
+}
+
+// in-place allreduce of n elements on the main stream
+int allreduce(gtsb_context *c, const char *what, void *buf, size_t n, ncclDataType_t type, ncclRedOp_t op) {
+  if (c->world == 1) return 0;
+  DistState *D = static_cast<DistState *>(c->dstate);
+  KernelTimer t_(what, c->stream);
+  NK(g_nccl.AllReduce(buf, buf, n, type, op, D->comm, c->stream));
+  return 0;
 }
 
 // ---- kernels that exist only for the partitioned graph
@@ -722,7 +740,8 @@ struct Plan {                     // what the ranks agreed on while building
   uint32_t big_rows_max = 0, deg_max = 0;   // most rows > BIG_ROW on one rank, longest row anywhere
   float cn_cutoff = 0.f, astat_cutoff = 0.f;
   int use_cn = 0;
-  bool facts_on_side = false;     // vinfo was computed and gathered on the side stream
+  bool facts_launched = false;    // the vertex facts were computed and gathered under the build
+  bool facts_on_side = false;     // ... on the side stream
   std::vector<uint64_t> vlo;      // [N+1] vertex-attribute slices by id (gtsb_set_vertices_slice_host)
   bool gather_attributes = false;
   bool any_input = false;         // gtsb_dist_any_input, agreed at the build setup
@@ -769,6 +788,7 @@ int dist_side_facts(gtsb_context *c, DistState *D, Plan &P) {
   c->stats.kernel_launches += 1;
   if (allgatherv(c, "nccl_allgather_vinfo", c->vinfo.p, sizeof(uint2), P.lo, side) != 0) return -1;
   if (side) CK(cudaEventRecord(D->ev_join, st));
+  P.facts_launched = true;
   P.facts_on_side = side;
   return 0;
 }
@@ -875,10 +895,10 @@ int dist_windows(gtsb_context *c, const Plan &P) {
   // window tables: sized by the largest share of rows / slots any rank holds (uniform growth)
   uint64_t rows_max = 0;
   for (int r = 0; r < N; r++) rows_max = P.lo[r + 1] - P.lo[r] > rows_max ? P.lo[r + 1] - P.lo[r] : rows_max;
-  bool grew = c->wcount.cap < ((rows_max + 63) / 64 + 2) * 4 || c->win_start.cap < ((rows_max < P.E_max + 1 ? rows_max : P.E_max + 1) + 2) * 4;
+  const uint64_t allocs = c->n_allocs;
+  bool grew = false;
   const int rc = injected_failure(c, "windows", grew) != 0 ? -1 : ensure_windows(c, rows_max, P.E_max + 1);
-  if (grew && agree(c, rc, "windows") != 0) return -1;
-  if (!grew && rc != 0) return -1;
+  if ((grew || c->n_allocs != allocs ? agree(c, rc, "windows") : rc) != 0) return -1;
   c->line_layout = true;
   c->csr_exported = false;
   c->have_graph = true;
@@ -1433,54 +1453,166 @@ int dist_general(gtsb_context *c, DistState *D, Plan &P) {
   return 0;
 }
 
-int dist_filter(gtsb_context *c, DistState *D, const Plan &P, float cn_cutoff, float astat_cutoff, int use_cn,
-                float cncutoff, int64_t ocutoff) {
-  const int N = c->world, me = c->rank;
+// work arrays of the filter: per-vertex ones for Vg vertices, proposals for E slots, big-row scratch
+// for big_rows rows of at most max_deg slots; the arguments of the kernels for this device's rows
+int ensure_filter_buffers(gtsb_context *c, uint64_t Vg, uint64_t E, uint32_t big_rows, uint32_t max_deg,
+                          FilterArgs &a) {
+  // proposals are rare (a pair needs two low copy numbers and an ambiguous order); room for E / 4,
+  // the single-device filter reruns the pairs pass with room for all E when that overflows
+  const uint64_t want = E / 4 + 65536 < E + 1 ? E / 4 + 65536 : E + 1;
+  const uint64_t prop_cap = want > c->proposals.cap / sizeof(uint2) ? want : c->proposals.cap / sizeof(uint2);
+  ENSURE(c->proposals, prop_cap * sizeof(uint2));
+  ENSURE(c->poly_cur, (Vg + 1) * 4);
+  ENSURE(c->poly_new, (Vg + 1) * 4);
+  ENSURE(c->gbits, Vg + 1);
+  ENSURE(c->fstat, Vg + 1);
+  ENSURE(c->work_a, (Vg + 1) * 4);
+  ENSURE(c->work_b, (Vg + 1) * 4);
+  ENSURE(c->vinfo, (Vg + 1) * sizeof(uint2));
+  ENSURE(c->vres, (Vg + 1) * 4);
+  ENSURE(c->vsum, Vg + 1);
+  ENSURE(c->dirty, Vg + 1);
+  const uint32_t blocks = (uint32_t) c->sm_count * 2;
+  if (big_rows) ENSURE(c->big_scratch, (size_t) (blocks < big_rows ? blocks : big_rows) * max_deg * BIG_SCRATCH_STRIDE);
+  a.big_blocks = c->n_big_rows && c->n_big_rows < blocks ? c->n_big_rows : blocks;
+  static const int split_hubs = [] {
+    const char *e = getenv("GTSB_HUBS");                 // 0: a block per hub row, as in round 1 (dev switch)
+    return (e != nullptr && atoi(e) == 0) ? 0 : 1;
+  }();
+  if (split_hubs && c->world == 1 && c->n_big_rows && c->max_deg > HUB_ROW) {
+    const uint64_t cap = E / HUB_LCH + c->n_big_rows + 1;
+    ENSURE(c->hub_cn, (E + 1) * 4);
+    ENSURE(c->hub_low, (E + 1) * 4);
+    ENSURE(c->hub_mark, E + 1);
+    ENSURE(c->hub_nlow, ((uint64_t) c->n_big_rows + 1) * 4);
+    ENSURE(c->hub_items, cap * sizeof(uint2));
+    a.hub_cn = c->hub_cn.as<float>();
+    a.hub_low = c->hub_low.as<uint32_t>();
+    a.hub_mark = c->hub_mark.as<uint8_t>();
+    a.hub_nlow = c->hub_nlow.as<uint32_t>();
+    a.hub_items = c->hub_items.as<uint2>();
+    a.hub_items_cap = (uint32_t) (cap > 0xFFFFFFFFull ? 0xFFFFFFFFull : cap);
+  }
+  a.g = graph_args(c);
+  a.proposals = c->proposals.as<uint2>();
+  a.proposals_cap = (uint32_t) (prop_cap > E + 1 ? E + 1 : prop_cap);
+  a.poly_cur = c->poly_cur.as<uint32_t>();
+  a.poly_new = c->poly_new.as<uint32_t>();
+  a.gbits = c->gbits.as<uint8_t>();
+  a.fstat = c->fstat.as<uint8_t>();
+  a.dirty = c->dirty.as<uint8_t>();
+  a.rep_pred = c->rep_pred.as<uint8_t>();
+  a.work_a = c->work_a.as<uint32_t>();
+  a.work_b = c->work_b.as<uint32_t>();
+  a.big_scratch = c->big_scratch.as<uint8_t>();
+  a.vinfo = c->vinfo.as<uint2>();
+  a.vres = c->vres.as<uint32_t>();
+  a.vsum = c->vsum.as<uint8_t>();
+  return 0;
+}
+
+// list: this rank's proposals, then every rank's, at their offsets off[r] (one rank: the same list)
+int gather_proposals(gtsb_context *c, const std::vector<uint64_t> &off, uint2 *&list) {
+  if (c->world == 1) return 0;
+  DistState *D = static_cast<DistState *>(c->dstate);
+  bool grew = false;
+  const int rc = injected_failure(c, "proposals", grew) != 0 ? -1
+                 : ensure_u(c, D->prop_all, (size_t) off[c->world] * sizeof(uint2), grew);
+  if (grew && agree(c, rc, "proposal list") != 0) return -1;
+  const uint64_t n = off[c->rank + 1] - off[c->rank];
+  if (n)
+    CK(cudaMemcpyAsync(D->prop_all.as<uint2>() + off[c->rank], list, (size_t) n * sizeof(uint2), cudaMemcpyDeviceToDevice,
+                       c->stream));
+  if (allgatherv(c, "nccl_allgather_proposals", D->prop_all.p, sizeof(uint2), off) != 0) return -1;
+  list = D->prop_all.as<uint2>();
+  return 0;
+}
+
+// room for every rank's fire-round updates, `cap` words a rank
+int fire_staging(gtsb_context *c, uint32_t cap) {
+  if (c->world == 1) return 0;
+  DistState *D = static_cast<DistState *>(c->dstate);
+  bool grew = false;
+  const int rc = injected_failure(c, "fire", grew) != 0 ? -1 : ensure_u(c, D->stage, (size_t) cap * 4 * c->world, grew);
+  return grew ? agree(c, rc, "fire round staging") : rc;
+}
+
+// the rows of a fire round's worklist (list, *n_dev <= cap of them), with their new status, to every rank
+int share_fire_status(gtsb_context *c, const uint32_t *list, const uint32_t *n_dev, uint32_t cap, uint8_t *fstat) {
+  if (c->world == 1) return 0;
+  DistState *D = static_cast<DistState *>(c->dstate);
+  cudaStream_t s = c->stream;
+  uint32_t *stage = D->stage.as<uint32_t>();
+  KernelTimer t_("nccl_allgather_fire_updates", s);
+  const uint32_t blocks = (cap + 255) / 256 < (uint32_t) c->sm_count * 8 ? (cap + 255) / 256 : (uint32_t) c->sm_count * 8;
+  k_dist_pack_fstat<<<blocks, 256, 0, s>>>(list, n_dev, cap, fstat, stage + (size_t) cap * c->rank);
+  NK(g_nccl.AllGather(stage + (size_t) cap * c->rank, stage, cap, ncclUint32, D->comm, s));
+  k_dist_apply_fstat<<<c->sm_count * 8, 256, 0, s>>>(stage, (uint64_t) cap * c->world, fstat);
+  c->stats.kernel_launches += 2;
+  return 0;
+}
+
+// The filter over the ranks of P (one rank: a single device, P from the context).  P.facts_launched:
+// the vertex facts were computed and gathered under the build (dist_side_facts); otherwise they are
+// computed here, with the repeat predicate when fused.
+int filter_ranks(gtsb_context *c, const Plan &P, bool fused, float cncutoff, int64_t ocutoff) {
+  const int N = c->world;
   const uint64_t Vg = c->V;
   cudaStream_t s = c->stream;
   uint32_t *cnt = c->counters.as<uint32_t>();
   std::vector<uint32_t> all;
   FilterArgs a{};
   // sized by what the fullest rank holds, so that every rank's buffers grow in the same step
-  bool grew = c->proposals.cap < proposal_capacity(P.E_max) * sizeof(uint2) || c->poly_cur.cap < (Vg + 1) * 4 ||
-                    c->vres.cap < (Vg + 1) * 4 ||
-                    (P.big_rows_max != 0 &&
-                     c->big_scratch.cap < (size_t) (P.big_rows_max < (uint32_t) c->sm_count * 2 ? P.big_rows_max
-                                                                                               : (uint32_t) c->sm_count * 2) *
-                                              P.deg_max * BIG_SCRATCH_STRIDE);
+  const uint64_t allocs = c->n_allocs;
+  bool grew = false;
   int rc = [&]() -> int {
     if (injected_failure(c, "filter", grew) != 0) return -1;
     if (await_vertices(c) != 0) return -1;
-    const uint32_t nb = c->n_big_rows, md = c->max_deg;
-    c->n_big_rows = P.big_rows_max;                      // scratch for the largest hub population of any rank
-    c->max_deg = P.deg_max;
-    const int e = ensure_filter_buffers(c, Vg, P.E_max, a);
-    c->n_big_rows = nb;
-    c->max_deg = md;
-    if (e != 0) return -1;
-    if (ensure_filter_buffers(c, Vg, P.E_max, a) != 0) return -1;      // arguments for this rank's rows
+    if (ensure_filter_buffers(c, Vg, P.E_max, P.big_rows_max, P.deg_max, a) != 0) return -1;
     CK(cudaMemsetAsync(cnt + CNT_PROPOSALS, 0, (CNT_NUM - CNT_PROPOSALS) * 4, s));
     CK(cudaMemsetAsync(c->poly_cur.p, 0xFF, (Vg + 1) * 4, s));
     CK(cudaMemsetAsync(c->poly_new.p, 0xFF, (Vg + 1) * 4, s));
     CK(cudaMemsetAsync(c->dirty.p, 0, Vg + 1, s));
     CK(cudaMemsetAsync(c->gbits.p, 0, Vg + 1, s));
-    CK(cudaMemsetAsync(c->fstat.p, 0x0C, Vg + 1, s));
+    CK(cudaMemsetAsync(c->fstat.p, 0x0C, Vg + 1, s));      // rows without slots: decided, nothing fires
     return 0;
   }();
-  if (grew && agree(c, rc, "filter buffers") != 0) return -1;
-  if (!grew && rc != 0) return -1;            // no allocation was due: not a memory problem, and not rank-local
+  // no allocation was due: a failure is not a memory problem, and not rank-local
+  if ((grew || c->n_allocs != allocs ? agree(c, rc, "filter buffers") : rc) != 0) return -1;
   a.ambig = c->ambig;
   a.cncutoff = cncutoff;
   a.ocutoff = ocutoff;
-  a.fused_repeats = 1;
+  a.fused_repeats = fused ? 1 : 0;
+  const uint64_t V = a.g.V, E = a.g.E;                    // this device's rows and slots
 
-  // phase 1: the neighbour facts were computed and gathered under the build (dist_side_facts)
-  if (P.facts_on_side) CK(cudaStreamWaitEvent(s, D->ev_join, 0));
+  // phase 1: who proposes whom (+ the static overlap answer of every small row)
+  if (!P.facts_launched) {
+    launch_vertex_facts(a, fused ? 1 : 0, P.cn_cutoff, P.astat_cutoff, P.use_cn, s);
+    c->stats.kernel_launches += V ? 1 : 0;
+  } else if (P.facts_on_side) {
+    CK(cudaStreamWaitEvent(s, static_cast<DistState *>(c->dstate)->ev_join, 0));
+  }
   launch_pairs(a, s);
-  c->stats.kernel_launches += 2 + (c->n_big_rows ? 1 : 0);
+  c->stats.kernel_launches += (E ? 2 : 0) + (E && c->n_big_rows ? 1 : 0);
   rc = [&]() -> int {
     if (read_counters(c) != 0) return -1;
     if (c->h_counters[CNT_ERROR] & 4u) return fail(c, "gtsb_filter: a contig is longer than 2^31-1");
+    // one device: more proposals than the list was sized for, once more with room for every slot (the
+    // ranks would have to agree on that)
+    if (c->h_counters[CNT_OVERFLOW] && N == 1) {
+      if (a.proposals_cap < E + 1) {
+        ENSURE(c->proposals, (E + 1) * sizeof(uint2));
+        a.proposals = c->proposals.as<uint2>();
+        a.proposals_cap = (uint32_t) (E + 1);
+        CK(cudaMemsetAsync(cnt + CNT_PROPOSALS, 0, 4, s));
+        CK(cudaMemsetAsync(cnt + CNT_OVERFLOW, 0, 4, s));
+        CK(cudaMemsetAsync(c->gbits.p, 0, Vg + 1, s));
+        launch_pairs(a, s);
+        c->stats.kernel_launches += (E ? 2 : 0) + (E && c->n_big_rows ? 1 : 0);
+        if (read_counters(c) != 0) return -1;
+      }
+      if (c->h_counters[CNT_OVERFLOW]) return fail(c, "gtsb_filter: proposal list overflow");
+    }
     if (c->h_counters[CNT_OVERFLOW])
       return fail(c, "gtsb_filter: more polymorphic proposals than a quarter of the slots (the partitioned filter sizes its list for that)");
     return 0;
@@ -1495,22 +1627,11 @@ int dist_filter(gtsb_context *c, DistState *D, const Plan &P, float cn_cutoff, f
   c->stats.proposals = nprop;
   c->stats.poly_sweeps = 0;
   if (nprop) {
-    bool pgrew = false;
-    rc = [&]() -> int {
-      if (injected_failure(c, "proposals", pgrew) != 0) return -1;
-      if (ensure_u(c, D->prop_all, (size_t) nprop * sizeof(uint2), pgrew) != 0) return -1;
-      return 0;
-    }();
-    if (pgrew && agree(c, rc, "proposal list") != 0) return -1;
-    if (my_prop)
-      CK(cudaMemcpyAsync(D->prop_all.as<uint2>() + p_off[me], a.proposals, (size_t) my_prop * sizeof(uint2),
-                         cudaMemcpyDeviceToDevice, s));
-    if (allgatherv(c, "nccl_allgather_proposals", D->prop_all.p, sizeof(uint2), p_off) != 0) return -1;
-    // every rank holds every proposal: the polyTime fix-point runs redundantly,
-    // identically, without any exchange
+    // every rank holds every proposal: the polyTime fix-point runs redundantly, identically, without any exchange
     FilterArgs pa = a;
-    pa.proposals = D->prop_all.as<uint2>();
+    if (gather_proposals(c, p_off, pa.proposals) != 0) return -1;
     for (;;) {
+      // a few sweeps per host synchronisation; converged when the last one changed nothing
       for (int k = 0; k < POLY_SWEEPS_PER_SYNC; k++) {
         CK(cudaMemsetAsync(cnt + CNT_POLY_CHANGED, 0, 4, s));
         launch_poly_sweep(pa, nprop, s);
@@ -1523,70 +1644,75 @@ int dist_filter(gtsb_context *c, DistState *D, const Plan &P, float cn_cutoff, f
     }
     launch_dirty(pa, nprop, s);
     c->stats.kernel_launches += 1;
-    KernelTimer t_("nccl_allreduce_dirty", s);
-    NK(g_nccl.AllReduce(c->dirty.p, c->dirty.p, Vg, ncclUint8, ncclMax, D->comm, s));
+    if (allreduce(c, "nccl_allreduce_dirty", c->dirty.p, Vg, ncclUint8, ncclMax) != 0) return -1;
   }
 
-  // phase 2
-  CK(cudaMemsetAsync(cnt + CNT_WORK_B, 0, 4, s));
-  launch_fire_init(a, cnt + CNT_WORK_B, s);
-  c->stats.kernel_launches += 1 + (c->n_big_rows ? 1 : 0);
+  // phase 2: fire candidates (static answer, recomputed next to polymorphic vertices), then the
+  // order-respecting fire fixpoint
+  static const int coop_env = [] {
+    const char *e = getenv("GTSB_FIRE");                 // 1: one launch per fire round (dev switch)
+    return (e != nullptr && atoi(e) == 1) ? 0 : 1;
+  }();
+  const bool coop = coop_env && N == 1;                  // one grid cannot span the ranks
+  // the worklist that fire_init_big and the dense round fill: its length lives in ring[0] when the
+  // cooperative rounds kernel follows (the counters were cleared above)
+  uint32_t *n_dense = coop ? cnt + CNT_RING0 : cnt + CNT_WORK_B;
+  CK(cudaMemsetAsync(n_dense, 0, 4, s));
+  launch_fire_init(a, n_dense, s);
+  c->stats.kernel_launches += (V ? 1 : 0) + (V && c->n_big_rows ? 1 : 0);
   if (allgatherv(c, "nccl_allgather_fstat", c->fstat.p, 1, P.lo) != 0) return -1;
   c->stats.fire_rounds = 0;
-  if (ocutoff >= 0) {
-    uint32_t *win = a.work_b, *wout = a.work_a;
-    int in_idx = CNT_WORK_B, out_idx = CNT_WORK_A;
-    launch_fire_dense(a, a.work_b, cnt + CNT_WORK_B, s);
-    c->stats.kernel_launches += c->E ? 1 : 0;
+  c->fire_ring_pending = false;
+  if (ocutoff >= 0 && Vg) {
+    launch_fire_dense(a, a.work_b, n_dense, s);
+    c->stats.kernel_launches += E ? 1 : 0;
     c->stats.fire_rounds++;
-    if (allgatherv(c, "nccl_allgather_fstat", c->fstat.p, 1, P.lo) != 0) return -1;
-    for (;;) {
-      // pending rows over all ranks; my own count bounds my next worklists (they only shrink)
-      const int rrc = read_counters(c);
-      const uint32_t n_in = c->h_counters[in_idx];
-      if (exchange(c, rrc, "fire round", &n_in, 1, all) != 0) return -1;
-      uint64_t pending = 0;
-      uint32_t cap = 0;
-      for (int r = 0; r < N; r++) {
-        pending += all[r];
-        cap = all[r] > cap ? all[r] : cap;
-      }
-      if (pending == 0) break;
-      if (c->stats.fire_rounds > Vg + 2) return fail(c, "gtsb_filter: fire rounds did not converge");
-      cap = (cap + 3u) & ~3u;
-      {
-        bool sgrew = false;
-        const int e = injected_failure(c, "fire", sgrew) != 0 ? -1 : ensure_u(c, D->stage, (size_t) cap * 4 * N, sgrew);
-        if (sgrew && agree(c, e, "fire round staging") != 0) return -1;
-      }
-      uint32_t *stage = D->stage.as<uint32_t>();
-      for (int k = 0; k < FIRE_ROUNDS_PER_SYNC; k++) {
-        CK(cudaMemsetAsync(cnt + out_idx, 0, 4, s));
-        launch_fire_round(a, win, cnt + in_idx, n_in, wout, cnt + out_idx, s);
-        c->stats.kernel_launches += (n_in ? 1 : 0) + 2;
-        c->stats.fire_rounds++;
-        {
-          // the rows of this round's worklist, with their new status, to every rank
-          KernelTimer t_("nccl_allgather_fire_updates", s);
-          const uint32_t blocks = (cap + 255) / 256 < (uint32_t) c->sm_count * 8 ? (cap + 255) / 256
-                                                                                 : (uint32_t) c->sm_count * 8;
-          k_dist_pack_fstat<<<blocks, 256, 0, s>>>(win, cnt + in_idx, cap, a.fstat, stage + (size_t) cap * me);
-          NK(g_nccl.AllGather(stage + (size_t) cap * me, stage, cap, ncclUint32, D->comm, s));
-          k_dist_apply_fstat<<<c->sm_count * 8, 256, 0, s>>>(stage, (uint64_t) cap * N, a.fstat);
+    if (coop && launch_fire_rounds_all(a, cnt + CNT_RING0, (uint32_t) (Vg + 2), s) == 0) {
+      c->stats.kernel_launches += 1;
+      c->fire_ring_pending = true;                       // the round count is read with the final counters
+    } else {
+      if (coop) CK(cudaMemcpyAsync(cnt + CNT_WORK_B, cnt + CNT_RING0, 4, cudaMemcpyDeviceToDevice, s));
+      if (allgatherv(c, "nccl_allgather_fstat", c->fstat.p, 1, P.lo) != 0) return -1;
+      uint32_t *win = a.work_b, *wout = a.work_a;
+      int in_idx = CNT_WORK_B, out_idx = CNT_WORK_A;
+      uint64_t last = ~0ull;
+      for (;;) {
+        // pending rows over all ranks; my own count bounds my next worklists (they only shrink), so a
+        // few rounds are queued per host synchronisation
+        const int rrc = read_counters(c);
+        const uint32_t n_in = c->h_counters[in_idx];
+        if (exchange(c, rrc, "fire round", &n_in, 1, all) != 0) return -1;
+        uint64_t pending = 0;
+        uint32_t cap = 0;
+        for (int r = 0; r < N; r++) {
+          pending += all[r];
+          cap = all[r] > cap ? all[r] : cap;
         }
-        uint32_t *t = win; win = wout; wout = t;
-        int ti = in_idx; in_idx = out_idx; out_idx = ti;
+        if (pending == 0) break;
+        if (pending >= last && c->stats.fire_rounds > Vg + 2) return fail(c, "gtsb_filter: fire rounds did not converge");
+        last = pending;
+        cap = (cap + 3u) & ~3u;
+        if (fire_staging(c, cap) != 0) return -1;
+        for (int k = 0; k < FIRE_ROUNDS_PER_SYNC; k++) {
+          CK(cudaMemsetAsync(cnt + out_idx, 0, 4, s));
+          launch_fire_round(a, win, cnt + in_idx, n_in, wout, cnt + out_idx, s);
+          c->stats.kernel_launches += n_in ? 1 : 0;
+          c->stats.fire_rounds++;
+          if (share_fire_status(c, win, cnt + in_idx, cap, a.fstat) != 0) return -1;
+          uint32_t *t = win; win = wout; wout = t;
+          int ti = in_idx; in_idx = out_idx; out_idx = ti;
+        }
       }
     }
   }
 
-  // final states
-  // the final pass reads a neighbour's fire bits and repeat predicate from the byte summary (and its
-  // polyTime from poly_cur, which every rank holds complete): one byte per vertex crosses NVLink
+  // final states.  The final pass reads a neighbour's fire bits and repeat predicate from the byte
+  // summary (and its polyTime from poly_cur, which every rank holds complete): one byte per vertex
+  // crosses NVLink
   launch_vres(a, s);
   if (allgatherv(c, "nccl_allgather_vsum", c->vsum.p, 1, P.lo) != 0) return -1;
   launch_finalize(a, s);
-  c->stats.kernel_launches += 2 + (c->n_big_rows ? 1 : 0);
+  c->stats.kernel_launches += (V ? 1 : 0) + (E ? 1 : 0) + (E && c->n_big_rows ? 1 : 0);
   return 0;
 }
 
@@ -1616,11 +1742,27 @@ int dist_pipeline(gtsb_context *c, float cn_cutoff, float astat_cutoff, int use_
     if (b > 0 && dist_general(c, D, P) != 0) return -1;
   }
   KernelTimer t_("PHASE_filter", c->stream);
-  if (dist_filter(c, D, P, cn_cutoff, astat_cutoff, use_cn, cncutoff, ocutoff) != 0) return -1;
-  {
-    KernelTimer t_("nccl_allreduce_vstate", c->stream);
-    NK(g_nccl.AllReduce(c->vstate.p, c->vstate.p, c->V, ncclUint8, ncclMax, D->comm, c->stream));
-  }
+  if (filter_ranks(c, P, true, cncutoff, ocutoff) != 0) return -1;
+  if (allreduce(c, "nccl_allreduce_vstate", c->vstate.p, c->V, ncclUint8, ncclMax) != 0) return -1;
+  CK(cudaGetLastError());
+  return 0;
+}
+
+int run_filter(gtsb_context *c, float pcutoff, float cncutoff, int64_t ocutoff, bool fused, float cn_cutoff,
+               float astat_cutoff, int use_cn) {
+  ProfScope ps_(c);
+  if (!c->have_graph) return fail(c, "gtsb_filter: no graph (call gtsb_build or gtsb_set_graph_host)");
+  if (get_ambig(c, pcutoff) != 0) return -1;
+  c->csr_exported = false;
+  Plan P;                                         // one rank: every row and slot is this device's
+  P.lo = {0, c->V};
+  P.E_max = c->E;
+  P.big_rows_max = c->n_big_rows;
+  P.deg_max = c->max_deg;
+  P.cn_cutoff = cn_cutoff;
+  P.astat_cutoff = astat_cutoff;
+  P.use_cn = use_cn;
+  if (filter_ranks(c, P, fused, cncutoff, ocutoff) != 0) return -1;
   CK(cudaGetLastError());
   return 0;
 }
