@@ -42,6 +42,7 @@ EXPORTS = [
     "gtsb_astat_stream_end", "gtsb_stream_set_slot", "gtsb_dist_any_input",
     "gtsb_dist_de_stream_begin", "gtsb_dist_astat_stream_begin",
     "gtsb_dot_write_begin", "gtsb_dot_write_next", "gtsb_dot_write_end",
+    "gtsb_fasta_stream_begin", "gtsb_dist_fasta_stream_begin", "gtsb_fasta_stream_end", "gtsb_get_vertex_names",
 ]
 
 
@@ -130,6 +131,10 @@ def load_library():
     L.gtsb_dot_write_begin.argtypes = [vp, i32, u64, C.POINTER(u64)]
     L.gtsb_dot_write_next.argtypes = [vp, C.POINTER(vp), C.POINTER(u64), C.POINTER(u64)]
     L.gtsb_dot_write_end.argtypes = [vp, i32]
+    L.gtsb_fasta_stream_begin.argtypes = [vp, u64]
+    L.gtsb_dist_fasta_stream_begin.argtypes = [vp, u64]
+    L.gtsb_fasta_stream_end.argtypes = [vp, C.POINTER(u64), C.POINTER(C.c_uint32)]
+    L.gtsb_get_vertex_names.argtypes = [vp, vp, vp, vp]
     _lib = L
     return L
 
@@ -291,6 +296,34 @@ def shard_file(path, world: int, rank: int, mail_weight: float = MAIL_WEIGHT):
         return _shard(read, n, world, rank, mail_weight)
 
 
+def _shard_fasta(read, n: int, world: int, rank: int):
+    """The cut search of shard_fasta_file over a byte-range reader (see _shard)."""
+    cuts = [0]
+    for r in range(1, world):
+        i = max(n * r // world, cuts[-1])
+        if 0 < i < n and read(i - 1, i) != b"\n":
+            i = _find_nl(read, n, i) + 1 or n
+        while 0 < i < n and read(i, i + 1) != b">":                 # the next line that starts a record
+            i = _find_nl(read, n, i) + 1 or n
+        cuts.append(i)
+    cuts.append(n)
+    return cuts[rank], cuts[rank + 1]
+
+
+def shard_fasta_file(path, world: int, rank: int):
+    """Rank `rank`'s chunk [lo, hi) of a contigs FASTA for parse_fasta_pieces on a partitioned context:
+    cuts near k * size / world, moved forward to the next line that starts with '>', so that every
+    chunk after the first starts a record.  Only bytes near the cuts are read."""
+    with open(path, "rb") as f:
+        n = f.seek(0, os.SEEK_END)
+
+        def read(a, b):
+            f.seek(a)
+            return f.read(b - a)
+
+        return _shard_fasta(read, n, world, rank)
+
+
 def read_pieces(path, lo: int, hi: int, piece: int = 1 << 26):
     """The bytes [lo, hi) of a file, `piece` bytes at a time (for parse_*_pieces)."""
     with open(path, "rb") as f:
@@ -314,6 +347,7 @@ class ScaffoldGraphB200:
             raise RuntimeError("gtsb_create failed: no usable CUDA device (no CPU fallback)")
         self.h = h
         self.V = 0
+        self.names_V = 0
         self._keep = []
         if want_win_rec:
             self._ck(self.L.gtsb_want_win_rec(self.h, 1))
@@ -446,6 +480,39 @@ class ScaffoldGraphB200:
         irr = self._stream(lambda: begin(self.h, _ptr(a), _ptr(cn)), pieces,
                            lambda irr: self.L.gtsb_astat_stream_end(self.h, _ptr(a), _ptr(cn), C.byref(irr)))
         return irr, a, cn
+
+    def parse_fasta_pieces(self, pieces, min_ctg_len: int = MIN_CONTIG_LEN):
+        """The contigs FASTA, given as consecutive pieces cut anywhere (see parse_de_pieces) -> (irregular
+        bits, V).  The records with seq_len > min_ctg_len are the vertices, their ids the order of
+        their headers (bytewise, gt_scaffolder_parser_count_distances); with irregular == 0 the names set
+        becomes their headers in id order, so that parse_de* / parse_astat* follow, and vertex_names()
+        returns them with seq_len.  irregular != 0 (GTSB_IRR_FASTA = 32: outside the canonical spelling,
+        16: two vertices with one header): nothing was set.  On a partitioned context every rank
+        streams its own chunk (shard_fasta_file) and all ranks get the same ids and names:
+
+            lo, hi = shard_fasta_file(path, world, rank)
+            irr, V = g.parse_fasta_pieces(read_pieces(path, lo, hi))"""
+        V = C.c_uint64(0)
+        dist = getattr(self, "world", 1) > 1
+        begin = self.L.gtsb_dist_fasta_stream_begin if dist else self.L.gtsb_fasta_stream_begin
+        irr = self._stream(lambda: begin(self.h, C.c_uint64(min_ctg_len)), pieces,
+                           lambda irr: self.L.gtsb_fasta_stream_end(self.h, C.byref(V), C.byref(irr)))
+        if irr == 0:
+            self.names_V = int(V.value)         # the names set's size; self.V stays the graph's
+        return irr, int(V.value)
+
+    def vertex_names(self):
+        """After a parse_fasta_pieces that set the names: (headers in id order as a list of bytes,
+        seq_len by id as uint32).  Sized by that read's V, not by the resident graph's."""
+        V = self.names_V
+        off = np.zeros(V + 1, np.uint64)
+        seq = np.zeros(V, np.uint32)
+        self._ck(self.L.gtsb_get_vertex_names(self.h, None, _ptr(off), _ptr(seq)))
+        blob = np.zeros(int(off[-1]) + 1, np.uint8)
+        self._ck(self.L.gtsb_get_vertex_names(self.h, _ptr(blob), None, None))
+        raw = blob.tobytes()
+        o = off.tolist()
+        return [raw[o[i]:o[i + 1]] for i in range(V)], seq
 
     def set_stream_slot(self, nbytes: int):
         """Bytes of one staging slot of the *_pieces calls (default 64 MiB)."""

@@ -40,7 +40,7 @@ struct Timer {
 // between two feeds lives here, so that other calls on the context, the whole-text calls included,
 // cannot disturb it.  The buffers stay allocated for the next read.
 struct TextStream {
-  enum Kind { CLOSED = 0, DE = 1, ASTAT = 2 };
+  enum Kind { CLOSED = 0, DE = 1, ASTAT = 2, FASTA = 3 };
   int kind = CLOSED;
   uint64_t slot = 64ull << 20;      // bytes of one step (carry included); 0: whole text, not staged
   char *host = nullptr;            // pinned: the step being filled, then 4 words the device reports into
@@ -65,6 +65,16 @@ struct TextStream {
   DevBuf root, ctg, dist, std_dev, rflags, num_pairs;   // grow geometrically, earlier records kept
   // .astat: 64-bit file offset + 1 of the winning piece per vertex, the values applied so far
   DevBuf last, astat, copy_num;
+  // FASTA: a step ends after its last '\n', or anywhere inside a sequence line longer than the slot;
+  // cont: the next step starts inside such a line.  Every record's header, header offsets and
+  // seq_len are appended to the fa_* columns in file order (seq_len summed over the record's lines,
+  // the open record's across steps); the length filter and the ids are the end's.
+  uint64_t min_len = 0;            // min_ctg_len: a record is a vertex iff seq_len > min_len
+  uint64_t fa_bytes = 0;           // header bytes appended so far
+  bool cont = false;
+  char first_byte = 0;             // the first byte fed (a partitioned chunk after the first starts with '>')
+  DevBuf fa_hdr, fa_seq, fa_hoff;  // per line of one step: header flag, sequence bytes, header byte offset
+  DevBuf fa_names, fa_off, fa_len; // the record columns: headers, R + 1 offsets, seq_len (u64)
   cudaEvent_t ev_copied = nullptr, ev_free[2] = {nullptr, nullptr};
 };
 
@@ -141,6 +151,12 @@ struct gtsb_context {
   uint64_t names_V = 0, names_mask = 0, names_bytes = 0;
   bool have_names = false, names_dup = false, have_num_pairs = false;
   TextStream ts, whole;
+  // the end of a FASTA read (gtsb_parse.cu / gtsb_dist.cu): the kept records (header length,
+  // seq_len, source record, header offsets, headers), the sort's keys, values, order, group
+  // boundaries, tied lists and run ids, and seq_len by vertex id of the names set it leaves
+  DevBuf fa_flag, fa_pos, fa_klen, fa_kseq, fa_ksrc, fa_koff, fa_knames, fa_key[2], fa_val[2], fa_ord, fa_tmp,
+      fa_bnd, fa_act[2], fa_head, fa_run, fa_hist, fa_scan64, names_seq;
+  bool have_names_seq = false;     // names_seq belongs to the names set (it came from a FASTA read)
   DotWrite dot;
 
   uint32_t *h_counters = nullptr;   // pinned
@@ -219,6 +235,16 @@ int stream_end_local(gtsb_context *c, TextStream &ts, const char *src, const cha
 void stream_close(TextStream &ts);
 void adopt_stream_records(gtsb_context *c, TextStream &ts, uint64_t R);
 void release_stream_records(TextStream &ts);
+// the FASTA read's end (gtsb_parse.cu): this rank's kept records into the fa_k* buffers (*K records,
+// *bytes header bytes); the ids of the K kept records held in the fa_k* buffers, and the names set
+// they make (IRR_DUP_NAME in *irregular: nothing set)
+int fasta_keep(gtsb_context *c, TextStream &ts, uint64_t *K, uint64_t *bytes);
+int fasta_ids(gtsb_context *c, uint64_t K, uint32_t *irregular);
+void fasta_release(gtsb_context *c);     // gtsb_destroy
+int fasta_offsets(gtsb_context *c, const uint32_t *len, uint64_t n, uint64_t *off);   // off = exclusive sum, u64
+// the end of a FASTA stream, one device and the ranks alike (gtsb_dist.cu, collective on a
+// partitioned context; at one rank its exchanges are the local status)
+int fasta_end(gtsb_context *c, const char *what, int rc, uint64_t *nof_vertices, uint32_t *irregular);
 // the end of a partitioned text read, stream or whole text (gtsb_dist.cu, collective).  rc: this
 // rank's status so far; stage: the GTSB_FAIL_AT place
 int dist_text_end(gtsb_context *c, TextStream &ts, const char *src, const char *what, int kind, const char *stage,

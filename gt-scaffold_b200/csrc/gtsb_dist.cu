@@ -1952,6 +1952,86 @@ int dist_text_end(gtsb_context *c, TextStream &ts, const char *src, const char *
   return 0;
 }
 
+// ---- the contigs FASTA: every rank reads its own chunk (consecutive byte ranges in rank order, every
+// chunk after the first starting a record) and keeps its records with seq_len > min_ctg_len; one
+// exchange of the counts, one allgatherv each of the header lengths, seq_len and headers in rank
+// order, and every rank sorts the whole set itself, as the polyTime sweeps run on every rank: ids,
+// names set and seq_len are identical everywhere and equal to one device's.  At one rank (one
+// device) the exchange is the local status and the gathers do nothing.
+int fasta_end(gtsb_context *c, const char *what, int rc, uint64_t *nof_vertices, uint32_t *irregular_out) {
+  TextStream &ts = c->ts;
+  uint64_t K = 0, B = 0;
+  if (rc == 0)
+    rc = [&]() -> int {
+      if (stream_end_local(c, ts, ts.host, what, TextStream::FASTA) != 0) return -1;
+      bool unused = false;
+      if (injected_failure(c, "fasta", unused) != 0) return -1;
+      return ts.irregular ? 0 : fasta_keep(c, ts, &K, &B);
+    }();
+  const uint32_t irregular = ts.irregular;
+  stream_close(ts);
+  if (nof_vertices != nullptr) *nof_vertices = 0;
+  if (irregular_out != nullptr) *irregular_out = 0;
+  const uint32_t mine[5] = {irregular, (uint32_t) K, (uint32_t) (K >> 32), (uint32_t) B, (uint32_t) (B >> 32)};
+  std::vector<uint32_t> all;
+  if (exchange(c, rc, what, mine, 5, all, true) != 0) return -1;
+  const int N = c->world, me = c->rank;
+  std::vector<uint64_t> klo(N + 1, 0), blo(N + 1, 0);
+  uint32_t irr = 0;
+  for (int r = 0; r < N; r++) {
+    const uint32_t *w = &all[(size_t) r * 5];
+    irr |= w[0];
+    klo[r + 1] = klo[r] + (w[1] | (uint64_t) w[2] << 32);
+    blo[r + 1] = blo[r] + (w[3] | (uint64_t) w[4] << 32);
+  }
+  if (irr) {                           // a refusal anywhere: the names set stays as it was on every rank
+    *irregular_out = irr;
+    return 0;
+  }
+  const uint64_t Kt = klo[N], Bt = blo[N];
+  if (Kt > GTSB_MAX_VERTICES)
+    return fail(c, "%s: %llu vertices, more than GTSB_MAX_VERTICES", what, (unsigned long long) Kt);
+  if (N > 1) {
+    // this rank's kept records to their place in the whole set, then the other ranks' beside them
+    DevBuf g[3];
+    rc = [&]() -> int {
+      ENSURE(g[0], (Kt + 1) * 4);
+      ENSURE(g[1], (Kt + 1) * 4);
+      ENSURE(g[2], Bt + 8);
+      cudaStream_t s = c->stream;
+      if (K) {
+        CK(cudaMemcpyAsync(g[0].as<uint32_t>() + klo[me], c->fa_klen.p, K * 4, cudaMemcpyDeviceToDevice, s));
+        CK(cudaMemcpyAsync(g[1].as<uint32_t>() + klo[me], c->fa_kseq.p, K * 4, cudaMemcpyDeviceToDevice, s));
+      }
+      if (B) CK(cudaMemcpyAsync(g[2].as<char>() + blo[me], c->fa_knames.p, B, cudaMemcpyDeviceToDevice, s));
+      return 0;
+    }();
+    if (rc == 0) {
+      DevBuf *k[3] = {&c->fa_klen, &c->fa_kseq, &c->fa_knames};
+      for (int i = 0; i < 3; i++) {
+        release(*k[i]);
+        *k[i] = g[i];
+      }
+    } else {
+      for (DevBuf &b : g) release(b);
+    }
+    if (agree(c, rc, what) != 0) return -1;
+    if (allgatherv(c, "nccl_allgather_fasta_len", c->fa_klen.p, 4, klo) != 0 ||
+        allgatherv(c, "nccl_allgather_fasta_seq", c->fa_kseq.p, 4, klo) != 0 ||
+        allgatherv(c, "nccl_allgather_fasta_names", c->fa_knames.p, 1, blo) != 0)
+      rc = -1;
+  }
+  if (rc == 0) rc = fasta_ids(c, Kt, &irr);
+  if (agree(c, rc, what) != 0) {
+    c->have_names = c->have_names_seq = false;
+    c->names_V = 0;
+    return -1;
+  }
+  *irregular_out = irr;
+  *nof_vertices = irr ? 0 : Kt;
+  return 0;
+}
+
 // ---- the `.dot` of the graph, every rank writing its own byte ranges (gtsb_dot_write_*, collective
 // begin and end).  Rank r formats the vertex lines of ids [V r/N, V (r+1)/N) and the edge lines of
 // eids [E r/N, E (r+1)/N).  Every rank stores its slots' edges into the receive buffer of their eid's

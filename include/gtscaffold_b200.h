@@ -152,6 +152,7 @@ int gtsb_set_states_host(gtsb_context *ctx, const uint8_t *vstate, const uint8_t
 #define GTSB_IRR_RANGE    4u   /* distance outside int32 / pair count outside uint32 */
 #define GTSB_IRR_FLOAT    8u   /* a value the device cannot prove it rounds as strtof does */
 #define GTSB_IRR_DUP_NAME 16u  /* two contigs with one header (bsearch's choice is unspecified) */
+#define GTSB_IRR_FASTA    32u  /* a contigs FASTA outside the canonical spelling (gtsb_fasta_stream_begin) */
 int gtsb_set_vertex_names_host(gtsb_context *ctx, uint64_t nof_vertices, const char *names,
                                const uint64_t *name_off);
 int gtsb_parse_de_host(gtsb_context *ctx, const char *text, uint64_t text_bytes,
@@ -231,6 +232,50 @@ int gtsb_stream_set_slot(gtsb_context *ctx, uint64_t bytes);
    ranks.  An end without an open stream fails on this rank alone, as on one device. */
 int gtsb_dist_de_stream_begin(gtsb_context *ctx);
 int gtsb_dist_astat_stream_begin(gtsb_context *ctx, const float *astat, const float *copy_num);
+
+/* ---- the contigs FASTA on the device: the vertices, their ids and the names set
+   (gt_scaffolder_parser_read_contigs, parser.c:420-494, with astat_is_annotated false, and the ids
+   of the qsort in gt_scaffolder_parser_count_distances, parser.c:172).
+
+     gtsb_fasta_stream_begin(ctx, min_ctg_len)   open a stream (an open one is discarded)
+     gtsb_stream_feed                            the next bytes of the file, as for .de text
+     gtsb_fasta_stream_end(ctx, &V, &irregular)  the result
+
+   A record is a '>' line and the sequence lines up to the next '>' line or the end; header = the
+   description after '>' up to its first ' ', seq_len = the record's sequence bytes without the
+   '\n's.  The vertices are the records with seq_len > min_ctg_len; vertex id = the rank of the
+   header among theirs in unsigned byte order (strcmp; a prefix sorts first).  On success the
+   context's names set becomes the V headers in id order -- what gtsb_set_vertex_names_host leaves
+   with them, so gtsb_parse_de_host / gtsb_parse_astat_host and their streams follow with no host
+   round trip -- and gtsb_get_vertex_names returns them with seq_len by id.
+   The device reads the CANONICAL spelling only: the text starts with '>'; no NUL (GTSB_IRR_NUL); no
+   '\r' and no other byte below 0x20 but '\n', none equal to 0x7f; no empty line; a description that
+   is not empty and does not start with ' '; sequence lines of [A-Za-z] only; the last line may lack
+   its '\n'.  Anything else sets GTSB_IRR_FASTA, two vertices with one header GTSB_IRR_DUP_NAME (the
+   reference's ids are unspecified then); end then returns 0 with *irregular != 0, *V = 0 and the
+   names set left as it was.  An empty text has no vertices.
+   Limits, which fail with a message: more than GTSB_MAX_VERTICES vertices, a vertex with seq_len of
+   2^31 or more, a header line longer than one staging slot (gtsb_stream_set_slot; sequence lines
+   have no length limit).  Pieces may be cut anywhere.  Errors as for the .de stream.  An error at
+   the end before the header sort -- the chunk rules, the limits, a failed exchange, an injected
+   failure -- leaves the names set as it was; an error in the sort or while the new names set is
+   written (on any rank, for a partitioned stream) leaves no names set.  Memory: the staging slots of the .de stream, per record 16 B and its
+   header, and at the end about 40 B per vertex plus twice the vertices' header bytes. */
+int gtsb_fasta_stream_begin(gtsb_context *ctx, uint64_t min_ctg_len);
+int gtsb_fasta_stream_end(gtsb_context *ctx, uint64_t *nof_vertices, uint32_t *irregular);
+/* the partitioned FASTA stream: every rank streams its own chunk -- consecutive byte ranges in rank
+   order, every non-empty chunk after the first starting with '>' and every chunk but the last
+   rank's ending right after a '\n' (checked at the end, as the .de chunk rule).  Begin and feed are
+   local; gtsb_fasta_stream_end is COLLECTIVE on such a stream, with the failure handling of the
+   partitioned .de stream (GTSB_FAIL_AT=<rank>:fasta injects one).  Each rank reads its own records,
+   then every rank sorts the whole set: V, the ids, the names set and seq_len are identical on every
+   rank and equal to one device's reading of the whole text.  *irregular is the OR over the ranks
+   (duplicates are found over the whole set); a refusal anywhere sets nothing anywhere. */
+int gtsb_dist_fasta_stream_begin(gtsb_context *ctx, uint64_t min_ctg_len);
+/* after a successful gtsb_fasta_stream_end: the headers in id order, concatenated (name_off[V]
+   bytes), their V + 1 offsets, and seq_len by id.  NULL pointers are skipped.  Fails when the
+   names set did not come from a FASTA read. */
+int gtsb_get_vertex_names(gtsb_context *ctx, char *names, uint64_t *name_off, uint32_t *seq_len);
 
 /* the records held by the context, file order (NULL pointers are skipped); num_pairs
    only after gtsb_parse_de_host or gtsb_de_stream_end */
